@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the UNMODIFIED reference (baseline/_ref) running its own stage-1 loop on the host cores
+    python bench.py --dump-outputs DIR ...    # also writes what the last timed step computed, DIR/<name>.npy
 
 Workload (BASELINE.json configs[3], SURVEY.md §8d cfg 4): SVTR-MRN, I = 6 experts, union charset C_i =
 [1899, 2224, 3844, 4968, 5041, 5153], per-GPU batch 256 (weak scaling), synthetic 32x256x4 crops, one
@@ -61,7 +62,13 @@ def parse():
     ap.add_argument("--mode", default="train", choices=["train", "infer", "stage0"],
                     help="train: router-training step (the BASELINE metric); infer: hard-routed forward + greedy decode (cfg 5); "
                          "stage0: expert-training step of the newest expert (SURVEY.md §8(f)3, il_modules/mrn.py:225-279)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all), so that "
+                         "two builds run with the same arguments can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def make_opt(precision, chunk, arch="svtr"):
@@ -280,6 +287,36 @@ def infer_sweep(learner, batches, dev):
     return rows
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(learner, loss, infer, stage0):
+    """What a caller holds after the last timed step, as host float32 arrays: the step's return values and, for the
+    training modes, the parameters the step updated and the gradients it computed."""
+    if infer:
+        r = loss[2]
+        out = {k: r[k] for k in ("ids", "lens", "conf", "index")}
+    elif stage0:
+        out = {"loss": loss[0], "params": learner._tp.params, "grads": learner._tp.grads}
+    else:
+        net = learner.net
+        out = {"loss_clf": loss[0], "taski_loss": loss[1], "router_params": net.router_arena(),
+               "router_grads": net.router_grad_arena()}
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes DIR/<name>.npy.  An array larger than an equal share of DUMP_LIMIT_BYTES is cut to every k-th element of
+    its flattened form: a fixed sample, the same on every run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // 4 // len(arrays)
+    for name, a in arrays.items():
+        if a.size > share:
+            a = a.reshape(-1)[:: -(-a.size // share)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ GPU arm
 def run_ours(args):
     from mrn_b200 import dist as mdist
@@ -297,6 +334,9 @@ def run_ours(args):
             raise SystemExit("--scaling strong needs --batch divisible by the number of GPUs")
         B = B // world
     opt = make_opt(args.precision, args.chunk, args.arch)
+    # the train-mode steps draw their DropPath masks from torch's device generator: a fixed seed gives every run with
+    # the same arguments the same masks, whichever --init is chosen
+    torch.manual_seed(111)
     sd = (synth.ctor_state_dict if args.init == "ctor" else synth.synth_state_dict)(CLASS_COUNTS, 111, arch=args.arch)
     T = 64 if args.arch == "svtr" else 63
     net = MRNNet(opt)
@@ -339,7 +379,7 @@ def run_ours(args):
         img, tgt, lens, dom = resident[k % n_batches]
         if infer:
             r = (learner.infer_batch if eager else infer_step)(img, "TF")
-            return r["conf"], r["lens"]
+            return r["conf"], r["lens"], r                  # the whole result rides along for --dump-outputs
         if stage0:
             l0 = (learner.train_step_stage0 if (eager or not use_graph) else learner.train_step_stage0_graphed)(img, tgt, lens)
             return l0, l0
@@ -434,6 +474,10 @@ def run_ours(args):
         e1.record()
         mdist.barrier(); torch.cuda.synchronize()
         ms_total = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
+    if args.dump_outputs and rank == 0:
+        # `loss` and the learner's state are those of the last step of the region `value` is timed on; the e2e steps
+        # below change the parameters again
+        dump_outputs(args.dump_outputs, step_outputs(learner, loss, infer, stage0))
     # ---- timed region 2: end to end from pinned host memory
     for k in range(2):
         step_e2e(k)

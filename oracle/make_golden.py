@@ -229,7 +229,7 @@ def run_stage0_case(name, class_counts, B, seed, bn_train=True, arch="svtr"):
     print(name, "->", path, os.path.getsize(path) // 1024, "KiB")
 
 
-def run_router_case(name, I, B, seed):
+def run_router_case(name, I, B, seed, sub=SUB):
     """DM_Router alone on random features (modules/dm_router.py:50-67) incl. input gradient."""
     shapes = synth.router_shapes(I)
     sd = {k: synth.synth_tensor(seed, k, s) for k, s in shapes.items()}
@@ -241,10 +241,10 @@ def run_router_case(name, I, B, seed):
         y = m(xr)
         w = synth.randn(seed, "router_dy", y.shape)
         (y * w).sum().backward()
-        g = dict(out=keep(y), dx=keep(xr.grad), I=np.int64(I), B=np.int64(B), seed=np.int64(seed),
-                 sub=np.int64(SUB), max_full=np.int64(MAX_FULL))
+        g = dict(out=keep(y, sub), dx=keep(xr.grad, sub), I=np.int64(I), B=np.int64(B), seed=np.int64(seed),
+                 sub=np.int64(sub), max_full=np.int64(MAX_FULL))
         for n_, p in m.named_parameters():
-            g["grad." + n_] = keep(p.grad)
+            g["grad." + n_] = keep(p.grad, sub)
             g["gradnorm." + n_] = np.float64(p.grad.double().norm().item())
     path = os.path.join(OUT, name + ".npz")
     np.savez_compressed(path, **g)
@@ -271,4 +271,4 @@ if __name__ == "__main__":
     if only and "router" not in only:
         sys.exit(0)
     run_router_case("dm_router_i3_b2", 3, 2, 5)
-    run_router_case("dm_router_i6_b1", 6, 1, 9)
+    run_router_case("dm_router_i6_b1", 6, 1, 9, sub=2 * SUB)      # every 22nd element keeps the file under 1 MB

@@ -162,18 +162,6 @@ def test_train_pack_arena_round_trips_the_expert_state_dict(arch):
     assert sum(float(v.abs().sum()) for k, v in g.items() if k != tp.entries[1][1]) == 0.0
 
 
-def test_load_config_on_the_reference_configs_when_present():
-    import os
-    from mrn_b200 import tiny_train
-    root = "/root/reference/config"
-    if not os.path.isdir(root):
-        pytest.skip("reference tree not present")
-    for name, fe in (("svtr_mrn.py", "SVTR"), ("crnn_mrn.py", "VGG")):
-        opt = tiny_train.load_config(os.path.join(root, name))
-        assert opt.il == "mrn" and opt.FeatureExtraction == fe and opt.Prediction == "CTC"
-        assert opt.batch_size == 256 and opt.imgH == 32 and opt.imgW == 256 and len(opt.lan_list) == 6
-
-
 def test_domain_ids_flatten_like_the_reference():
     import torch
     from mrn_b200.il_modules.mrn import _domain_ids
