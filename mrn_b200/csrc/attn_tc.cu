@@ -10,8 +10,7 @@
 // Warp roles: warp 0 TMA producer, warp 1 TMEM alloc + MMA issuer, warps 2..9 softmax / epilogue: two warps per TMEM
 // lane quarter, each owning one 64-key half of the block (and one 16-dim half of O); the partners exchange their
 // half-row maxima through shared memory.  The softmax chain is latency-bound, so the extra warps are what buys speed.
-#include "common.cuh"
-#include <cuda.h>
+#include "sm100.cuh"
 
 namespace {
 
@@ -21,75 +20,6 @@ constexpr int P_BYTES = 128 * KT * 2;           // 32 KiB
 constexpr int TMEM_COLS = 256;
 constexpr uint32_t O_COL = 128;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");   // suspend-time hint: no hot spin
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();   // > 2 s: protocol bug -> fail loudly, never hang
-  }
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
-}
-// layout_type: 2 = SWIZZLE_128B, 4 = SWIZZLE_64B ; sbo = byte distance between 8-row (K-major) / 8-k (MN-major) atoms
-__device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t sbo_bytes, uint32_t layout_type) {
-  uint64_t d = 0;
-  d |= (uint64_t)((addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)layout_type << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ float max3(float a, float b, float c) {
-  float r;
-  asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));      // FMNMX3
-  return r;
-}
-
 // named barrier 1 + q for the two partner warps (64 threads) of TMEM lane quarter q; immediate ids keep the CTA at 5 barriers
 __device__ __forceinline__ void pair_sync(int q) {
   switch (q) {
@@ -98,12 +28,6 @@ __device__ __forceinline__ void pair_sync(int q) {
     case 2: asm volatile("bar.sync 3, 64;" ::: "memory"); break;
     default: asm volatile("bar.sync 4, 64;" ::: "memory"); break;
   }
-}
-
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
 }
 
 constexpr int ATT_THREADS = 64 + 256;
@@ -117,9 +41,7 @@ __global__ void __launch_bounds__(ATT_THREADS)
 attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict__ out, int N, int d, int heads, int total) {
   constexpr int W = 64;            // SVTR token grid width for 32x256 crops (modules/svtr.py:348): shifts, not divisions
   extern __shared__ uint8_t smem_raw[];
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   uint8_t* sQ = smem;                          // 8 KiB
   uint8_t* sKV = smem + TILE_BYTES;            // 2 slots x (K 8 KiB + V 8 KiB)
   uint8_t* sP = smem + TILE_BYTES + 4 * TILE_BYTES;   // 32 KiB, 1024-aligned (offset 40 KiB)
@@ -143,16 +65,13 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
     mbar_init(&q_full, 1); mbar_init(&q_empty, 1);
     for (int s = 0; s < 2; ++s) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 1); }
     mbar_init(&s_full, 1); mbar_init(&s_empty, 256); mbar_init(&p_full, 256); mbar_init(&o_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tm)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tm);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"((uint32_t)TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(&tmem_base_sh, TMEM_COLS);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
 
   if (warp == 0) {
@@ -177,17 +96,18 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
   } else if (warp == 1) {
     if (lane == 0) {
       // S = Q K^T : M128 N128, A and B K-major ; O = P V : M128 N32, A K-major, B MN-major
-      constexpr uint32_t idesc_s = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(KT >> 3) << 17) | ((uint32_t)(QT >> 4) << 24);
-      constexpr uint32_t idesc_o = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((uint32_t)(HD >> 3) << 17) | ((uint32_t)(QT >> 4) << 24);
-      const uint64_t qdesc = make_desc(smem_u32(sQ), 512, 4);
-      const uint64_t pdesc = make_desc(smem_u32(sP), 1024, 2);
+      constexpr uint32_t idesc_s = umma_idesc(UMMA_BF16, QT, KT);
+      constexpr uint32_t idesc_o = umma_idesc(UMMA_BF16, QT, HD, false, true);
+      // Q, K, V tiles: rows of 64 B (SWIZZLE_64B), atoms 512 B apart
+      const uint64_t qdesc = umma_smem_desc(smem_u32(sQ), 16, 512, UMMA_SWIZZLE_64B);
+      const uint64_t pdesc = umma_desc_k128(smem_u32(sP));
       // blocks are numbered jc across items: S(jc + 1) goes out as soon as the softmax warps have pulled S(jc) out of TMEM
       // (for the first block of an item also: its Q tile has landed), then P(jc) V(jc)
       auto issue_s = [&](uint32_t jc) {
         const int s = jc & 1;
         mbar_wait(&kv_full[s], (jc >> 1) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint64_t kdesc = make_desc(smem_u32(sKV + s * 2 * TILE_BYTES), 512, 4);
+        tc_fence_after();
+        const uint64_t kdesc = umma_smem_desc(smem_u32(sKV + s * 2 * TILE_BYTES), 16, 512, UMMA_SWIZZLE_64B);
 #pragma unroll
         for (int k = 0; k < HD / 16; ++k) umma_bf16(tmem_base, qdesc + (uint64_t)(k * 2), kdesc + (uint64_t)(k * 2), idesc_s, k);
         umma_commit(&s_full);
@@ -210,9 +130,9 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
             if (j + 2 == nb) umma_commit(&q_empty);               // last S of this item issued: Q is free once it retires
           }
           mbar_wait(&p_full, jc & 1u);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const int s = jc & 1;
-          const uint64_t vdesc = make_desc(smem_u32(sKV + s * 2 * TILE_BYTES + TILE_BYTES), 512, 4);
+          const uint64_t vdesc = umma_smem_desc(smem_u32(sKV + s * 2 * TILE_BYTES + TILE_BYTES), 16, 512, UMMA_SWIZZLE_64B);
 #pragma unroll
           for (int k = 0; k < KT / 16; ++k) {
             // P: two 64-key halves of 16 KiB, +32 B per 16 keys inside the 128 B row; V: +16 key rows of 64 B
@@ -259,7 +179,7 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
     for (int j = 0; j < HD / 2; ++j) acc[j] = 0.f;
     for (int j = 0; j < nb; ++j, ++jc) {
       mbar_wait(&s_full, jc & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       // Local window as a 32-bit validity mask per 32-key chunk (a chunk lies inside one row of the token grid):
       // bit i set <=> |kh - qh| <= 3 and |kw0 + i - qw| <= 5.
       uint32_t vmask[2];
@@ -301,12 +221,12 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
         // deferred accumulation of the previous block: O_{j-1} = P_{j-1} V_{j-1} had all of pass 1 to complete, and
         // its completion also frees the P tile that pass 2 below overwrites
         mbar_wait(&o_full, (jc - 1u) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         uint32_t o[16];
         tmem_ld16(lane_addr + O_COL + (uint32_t)(ch * 16), o);
 #pragma unroll
         for (int i = 0; i < HD / 2; ++i) acc[i] = fmaf(acc[i], corr_prev, __uint_as_float(o[i]));
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
       }
       // pass 2: P = exp2(s*scale*log2e - m) -> bf16 -> swizzled smem (this warp's 64-key half = one 16 KiB P tile half)
 #pragma unroll
@@ -338,7 +258,7 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
           *reinterpret_cast<uint4*>(prow + piece * 16) = make_uint4(pk[p4 * 4], pk[p4 * 4 + 1], pk[p4 * 4 + 2], pk[p4 * 4 + 3]);
         }
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       mbar_arrive(&s_empty);                                      // this warp's half of S_j is consumed
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // generic-proxy smem writes -> visible to UMMA
       mbar_arrive(&p_full);
@@ -348,12 +268,12 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
     }
     {
       mbar_wait(&o_full, (jc - 1u) & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       uint32_t o[16];
       tmem_ld16(lane_addr + O_COL + (uint32_t)(ch * 16), o);
 #pragma unroll
       for (int i = 0; i < HD / 2; ++i) acc[i] = fmaf(acc[i], corr_prev, __uint_as_float(o[i]));
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
     }
     xch[2][ch][r] = l;
     pair_sync(q);
@@ -372,25 +292,9 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
       pair_sync(q);                                                // xch[2] is rewritten by the next item
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS) : "memory");
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
+  if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
 }  // namespace
@@ -398,16 +302,12 @@ EncodeTiledFn encode_fn() {
 // qkv [groups*N, 3d] bf16 -> out [groups*N, d] bf16 ; N % 128 == 0, head_dim 32
 int mrnb_attention_tc(const void* qkv, void* out, int groups, int N, int d, int heads, int H, int W, int local, cudaStream_t st) {
   MRNB_CHECK_ARG(qkv && out && groups > 0 && N % 128 == 0 && d == heads * HD && H * W == N && W == 64, "attention_tc: bad argument (token grid width must be 64)");
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) { mrnb_set_error("attention_tc: cuTensorMapEncodeTiled unavailable"); return MRNB_ERR_UNSUPPORTED; }
   CUtensorMap tm;
   cuuint64_t dims[2] = {(cuuint64_t)(3 * d), (cuuint64_t)((long)groups * N)};
   cuuint64_t strides[1] = {(cuuint64_t)(3 * d) * 2};
   cuuint32_t box[2] = {HD, 128}, es[2] = {1, 1};
-  CUresult r = fn(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(qkv), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("attention_tc: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
+  MRNB_TRY(encode_tensor_map("attention_tc", &tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, qkv, dims, strides, box, es,
+                             CU_TENSOR_MAP_SWIZZLE_64B));
   const size_t smem = 1024 + TILE_BYTES + 4 * TILE_BYTES + P_BYTES;
   static bool attr = false;
   if (!attr) {

@@ -11,70 +11,13 @@
 // One persistent CTA walks work items (g = b * heads + h, 128-query tile); operands arrive by TMA as 32-wide head slices
 // of the [rows, ld] token tensors (64-wide box, the upper half zero-filled by the hardware, only the two non-zero
 // k-steps are issued); shared memory is double buffered so the loads of item i + 1 overlap the epilogue of item i.
-#include "common.cuh"
 #include "gemm_tc2.h"
-#include <cuda.h>
+#include "sm100.cuh"
 
 namespace {
 
 constexpr int BM = 128, BK = 64;
 typedef __nv_bfloat16 bf16;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();      // > 2 s: protocol bug -> kernel error, never a hang
-  }
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t make_desc_k(uint32_t addr) {       // K-major, 128-byte swizzle, 8-row atoms 1024 B apart
-  uint64_t d = 0;
-  d |= (uint64_t)((addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)(16 >> 4) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,"
-      "%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]),
-        "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]),
-        "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 
 struct SpArgs {
   bf16* P;                 // FWD: out probabilities; BWD: in probabilities      [GH][N][N]
@@ -93,8 +36,6 @@ constexpr int EPI_WARPS = 16, NTHREADS = 64 + EPI_WARPS * 32;
 
 __device__ __forceinline__ void epi_sync() { asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory"); }
 
-__device__ __forceinline__ float ex2f(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-
 // MODE 0: forward, all keys visible.  MODE 2: forward, Local window.  MODE 1: backward (dP -> dS).
 template <int N, int MODE>
 __global__ void __launch_bounds__(NTHREADS)
@@ -102,9 +43,7 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   extern __shared__ uint8_t smem_raw[];
   constexpr int A_BYTES = BM * BK * 2, B_BYTES = N * BK * 2, STAGE_BYTES = A_BYTES + B_BYTES;
   constexpr int MT = N / BM;
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   __shared__ __align__(8) uint64_t full_bar[2];
   __shared__ __align__(8) uint64_t empty_bar[2];
   __shared__ __align__(8) uint64_t tmem_full_bar;
@@ -116,17 +55,14 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (threadIdx.x == 0) {
     for (int s = 0; s < 2; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     mbar_init(&tmem_full_bar, 1); mbar_init(&tmem_empty_bar, EPI_WARPS);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"((uint32_t)N) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(&tmem_base_sh, N);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
 
   if (warp == 0) {
@@ -148,18 +84,18 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   } else if (warp == 1) {
     if (lane == 0) {
       constexpr int UN = N >= 256 ? 256 : N;                      // columns per MMA instruction
-      constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(UN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+      constexpr uint32_t idesc = umma_idesc(UMMA_BF16, BM, UN);
       uint32_t it = 0;
       for (long t = blockIdx.x; t < a.items; t += gridDim.x, ++it) {
         const int s = it & 1;
         mbar_wait(&tmem_empty_bar, (it & 1u) ^ 1u);               // the epilogue has drained the accumulator
         mbar_wait(&full_bar[s], (it >> 1) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
-        const uint64_t adesc = make_desc_k(sa);
+        const uint64_t adesc = umma_desc_k128(sa);
 #pragma unroll
         for (int nb = 0; nb < N / UN; ++nb) {
-          const uint64_t bdesc = make_desc_k(sa + A_BYTES + nb * UN * BK * 2);
+          const uint64_t bdesc = umma_desc_k128(sa + A_BYTES + nb * UN * BK * 2);
 #pragma unroll
           for (int k = 0; k < 2; ++k)                              // head_dim 32 = two 16-wide k-steps; the rest of the box is zero
             umma_bf16(tmem_base + (uint32_t)(nb * UN), adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, k != 0 ? 1u : 0u);
@@ -179,7 +115,7 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int n = m0 + rr;                                       // query row inside the (sample, head)
       const long prow = ((long)g * N + n) * N;
       mbar_wait(&tmem_full_bar, it & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
       if (MODE != 1) {
         constexpr bool LOCAL = MODE == 2;
@@ -217,7 +153,7 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const uint32_t vm = chunk_mask(c0);
           if (vm == 0u) continue;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) if (!LOCAL || ((vm >> j) & 1u)) sum += ex2f(fmaf(__uint_as_float(r[j]), sc2, -mx));
+          for (int j = 0; j < 32; ++j) if (!LOCAL || ((vm >> j) & 1u)) sum += ex2_approx(fmaf(__uint_as_float(r[j]), sc2, -mx));
         }
         red_sum[cg][rr] = sum;
         epi_sync();
@@ -236,8 +172,8 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           uint32_t pk[16];
 #pragma unroll
           for (int j = 0; j < 32; j += 2) {
-            const float p0 = (!LOCAL || ((vm >> j) & 1u)) ? ex2f(fmaf(__uint_as_float(r[j]), sc2, -mx)) * inv : 0.f;
-            const float p1 = (!LOCAL || ((vm >> (j + 1)) & 1u)) ? ex2f(fmaf(__uint_as_float(r[j + 1]), sc2, -mx)) * inv : 0.f;
+            const float p0 = (!LOCAL || ((vm >> j) & 1u)) ? ex2_approx(fmaf(__uint_as_float(r[j]), sc2, -mx)) * inv : 0.f;
+            const float p1 = (!LOCAL || ((vm >> (j + 1)) & 1u)) ? ex2_approx(fmaf(__uint_as_float(r[j + 1]), sc2, -mx)) * inv : 0.f;
             __nv_bfloat162 hh = __floats2bfloat162_rn(p0, p1);
             pk[j >> 1] = *reinterpret_cast<uint32_t*>(&hh);
           }
@@ -280,44 +216,23 @@ attn_sp_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
         }
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty_bar);
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)N) : "memory");
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, N);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 // rows of one head: (k, row, head, sample) over a [B * rows, ld] bf16 tensor whose heads are 32-wide column slices
 int encode_head(CUtensorMap* map, const void* ptr, long rows, long ld, int heads, long batch) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) { mrnb_set_error("attn_sp: cuTensorMapEncodeTiled unavailable"); return MRNB_ERR_UNSUPPORTED; }
   if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld * 2) % 16) { mrnb_set_error("attn_sp: misaligned operand"); return MRNB_ERR_ARG; }
   cuuint64_t dims[4] = {32, (cuuint64_t)rows, (cuuint64_t)heads, (cuuint64_t)batch};
   cuuint64_t strides[3] = {(cuuint64_t)ld * 2, 64, (cuuint64_t)rows * ld * 2};
   cuuint32_t box[4] = {64, 128, 1, 1}, es[4] = {1, 1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("attn_sp: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("attn_sp", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, dims, strides, box, es, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 template <int N, int MODE>

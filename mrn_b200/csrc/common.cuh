@@ -154,19 +154,6 @@ template <typename T> __device__ __forceinline__ T from_f32(float v);
 template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
-// Wall-clock guard for mbarrier waits: first call latches the start time, later calls report > 2 s elapsed.
-// (MRNB_WAIT_TRAP_NS: builds for compute-sanitizer runs, whose instrumentation slows kernels by orders of magnitude,
-// raise the limit -- tools/sanitize.sh.)
-#ifndef MRNB_WAIT_TRAP_NS
-#define MRNB_WAIT_TRAP_NS 2000000000ull
-#endif
-__device__ __forceinline__ bool mrnb_wait_expired(uint64_t& t0) {
-  uint64_t now;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-  if (t0 == 0) { t0 = now; return false; }
-  return now - t0 > (unsigned long long)(MRNB_WAIT_TRAP_NS);
-}
-
 // log(exp(a)+exp(b)) with -inf handling
 __device__ __forceinline__ float log_add(float a, float b) {
   const float m = fmaxf(a, b);            // fmaxf drops a NaN operand ...

@@ -12,7 +12,7 @@
 // E_i[b,t] = sum_c softmax(logits)[c] * pad_i[c].  With those, the router-stage gradient
 //   dL/dgate[b,i] = scale_b * sum_t ( E_i[b,t] - sum_s occ[b,t,s] * pad_i[b,t,ext_s] )
 // needs no second pass over the logits (SURVEY.md Appendix A.5 identity, re-associated).
-#include "common.cuh"
+#include "sm100.cuh"
 
 namespace {
 
@@ -45,11 +45,6 @@ __device__ __forceinline__ void acc_merge(float& m, float& s, float (&A)[I], flo
   if (best2 > best || (best2 == best && besti2 < besti)) { best = best2; besti = besti2; }
 }
 
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 constexpr float LOG2E = 1.4426950408889634f;
 
 // Vector pass over one charset segment [lo, hi) in which experts i < K are past their charset (pad value 1.0) and
@@ -303,34 +298,6 @@ constexpr int TMA_CONSUMERS = 704;             // 22 consumer warps: the per-chu
 constexpr int TMA_CHUNK = 4 * TMA_CONSUMERS;   // columns per stage = 4 per consumer thread
 constexpr int TMA_MAX_CHUNKS = 8;
 
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init_(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx_(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_addr(bar)), "r"(parity), "r"(0x989680u) : "memory");
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();      // protocol bug: fail loudly, never hang
-  }
-}
-__device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_addr(dst)), "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(smem_addr(bar)) : "memory");
-}
-
 constexpr int TMA_EPI_WARPS = 4;                          // epilogue warp e finishes rows it = e (mod 4)
 constexpr int TMA_THREADS = TMA_CONSUMERS + 32 + 32 * TMA_EPI_WARPS;      // + producer warp + epilogue warps
 
@@ -349,10 +316,10 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
 
   for (int k = tid; k < nchunks * I * TMA_CHUNK; k += blockDim.x) stage[k] = 1.0f;      // pad value, written once
   if (tid == 0) {
-    for (int j = 0; j < nchunks; ++j) { mbar_init_(&full_bar[j], 1); mbar_init_(&empty_bar[j], TMA_CONSUMERS / 32); }
-    for (int k = 0; k < TMA_EPI_WARPS; ++k) mbar_init_(&rowdone_bar[k], TMA_CONSUMERS / 32);
-    for (int k = 0; k < 2; ++k) mbar_init_(&partfree_bar[k], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int j = 0; j < nchunks; ++j) { mbar_init(&full_bar[j], 1); mbar_init(&empty_bar[j], TMA_CONSUMERS / 32); }
+    for (int k = 0; k < TMA_EPI_WARPS; ++k) mbar_init(&rowdone_bar[k], TMA_CONSUMERS / 32);
+    for (int k = 0; k < 2; ++k) mbar_init(&partfree_bar[k], 1);
+    fence_mbarrier_init();
   }
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy fill before async-proxy (TMA) writes
   __syncthreads();
@@ -392,10 +359,10 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
           int n = myC - j * TMA_CHUNK;
           n = n < 0 ? 0 : (n > TMA_CHUNK ? TMA_CHUNK : n);
           const uint32_t nb = (lane < I && myg != 0.f) ? (uint32_t)((n + 3) & ~3) * 4u : 0u;
-          mbar_wait_(&empty_bar[j], (it & 1u) ^ 1u);
+          mbar_wait(&empty_bar[j], (it & 1u) ^ 1u);
           if (lane == 0) {
-            if (total == 0) mbar_arrive_(&full_bar[j]);
-            else mbar_expect_tx_(&full_bar[j], total);
+            if (total == 0) mbar_arrive(&full_bar[j]);
+            else mbar_expect_tx(&full_bar[j], total);
           }
           __syncwarp();
           if (nb) bulk_load(stage + ((size_t)j * I + lane) * TMA_CHUNK, src + j * TMA_CHUNK, nb, &full_bar[j]);
@@ -438,7 +405,7 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
           for (int i = 0; i < I; ++i) zlab[base + i] = 0.f;
         }
       }
-      mbar_wait_(&rowdone_bar[ew], (it / TMA_EPI_WARPS) & 1u);
+      mbar_wait(&rowdone_bar[ew], (it / TMA_EPI_WARPS) & 1u);
       float m = -INFINITY, s = 0.f, best = -INFINITY;
       int besti = 0x7fffffff;
       float A[I];
@@ -452,7 +419,7 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
                      __float_as_int(pb[3 * TMA_CONSUMERS + k]));
       }
       __syncwarp();
-      if (lane == 0) mbar_arrive_(&partfree_bar[e]);             // partial buffer e may be rewritten (row it + 2)
+      if (lane == 0) mbar_arrive(&partfree_bar[e]);             // partial buffer e may be rewritten (row it + 2)
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
         const float m2 = __shfl_xor_sync(0xffffffffu, m, o);
@@ -510,13 +477,13 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
     float* lrow = logits ? logits + (long)row * ldo : nullptr;
 
     for (int j = 0; j < nchunks; ++j) {
-      mbar_wait_(&full_bar[j], it & 1u);
+      mbar_wait(&full_bar[j], it & 1u);
       const int c0 = j * TMA_CHUNK + tid * 4;
       float4 v[I];
 #pragma unroll
       for (int i = 0; i < I; ++i) v[i] = *reinterpret_cast<const float4*>(stage + ((size_t)j * I + i) * TMA_CHUNK + tid * 4);
       __syncwarp();
-      if (lane == 0) mbar_arrive_(&empty_bar[j]);              // stage j may be refilled with the next row
+      if (lane == 0) mbar_arrive(&empty_bar[j]);              // stage j may be refilled with the next row
       if ((smask >> j) & 1u) {                                 // rare: re-impose the pad on the copied ld padding
 #pragma unroll
         for (int i = 0; i < I; ++i) {
@@ -575,13 +542,13 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
     }
     // ---- hand the per-thread partials to this row's epilogue warp and move on to the next row
     const int buf = it & 1u;
-    mbar_wait_(&partfree_bar[buf], ((it >> 1) & 1u) ^ 1u);
+    mbar_wait(&partfree_bar[buf], ((it >> 1) & 1u) ^ 1u);
     float* pw = part + (size_t)buf * PK * TMA_CONSUMERS + tid;
     pw[0] = m; pw[TMA_CONSUMERS] = s; pw[2 * TMA_CONSUMERS] = best; pw[3 * TMA_CONSUMERS] = __int_as_float(besti);
 #pragma unroll
     for (int i = 0; i < I; ++i) pw[(4 + i) * TMA_CONSUMERS] = A[i];
     __syncwarp();
-    if (lane == 0) mbar_arrive_(&rowdone_bar[it % TMA_EPI_WARPS]);
+    if (lane == 0) mbar_arrive(&rowdone_bar[it % TMA_EPI_WARPS]);
   }
 }
 

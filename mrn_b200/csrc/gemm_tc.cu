@@ -10,9 +10,8 @@
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..5 = epilogue
 // (TMEM lane quarter = warp_id % 4).  Pipelines: smem full/empty mbarriers (TMA <-> MMA) and one TMEM-full
 // mbarrier (MMA -> epilogue).  sm_100a only.
-#include "common.cuh"
 #include "gemm_tc.h"
-#include <cuda.h>
+#include "sm100.cuh"
 
 namespace {
 
@@ -20,106 +19,8 @@ constexpr int BM = 128, BK = 64, UMMA_K = 16;
 constexpr int MAX_STAGES = 2;          // 2 x 32 KiB ring + 32 KiB staging: two persistent CTAs per SM
 constexpr int A_STAGE_BYTES = BM * BK * 2;   // 16 KiB
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)      // suspend-time hint: sleep in hardware, do not spin
-      : "memory");
-  return ok != 0;
-}
-// Bounded wait: a protocol bug traps (kernel error) instead of hanging the GPU.
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0; !mbar_try_wait(bar, parity); ++spin) {
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();   // > 2 s: protocol bug -> fail loudly, never hang
-  }
-}
-
-__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-
-__device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-
-// K-major, 128B-swizzled operand tile: rows of 128 B, 8-row swizzle atoms 1024 B apart (SBO), LBO unused.
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);        // start address, bits [0,14)
-  d |= (uint64_t)1 << 16;                              // leading byte offset (ignored for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                    // stride byte offset, bits [32,46)
-  d |= (uint64_t)1 << 46;                              // descriptor version (Blackwell)
-  d |= (uint64_t)2 << 61;                              // layout type: SWIZZLE_128B
-  return d;
-}
-
-// kind::f16 instruction descriptor: D = fp32, A = B = bf16, both K-major, M = 128, N = BN
-__host__ __device__ constexpr uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-}
-
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
 // Output tensor maps of the TMA-store epilogue (MODE 3: one fp32 [M, C_e] map per expert, box 32 x 32, 128B swizzle)
 struct TcOutMaps { CUtensorMap m[8]; };
-
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1) : "memory");
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
 
 struct TcEpi {
   const float* bias; long bias_gs;
@@ -177,9 +78,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   constexpr int B_STAGE_BYTES = BN * BK * 2;
   constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
   constexpr int TMEM_COLS = 2 * BN;
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   __shared__ __align__(8) uint64_t full_bar[MAX_STAGES];
   __shared__ __align__(8) uint64_t empty_bar[MAX_STAGES];
   __shared__ __align__(8) uint64_t tmem_full_bar[2];
@@ -197,18 +96,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (threadIdx.x == 0) {
     for (int s = 0; s < stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(&tmem_full_bar[b], 1); mbar_init(&tmem_empty_bar[b], EPI_WARPS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmW);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"((uint32_t)TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(&tmem_base_sh, TMEM_COLS);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
 
   if (warp == 0) {
@@ -241,7 +136,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(BN);
+      constexpr uint32_t idesc = umma_idesc(UMMA_BF16, BM, BN);
       uint32_t it = 0;
       int i = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x, ++i) {
@@ -251,15 +146,15 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         const int buf = i & 1;
         mbar_wait(&tmem_empty_bar[buf], (((uint32_t)i >> 1) & 1u) ^ 1u);      // epilogue has drained this accumulator
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t acc = tmem_base + (uint32_t)(buf * BN);
         for (int kb = 0; kb < KB; ++kb, ++it) {
           const int s = it % stages;
           const uint32_t ph = (it / stages) & 1u;
           mbar_wait(&full_bar[s], ph);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
-          const uint64_t adesc = make_smem_desc(sa), bdesc = make_smem_desc(sa + A_STAGE_BYTES);
+          const uint64_t adesc = umma_desc_k128(sa), bdesc = umma_desc_k128(sa + A_STAGE_BYTES);
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
             // advance 16 bf16 = 32 B along K inside the 128 B swizzle row: +2 in the (>>4) address field
@@ -315,7 +210,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
       const float rs = (MODE != 3 && interior && ep.rowscale) ? ep.rowscale[(long)g * ep.rowscale_gs + m0 / ep.rows_per_scale] : 1.0f;
       mbar_wait(&tmem_full_bar[buf], ((uint32_t)i >> 1) & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const uint32_t tcol = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * BN + ch * CW);
       float4 keep[LNF ? NP * 8 : 1];
 #pragma unroll
@@ -328,7 +223,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           uint32_t r[32];
           tmem_ld32(tcol + (uint32_t)(ps * 32), r);
           if (ps == NP - 1) {
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&tmem_empty_bar[buf]);  // this warp's share of the accumulator is out of TMEM
           }
@@ -555,11 +450,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   }
   if (MODE == 3 && warp >= 2 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // bulk stores of this thread are complete
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS) : "memory");
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -600,7 +493,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(LSEQ_THREADS, 1)
 lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
   constexpr int LH = 256;
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   uint8_t* sW = smem;                                        // 4 k-blocks x [256 gate rows x 64 k]
   uint8_t* sA = smem + LSEQ_W_BYTES;                         // 4 k-blocks x [128 samples x 64 k]
   float* staging = reinterpret_cast<float*>(smem + LSEQ_W_BYTES + LSEQ_A_BYTES);
@@ -613,16 +506,13 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
   const int e = g >> 1, dir = g & 1;
   if (threadIdx.x == 0) {
     mbar_init(&w_full, 1); mbar_init(&acc_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmW);
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(256u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 0) tmem_alloc(&tmem_base_sh, 256);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
   if (threadIdx.x == 0) {
     mbar_expect_tx(&w_full, LSEQ_W_BYTES);
@@ -650,10 +540,10 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
     __syncthreads();
     if (threadIdx.x == 0) {
       if (it == 0) mbar_wait(&w_full, 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      constexpr uint32_t idesc = make_idesc(256);
+      tc_fence_after();
+      constexpr uint32_t idesc = umma_idesc(UMMA_BF16, BM, 256);
       for (int kb = 0; kb < 4; ++kb) {
-        const uint64_t ad = make_smem_desc(smem_u32(sA + kb * A_STAGE_BYTES)), bd = make_smem_desc(smem_u32(sW + kb * (256 * BK * 2)));
+        const uint64_t ad = umma_desc_k128(smem_u32(sA + kb * A_STAGE_BYTES)), bd = umma_desc_k128(smem_u32(sW + kb * (256 * BK * 2)));
 #pragma unroll
         for (int k = 0; k < BK / UMMA_K; ++k) umma_bf16(tmem_base, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
       }
@@ -677,7 +567,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
         pvv[itr] = *reinterpret_cast<const uint2*>(prep0 + (long)(m0 + q * 32 + itr * 4 + rsel) * p.pre_row);
       }
       mbar_wait(&acc_full, it & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
 #pragma unroll 1
       for (int ps = 0; ps < 4; ++ps) {
         const int col = nq * 256 + ch * 128 + ps * 32 + p8 * 4;  // interleaved gate column of the chain: unit j = col / 4
@@ -720,7 +610,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
         for (int itr = 0; itr < 8; ++itr) pvv[itr] = pvn[itr];
         __syncwarp();
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       if (s + 1 < p.CT) {
         // next step's input pre-activations (128 rows x 512 B of this CTA's gate columns): HBM -> L2 while the barrier settles
         const int tn = dir ? p.CT - 2 - s : s + 1;
@@ -734,33 +624,13 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap tmW, const LstmSeqArgs p) {
     // h_s of all four gate-column quarters becomes visible to the cluster; the accumulator and the operand tile are free
     cluster_sync_all();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
+  if (warp == 0) tmem_dealloc(tmem_base, 256);
 }
 
 // 3-D map over a [groups][rows][K] bf16 operand (K contiguous): box = 64 x box_rows x 1, 128B swizzle, zero OOB fill
 int make_map(CUtensorMap* map, const void* ptr, long K, long rows, long groups, long ld, long gstride, int box_rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) { mrnb_set_error("tc_gemm: cuTensorMapEncodeTiled is not available from the driver"); return MRNB_ERR_UNSUPPORTED; }
   if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld % 8) || (groups > 1 && gstride % 8)) {
     mrnb_set_error("tc_gemm: operand must be 16-byte aligned with ld %% 8 == 0 (ptr=%p ld=%ld gstride=%ld)", ptr, ld, gstride);
     return MRNB_ERR_ARG;
@@ -769,16 +639,10 @@ int make_map(CUtensorMap* map, const void* ptr, long K, long rows, long groups, 
   cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)(groups > 1 ? gstride : rows * ld) * 2};
   cuuint32_t box[3] = {(cuuint32_t)BK, (cuuint32_t)box_rows, 1};
   cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("tc_gemm: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("tc_gemm", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, ptr, dims, strides, box, estr, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 int make_conv_map(CUtensorMap* map, const void* ptr, const MrnbTcConv& c) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) { mrnb_set_error("tc_gemm: cuTensorMapEncodeTiled is not available from the driver"); return MRNB_ERR_UNSUPPORTED; }
   cuuint64_t dims[4], strides[3];
   for (int j = 0; j < 4; ++j) dims[j] = (cuuint64_t)c.dims[j];
   for (int j = 0; j < 3; ++j) strides[j] = (cuuint64_t)c.strides[j] * 2;
@@ -790,16 +654,13 @@ int make_conv_map(CUtensorMap* map, const void* ptr, const MrnbTcConv& c) {
     mrnb_set_error("tc_gemm: bad convolution view");
     return MRNB_ERR_ARG;
   }
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("tc_gemm: cuTensorMapEncodeTiled (conv) failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("tc_gemm (conv)", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, dims, strides, box, estr,
+                           CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 // 2-D map over an fp32 [rows][cols] output (row pitch ld floats): box 32 x 32, 128B swizzle -- the TMA-store epilogue
 bool make_out_map(CUtensorMap* map, void* ptr, long cols, long rows, long ld) {
-  EncodeTiledFn fn = get_encode_fn();
+  EncodeTiledFn fn = tensor_map_encoder();
   if (!fn || (reinterpret_cast<uintptr_t>(ptr) & 15) || (ld % 4)) return false;
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)ld * 4};

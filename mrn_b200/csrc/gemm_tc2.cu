@@ -10,10 +10,9 @@
 //   * two-level output addressing (same MrnbAxis as gemm_f32.cu), split-K with fp32 atomics, and an epilogue with
 //     bias over n or m, exact GELU, an elementwise multiplier and a residual at the output address.
 // bf16 operands, fp32 accumulation in TMEM.  One 128 x BN output tile per CTA (router GEMMs have K >= 256).
-#include "common.cuh"
 #include "gemm_f32.h"
 #include "gemm_tc2.h"
-#include <cuda.h>
+#include "sm100.cuh"
 
 namespace {
 
@@ -22,70 +21,6 @@ constexpr int BM = 128, BK = 64, UMMA_K = 16;
 __host__ __device__ constexpr int stages_for(int bn) { return bn > 128 ? 4 : 3; }
 constexpr int A_BYTES = BM * BK * 2;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");   // suspend-time hint: no hot spin
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();   // > 2 s: protocol bug -> fail loudly, never hang        // protocol bug -> kernel error, not a hung GPU
-  }
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-// 128B-swizzled operand descriptors (cute::UMMA::SmemDescriptor bit layout).
-//  K-major : rows of 128 B (64 k), 8-row atoms 1024 B apart along M/N (SBO); LBO unused.
-//  MN-major: rows of 128 B (64 m/n), one row per k, 8-k atoms 1024 B apart (SBO); 64-wide MN chunks LBO apart.
-__device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t lbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,"
-      "%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]),
-        "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]),
-        "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
@@ -140,9 +75,7 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   constexpr int B_BYTES = BN * BK * 2;
   constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   constexpr int STAGES = stages_for(BN);
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   __shared__ __align__(8) uint64_t full_bar[STAGES];
   __shared__ __align__(8) uint64_t empty_bar[STAGES];
   __shared__ __align__(8) uint64_t tmem_full_bar[2];
@@ -156,17 +89,14 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(&tmem_full_bar[a], 1); mbar_init(&tmem_empty_bar[a], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"((uint32_t)(2 * BN)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(&tmem_base_sh, 2 * BN);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
 
   auto tile_coords = [&](long t, int& n0, int& m0, int& g, int& kb0, int& KB) {
@@ -218,24 +148,25 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((A_MN ? 1u : 0u) << 15) | ((B_MN ? 1u : 0u) << 16) |
-                                 ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+      constexpr uint32_t idesc = umma_idesc(UMMA_BF16, BM, BN, A_MN, B_MN);
       uint32_t it = 0, ti = 0;
       for (long t = blockIdx.x; t < total; t += gridDim.x, ++ti) {
         int n0, m0, g, kb0, KB;
         tile_coords(t, n0, m0, g, kb0, KB);
         const uint32_t acc = ti & 1u;
         mbar_wait(&tmem_empty_bar[acc], ((ti >> 1) & 1u) ^ 1u);       // epilogue has drained this accumulator
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * (uint32_t)BN;
         for (int i = 0; i < KB; ++i, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1u;
           mbar_wait(&full_bar[s], ph);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
-          const uint64_t adesc = make_desc(sa, A_MN ? BK * 128 : 16);
-          const uint64_t bdesc = make_desc(sa + A_BYTES, B_MN ? BK * 128 : 16);
+          // 128B-swizzled tiles.  K-major: rows of 128 B (64 k), 8-row atoms 1024 B apart along M/N; MN-major: rows of
+          // 128 B (64 m/n), one row per k, 8-k atoms 1024 B apart, 64-wide MN chunks BK * 128 B apart (LBO)
+          const uint64_t adesc = umma_smem_desc(sa, A_MN ? BK * 128 : 16, 1024, UMMA_SWIZZLE_128B);
+          const uint64_t bdesc = umma_smem_desc(sa + A_BYTES, B_MN ? BK * 128 : 16, 1024, UMMA_SWIZZLE_128B);
 #pragma unroll
           for (int k = 0; k < BK / UMMA_K; ++k) {
             // K-major: +32 B inside the swizzled row; MN-major: +16 k-rows of 128 B
@@ -258,7 +189,7 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const uint32_t acc = ti & 1u;
       const int row = m0 + q * 32 + lane;
       mbar_wait(&tmem_full_bar[acc], (ti >> 1) & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const bool rok = row < ep.M;
       const long og = ep.g_inner > 0 ? (long)(g / ep.g_inner) * ep.c_gs + (long)(g % ep.g_inner) * ep.c_gs2 : (long)g * ep.c_gs;
       const long om = rok ? og + (long)(row / ep.cm.inner) * ep.cm.so + (long)(row % ep.cm.inner) * ep.cm.si : 0;
@@ -411,37 +342,17 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         }
       }
       // this warp has read its 32 lanes of the accumulator: hand the buffer back to the MMA warp
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&tmem_empty_bar[acc])) : "memory");
-      }
+      if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]);
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN)) : "memory");
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
+  if (warp == 1) tmem_dealloc(tmem_base, 2 * BN);
 }
 
 int encode(CUtensorMap* map, const MrnbTcOperand& op) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) { mrnb_set_error("tc_gemm2: cuTensorMapEncodeTiled unavailable"); return MRNB_ERR_UNSUPPORTED; }
   cuuint64_t dims[4], strides[3];
   cuuint32_t box[4], es[4] = {1, 1, 1, 1};
   for (int j = 0; j < 4; ++j) { dims[j] = (cuuint64_t)op.dims[j]; box[j] = (cuuint32_t)op.box[j]; }
@@ -452,11 +363,7 @@ int encode(CUtensorMap* map, const MrnbTcOperand& op) {
   }
   for (int j = 0; j < 3; ++j)
     if ((op.strides[j] * 2) % 16) { mrnb_set_error("tc_gemm2: stride %d not a multiple of 16 bytes", j); return MRNB_ERR_ARG; }
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(op.ptr), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("tc_gemm2: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("tc_gemm2", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, op.ptr, dims, strides, box, es, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 template <int BN, bool A_MN, bool B_MN>

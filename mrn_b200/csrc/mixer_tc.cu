@@ -27,9 +27,8 @@
 //     S of the next head is issued behind the last P V of the current one.
 // Shared memory: A, q/k/v of one (OVL: two) head(s) for all tokens (3 x N x 64 B each), one probability / head-output
 // tile per stream, the q|k|v and proj weights of the current head(s), epilogue staging.
-#include "common.cuh"
 #include "mixer_tc.h"
-#include <cuda.h>
+#include "sm100.cuh"
 #include <stdlib.h>
 #include <type_traits>
 
@@ -47,92 +46,6 @@ constexpr int REGS_CTRL = 80, REGS_SOFTMAX = 168, REGS_EPI = 96;       // 128 * 
 constexpr uint32_t Y_COL = 0, S0_COL = 256, S1_COL = 320, O0_COL = 384, O1_COL = 416, STG0_COL = 256, STG1_COL = 352;
 constexpr uint32_t STGX_COL = 448;      // OVL: dedicated 64-column staging of the q|k (64) / v (32) parts of one 128-token tile
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();   // > 2 s: protocol bug -> fail loudly, never hang
-  }
-}
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-// layout_type: 2 = SWIZZLE_128B (rows of 128 B, 8-row atoms 1024 B apart), 4 = SWIZZLE_64B (rows of 64 B, atoms 512 B apart)
-__device__ __forceinline__ uint64_t make_desc(uint32_t addr, uint32_t sbo_bytes, uint32_t layout_type) {
-  uint64_t d = 0;
-  d |= (uint64_t)((addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)layout_type << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]), "r"(r[19]),
-        "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]),
-        "r"(r[30]), "r"(r[31])
-      : "memory");
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ float max3(float a, float b, float c) {
-  float r;
-  asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
-  return r;
-}
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 // named barrier 1 + q for the two partner warps (64 threads) of TMEM lane quarter q
 __device__ __forceinline__ void pair_sync(int q) {
   switch (q) {
@@ -142,15 +55,6 @@ __device__ __forceinline__ void pair_sync(int q) {
     default: asm volatile("bar.sync 4, 64;" ::: "memory"); break;
   }
 }
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-// kind::f16 instruction descriptor: D = fp32, A = B = bf16, K-major A, M = 128; b_mn = 1: B operand MN-major
-__host__ __device__ constexpr uint32_t make_idesc(int n, int b_mn = 0) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-
 template <int D>
 struct MCfg {
   static constexpr int N = 32768 / D;                       // tokens per unit: 512 / 256 / 128
@@ -197,14 +101,6 @@ struct MixParams {
       ep.trace[(slot_) * 256 + (idx_)] = now__;                                                    \
     }                                                                                              \
   } while (0)
-
-__device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
 
 // Y epilogue of ONE 128-token query tile for the 32 rows of the calling warp (TMEM lane quarter q):
 //   x <- x + rs * (Y + b_proj) in place  [+ LayerNorm 2 -> ln_out (bf16)]
@@ -384,9 +280,7 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 const __grid_constant__ CUtensorMap tmWp, const MixParams ep) {
   using K = MCfg<D>;
   extern __shared__ uint8_t smem_raw[];
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   uint8_t* sA = smem;
   uint8_t* sQ = sA + K::A_BYTES;                            // [N rows x 64 B]; then sK, sV
   uint8_t* sK = sQ + K::NT * K::HT_BYTES;
@@ -415,15 +309,12 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     }
     mbar_init(&qkv_ready, EPI_WARPS * 32); mbar_init(&y_full, 2); mbar_init(&st1_done, 1);
     for (int b = 0; b < 4; ++b) mbar_init(&y_empty[b], 4);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmWq)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmWp)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmWq);
+    prefetch_tmap(&tmWp);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(&tmem_base_sh, 512);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -489,7 +380,7 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     // dedicated staging columns; the Y-epilogue warpgroup drains each part into the q/k/v buffer of the head's parity.
     if constexpr (K::OVL) {
       if (lane == 0) {
-        constexpr uint32_t idesc_qk = make_idesc(64), idesc_v = make_idesc(32);
+        constexpr uint32_t idesc_qk = umma_idesc(UMMA_BF16, 128, 64), idesc_v = umma_idesc(UMMA_BF16, 128, 32);
         uint32_t hc = 0, tc = 0, pc = 0;
         for (int u = blockIdx.x; u < total; u += gridDim.x) {
           for (int h = 0; h < K::HEADS; ++h, ++hc) {
@@ -503,8 +394,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 mbar_wait(&stg_empty[0], (pc & 1u) ^ 1u);
                 tc_fence_after();
                 for (int kb = 0; kb < K::KB; ++kb) {
-                  const uint64_t ad = make_desc(smem_u32(sA + kb * 16384), 1024, 2);
-                  const uint64_t bd = make_desc(smem_u32(sWq + kb * K::WQ_KB_BYTES + part * 8192), 1024, 2);
+                  const uint64_t ad = umma_desc_k128(smem_u32(sA + kb * 16384));
+                  const uint64_t bd = umma_desc_k128(smem_u32(sWq + kb * K::WQ_KB_BYTES + part * 8192));
 #pragma unroll
                   for (int k = 0; k < 4; ++k)
                     umma_bf16(tmem_base + STGX_COL, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), part ? idesc_v : idesc_qk, (kb | k) != 0);
@@ -524,7 +415,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     // thread, so every dependency edge is a hardware-sleeping mbarrier wait (no polling between the streams).
     if (lane == 0) {
       const int s = warp == 1 ? 0 : 1;
-      constexpr uint32_t idesc_qkv = make_idesc(96), idesc_s = make_idesc(64), idesc_o = make_idesc(HD, 1), idesc_y = make_idesc(D);
+      constexpr uint32_t idesc_qkv = umma_idesc(UMMA_BF16, 128, 96), idesc_s = umma_idesc(UMMA_BF16, 128, 64);
+      constexpr uint32_t idesc_o = umma_idesc(UMMA_BF16, 128, HD, false, true), idesc_y = umma_idesc(UMMA_BF16, 128, D);
       const uint32_t s_col = s ? S1_COL : S0_COL, o_col = s ? O1_COL : O0_COL;
       uint32_t hc = 0, mc = 0, pc = 0, qc = 0;
       bool s_early = false;                                    // OVL: the first S of the coming head is already issued
@@ -543,8 +435,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
               mbar_wait(&stg_empty[sb], ((mc >> 1) & 1u) ^ 1u);
               tc_fence_after();
               for (int kb = 0; kb < K::KB; ++kb) {
-                const uint64_t ad = make_desc(smem_u32(sA + (mt * K::KB + kb) * 16384), 1024, 2);
-                const uint64_t bd = make_desc(smem_u32(sWq + kb * K::WQ_KB_BYTES), 1024, 2);
+                const uint64_t ad = umma_desc_k128(smem_u32(sA + (mt * K::KB + kb) * 16384));
+                const uint64_t bd = umma_desc_k128(smem_u32(sWq + kb * K::WQ_KB_BYTES));
 #pragma unroll
                 for (int k = 0; k < 4; ++k) umma_bf16(tmem_base + stg_col, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), idesc_qkv, (kb | k) != 0);
               }
@@ -563,8 +455,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           uint8_t* const sKh = sK + (K::OVL ? buf * K::QKV1_BYTES : 0);
           uint8_t* const sVh = sV + (K::OVL ? buf * K::QKV1_BYTES : 0);
           auto issue_s_from = [&](const uint8_t* q_, const uint8_t* k_, int qt, int kr) {
-            const uint64_t qd = make_desc(smem_u32(q_ + qt * K::HT_BYTES), 512, 4);
-            const uint64_t kd = make_desc(smem_u32(k_ + kr * 4096), 512, 4);
+            const uint64_t qd = umma_smem_desc(smem_u32(q_ + qt * K::HT_BYTES), 16, 512, UMMA_SWIZZLE_64B);
+            const uint64_t kd = umma_smem_desc(smem_u32(k_ + kr * 4096), 16, 512, UMMA_SWIZZLE_64B);
 #pragma unroll
             for (int k = 0; k < HD / 16; ++k) umma_bf16(tmem_base + s_col, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc_s, k);
             umma_commit(&s_full[s]);
@@ -591,8 +483,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
               {
                 // O (+)= P V: the accumulator lives in TMEM for the whole query tile (the softmax warps rescale it in
                 // place on the rare occasions the running reference maximum moves)
-                const uint64_t pd = make_desc(smem_u32(sP + s * K::P_TILE), 1024, 2);
-                const uint64_t vd = make_desc(smem_u32(sVh + kr * 4096), 512, 4);
+                const uint64_t pd = umma_desc_k128(smem_u32(sP + s * K::P_TILE));
+                const uint64_t vd = umma_smem_desc(smem_u32(sVh + kr * 4096), 16, 512, UMMA_SWIZZLE_64B);
 #pragma unroll
                 for (int k = 0; k < 64 / 16; ++k)             // P: +32 B per 16 keys inside the 128 B row; V: +16 key rows of 64 B
                   umma_bf16(tmem_base + o_col, pd + (uint64_t)(k * 2), vd + (uint64_t)((k * 16 * 64) >> 4), idesc_o, (!first_of_tile) || k != 0);
@@ -621,8 +513,8 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 // first head: the previous unit's epilogue must have drained THIS tile's Y columns (released tile by tile).
                 // OVL: the stream's own softmax warps run that epilogue before they hand over this head output
                 if (!K::OVL && h == 0) { mbar_wait(&y_empty[qt], ((uint32_t)i & 1u) ^ 1u); tc_fence_after(); }
-                const uint64_t od = make_desc(smem_u32(sP + s * K::P_TILE), 512, 4);
-                const uint64_t wd = make_desc(smem_u32(sWp + buf * K::WP_BYTES), 512, 4);
+                const uint64_t od = umma_smem_desc(smem_u32(sP + s * K::P_TILE), 16, 512, UMMA_SWIZZLE_64B);
+                const uint64_t wd = umma_smem_desc(smem_u32(sWp + buf * K::WP_BYTES), 16, 512, UMMA_SWIZZLE_64B);
 #pragma unroll
                 for (int k = 0; k < HD / 16; ++k)
                   umma_bf16(tmem_base + Y_COL + (uint32_t)(qt * D), od + (uint64_t)(k * 2), wd + (uint64_t)(k * 2), idesc_y, (h | k) != 0);
@@ -968,38 +860,18 @@ mixer_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
 void* g_mixer_trace = nullptr;
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 // [groups][rows][K] bf16, k contiguous: box = box_k x box_rows x 1
 int map3(CUtensorMap* map, const void* ptr, long K, long rows, long groups, int box_k, int box_rows, CUtensorMapSwizzle sw) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) { mrnb_set_error("mixer_tc: cuTensorMapEncodeTiled unavailable"); return MRNB_ERR_UNSUPPORTED; }
   if (reinterpret_cast<uintptr_t>(ptr) & 15) { mrnb_set_error("mixer_tc: misaligned operand"); return MRNB_ERR_ARG; }
   cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)groups};
   cuuint64_t strides[2] = {(cuuint64_t)K * 2, (cuuint64_t)rows * K * 2};
   cuuint32_t box[3] = {(cuuint32_t)box_k, (cuuint32_t)box_rows, 1}, es[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("mixer_tc: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("mixer_tc", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, ptr, dims, strides, box, es, sw);
 }
 
 template <int D, bool LOCAL, bool LNF>

@@ -14,9 +14,8 @@
 // epilogue of tile i runs while the GELU warps already work on tile i + 1 (ncu source view of the previous single-epilogue
 // version: 31 % of the epilogue warps' samples sat in the O -> x / LayerNorm code, serialised with the GELU chunks); the
 // O accumulator is double buffered in TMEM for d <= 128.
-#include "common.cuh"
 #include "mlp_tc.h"
-#include <cuda.h>
+#include "sm100.cuh"
 
 namespace {
 
@@ -25,84 +24,9 @@ constexpr int EPI_WARPS = 8, NTHREADS = 512;
 constexpr int REGS_CTRL = 80, REGS_GELU = 168, REGS_OUT = 96;       // 128 * (80 + 2 * 168 + 96) = 65536
 constexpr int TILE16K = 128 * 64 * 2;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint64_t t0 = 0;
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    if (ok) return;
-    if ((spin & 63u) == 63u && mrnb_wait_expired(t0)) __trap();   // > 2 s: protocol bug -> fail loudly, never hang
-  }
-}
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-// K-major SWIZZLE_128B tile: rows of 128 B, 8-row atoms 1024 B apart
-__device__ __forceinline__ uint64_t make_desc(uint32_t addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((addr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 // 16-byte-chunk swizzle key of row rl in the staged fp32 tiles (row pitch a multiple of 128 B): a quarter warp touches
 // rows {2k, 2k+1} x 4 consecutive chunks, so bit 2 separates the two rows and bits 0-1 the row pairs -> conflict free
 __device__ __forceinline__ int xs_key(int rl) { return ((rl & 1) << 2) | ((rl >> 1) & 3); }
-__host__ __device__ constexpr uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-}
-
 struct MlpParams {
   const float* b1; const float* b2; long b_gs1, b_gs2;        // [groups][4D], [groups][D]
   float* x; long x_gs;                                        // fp32 residual stream, in place: [g][rows][D]
@@ -147,9 +71,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
               const __grid_constant__ CUtensorMap tmW2, const MlpParams ep) {
   using K = Cfg<D>;
   extern __shared__ uint8_t smem_raw[];
-  // 1 KiB alignment by OFFSET (not by integer round-trip of the pointer): the compiler keeps the shared address space,
-  // so staging / operand tiles are accessed with LDS / STS instead of generic LD / ST
-  uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   uint8_t* sA = smem;
   uint8_t* sP = smem + K::A_BYTES;
   uint8_t* ring = sP + K::P_BYTES;
@@ -168,18 +90,15 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
     for (int b = 0; b < 2; ++b) { mbar_init(&s_full[b], 1); mbar_init(&s_empty[b], EPI_WARPS); }
     mbar_init(&p_full, EPI_WARPS); mbar_init(&p_empty, 1);
     for (int b = 0; b < 2; ++b) { mbar_init(&o_full[b], 1); mbar_init(&o_empty[b], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW1)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW2)) : "memory");
+    fence_mbarrier_init();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmW1);
+    prefetch_tmap(&tmW2);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(&tmem_base_sh, 512);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_sh;
 
   if (warp < 4) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_CTRL));
@@ -189,7 +108,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       uint32_t it = 0;
       auto load_w = [&](const CUtensorMap* map, int c0, int c1, int g, uint32_t bytes) {
         const int s = it % K::RS;
-        mbar_wait(&w_empty[s], ((it / K::RS) & 1u) ^ 1u);
+        mbar_wait_nohint(&w_empty[s], ((it / K::RS) & 1u) ^ 1u);
         mbar_expect_tx(&w_full[s], bytes);
         tma_load_3d(ring + (size_t)s * K::SLOT, map, &w_full[s], c0, c1, g);
         ++it;
@@ -198,7 +117,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       //   { W1_{c+1}  |  at the last chunk: A and W1_0 of the NEXT tile (its S_0 is issued before this tile's last P W2) } ; W2_c
       auto load_a = [&](int ti, int t) {
         const int g = t / m_tiles, m0 = (t % m_tiles) * BM;
-        mbar_wait(&a_empty, ((uint32_t)ti & 1u) ^ 1u);
+        mbar_wait_nohint(&a_empty, ((uint32_t)ti & 1u) ^ 1u);
         mbar_expect_tx(&a_full, K::A_BYTES);
         for (int kb = 0; kb < K::KB; ++kb) tma_load_3d(sA + kb * TILE16K, &tmA, &a_full, kb * BK, m0, g);
         for (int kb = 0; kb < K::KB; ++kb) load_w(&tmW1, kb * BK, 0, g, TILE16K);
@@ -221,51 +140,51 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   } else if (warp == 1) {
     // ============================== MMA issuer ==============================
     if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc(HC);
-      constexpr uint32_t idesc_o = make_idesc(K::W2ROWS) & ~((7u << 7) | (7u << 10));   // second GEMM in f16 x f16: P (GELU output) and W2 are f16
+      constexpr uint32_t idesc_s = umma_idesc(UMMA_BF16, BM, HC);
+      constexpr uint32_t idesc_o = umma_idesc(UMMA_F16, BM, K::W2ROWS);      // second GEMM in f16 x f16: P (GELU output) and W2 are f16
       uint32_t it = 0;
       int i = 0;
       auto issue_s = [&](int ti, int c) {
           const int b = c & 1;
           const uint32_t u = (uint32_t)(ti * (K::C / 2) + (c >> 1));
-          mbar_wait(&s_empty[b], (u & 1u) ^ 1u);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          mbar_wait_nohint(&s_empty[b], (u & 1u) ^ 1u);
+          tc_fence_after();
           for (int kb = 0; kb < K::KB; ++kb, ++it) {
             const int s = it % K::RS;
-            mbar_wait(&w_full[s], (it / K::RS) & 1u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint64_t ad = make_desc(smem_u32(sA + kb * TILE16K)), bd = make_desc(smem_u32(ring + (size_t)s * K::SLOT));
+            mbar_wait_nohint(&w_full[s], (it / K::RS) & 1u);
+            tc_fence_after();
+            const uint64_t ad = umma_desc_k128(smem_u32(sA + kb * TILE16K)), bd = umma_desc_k128(smem_u32(ring + (size_t)s * K::SLOT));
 #pragma unroll
             for (int k = 0; k < 4; ++k) umma_bf16(tmem_base + (uint32_t)(b * HC), ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), idesc_s, (kb | k) != 0);
             umma_commit(&w_empty[s]);
           }
           umma_commit(&s_full[b]);
       };
-      if ((int)blockIdx.x < total) { mbar_wait(&a_full, 0u); issue_s(0, 0); }
+      if ((int)blockIdx.x < total) { mbar_wait_nohint(&a_full, 0u); issue_s(0, 0); }
       for (int t = blockIdx.x; t < total; t += gridDim.x, ++i) {
         for (int c = 0; c < K::C; ++c) {
           if (c + 1 < K::C) {
             issue_s(i, c + 1);
           } else if (t + (int)gridDim.x < total) {
             // S_0 of the NEXT tile goes out before this tile's last P W2: the GELU warps find it ready at the tile boundary
-            mbar_wait(&a_full, (uint32_t)(i + 1) & 1u);
+            mbar_wait_nohint(&a_full, (uint32_t)(i + 1) & 1u);
             issue_s(i + 1, 0);
           }
           if (c + 1 == K::C - 1) umma_commit(&a_empty);                   // last S of this tile issued: A is free once it retires
           const uint32_t up = (uint32_t)(i * K::C + c);
           MRNB_TRACE(0, (int)up);                          // MMA: S_{c+1} issued, start waiting for P_c
-          mbar_wait(&p_full, up & 1u);
+          mbar_wait_nohint(&p_full, up & 1u);
           MRNB_TRACE(1, (int)up);                          // MMA: P_c available
           // O accumulator of this tile: buffer i % OB, free once the output epilogue of tile i - OB has drained it
           const uint32_t ob = K::OB == 2 ? ((uint32_t)i & 1u) : 0u, on = K::OB == 2 ? ((uint32_t)i >> 1) : (uint32_t)i;
-          if (c == 0) mbar_wait(&o_empty[ob], (on & 1u) ^ 1u);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          if (c == 0) mbar_wait_nohint(&o_empty[ob], (on & 1u) ^ 1u);
+          tc_fence_after();
           for (int kk = 0; kk < 2; ++kk) {
             for (int nh = 0; nh < K::NH; ++nh, ++it) {
               const int s = it % K::RS;
-              mbar_wait(&w_full[s], (it / K::RS) & 1u);
-              asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-              const uint64_t ad = make_desc(smem_u32(sP + kk * TILE16K)), bd = make_desc(smem_u32(ring + (size_t)s * K::SLOT));
+              mbar_wait_nohint(&w_full[s], (it / K::RS) & 1u);
+              tc_fence_after();
+              const uint64_t ad = umma_desc_k128(smem_u32(sP + kk * TILE16K)), bd = umma_desc_k128(smem_u32(ring + (size_t)s * K::SLOT));
 #pragma unroll
               for (int k = 0; k < 4; ++k)
                 umma_bf16(tmem_base + K::O_COL + ob * (uint32_t)D + (uint32_t)(nh * K::W2ROWS), ad + (uint64_t)(k * 2),
@@ -300,13 +219,13 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         const int b = c & 1;
         const uint32_t u = (uint32_t)(i * (K::C / 2) + (c >> 1));
         if (warp == 4 && lane == 0) MRNB_TRACE(3, i * K::C + c);   // epi: start waiting for S_c
-        mbar_wait(&s_full[b], u & 1u);
+        mbar_wait_nohint(&s_full[b], u & 1u);
         if (warp == 4 && lane == 0) MRNB_TRACE(4, i * K::C + c);   // epi: S_c ready
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         uint32_t v0[32], v1[32];
         tmem_ld32(lane_addr + (uint32_t)(b * HC + ch * 64), v0);
         tmem_ld32(lane_addr + (uint32_t)(b * HC + ch * 64 + 32), v1);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&s_empty[b]);
         // +b1 (fp32), then GELU two values at a time in f16x2; P is handed to the tensor core as an f16 operand
@@ -326,7 +245,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         }
         const uint32_t up = (uint32_t)(i * K::C + c);
         if (warp == 4 && lane == 0) MRNB_TRACE(5, (int)up);        // epi: GELU done
-        mbar_wait(&p_empty, (up & 1u) ^ 1u);                   // previous P has been consumed by its MMAs (GELU already done)
+        mbar_wait_nohint(&p_empty, (up & 1u) ^ 1u);                   // previous P has been consumed by its MMAs (GELU already done)
         if (warp == 4 && lane == 0) MRNB_TRACE(6, (int)up);        // epi: P buffer free
         uint8_t* prow = sP + ch * TILE16K + r * 128;
 #pragma unroll
@@ -377,9 +296,9 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
         for (int k = 0; k < D / 32; ++k) asm volatile("prefetch.global.L2 [%0];" ::"l"(xl2 + (long)(k * 32 + lane) * 128));
       }
-      mbar_wait(&o_full[ob], on & 1u);
+      mbar_wait_nohint(&o_full[ob], on & 1u);
       if (warp == 12 && lane == 0) MRNB_TRACE(8, i);               // out: O ready
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       __nv_bfloat16* ct = (!LNF && ep.cast_out) ? ep.cast_out + (long)g * ep.ln_gs + (long)(m0 + q * 32) * D : nullptr;
       float sum[4] = {0.f, 0.f, 0.f, 0.f}, sq[4] = {0.f, 0.f, 0.f, 0.f};
       constexpr bool XS = LNF && K::XT_BYTES > 0;              // residual rows staged in shared memory (LayerNorm variants:
@@ -408,7 +327,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         uint32_t v[16];
         tmem_ld16(lane_addr + K::O_COL + ob * (uint32_t)D + (uint32_t)(c * 16), v);
         if (c == D / 16 - 1) {
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(&o_empty[ob]);            // accumulator drained: a later tile may overwrite it
         }
@@ -473,38 +392,17 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
 int map3(CUtensorMap* map, const void* ptr, long K, long rows, long groups, long ld, long gstride, int box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) { mrnb_set_error("mlp_tc: cuTensorMapEncodeTiled unavailable"); return MRNB_ERR_UNSUPPORTED; }
   if ((reinterpret_cast<uintptr_t>(ptr) & 15) || (ld % 8) || (gstride % 8)) { mrnb_set_error("mlp_tc: misaligned operand"); return MRNB_ERR_ARG; }
   cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)groups};
   cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)gstride * 2};
   cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1}, es[3] = {1, 1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, es,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { mrnb_set_error("mlp_tc: cuTensorMapEncodeTiled failed (%d)", (int)r); return MRNB_ERR_ARG; }
-  return MRNB_OK;
+  return encode_tensor_map("mlp_tc", map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, ptr, dims, strides, box, es, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 template <int D, bool LNF>
