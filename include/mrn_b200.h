@@ -368,6 +368,15 @@ int mrnb_svtr_attention_f32(const float* qkv, float* out, int groups, int N, int
 /* tcgen05 attention (bf16 mode): qkv [groups*N, 3d] bf16 -> out [groups*N, d] bf16; N % 128 == 0, head_dim 32. */
 int mrnb_svtr_attention_bf16(const void* qkv, void* out, int groups, int N, int d, int heads, int H, int W, int local,
                              cudaStream_t stream);
+/* Training attention of one SVTR stage on the tensor cores (bf16 mode of the stage-0 step), head_dim 32, d = 32 * heads,
+ * N in {128, 256, 512} tokens on an (N / W) x W grid, W a power of two >= 32.
+ *   forward : qkv [B*N, 3d] bf16 -> P [B*heads, N, N] bf16 = softmax(32^-0.5 q k^T [+ Local 7x11 window]), O [B*N, d] bf16 = P v
+ *   backward: dO fp32 and its bf16 copy dO16 [B*N, d], with the forward's qkv, O and P -> dS [B*heads, N, N] bf16 =
+ *             P (dO v^T - dO.O), dqkv [B*N, 3d] bf16 = (dQ | dK | dV). */
+int mrnb_attn_tc_train_forward(const void* qkv, void* P, void* O, int B, int N, int d, int heads, int W, int local,
+                               cudaStream_t stream);
+int mrnb_attn_tc_train_backward(const void* qkv, const void* O, const float* dO, const void* dO16, const void* P, void* dS,
+                                void* dqkv, int B, int N, int d, int heads, cudaStream_t stream);
 int mrnb_cast_f32_to_bf16(const float* x, void* y, long n, cudaStream_t stream);
 int mrnb_cast_f32_to_f16(const float* x, void* y, long n, cudaStream_t stream);
 

@@ -115,6 +115,8 @@ _SIGNATURES = {
     "mrnb_layernorm_f32": (_i, [_vp, _vp, _vp, _vp, _l, _i, _f, _vp]),
     "mrnb_svtr_attention_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "mrnb_svtr_attention_bf16": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "mrnb_attn_tc_train_forward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "mrnb_attn_tc_train_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     "mrnb_cast_f32_to_bf16": (_i, [_vp, _vp, _l, _vp]),
     "mrnb_cast_f32_to_f16": (_i, [_vp, _vp, _l, _vp]),
 }

@@ -198,9 +198,9 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
           vmask[cc] = mk;
         }
       }
-      // pass 1: maximum over the chunks this warp visits.  The Local window mask is NOT applied here: any reference
-      // >= the true row maximum keeps exp2() <= 1, and the keys of a visited chunk sit next to the window, so the
-      // reference stays within a few units of the masked maximum (the bf16 / fp32 exponent range is ample).
+      // pass 1: maximum over the visible keys of the chunks this warp visits.  The Local window mask must apply here:
+      // a masked key next to the window can score tens of log2 units above every visible one (peaked scores), and a
+      // reference that high flushes all visible exp2() terms to zero -> l = 0 and a NaN / inf output row.
       float bmax = -INFINITY;
 #pragma unroll
       for (int cc = 0; cc < 2; ++cc) {
@@ -208,7 +208,14 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tm, __nv_bfloat16* __restrict
         uint32_t v[32];
         tmem_ld32(lane_addr + (uint32_t)((ch * 2 + cc) * 32), v);
 #pragma unroll
-        for (int i = 0; i < 32; i += 2) bmax = max3(bmax, __uint_as_float(v[i]), __uint_as_float(v[i + 1]));
+        for (int i = 0; i < 32; i += 2) {
+          float s0 = __uint_as_float(v[i]), s1 = __uint_as_float(v[i + 1]);
+          if (LOCAL) {
+            if (!((vmask[cc] >> i) & 1u)) s0 = -INFINITY;
+            if (!((vmask[cc] >> (i + 1)) & 1u)) s1 = -INFINITY;
+          }
+          bmax = max3(bmax, s0, s1);
+        }
       }
       xch[jc & 1][ch][r] = bmax;
       pair_sync(q);                                              // the two warps of this lane quarter

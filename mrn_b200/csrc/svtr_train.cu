@@ -1167,3 +1167,19 @@ extern "C" int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtr
   mrnb_set_error("svtr_train_backward: unknown precision %d", prec);
   return MRNB_ERR_ARG;
 }
+
+// ---- C-ABI test entries: the bf16 training attention of one stage, forwarded unchanged to attn_tc_forward /
+// attn_tc_backward so the score kernel and the four value-side head GEMMs can be compared with a reference on their own
+extern "C" int mrnb_attn_tc_train_forward(const void* qkv, void* P, void* O, int B, int N, int d, int heads, int W, int local,
+                                          cudaStream_t stream) {
+  MRNB_CHECK_ARG(qkv && P && O && B > 0 && heads > 0 && d == 32 * heads, "attn_tc_train_forward: bad argument");
+  return attn_tc_forward((const bf16*)qkv, (bf16*)P, (bf16*)O, B, N, d, heads, W, local != 0, stream);
+}
+
+extern "C" int mrnb_attn_tc_train_backward(const void* qkv, const void* O, const float* dO, const void* dO16, const void* P,
+                                           void* dS, void* dqkv, int B, int N, int d, int heads, cudaStream_t stream) {
+  MRNB_CHECK_ARG(qkv && O && dO && dO16 && P && dS && dqkv && B > 0 && heads > 0 && d == 32 * heads,
+                 "attn_tc_train_backward: bad argument");
+  return attn_tc_backward((const bf16*)qkv, (const bf16*)O, dO, (const bf16*)dO16, (const bf16*)P, (bf16*)dS, (bf16*)dqkv, B, N,
+                          d, heads, stream);
+}

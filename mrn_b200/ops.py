@@ -90,12 +90,23 @@ def cast_f16(x: torch.Tensor) -> torch.Tensor:
     return y
 
 
-def linear_bf16(a, w, bias=None, residual=None, gelu=False, out_f32=True):
+def _out(out, shape, device, dtype):
+    """A caller-supplied output (e.g. NaN pre-filled by a test, so that an element the kernel never writes shows) or a
+    fresh one."""
+    if out is None:
+        return torch.empty(shape, device=device, dtype=dtype)
+    if tuple(out.shape) != tuple(shape) or out.dtype != dtype or not out.is_contiguous() or out.device != device:
+        raise RuntimeError("out: expected a contiguous %s tensor of shape %s on %s, got %s %s on %s"
+                           % (dtype, tuple(shape), device, out.dtype, tuple(out.shape), out.device))
+    return out
+
+
+def linear_bf16(a, w, bias=None, residual=None, gelu=False, out_f32=True, out=None):
     assert a.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and a.is_contiguous() and w.is_contiguous()
     _chk_f32(bias, residual)
     M, K = a.shape
     N = w.shape[0]
-    out = torch.empty(M, N, device=a.device, dtype=torch.float32 if out_f32 else torch.bfloat16)
+    out = _out(out, (M, N), a.device, torch.float32 if out_f32 else torch.bfloat16)
     L.check(L.load().mrnb_linear_bf16(_p(a), _p(w), _p(bias), _p(residual), _p(out), int(out_f32), M, N, K, int(gelu),
                                       _stream()), "linear_bf16")
     return out
@@ -150,13 +161,42 @@ def svtr_attention(qkv, heads, H, W, local):
     return out
 
 
-def svtr_attention_bf16(qkv, heads, H, W, local):
+def svtr_attention_bf16(qkv, heads, H, W, local, out=None):
     assert qkv.dtype == torch.bfloat16 and qkv.is_contiguous()
     G, N, d3 = qkv.shape
-    out = torch.empty(G, N, d3 // 3, device=qkv.device, dtype=torch.bfloat16)
+    out = _out(out, (G, N, d3 // 3), qkv.device, torch.bfloat16)
     L.check(L.load().mrnb_svtr_attention_bf16(_p(qkv), _p(out), G, N, d3 // 3, heads, H, W, int(local), _stream()),
             "attention_bf16")
     return out
+
+
+def attn_tc_train_forward(qkv, heads, W, local, P=None, O=None):
+    """Training attention forward of one stage (bf16 mode): qkv [B, N, 3d] bf16 -> (P [B*heads, N, N] bf16 = the
+    probabilities kept for the backward, O [B, N, d] bf16)."""
+    assert qkv.dtype == torch.bfloat16 and qkv.is_contiguous()
+    B, N, d3 = qkv.shape
+    d = d3 // 3
+    P = _out(P, (B * heads, N, N), qkv.device, torch.bfloat16)
+    O = _out(O, (B, N, d), qkv.device, torch.bfloat16)
+    L.check(L.load().mrnb_attn_tc_train_forward(_p(qkv), _p(P), _p(O), B, N, d, heads, W, int(local), _stream()),
+            "attn_tc_train_forward")
+    return P, O
+
+
+def attn_tc_train_backward(qkv, O, P, dO, dO16, heads, dS=None, dqkv=None):
+    """Training attention backward of one stage (bf16 mode): dO [B, N, d] fp32 and its bf16 copy dO16, with the
+    forward's qkv, O and P -> (dS [B*heads, N, N] bf16, dqkv [B, N, 3d] bf16 = dQ | dK | dV)."""
+    assert qkv.dtype == O.dtype == P.dtype == dO16.dtype == torch.bfloat16
+    assert qkv.is_contiguous() and O.is_contiguous() and P.is_contiguous() and dO16.is_contiguous()
+    _chk_f32(dO)
+    B, N, d3 = qkv.shape
+    d = d3 // 3
+    assert O.shape == dO.shape == dO16.shape == (B, N, d) and P.shape == (B * heads, N, N)
+    dS = _out(dS, (B * heads, N, N), qkv.device, torch.bfloat16)
+    dqkv = _out(dqkv, (B, N, d3), qkv.device, torch.bfloat16)
+    L.check(L.load().mrnb_attn_tc_train_backward(_p(qkv), _p(O), _p(dO), _p(dO16), _p(P), _p(dS), _p(dqkv), B, N, d, heads,
+                                                 _stream()), "attn_tc_train_backward")
+    return dS, dqkv
 
 
 # ------------------------------------------------------------------------------------------------ SVTR experts
