@@ -317,6 +317,23 @@ int mrnb_ctc_dense_grad(const float* logits, long ldl, const float* lse, const f
 int mrnb_greedy_decode(const int* amax, const float* maxprob, int B, int T, int* out_ids, int* out_len, float* conf,
                        cudaStream_t stream);
 
+/* CTC prefix beam search (N-best decoding).  No counterpart in the reference: an addition to its greedy decode,
+ * test.py:211-221.  Opt-in; the default decode stays mrnb_greedy_decode.
+ *
+ * mrnb_ctc_topk: per-frame candidate pruning on the same expert table and gate as mrnb_gate_combine (z, ld, Ci are HOST
+ *   arrays; experts with a zero gate are not read) and the lse [B,T] it wrote.  The combined value is recomputed with
+ *   the combine's expression, so top_ids[...,0] equals its amax wherever amax != 0.  Writes top_ids [B,T,K] int32 (the K
+ *   non-blank classes with the highest combined value, ties to the smaller class; -1 past the C-1 real classes),
+ *   top_lp [B,T,K] = value - lse (-inf in unused slots) and blank_lp [B,T].  1 <= K <= 32.
+ * mrnb_ctc_beam_search: CTC prefix beam search in log space over blank + the K candidates of every frame, beam width W,
+ *   the n_best best labelings out: ids [B,n_best,T] compact (-1 padded), len [B,n_best], score [B,n_best] = log p of
+ *   the labeling over the kept alignments.  Ties: stay before extension, then the parent's rank, then the class index
+ *   (class indices < 2^26).  1 <= K <= 32, 1 <= W <= 32, 1 <= n_best <= W, 1 <= T <= 128.  No workspace. */
+int mrnb_ctc_topk(const float* const* z, const long* ld, const int* Ci, int n_experts, const float* gate, const float* lse,
+                  int B, int T, int K, int* top_ids, float* top_lp, float* blank_lp, cudaStream_t stream);
+int mrnb_ctc_beam_search(const int* top_ids, const float* top_lp, const float* blank_lp, int B, int T, int K, int W,
+                         int n_best, int* out_ids, int* out_len, float* out_score, cudaStream_t stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * Image preparation on the device.  Replaces data/dataset.py:235-246 (ResizeNormalize: PIL Image.resize((imgW, imgH),
  * BICUBIC) on the RGBA crop -> torchvision ToTensor -> sub_(0.5).div_(0.5)) as applied per image by AlignCollate

@@ -104,6 +104,8 @@ _SIGNATURES = {
     "mrnb_ctc_lattice": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp, _vp]),
     "mrnb_ctc_dense_grad": (_i, [_vp, _l, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _l, _vp]),
     "mrnb_greedy_decode": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
+    "mrnb_ctc_topk": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "mrnb_ctc_beam_search": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "mrnb_resize_workspace_bytes": (_sz, [_i, _i, _i]),
     "mrnb_resize_normalize_rgba": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
     "mrnb_clip_adam": (_i, [_vp, _vp, _vp, _vp, _l, _f, _f, _f, _f, _f, _i, _vp, _vp, _vp]),

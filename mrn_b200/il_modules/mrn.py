@@ -5,7 +5,8 @@ What runs where
   * stage 1 (router training, il_modules/mrn.py:298-384) -- the north-star hot path -- is one fused device step:
     grouped frozen experts -> DM-Router -> gate -> fused combine + CTC -> analytic gate gradient -> router backward
     -> [NCCL all-reduce of the gradient arena] -> clip + Adam.  No autograd graph, no host sync inside the step.
-  * validation (test.py:139-279) uses the hard route + device-side greedy decode (one D2H copy per batch).
+  * validation (test.py:139-279) uses the hard route + device-side greedy decode (one D2H copy per batch), or with
+    opt.decode = "beam" the device CTC prefix beam search (an addition beyond the reference).
   * stage 0 (training the newest expert end to end, il_modules/mrn.py:225-279; SURVEY.md §8(f)3) for SVTR experts:
     activation-keeping forward -> fused log-softmax + CTC -> dense CTC gradient -> hand-written backward to every
     parameter of the expert (mrnb_svtr_train_forward / _backward) -> [NCCL all-reduce of the expert's gradient arena]
@@ -527,33 +528,48 @@ class MRN(object):
                 train_taski_loss_avg.reset()
 
     # ---- evaluation ----------------------------------------------------------------------------------
-    def infer_batch(self, image, val_choose="TF", labels_index=None, labels_length=None):
-        """Hard-routed (TF) or last-expert (FF) inference + device-side greedy decode.
-        Returns dict(ids, lens, conf, index, loss) -- ids compact [B,T] (-1 padded)."""
+    def infer_batch(self, image, val_choose="TF", labels_index=None, labels_length=None, decode="greedy", beam_width=8,
+                    beam_topk=16, n_best=1):
+        """Hard-routed (TF) or last-expert (FF) inference + device-side decode.
+        Returns dict(ids, lens, conf, index, loss) -- ids compact [B,T] (-1 padded).
+        decode="greedy": best path (test.py:211-221).  decode="beam": CTC prefix beam search of width beam_width over the
+        beam_topk best classes of every frame; ids / lens / conf = exp(score) are the best labeling's, and n_best > 1 adds
+        nbest_ids [B,n_best,T], nbest_lens [B,n_best] and nbest_scores [B,n_best] (log-probabilities, best first)."""
+        if decode not in ("greedy", "beam"):
+            raise ValueError("decode must be 'greedy' or 'beam', got %r" % (decode,))
+        beam = decode == "beam"
         net = self.net
         if val_choose == "FF":
             out = net(image, cross=False, is_train=False)
             gate = torch.ones(image.shape[0], 1, device=image.device)
-            r = ops.gate_combine([out["logits"]], gate, labels_index, labels_length, want_decode=True)
-            index = None
+            r = ops.gate_combine([out["logits"]], gate, labels_index, labels_length, want_decode=not beam)
+            experts, index = [out["logits"]], None
         else:
             r = net.route_and_combine(image, is_train=False, want_logits=False, targets=labels_index, lengths=labels_length,
-                                      want_decode=True)
-            index = r["index"]
+                                      want_decode=not beam)
+            experts, gate, index = r["expert_logits"], r["combine_gate"], r["index"]
         loss = None
         if labels_index is not None:
             loss = ops.ctc_lattice(r["lpe"], labels_index, labels_length)["loss"]
-        ids, lens, conf = ops.greedy_decode(r["amax"], r["maxprob"])
-        return dict(ids=ids, lens=lens, conf=conf, index=index, loss=loss)
+        if not beam:
+            ids, lens, conf = ops.greedy_decode(r["amax"], r["maxprob"])
+            return dict(ids=ids, lens=lens, conf=conf, index=index, loss=loss)
+        top_ids, top_lp, blank_lp = ops.ctc_topk(experts, gate, r["lse"], beam_topk)
+        nb_ids, nb_lens, nb_scores = ops.ctc_beam_search(top_ids, top_lp, blank_lp, beam_width, n_best)
+        res = dict(ids=nb_ids[:, 0], lens=nb_lens[:, 0], conf=nb_scores[:, 0].exp(), index=index, loss=loss)
+        if n_best > 1:
+            res.update(nbest_ids=nb_ids, nbest_lens=nb_lens, nbest_scores=nb_scores)
+        return res
 
-    def infer_batch_graphed(self, image, val_choose="TF"):
-        """infer_batch replayed from a CUDA graph captured per (batch size, route): small batches are launch-bound
+    def infer_batch_graphed(self, image, val_choose="TF", decode="greedy", beam_width=8, beam_topk=16, n_best=1):
+        """infer_batch replayed from a CUDA graph captured per (batch size, route, decode settings): small batches are launch-bound
         (~95 kernels), and a replay costs one launch.  The graph owns static input / output buffers; the returned
         tensors are views of the static outputs and stay valid until the next replay for the same batch size.
         Eval-mode experts only (train-mode BatchNorm / DropPath state is not captured)."""
         if any(self.net._experts_train_mode()):
             raise RuntimeError("infer_batch_graphed needs eval-mode experts (call model.eval() first)")
-        key = (int(image.shape[0]), val_choose, str(image.device))
+        dec = dict(decode=decode, beam_width=beam_width, beam_topk=beam_topk, n_best=n_best)
+        key = (int(image.shape[0]), val_choose, str(image.device)) + tuple(dec.values())
         cache = self.__dict__.setdefault("_infer_graphs", {})
         ent = cache.get(key)
         if ent is None:
@@ -562,12 +578,12 @@ class MRN(object):
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):             # warm-up on a side stream: lazy allocations, attribute setup, packs
                 for _ in range(2):
-                    self.infer_batch(static_in, val_choose)
+                    self.infer_batch(static_in, val_choose, **dec)
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                out = self.infer_batch(static_in, val_choose)
+                out = self.infer_batch(static_in, val_choose, **dec)
             ent = cache[key] = (graph, static_in, out)
         graph, static_in, out = ent
         static_in.copy_(image, non_blocking=True)
@@ -575,7 +591,10 @@ class MRN(object):
         return out
 
     def validation(self, eval_loader, val_choose="TF"):
-        """test.py:139-279 with the decode / confidence on the device."""
+        """test.py:139-279 with the decode / confidence on the device.  opt.decode ("greedy", the default, or "beam"),
+        opt.beam_width (8) and opt.beam_topk (16) choose the decoder; a config without them decodes greedily."""
+        dec = dict(decode=getattr(self.opt, "decode", "greedy"), beam_width=int(getattr(self.opt, "beam_width", 8)),
+                   beam_topk=int(getattr(self.opt, "beam_topk", 16)))
         n_correct, norm_ED, length_of_data, infer_time = 0, 0.0, 0, 0.0
         valid_loss_avg = Averager()
         preds_str, confidence, labels = [], [], []
@@ -585,7 +604,7 @@ class MRN(object):
             image = image_tensors.to(self.device, non_blocking=True)
             labels_index, labels_length = self.converter.encode(labels, batch_max_length=self.opt.batch_max_length)
             t0 = time.time()
-            r = self.infer_batch(image, val_choose, labels_index, labels_length)
+            r = self.infer_batch(image, val_choose, labels_index, labels_length, **dec)
             preds_str = self.converter.decode_compact(r["ids"], r["lens"])       # the batch's single D2H sync
             infer_time += time.time() - t0
             valid_loss_avg.add(r["loss"])

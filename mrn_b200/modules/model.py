@@ -387,5 +387,5 @@ class MRNNet(nn.Module):
             if sparse:
                 logits = ops.svtr_heads(self._cache.pack, image.shape[0], index)
         r = ops.gate_combine(logits, g, targets, lengths, want_logits=want_logits, want_E=want_E, want_decode=want_decode)
-        r.update(index=idx_out, gate=gate, scores=scores, features=feats, expert_logits=logits)
+        r.update(index=idx_out, gate=gate, scores=scores, features=feats, expert_logits=logits, combine_gate=g)
         return r

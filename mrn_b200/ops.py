@@ -909,6 +909,45 @@ def greedy_decode(amax, maxprob):
     return ids, lens, conf
 
 
+def ctc_topk(logits: Sequence[torch.Tensor], gate: torch.Tensor, lse: torch.Tensor, K: int, out=None):
+    """Per-frame CTC candidates for the beam search: the K best non-blank classes of the combined logits (same expert
+    table and gate as gate_combine, lse from it).  Returns (top_ids [B,T,K] int32, top_lp [B,T,K], blank_lp [B,T]);
+    `out` may supply those three tensors."""
+    _chk_f32(gate, lse)
+    B, T, _ = logits[0].shape
+    dev = gate.device
+    ptrs, lds, cs = _expert_tables(logits)
+    if tuple(gate.shape) != (B, len(logits)) or tuple(lse.shape) != (B, T):
+        raise RuntimeError("ctc_topk: gate must be [B,I] and lse [B,T]")
+    o = out or (None, None, None)
+    top_ids = _out(o[0], (B, T, K), dev, torch.int32)
+    top_lp = _out(o[1], (B, T, K), dev, torch.float32)
+    blank_lp = _out(o[2], (B, T), dev, torch.float32)
+    L.check(L.load().mrnb_ctc_topk(ptrs, lds, cs, len(logits), _p(gate), _p(lse), B, T, K, _p(top_ids), _p(top_lp),
+                                   _p(blank_lp), _stream()), "ctc_topk")
+    return top_ids, top_lp, blank_lp
+
+
+def ctc_beam_search(top_ids: torch.Tensor, top_lp: torch.Tensor, blank_lp: torch.Tensor, W: int, n_best: int = 1,
+                    out=None):
+    """CTC prefix beam search of width W over the ctc_topk candidates.  Returns (ids [B,n_best,T] int32 compact and
+    -1 padded, lens [B,n_best] int32, scores [B,n_best] = log p of each labeling), best first; `out` may supply them."""
+    _chk_f32(top_lp, blank_lp)
+    if top_ids.dtype != torch.int32 or not top_ids.is_contiguous():
+        raise RuntimeError("ctc_beam_search: top_ids must be a contiguous int32 tensor")
+    B, T, K = top_ids.shape
+    if tuple(top_lp.shape) != (B, T, K) or tuple(blank_lp.shape) != (B, T):
+        raise RuntimeError("ctc_beam_search: top_lp must be [B,T,K] and blank_lp [B,T]")
+    dev = top_ids.device
+    o = out or (None, None, None)
+    ids = _out(o[0], (B, n_best, T), dev, torch.int32)
+    lens = _out(o[1], (B, n_best), dev, torch.int32)
+    scores = _out(o[2], (B, n_best), dev, torch.float32)
+    L.check(L.load().mrnb_ctc_beam_search(_p(top_ids), _p(top_lp), _p(blank_lp), B, T, K, int(W), int(n_best), _p(ids),
+                                          _p(lens), _p(scores), _stream()), "ctc_beam_search")
+    return ids, lens, scores
+
+
 # ------------------------------------------------------------------------------------------------ optimiser
 def clip_adam(params, grads, exp_avg, exp_avg_sq, lr, step, max_norm=5.0, betas=(0.9, 0.999), eps=1e-8, scratch=None,
               norm_out=None):
