@@ -166,25 +166,6 @@ __global__ void pool_kernel(const AT* __restrict__ in, AT* __restrict__ out, int
   store8<AT>(out + (size_t)i * 8, m);
 }
 
-// fp32 mode: im2col of an NHWC activation, col[(n, oh, owp), (kh, kw, c)], stride 1, OWp >= OW columns (extra = pad)
-__global__ void im2col_nhwc_kernel(const float* __restrict__ x, float* __restrict__ col, int H, int W, int C, int KH, int KW,
-                                   int pad, int OH, int OWp, long total4) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const int c = (int)(i % c4) * 4;
-  long r = i / c4;
-  const int kw = (int)(r % KW); r /= KW;
-  const int kh = (int)(r % KH); r /= KH;
-  const int ow = (int)(r % OWp); r /= OWp;
-  const int oh = (int)(r % OH);
-  const long n = r / OH;
-  const int ih = oh - pad + kh, iw = ow - pad + kw;
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (ih >= 0 && ih < H && iw >= 0 && iw < W) v = *reinterpret_cast<const float4*>(x + ((n * H + ih) * W + iw) * C + c);
-  *reinterpret_cast<float4*>(col + i * 4) = v;
-}
-
 // per-channel sum / sum of squares over the rows of x [I][rows][512] (BatchNorm2d batch statistics), fp64 atomics
 template <typename AT>
 __global__ void __launch_bounds__(256)
@@ -327,8 +308,8 @@ int conv_layer(const ConvSpec& c, int I, int B, const AT* in, const float* W32, 
   } else {
     for (int e = 0; e < I; ++e) {
       const long total4 = rows * K / 4;
-      im2col_nhwc_kernel<<<cdiv(total4, 256), 256, 0, st>>>(reinterpret_cast<const float*>(in) + (long)e * B * c.H * c.W * c.Cin,
-                                                            col, c.H, c.W, c.Cin, c.KS, c.KS, c.pad, c.OH, c.OWp, total4);
+      im2col_nhwc_kernel<float><<<cdiv(total4, 256), 256, 0, st>>>(reinterpret_cast<const float*>(in) + (long)e * B * c.H * c.W * c.Cin,
+                                                                   col, c.H, c.W, c.Cin, c.KS, c.KS, c.pad, 1, 1, c.OH, c.OWp, total4);
       MRNB_CHECK_LAUNCH("im2col_nhwc_kernel");
       LinearArgs a{};
       a.A = col; a.lda = K; a.W32 = W32 + (long)e * c.Cout * K; a.bias = bias ? bias + (long)e * c.Cout : nullptr;
@@ -438,7 +419,7 @@ int crnn_forward_t(const MrnbCrnnPack& P, const float* image, int B, int bn_batc
         MRNB_CHECK_LAUNCH("bn_stats512_kernel");
       }
       bn_finalize_kernel<<<cdiv(I * 512, 128), 128, 0, st>>>(stats, P.p[bnw], P.p[bnw + 1], (float*)P.p[bnw + 2],
-                                                             (float*)P.p[bnw + 3], ss, I, 512, (double)rows4, bn_batch_stats,
+                                                             (float*)P.p[bnw + 3], ss, nullptr, I, 512, (double)rows4, bn_batch_stats,
                                                              update_running, 1e-5f);
       MRNB_CHECK_LAUNCH("bn_finalize_kernel");
       // layer 0: 12-13 -> X [4,64,512]; layer 1: 15-17 (+ MaxPool (2,1)) -> Y [2,64,512]

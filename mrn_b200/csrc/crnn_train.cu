@@ -32,76 +32,6 @@ __global__ void nchw_to_nhwc4_kernel(const float* __restrict__ img, float* __res
   *reinterpret_cast<float4*>(out + i * 4) = make_float4(s[0], s[HW], s[2L * HW], s[3L * HW]);
 }
 
-// stride-1 convolution: col[(b,oh,ow), (kh,kw,c)] from NHWC x, zero padding `pad`
-template <typename OT>
-__global__ void im2col_s1_kernel(const float* __restrict__ x, OT* __restrict__ col, int H, int W, int C, int KH, int KW, int pad,
-                                 int Ho, int Wo, long total4) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const int c = (int)(i % c4) * 4;
-  long r = i / c4;
-  const int tap = (int)(r % (KH * KW)); r /= (KH * KW);
-  const int ow = (int)(r % Wo); r /= Wo;
-  const int oh = (int)(r % Ho);
-  const long b = r / Ho;
-  const int ih = oh - pad + tap / KW, iw = ow - pad + tap % KW;
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (ih >= 0 && ih < H && iw >= 0 && iw < W) v = *reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
-  if constexpr (sizeof(OT) == 4) {
-    *reinterpret_cast<float4*>(col + i * 4) = v;
-  } else {                                        // four bf16 values = one 8-byte store
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
-    *reinterpret_cast<uint2*>(col + i * 4) = make_uint2(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1));
-  }
-}
-
-// bf16 im2col for the GEMM convolutions, eight channels per thread (two 16-byte loads, one 16-byte store); the channel
-// count and the tap count are template parameters so that only the (row -> b, oh, ow) split divides by runtime values.
-template <int C, int KH, int KW>
-__global__ void __launch_bounds__(256)
-im2col_s1_bf16_kernel(const float* __restrict__ x, bf16* __restrict__ col, int H, int W, int pad, int Ho, int Wo, long pairs) {
-  constexpr int G = C / 8, KK = KH * KW;
-  const long pair = (long)blockIdx.x * (256 / G) + threadIdx.x / G;      // (output pixel, tap)
-  if (pair >= pairs) return;
-  const int c = (threadIdx.x % G) * 8;
-  const int tap = (int)(pair % KK);
-  long r = pair / KK;
-  const int ow = (int)(r % Wo); r /= Wo;
-  const int oh = (int)(r % Ho);
-  const long b = r / Ho;
-  const int ih = oh - pad + tap / KW, iw = ow - pad + tap % KW;
-  uint4 o = make_uint4(0u, 0u, 0u, 0u);
-  if (ih >= 0 && ih < H && iw >= 0 && iw < W) {
-    const float4* src = reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
-    const float4 v0 = src[0], v1 = src[1];
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v0.x, v0.y), h1 = __floats2bfloat162_rn(v0.z, v0.w);
-    __nv_bfloat162 h2 = __floats2bfloat162_rn(v1.x, v1.y), h3 = __floats2bfloat162_rn(v1.z, v1.w);
-    o = make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1), *reinterpret_cast<uint32_t*>(&h2),
-                   *reinterpret_cast<uint32_t*>(&h3));
-  }
-  *reinterpret_cast<uint4*>(col + pair * C + c) = o;
-}
-
-template <typename AT>
-int launch_im2col(const float* x, AT* col, int H, int W, int C, int KH, int KW, int pad, int Ho, int Wo, long rows, cudaStream_t st) {
-  if constexpr (sizeof(AT) == 2) {
-    const long pairs = rows * KH * KW;
-#define IM2COL_CASE(C_, KH_, KW_)                                                                                        \
-    if (C == C_ && KH == KH_ && KW == KW_) {                                                                             \
-      im2col_s1_bf16_kernel<C_, KH_, KW_><<<cdiv(pairs, 256 / (C_ / 8)), 256, 0, st>>>(x, col, H, W, pad, Ho, Wo, pairs); \
-      MRNB_CHECK_LAUNCH("im2col_s1_bf16_kernel");                                                                         \
-      return MRNB_OK;                                                                                                    \
-    }
-    IM2COL_CASE(64, 3, 3) IM2COL_CASE(128, 3, 3) IM2COL_CASE(256, 3, 3) IM2COL_CASE(512, 3, 3) IM2COL_CASE(512, 2, 2)
-#undef IM2COL_CASE
-  }
-  const long c4 = rows * KH * KW * C / 4;
-  im2col_s1_kernel<AT><<<cdiv(c4, 256), 256, 0, st>>>(x, col, H, W, C, KH, KW, pad, Ho, Wo, c4);
-  MRNB_CHECK_LAUNCH("im2col_s1_kernel");
-  return MRNB_OK;
-}
-
 // conv0 on the tensor cores (bf16 mode): 3x3 pad-1 im2col of the 4-channel NHWC image with the 36 taps zero-padded to
 // K = 64 (one 128-byte swizzle row): col[(b,oh,ow), (kh,kw,c) | 0...].  Thread = (output pixel, group of 8 columns).
 __global__ void im2col_c4_pad64_kernel(const float* __restrict__ x, bf16* __restrict__ col, int H, int W, long rows) {
@@ -132,44 +62,6 @@ __global__ void im2col_c4_pad64_kernel(const float* __restrict__ x, bf16* __rest
   }
   *reinterpret_cast<uint4*>(col + i * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
 }
-// [64, 36] fp32 -> [64, 64] bf16 (zero padded);  and back: [64, 64] fp32 gradient -> its first 36 columns
-__global__ void pad_w0_kernel(const float* __restrict__ w, bf16* __restrict__ wp) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 64 * 64) return;
-  const int o = i >> 6, k = i & 63;
-  wp[i] = __float2bfloat16_rn(k < 36 ? w[o * 36 + k] : 0.f);
-}
-__global__ void unpad_dw0_kernel(const float* __restrict__ dwp, float* __restrict__ dw) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 64 * 36) return;
-  dw[i] = dwp[(i / 36) * 64 + i % 36];
-}
-
-// transpose: dx[b,ih,iw,c] = sum over taps of dcol[(b, ih + pad - kh, iw + pad - kw), (kh,kw,c)]
-__global__ void col2im_s1_kernel(const float* __restrict__ dcol, float* __restrict__ dx, int H, int W, int C, int KH, int KW,
-                                 int pad, int Ho, int Wo, long total4) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const int c = (int)(i % c4) * 4;
-  long r = i / c4;
-  const int iw = (int)(r % W); r /= W;
-  const int ih = (int)(r % H);
-  const long b = r / H;
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int kh = 0; kh < KH; ++kh) {
-    const int oh = ih + pad - kh;
-    if (oh < 0 || oh >= Ho) continue;
-    for (int kw = 0; kw < KW; ++kw) {
-      const int ow = iw + pad - kw;
-      if (ow < 0 || ow >= Wo) continue;
-      const float4 v = *reinterpret_cast<const float4*>(dcol + (((b * Ho + oh) * Wo + ow) * (KH * KW) + kh * KW + kw) * C + c);
-      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-    }
-  }
-  *reinterpret_cast<float4*>(dx + i * 4) = acc;
-}
-
 __global__ void relu_kernel(float* __restrict__ x, long n4) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n4) return;
@@ -266,34 +158,10 @@ bn_relu_bwd_reduce_kernel(const float* __restrict__ raw, const float* __restrict
     atomicAdd(sums + c * 2, a); atomicAdd(sums + c * 2 + 1, b);
   }
 }
-__global__ void bn_relu_bwd_apply_kernel(const float* __restrict__ raw, float* __restrict__ d, bf16* __restrict__ d16,
-                                         const float* __restrict__ ss, const float* __restrict__ mr,
-                                         const double* __restrict__ sums, double count, int use_batch,
-                                         float* __restrict__ dgamma, float* __restrict__ dbeta, int C, long total) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < C) { dgamma[i] = (float)sums[i * 2 + 1]; dbeta[i] = (float)sums[i * 2]; }
-  if (i >= total) return;
-  const int c = (int)(i % C);
-  float dz = d[i];
-  if (use_batch) {
-    const float xh = (raw[i] - mr[c * 2]) * mr[c * 2 + 1];
-    dz = dz - (float)(sums[c * 2] / count) - xh * (float)(sums[c * 2 + 1] / count);
-  }
-  const float v = ss[c * 2] * dz;
-  d[i] = v;
-  if (d16) d16[i] = __float2bfloat16_rn(v);
-}
-
 __global__ void add_vec_kernel(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ o, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) o[i] = a[i] + b[i];
 }
-template <typename OT>
-__global__ void cast_to_kernel(const float* __restrict__ x, OT* __restrict__ y, long n) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) y[i] = from_f32<OT>(x[i]);
-}
-
 // ------------------------------------------------------------------------------------------------
 // LSTM cell, both directions per launch.  gates G [B,63,2048] hold the pre-activations on entry and the activated
 // gates (sigmoid i, f, o; tanh g) on exit; c, rec [B,63,512].  Direction 0 walks t = s, direction 1 walks t = 62 - s.
@@ -448,13 +316,12 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
     const ConvL& L = LAYERS[l];
     const int Ho = out_h(L), Wo = out_w(L), K = L.KH * L.KW * L.Cin;
     const int rows = B * Ho * Wo;
-    const long c4 = (long)rows * K / 4;
     const long n = (long)rows * L.Cout;
     float* dst = L.bn >= 0 ? w.raw[L.bn] : w.act[l];
     if (l == 0 && TC) {    // K = 36 zero-padded to 64: one swizzled k-block on the tensor cores
       im2col_c4_pad64_kernel<<<cdiv((long)rows * 8, 256), 256, 0, st>>>(in, reinterpret_cast<bf16*>(w.col), L.H, L.W, rows);
       MRNB_CHECK_LAUNCH("im2col_c4_pad64_kernel");
-      pad_w0_kernel<<<16, 256, 0, st>>>(P.p[L.w_slot], w.w0pad16);
+      pad_w0_kernel<<<16, 256, 0, st>>>(P.p[L.w_slot], w.w0pad16, 64);
       MRNB_CHECK_LAUNCH("pad_w0_kernel");
       LinearArgs a{};
       a.A = w.col; a.lda = 64; a.a_gstride = (long)rows * 64;
@@ -465,13 +332,12 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
       MRNB_TRY(linear<AT>(a, st));
     } else if (l == 0) {   // fp32 mode: CUDA cores
       float* colf = reinterpret_cast<float*>(w.dcol);
-      im2col_s1_kernel<float><<<cdiv(c4, 256), 256, 0, st>>>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, Ho, Wo, c4);
-      MRNB_CHECK_LAUNCH("im2col_s1_kernel");
+      MRNB_TRY(launch_im2col<float>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
       MrnbGemm g = mrnb_gemm_nt(colf, K, P.p[L.w_slot], K, dst, L.Cout, rows, L.Cout, K);
       g.bias_n = P.p[L.b_slot]; g.act = 2;
       MRNB_TRY(mrnb_sgemm(g, st));
     } else {
-      MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, Ho, Wo, rows, st));
+      MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
       MRNB_TRY(lin<AT>(w.col, K, P.p[L.w_slot], P.h[L.w_slot], L.b_slot >= 0 ? P.p[L.b_slot] : nullptr, dst, L.Cout, true, rows,
                        L.Cout, K, nullptr, nullptr, 1, st));
       if (L.bn < 0) {
@@ -483,9 +349,9 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
       const int q = L.bn;
       const int sw = q == 0 ? MRNB_T_BN4_W : MRNB_T_BN5_W;
       if (bn_batch) MRNB_TRY(launch_colstats(dst, rows, 512, w.stats + q * 1024, st));
-      bn_finalize_train_kernel<<<2, 256, 0, st>>>(w.stats + q * 1024, P.p[sw], P.p[sw + 1], P.bn_mean[q], P.bn_var[q],
-                                                  w.ss + q * 1024, w.mr + q * 1024, 512, (double)rows, bn_batch, update_running, 1e-5f);
-      MRNB_CHECK_LAUNCH("bn_finalize_train_kernel");
+      bn_finalize_kernel<<<2, 256, 0, st>>>(w.stats + q * 1024, P.p[sw], P.p[sw + 1], P.bn_mean[q], P.bn_var[q], w.ss + q * 1024,
+                                            w.mr + q * 1024, 1, 512, (double)rows, bn_batch != 0, update_running != 0, 1e-5f);
+      MRNB_CHECK_LAUNCH("bn_finalize_kernel");
       bn_relu_kernel<<<cdiv(n, 256), 256, 0, st>>>(dst, w.ss + q * 1024, w.act[l], 512, n);
       MRNB_CHECK_LAUNCH("bn_relu_kernel");
     }
@@ -500,8 +366,8 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
   const int M = B * T63;
   const AT* x = nullptr;
   if (TC) {
-    cast_to_kernel<AT><<<cdiv((long)M * 512, 256), 256, 0, st>>>(w.act[6], w.vis16, (long)M * 512);
-    MRNB_CHECK_LAUNCH("cast_to_kernel");
+    cast_kernel<AT><<<cdiv((long)M * 512, 256), 256, 0, st>>>(w.act[6], w.vis16, (long)M * 512);
+    MRNB_CHECK_LAUNCH("cast_kernel");
     x = w.vis16;
   } else {
     x = reinterpret_cast<const AT*>(w.act[6]);
@@ -548,8 +414,8 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
     }
     const AT* r = nullptr;
     if (TC) {
-      cast_to_kernel<AT><<<cdiv((long)M * 512, 256), 256, 0, st>>>(w.rec[k], w.rec16[k], (long)M * 512);
-      MRNB_CHECK_LAUNCH("cast_to_kernel");
+      cast_kernel<AT><<<cdiv((long)M * 512, 256), 256, 0, st>>>(w.rec[k], w.rec16[k], (long)M * 512);
+      MRNB_CHECK_LAUNCH("cast_kernel");
       r = w.rec16[k];
     } else {
       r = reinterpret_cast<const AT*>(w.rec[k]);
@@ -658,8 +524,8 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
       MRNB_CHECK_LAUNCH("maxpool_relu_bwd_kernel");
       float* t = d; d = other; other = t;
       if (d16 && L.bn < 0) {
-        cast_to_kernel<bf16><<<cdiv(n, 256), 256, 0, st>>>(d, d16, n);
-        MRNB_CHECK_LAUNCH("cast_to_kernel");
+        cast_kernel<bf16><<<cdiv(n, 256), 256, 0, st>>>(d, d16, n);
+        MRNB_CHECK_LAUNCH("cast_kernel");
       }
     } else {
       relu_bwd_kernel<<<cdiv(n, 256), 256, 0, st>>>(w.act[l], d, L.bn < 0 ? d16 : nullptr, n);
@@ -671,37 +537,37 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
       int chunks = rows / 256; if (chunks < 1) chunks = 1; if (chunks > 64) chunks = 64;
       bn_relu_bwd_reduce_kernel<<<dim3(16, chunks), dim3(32, 8), 0, st>>>(w.raw[q], d, w.mr + q * 1024, rows, 512, w.bsums + q * 1024);
       MRNB_CHECK_LAUNCH("bn_relu_bwd_reduce_kernel");
-      bn_relu_bwd_apply_kernel<<<cdiv(n, 256), 256, 0, st>>>(w.raw[q], d, d16, w.ss + q * 1024, w.mr + q * 1024, w.bsums + q * 1024,
-                                                             (double)rows, bn_batch, gpt(G, sw), gpt(G, sw + 1), 512, n);
-      MRNB_CHECK_LAUNCH("bn_relu_bwd_apply_kernel");
+      bn_bwd_apply_kernel<<<cdiv(n, 256), 256, 0, st>>>(w.raw[q], d, w.ss + q * 1024, w.mr + q * 1024, w.bsums + q * 1024, (double)rows,
+                                                        bn_batch, gpt(G, sw), gpt(G, sw + 1), 512, n, d16);
+      MRNB_CHECK_LAUNCH("bn_bwd_apply_kernel");
     }
     // conv backward
     if (L.b_slot >= 0) MRNB_TRY(launch_colsum<float>(d, L.Cout, rows, L.Cout, gpt(G, L.b_slot), st));
     const float* in = l == 0 ? w.img4 : w.pool[l - 1];
-    const long c4 = (long)rows * K / 4;
     if (l == 0 && TC) {
       im2col_c4_pad64_kernel<<<cdiv((long)rows * 8, 256), 256, 0, st>>>(in, reinterpret_cast<bf16*>(w.col), L.H, L.W, rows);
       MRNB_CHECK_LAUNCH("im2col_c4_pad64_kernel");
       cudaMemsetAsync(w.dw0pad, 0, 64 * 64 * sizeof(float), st);
       MRNB_TRY(gemm_dw_tc(d16, 64, reinterpret_cast<const bf16*>(w.col), 64, w.dw0pad, rows, 64, 64, st));
-      unpad_dw0_kernel<<<9, 256, 0, st>>>(w.dw0pad, gpt(G, L.w_slot));
+      unpad_dw0_kernel<<<9, 256, 0, st>>>(w.dw0pad, gpt(G, L.w_slot), 64);
       MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
       break;
     }
     if (l == 0) {
       float* colf = w.dcol;
-      im2col_s1_kernel<float><<<cdiv(c4, 256), 256, 0, st>>>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, Ho, Wo, c4);
-      MRNB_CHECK_LAUNCH("im2col_s1_kernel");
+      MRNB_TRY(launch_im2col<float>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
       MRNB_TRY(gemm_dw_f32(d, L.Cout, colf, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
       break;                                   // no gradient w.r.t. the image
     }
     Grad gd{d, d16, L.Cout};
-    MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, Ho, Wo, rows, st));
+    MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
     MRNB_TRY(gemm_dw<AT>(gd, w.col, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
     MRNB_TRY(gemm_dx<AT>(gd, P.p[L.w_slot], P.h[L.w_slot], w.dcol, nullptr, K, rows, L.Cout, K, st));
     const long in4 = (long)B * L.H * L.W * L.Cin / 4;
-    col2im_s1_kernel<<<cdiv(in4, 256), 256, 0, st>>>(w.dcol, other, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, Ho, Wo, in4);
-    MRNB_CHECK_LAUNCH("col2im_s1_kernel");
+    // LAYERS has 3 x 3 windows and the 2 x 2 of conv6
+    const auto col2im = L.KH == 2 ? col2im_nhwc_kernel<2, 2> : col2im_nhwc_kernel<3, 3>;
+    col2im<<<cdiv(in4, 256), 256, 0, st>>>(w.dcol, other, L.H, L.W, L.Cin, L.pad, 1, 1, Ho, Wo, in4);
+    MRNB_CHECK_LAUNCH("col2im_nhwc_kernel");
     float* t = d; d = other; other = t;
   }
   return MRNB_OK;

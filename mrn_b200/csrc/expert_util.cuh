@@ -1,5 +1,6 @@
-// Helpers shared by the expert recognisers (svtr.cu, crnn.cu): grouped Linear dispatch (CUDA-core fp32 engine or
-// tcgen05 bf16 engine), workspace carving, BatchNorm finalisation.  Everything here has internal linkage.
+// Helpers shared by the expert recognisers (svtr.cu, crnn.cu) and, through train_util.cuh, their training paths: grouped
+// Linear dispatch (CUDA-core fp32 engine or tcgen05 bf16 engine), workspace carving, the NHWC im2col, BatchNorm
+// finalisation and the fp32 -> AT cast.  Everything here has internal linkage.
 #pragma once
 #include "common.cuh"
 #include "gemm_f32.h"
@@ -61,13 +62,41 @@ struct Workspace {
   }
 };
 
+// im2col of a KH x KW convolution with zero padding `pad` and stride (sh, sw) over NHWC x[B,H,W,C]:
+// col[(b,oh,ow), (kh,kw,c)] with ih = oh*sh - pad + kh, iw = ow*sw - pad + kw, zero outside the image.  Four channels
+// per thread (C % 4 == 0).  Output columns ow >= the true output width (a padded frame axis) are filled by the same rule.
+template <typename OT>
+__global__ void im2col_nhwc_kernel(const float* __restrict__ x, OT* __restrict__ col, int H, int W, int C, int KH, int KW,
+                                   int pad, int sh, int sw, int Ho, int Wo, long total4) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total4) return;
+  const int c4 = C / 4;
+  const int c = (int)(i % c4) * 4;
+  long r = i / c4;
+  const int tap = (int)(r % (KH * KW)); r /= (KH * KW);
+  const int ow = (int)(r % Wo); r /= Wo;
+  const int oh = (int)(r % Ho);
+  const long b = r / Ho;
+  const int ih = oh * sh - pad + tap / KW, iw = ow * sw - pad + tap % KW;
+  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (ih >= 0 && ih < H && iw >= 0 && iw < W) v = *reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
+  if constexpr (sizeof(OT) == 4) {
+    *reinterpret_cast<float4*>(col + i * 4) = v;
+  } else {                                        // four bf16 values = one 8-byte store
+    __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
+    *reinterpret_cast<uint2*>(col + i * 4) = make_uint2(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1));
+  }
+}
+
 // BN finalize: scale/shift per (expert, channel) from batch statistics (train) or running statistics (eval);
 // in train mode also the running-stat update with momentum 0.1 and the unbiased variance (nn.BatchNorm2d).
-// use_batch_stats / update_running are per-expert bit masks (bit e = expert e).
+// use_batch_stats / update_running are per-expert bit masks (bit e = expert e).  mean_rstd, when not null, receives
+// (mean, 1/sqrt(var + eps)) per (expert, channel) for the BatchNorm backward.
 __global__ void bn_finalize_kernel(const double* __restrict__ stats, const float* __restrict__ gamma,
                                    const float* __restrict__ beta, float* __restrict__ run_mean,
-                                   float* __restrict__ run_var, float* __restrict__ scale_shift /*[I,C,2]*/, int I, int C,
-                                   double count, int use_batch_stats, int update_running, float eps) {
+                                   float* __restrict__ run_var, float* __restrict__ scale_shift /*[I,C,2]*/,
+                                   float* __restrict__ mean_rstd /*[I,C,2] or null*/, int I, int C, double count,
+                                   int use_batch_stats, int update_running, float eps) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= I * C) return;
   float mean, var;
@@ -84,9 +113,11 @@ __global__ void bn_finalize_kernel(const double* __restrict__ stats, const float
   } else {
     mean = run_mean[idx]; var = run_var[idx];
   }
-  const float sc = gamma[idx] * rsqrtf(var + eps);
+  const float rstd = rsqrtf(var + eps);
+  const float sc = gamma[idx] * rstd;
   scale_shift[idx * 2] = sc;
   scale_shift[idx * 2 + 1] = beta[idx] - mean * sc;
+  if (mean_rstd) { mean_rstd[idx * 2] = mean; mean_rstd[idx * 2 + 1] = rstd; }
 }
 
 template <typename AT>

@@ -732,7 +732,7 @@ int svtr_forward_t(const MrnbSvtrPack& P, const float* image, int B, int Bc, int
                                                                       bn_batch_stats ? st0 : nullptr, B);
     MRNB_CHECK_LAUNCH("conv0_kernel");
     bn_finalize_kernel<<<cdiv(I * 32, 128), 128, 0, st>>>(st0, P.p[MRNB_P_BN0_W], P.p[MRNB_P_BN0_B],
-                                                          (float*)P.p[MRNB_P_BN0_MEAN], (float*)P.p[MRNB_P_BN0_VAR], ss0, I,
+                                                          (float*)P.p[MRNB_P_BN0_MEAN], (float*)P.p[MRNB_P_BN0_VAR], ss0, nullptr, I,
                                                           32, (double)B * 16 * 128, bn_batch_stats, update_running, 1e-5f);
     MRNB_CHECK_LAUNCH("bn_finalize_kernel");
     const long total8 = (long)I * B * 16 * 130 * 4;
@@ -760,7 +760,7 @@ int svtr_forward_t(const MrnbSvtrPack& P, const float* image, int B, int Bc, int
                                                          bn_batch_stats ? st0 : nullptr, B);
     MRNB_CHECK_LAUNCH("conv0_kernel");
     bn_finalize_kernel<<<cdiv(I * 32, 128), 128, 0, st>>>(st0, P.p[MRNB_P_BN0_W], P.p[MRNB_P_BN0_B],
-                                                          (float*)P.p[MRNB_P_BN0_MEAN], (float*)P.p[MRNB_P_BN0_VAR], ss0, I,
+                                                          (float*)P.p[MRNB_P_BN0_MEAN], (float*)P.p[MRNB_P_BN0_VAR], ss0, nullptr, I,
                                                           32, (double)B * 16 * 128, bn_batch_stats, update_running, 1e-5f);
     MRNB_CHECK_LAUNCH("bn_finalize_kernel");
     const size_t smem = (12872 + 288 * 64) * sizeof(float);
@@ -771,7 +771,7 @@ int svtr_forward_t(const MrnbSvtrPack& P, const float* image, int B, int Bc, int
     MRNB_CHECK_LAUNCH("conv1_kernel");
   }
   bn_finalize_kernel<<<cdiv(I * 64, 128), 128, 0, st>>>(st1, P.p[MRNB_P_BN1_W], P.p[MRNB_P_BN1_B],
-                                                        (float*)P.p[MRNB_P_BN1_MEAN], (float*)P.p[MRNB_P_BN1_VAR], ss1, I,
+                                                        (float*)P.p[MRNB_P_BN1_MEAN], (float*)P.p[MRNB_P_BN1_VAR], ss1, nullptr, I,
                                                         64, (double)B * 8 * 64, bn_batch_stats, update_running, 1e-5f);
   MRNB_CHECK_LAUNCH("bn_finalize_kernel");
   {

@@ -35,7 +35,7 @@ static const int DIMS[3] = {64, 128, 256}, DEPTH[3] = {3, 6, 3}, HEADS[3] = {2, 
 static const int OUTS[3] = {128, 256, 512};
 
 // ------------------------------------------------------------------------------------------------
-// im2col / col2im
+// conv0 im2col of the NCHW image
 // ------------------------------------------------------------------------------------------------
 // conv0 (4->32, 3x3 s2 p1) on the NCHW image: col[(b,oh,ow), c*9 + kh*3 + kw]  (nn.Conv2d weight order)
 __global__ void im2col_img_kernel(const float* __restrict__ img, float* __restrict__ col, long total) {
@@ -79,122 +79,8 @@ __global__ void im2col_img_pad64_kernel(const float* __restrict__ img, __nv_bflo
   }
   *reinterpret_cast<uint4*>(col + i * 8) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
 }
-// conv0 weight [32, 36] fp32 -> [32, 64] bf16 zero padded; its gradient [32, 64] fp32 -> the first 36 columns
-__global__ void pad_w0_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wp) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 32 * 64) return;
-  const int o = i >> 6, k = i & 63;
-  wp[i] = __float2bfloat16_rn(k < 36 ? w[o * 36 + k] : 0.f);
-}
-__global__ void unpad_dw0_kernel(const float* __restrict__ dwp, float* __restrict__ dw) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 32 * 36) return;
-  dw[i] = dwp[(i / 36) * 64 + i % 36];
-}
-
-// 3x3 pad-1 convolution with stride (sh, sw) over NHWC x[B,H,W,C]: col[(b,oh,ow), (kh,kw,c)]
-template <typename OT>
-__global__ void im2col_nhwc_kernel(const float* __restrict__ x, OT* __restrict__ col, int H, int W, int C, int Ho, int Wo,
-                                   int sh, int sw, long total4) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const int c = (int)(i % c4) * 4;
-  long r = i / c4;
-  const int tap = (int)(r % 9); r /= 9;
-  const int ow = (int)(r % Wo); r /= Wo;
-  const int oh = (int)(r % Ho);
-  const long b = r / Ho;
-  const int ih = oh * sh - 1 + tap / 3, iw = ow * sw - 1 + tap % 3;
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (ih >= 0 && ih < H && iw >= 0 && iw < W) v = *reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
-  if constexpr (sizeof(OT) == 4) {
-    *reinterpret_cast<float4*>(col + i * 4) = v;
-  } else {                                        // four bf16 values = one 8-byte store
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
-    *reinterpret_cast<uint2*>(col + i * 4) = make_uint2(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1));
-  }
-}
-
-// bf16 variant, eight channels per thread (two 16-byte loads, one 16-byte store), channel count as a template parameter
-template <int C>
-__global__ void __launch_bounds__(256)
-im2col_nhwc_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col, int H, int W, int Ho, int Wo, int sh,
-                        int sw, long pairs) {
-  constexpr int G = C / 8;
-  const long pair = (long)blockIdx.x * (256 / G) + threadIdx.x / G;      // (output pixel, tap)
-  if (pair >= pairs) return;
-  const int c = (threadIdx.x % G) * 8;
-  const int tap = (int)(pair % 9);
-  long r = pair / 9;
-  const int ow = (int)(r % Wo); r /= Wo;
-  const int oh = (int)(r % Ho);
-  const long b = r / Ho;
-  const int ih = oh * sh - 1 + tap / 3, iw = ow * sw - 1 + tap % 3;
-  uint4 o = make_uint4(0u, 0u, 0u, 0u);
-  if (ih >= 0 && ih < H && iw >= 0 && iw < W) {
-    const float4* src = reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
-    const float4 v0 = src[0], v1 = src[1];
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(v0.x, v0.y), h1 = __floats2bfloat162_rn(v0.z, v0.w);
-    __nv_bfloat162 h2 = __floats2bfloat162_rn(v1.x, v1.y), h3 = __floats2bfloat162_rn(v1.z, v1.w);
-    o = make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1), *reinterpret_cast<uint32_t*>(&h2),
-                   *reinterpret_cast<uint32_t*>(&h3));
-  }
-  *reinterpret_cast<uint4*>(col + pair * C + c) = o;
-}
-
-template <typename AT>
-int launch_im2col_nhwc(const float* x, AT* col, int H, int W, int C, int Ho, int Wo, int sh, int sw, long rows, cudaStream_t st) {
-  if constexpr (sizeof(AT) == 2) {
-    const long pairs = rows * 9;
-#define IM2COL_CASE(C_)                                                                                             \
-    if (C == C_) {                                                                                                  \
-      im2col_nhwc_bf16_kernel<C_><<<cdiv(pairs, 256 / (C_ / 8)), 256, 0, st>>>(x, col, H, W, Ho, Wo, sh, sw, pairs); \
-      MRNB_CHECK_LAUNCH("im2col_nhwc_bf16_kernel");                                                                  \
-      return MRNB_OK;                                                                                               \
-    }
-    IM2COL_CASE(32) IM2COL_CASE(64) IM2COL_CASE(128) IM2COL_CASE(256)
-#undef IM2COL_CASE
-  }
-  const long c4 = rows * 9 * C / 4;
-  im2col_nhwc_kernel<AT><<<cdiv(c4, 256), 256, 0, st>>>(x, col, H, W, C, Ho, Wo, sh, sw, c4);
-  MRNB_CHECK_LAUNCH("im2col_nhwc_kernel");
-  return MRNB_OK;
-}
-
-// transpose of the above: dx[b,ih,iw,c] = sum over the (oh,ow,tap) that read this pixel of dcol
-__global__ void col2im_nhwc_kernel(const float* __restrict__ dcol, float* __restrict__ dx, int H, int W, int C, int Ho,
-                                   int Wo, int sh, int sw, long total4) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total4) return;
-  const int c4 = C / 4;
-  const int c = (int)(i % c4) * 4;
-  long r = i / c4;
-  const int iw = (int)(r % W); r /= W;
-  const int ih = (int)(r % H);
-  const long b = r / H;
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-  for (int kh = 0; kh < 3; ++kh) {
-    const int th = ih + 1 - kh;
-    if (th < 0 || th % sh != 0) continue;
-    const int oh = th / sh;
-    if (oh >= Ho) continue;
-#pragma unroll
-    for (int kw = 0; kw < 3; ++kw) {
-      const int tw = iw + 1 - kw;
-      if (tw < 0 || tw % sw != 0) continue;
-      const int ow = tw / sw;
-      if (ow >= Wo) continue;
-      const float4 v = *reinterpret_cast<const float4*>(dcol + (((b * Ho + oh) * Wo + ow) * 9 + kh * 3 + kw) * C + c);
-      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-    }
-  }
-  *reinterpret_cast<float4*>(dx + i * 4) = acc;
-}
-
 // ------------------------------------------------------------------------------------------------
-// BatchNorm (train): finalize keeps (scale, shift) and (mean, rstd); GELU applied on top.
+// BatchNorm (train) with GELU on top (finalize: expert_util.cuh, backward apply pass: train_util.cuh)
 // ------------------------------------------------------------------------------------------------
 // act = GELU(raw * sc + sh) (+ pos[(row % pos_rows), c])      [rows, C] fp32, C % 4 == 0
 __global__ void bn_gelu_kernel(const float* __restrict__ raw, const float* __restrict__ ss, const float* __restrict__ pos,
@@ -240,26 +126,6 @@ bn_bwd_reduce_kernel(const float* __restrict__ raw, float* __restrict__ d, const
     for (int k = 0; k < 8; ++k) { a += sh[k][threadIdx.x][0]; b += sh[k][threadIdx.x][1]; }
     atomicAdd(sums + c * 2, a); atomicAdd(sums + c * 2 + 1, b);
   }
-}
-
-// draw = gamma*rstd * (dz - S1/n - xhat * S2/n)   (batch statistics)   or   gamma*rstd * dz   (running statistics);
-// dgamma = S2, dbeta = S1
-__global__ void bn_bwd_apply_kernel(const float* __restrict__ raw, float* __restrict__ d, const float* __restrict__ ss,
-                                    const float* __restrict__ mr, const double* __restrict__ sums, double count,
-                                    int use_batch, float* __restrict__ dgamma, float* __restrict__ dbeta, int C, long total,
-                                    __nv_bfloat16* __restrict__ d16 = nullptr) {
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < C) { dgamma[i] = (float)sums[i * 2 + 1]; dbeta[i] = (float)sums[i * 2]; }
-  if (i >= total) return;
-  const int c = (int)(i % C);
-  const float sc = ss[c * 2];
-  float dz = d[i];
-  if (use_batch) {
-    const float xh = (raw[i] - mr[c * 2]) * mr[c * 2 + 1];
-    dz = dz - (float)(sums[c * 2] / count) - xh * (float)(sums[c * 2 + 1] / count);
-  }
-  d[i] = sc * dz;
-  if (d16) d16[i] = __float2bfloat16_rn(sc * dz);
 }
 
 // dpos[n,c] = sum_b dx[b,n,c]
@@ -844,7 +710,7 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
       const long rows0 = (long)B * 2048;
       im2col_img_pad64_kernel<<<cdiv(rows0 * 8, 256), 256, 0, st>>>(image, w.big, rows0);
       MRNB_CHECK_LAUNCH("im2col_img_pad64_kernel");
-      pad_w0_kernel<<<8, 256, 0, st>>>(P.p[MRNB_P_CONV0_W], w.w0pad16);
+      pad_w0_kernel<<<8, 256, 0, st>>>(P.p[MRNB_P_CONV0_W], w.w0pad16, 32);
       MRNB_CHECK_LAUNCH("pad_w0_kernel");
       MrnbTcGemm2 g0{};
       g0.a = mrnb_operand_k2d(w.big, rows0, 64, 64, 128, 1);
@@ -861,18 +727,17 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
       MRNB_TRY(mrnb_sgemm(g, st));
     }
     if (bn_batch) MRNB_TRY(launch_colstats(w.raw0, (long)B * 2048, 32, w.stats, st));
-    bn_finalize_train_kernel<<<1, 64, 0, st>>>(w.stats, P.p[MRNB_P_BN0_W], P.p[MRNB_P_BN0_B], (float*)P.p[MRNB_P_BN0_MEAN],
-                                               (float*)P.p[MRNB_P_BN0_VAR], w.ss, w.mr, 32, (double)B * 2048, bn_batch,
-                                               update_running, 1e-5f);
-    MRNB_CHECK_LAUNCH("bn_finalize_train_kernel");
+    bn_finalize_kernel<<<1, 64, 0, st>>>(w.stats, P.p[MRNB_P_BN0_W], P.p[MRNB_P_BN0_B], (float*)P.p[MRNB_P_BN0_MEAN],
+                                         (float*)P.p[MRNB_P_BN0_VAR], w.ss, w.mr, 1, 32, (double)B * 2048, bn_batch != 0,
+                                         update_running != 0, 1e-5f);
+    MRNB_CHECK_LAUNCH("bn_finalize_kernel");
     const long t4 = (long)B * 2048 * 32 / 4;
     bn_gelu_kernel<<<cdiv(t4, 256), 256, 0, st>>>(w.raw0, w.ss, nullptr, 1, w.act0, 32, t4);
     MRNB_CHECK_LAUNCH("bn_gelu_kernel");
-    const long c4 = (long)B * 512 * 288 / 4;
     if constexpr (sizeof(AT) == 2) {
       // conv1 (K = 288) on the tensor cores: bf16 im2col, the contraction rounded up to 320 (TMA zero-fills both operands)
       MRNB_CHECK_ARG(P.h[MRNB_P_CONV1_W], "svtr_train: bf16 mode needs the 16-bit weight shadow");
-      MRNB_TRY(launch_im2col_nhwc<AT>(w.act0, w.big, 16, 128, 32, 8, 64, 2, 2, (long)B * 512, st));
+      MRNB_TRY(launch_im2col<AT>(w.act0, w.big, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, (long)B * 512, st));
       MrnbTcGemm2 g1{};
       g1.a = mrnb_operand_k2d(w.big, (long)B * 512, 288, 288, 128, 1);
       g1.b = mrnb_operand_k2d(P.h[MRNB_P_CONV1_W], 64, 288, 288, 64, 1);
@@ -880,17 +745,16 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
       g1.M = B * 512; g1.N = 64; g1.K = 320; g1.groups = 1; g1.splitk = 1; g1.alpha = 1.f;
       MRNB_TRY(mrnb_tc_gemm2(g1, st));
     } else {
-      im2col_nhwc_kernel<float><<<cdiv(c4, 256), 256, 0, st>>>(w.act0, w.colf, 16, 128, 32, 8, 64, 2, 2, c4);
-      MRNB_CHECK_LAUNCH("im2col_nhwc_kernel");
+      MRNB_TRY(launch_im2col<float>(w.act0, w.colf, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, (long)B * 512, st));
       MrnbGemm g1 = mrnb_gemm_nt(w.colf, 288, P.p[MRNB_P_CONV1_W], 288, w.raw1, 64, B * 512, 64, 288);
       g1.bias_n = P.p[MRNB_P_CONV1_B];
       MRNB_TRY(mrnb_sgemm(g1, st));
     }
     if (bn_batch) MRNB_TRY(launch_colstats(w.raw1, (long)B * 512, 64, w.stats + 64, st));
-    bn_finalize_train_kernel<<<1, 64, 0, st>>>(w.stats + 64, P.p[MRNB_P_BN1_W], P.p[MRNB_P_BN1_B],
-                                               (float*)P.p[MRNB_P_BN1_MEAN], (float*)P.p[MRNB_P_BN1_VAR], w.ss + 64,
-                                               w.mr + 64, 64, (double)B * 512, bn_batch, update_running, 1e-5f);
-    MRNB_CHECK_LAUNCH("bn_finalize_train_kernel");
+    bn_finalize_kernel<<<1, 64, 0, st>>>(w.stats + 64, P.p[MRNB_P_BN1_W], P.p[MRNB_P_BN1_B], (float*)P.p[MRNB_P_BN1_MEAN],
+                                         (float*)P.p[MRNB_P_BN1_VAR], w.ss + 64, w.mr + 64, 1, 64, (double)B * 512,
+                                         bn_batch != 0, update_running != 0, 1e-5f);
+    MRNB_CHECK_LAUNCH("bn_finalize_kernel");
     bn_gelu_kernel<<<cdiv(u / 4, 256), 256, 0, st>>>(w.raw1, w.ss + 64, P.p[MRNB_P_POS_EMBED], 512, w.stage_in[0], 64, u / 4);
     MRNB_CHECK_LAUNCH("bn_gelu_kernel");
     mrnb_prof_end(MRNB_PROF_CONV, st);
@@ -924,8 +788,7 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
     const int Co = OUTS[s], Ho = H / 2;
     const int orows = B * Ho * Wd;
     const int ps = MRNB_P_SUB0 + s * MRNB_PS_COUNT;
-    const long c4 = (long)orows * 9 * d / 4;
-    MRNB_TRY(launch_im2col_nhwc<AT>(w.xout[blk - 1], w.big, H, Wd, d, Ho, Wd, 2, 1, (long)orows, st));
+    MRNB_TRY(launch_im2col<AT>(w.xout[blk - 1], w.big, H, Wd, d, 3, 3, 1, 2, 1, Ho, Wd, (long)orows, st));
     MRNB_TRY(lin<AT>(w.big, 9 * d, P.p[ps + MRNB_PS_CONV_W], P.h[ps + MRNB_PS_CONV_W], P.p[ps + MRNB_PS_CONV_B], w.cv[s], Co,
                      true, orows, Co, 9 * d, nullptr, nullptr, 1, st));
     if (s < 2) MRNB_TRY(launch_ln_fwd<float>(w.cv[s], w.stage_in[s + 1], P.p[ps + MRNB_PS_NORM_W], P.p[ps + MRNB_PS_NORM_B], orows, Co, 1e-5f, st));
@@ -988,11 +851,10 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
     {
       Grad gcv{dcv, w.dy16, Co};
       MRNB_TRY(launch_colsum<float>(dcv, Co, orows, Co, gp(G, ps + MRNB_PS_CONV_B), st));
-      const long c4 = (long)orows * 9 * d / 4;
-      MRNB_TRY(launch_im2col_nhwc<AT>(w.xout[blk - 1], w.big, H, Wd, d, Ho, Wd, 2, 1, (long)orows, st));
+      MRNB_TRY(launch_im2col<AT>(w.xout[blk - 1], w.big, H, Wd, d, 3, 3, 1, 2, 1, Ho, Wd, (long)orows, st));
       MRNB_TRY(gemm_dw<AT>(gcv, w.big, 9 * d, gp(G, ps + MRNB_PS_CONV_W), orows, Co, 9 * d, st));
       MRNB_TRY(gemm_dx<AT>(gcv, P.p[ps + MRNB_PS_CONV_W], P.h[ps + MRNB_PS_CONV_W], w.dbig, nullptr, 9 * d, orows, Co, 9 * d, st));
-      col2im_nhwc_kernel<<<cdiv(u / 4, 256), 256, 0, st>>>(w.dbig, dx, H, Wd, d, Ho, Wd, 2, 1, u / 4);
+      col2im_nhwc_kernel<3, 3><<<cdiv(u / 4, 256), 256, 0, st>>>(w.dbig, dx, H, Wd, d, 1, 2, 1, Ho, Wd, u / 4);
       MRNB_CHECK_LAUNCH("col2im_nhwc_kernel");
     }
     for (int j = DEPTH[s] - 1; j >= 0; --j) {
@@ -1081,20 +943,18 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
                                                       gp(G, MRNB_P_BN1_W), gp(G, MRNB_P_BN1_B), 64, u, TC ? w.dy16 : nullptr);
     MRNB_CHECK_LAUNCH("bn_bwd_apply_kernel");
     MRNB_TRY(launch_colsum<float>(dx, 64, r1, 64, gp(G, MRNB_P_CONV1_B), st));
-    const long c4 = r1 * 288 / 4;
     if constexpr (TC) {
-      MRNB_TRY(launch_im2col_nhwc<AT>(w.act0, w.big, 16, 128, 32, 8, 64, 2, 2, (long)B * 512, st));
+      MRNB_TRY(launch_im2col<AT>(w.act0, w.big, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
       MRNB_TRY(gemm_dw_tc(w.dy16, 64, w.big, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
       MRNB_TRY(gemm_dx_tc(w.dy16, 64, P.h[MRNB_P_CONV1_W], w.dbig, nullptr, 288, (int)r1, 64, 288, st));
     } else {
-      im2col_nhwc_kernel<float><<<cdiv(c4, 256), 256, 0, st>>>(w.act0, w.colf, 16, 128, 32, 8, 64, 2, 2, c4);
-      MRNB_CHECK_LAUNCH("im2col_nhwc_kernel");
+      MRNB_TRY(launch_im2col<float>(w.act0, w.colf, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
       MRNB_TRY(gemm_dw_f32(dx, 64, w.colf, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
       MRNB_TRY(gemm_dx_f32(dx, 64, P.p[MRNB_P_CONV1_W], w.dbig, 288, (int)r1, 64, 288, st));
     }
     float* dact0 = w.dy;                                   // [B,16,128,32]
     const long n0 = (long)B * 2048 * 32;
-    col2im_nhwc_kernel<<<cdiv(n0 / 4, 256), 256, 0, st>>>(w.dbig, dact0, 16, 128, 32, 8, 64, 2, 2, n0 / 4);
+    col2im_nhwc_kernel<3, 3><<<cdiv(n0 / 4, 256), 256, 0, st>>>(w.dbig, dact0, 16, 128, 32, 1, 2, 2, 8, 64, n0 / 4);
     MRNB_CHECK_LAUNCH("col2im_nhwc_kernel");
     const long r0 = (long)B * 2048;
     chunks = (int)(r0 / 256); if (chunks < 1) chunks = 1; if (chunks > 148) chunks = 148;
@@ -1109,7 +969,7 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
       MRNB_CHECK_LAUNCH("im2col_img_pad64_kernel");
       cudaMemsetAsync(w.dw0pad, 0, 32 * 64 * sizeof(float), st);
       MRNB_TRY(gemm_dw_tc(w.dbig16, 32, w.big, 64, w.dw0pad, (int)r0, 32, 64, st));
-      unpad_dw0_kernel<<<5, 256, 0, st>>>(w.dw0pad, gp(G, MRNB_P_CONV0_W));
+      unpad_dw0_kernel<<<5, 256, 0, st>>>(w.dw0pad, gp(G, MRNB_P_CONV0_W), 32);
       MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
     } else {
       const long total = r0 * 36;

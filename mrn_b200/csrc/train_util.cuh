@@ -1,6 +1,7 @@
 // Building blocks shared by the expert-training translation units (svtr_train.cu, crnn_train.cu): column sums (bias
-// gradients, BatchNorm statistics), BatchNorm finalisation, the forward / backward GEMM dispatch (CUDA-core fp32 engine or
-// tcgen05 bf16 engines) and small casts.  Everything has internal linkage.
+// gradients, BatchNorm statistics), the forward / backward GEMM dispatch (CUDA-core fp32 engine or tcgen05 bf16 engines),
+// small casts, the convolution lowering (bf16 im2col, col2im, conv0 weight padding) and the BatchNorm-backward apply
+// pass.  Everything has internal linkage.
 #pragma once
 #include "common.cuh"
 #include "gemm_f32.h"
@@ -93,32 +94,6 @@ int launch_colstats(const float* x, long rows, int C, double* stats, cudaStream_
   colsum_kernel<float, true><<<dim3(cdiv(C, 32), chunks), dim3(32, 8), 0, st>>>(x, C, rows, C, nullptr, stats);
   MRNB_CHECK_LAUNCH("colsum_kernel");
   return MRNB_OK;
-}
-
-// BatchNorm (train): finalize keeps (scale, shift) and (mean, rstd)
-__global__ void bn_finalize_train_kernel(const double* __restrict__ stats, const float* __restrict__ gamma,
-                                         const float* __restrict__ beta, float* __restrict__ run_mean,
-                                         float* __restrict__ run_var, float* __restrict__ ss, float* __restrict__ mr, int C,
-                                         double count, int use_batch, int update_running, float eps) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= C) return;
-  float mean, var;
-  if (use_batch) {
-    const double m = stats[c * 2] / count;
-    double v = stats[c * 2 + 1] / count - m * m;
-    if (v < 0) v = 0;
-    mean = (float)m; var = (float)v;
-    if (update_running) {
-      run_mean[c] = 0.9f * run_mean[c] + 0.1f * mean;
-      run_var[c] = 0.9f * run_var[c] + 0.1f * (float)(v * count / (count - 1.0));
-    }
-  } else {
-    mean = run_mean[c]; var = run_var[c];
-  }
-  const float rstd = rsqrtf(var + eps);
-  const float sc = gamma[c] * rstd;
-  ss[c * 2] = sc; ss[c * 2 + 1] = beta[c] - mean * sc;
-  mr[c * 2] = mean; mr[c * 2 + 1] = rstd;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -235,5 +210,130 @@ __global__ void cast_pad_rows_kernel(const float* __restrict__ x, long ld, int C
     pk[u] = *reinterpret_cast<uint32_t*>(&hh);
   }
   *reinterpret_cast<uint4*>(y + r * ld16 + c) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Convolution lowering.  The forward GEMM reads im2col_nhwc_kernel's layout col[(b,oh,ow), (kh,kw,c)] (expert_util.cuh);
+// col2im is its transpose.
+// ------------------------------------------------------------------------------------------------
+// bf16 im2col, eight channels per thread (two 16-byte loads, one 16-byte store); the channel count and the window are
+// template parameters so that only the (row -> b, oh, ow) split divides by runtime values.
+template <int C, int KH, int KW>
+__global__ void __launch_bounds__(256)
+im2col_nhwc_bf16_kernel(const float* __restrict__ x, bf16* __restrict__ col, int H, int W, int pad, int sh, int sw, int Ho,
+                        int Wo, long pairs) {
+  constexpr int G = C / 8, KK = KH * KW;
+  const long pair = (long)blockIdx.x * (256 / G) + threadIdx.x / G;      // (output pixel, tap)
+  if (pair >= pairs) return;
+  const int c = (threadIdx.x % G) * 8;
+  const int tap = (int)(pair % KK);
+  long r = pair / KK;
+  const int ow = (int)(r % Wo); r /= Wo;
+  const int oh = (int)(r % Ho);
+  const long b = r / Ho;
+  const int ih = oh * sh - pad + tap / KW, iw = ow * sw - pad + tap % KW;
+  uint4 o = make_uint4(0u, 0u, 0u, 0u);
+  if (ih >= 0 && ih < H && iw >= 0 && iw < W) {
+    const float4* src = reinterpret_cast<const float4*>(x + ((b * H + ih) * W + iw) * C + c);
+    const float4 v0 = src[0], v1 = src[1];
+    __nv_bfloat162 h0 = __floats2bfloat162_rn(v0.x, v0.y), h1 = __floats2bfloat162_rn(v0.z, v0.w);
+    __nv_bfloat162 h2 = __floats2bfloat162_rn(v1.x, v1.y), h3 = __floats2bfloat162_rn(v1.z, v1.w);
+    o = make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1), *reinterpret_cast<uint32_t*>(&h2),
+                   *reinterpret_cast<uint32_t*>(&h3));
+  }
+  *reinterpret_cast<uint4*>(col + pair * C + c) = o;
+}
+
+// im2col of `rows` output pixels into the AT GEMM operand.  bf16 mode uses the eight-channel kernel for the channel counts
+// and windows of the SVTR and CRNN convolutions; everything else takes the four-channel kernel.
+template <typename AT>
+int launch_im2col(const float* x, AT* col, int H, int W, int C, int KH, int KW, int pad, int sh, int sw, int Ho, int Wo,
+                  long rows, cudaStream_t st) {
+  if constexpr (sizeof(AT) == 2) {
+    const long pairs = rows * KH * KW;
+#define IM2COL_CASE(C_, KH_, KW_)                                                                                                 \
+    if (C == C_ && KH == KH_ && KW == KW_) {                                                                                      \
+      im2col_nhwc_bf16_kernel<C_, KH_, KW_><<<cdiv(pairs, 256 / (C_ / 8)), 256, 0, st>>>(x, col, H, W, pad, sh, sw, Ho, Wo, pairs); \
+      MRNB_CHECK_LAUNCH("im2col_nhwc_bf16_kernel");                                                                               \
+      return MRNB_OK;                                                                                                             \
+    }
+    IM2COL_CASE(32, 3, 3) IM2COL_CASE(64, 3, 3) IM2COL_CASE(128, 3, 3) IM2COL_CASE(256, 3, 3) IM2COL_CASE(512, 3, 3)
+    IM2COL_CASE(512, 2, 2)
+#undef IM2COL_CASE
+  }
+  const long c4 = rows * KH * KW * C / 4;
+  im2col_nhwc_kernel<AT><<<cdiv(c4, 256), 256, 0, st>>>(x, col, H, W, C, KH, KW, pad, sh, sw, Ho, Wo, c4);
+  MRNB_CHECK_LAUNCH("im2col_nhwc_kernel");
+  return MRNB_OK;
+}
+
+// transpose of the im2col: dx[b,ih,iw,c] = sum of dcol over the (oh, ow, kh, kw) that read this pixel, taps in ascending
+// (kh, kw) order.  Four channels per thread.
+template <int KH, int KW>
+__global__ void col2im_nhwc_kernel(const float* __restrict__ dcol, float* __restrict__ dx, int H, int W, int C, int pad,
+                                   int sh, int sw, int Ho, int Wo, long total4) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total4) return;
+  const int c4 = C / 4;
+  const int c = (int)(i % c4) * 4;
+  long r = i / c4;
+  const int iw = (int)(r % W); r /= W;
+  const int ih = (int)(r % H);
+  const long b = r / H;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+  for (int kh = 0; kh < KH; ++kh) {
+    const int th = ih + pad - kh;
+    if (th < 0 || th % sh != 0) continue;
+    const int oh = th / sh;
+    if (oh >= Ho) continue;
+#pragma unroll
+    for (int kw = 0; kw < KW; ++kw) {
+      const int tw = iw + pad - kw;
+      if (tw < 0 || tw % sw != 0) continue;
+      const int ow = tw / sw;
+      if (ow >= Wo) continue;
+      const float4 v = *reinterpret_cast<const float4*>(dcol + (((b * Ho + oh) * Wo + ow) * (KH * KW) + kh * KW + kw) * C + c);
+      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+  }
+  *reinterpret_cast<float4*>(dx + i * 4) = acc;
+}
+
+// conv0 on the tensor cores: its weight [cout, 36] fp32 -> [cout, 64] bf16, the 36 taps zero padded to one 64-wide
+// k-block; and back, the gradient [cout, 64] fp32 -> its first 36 columns
+__global__ void pad_w0_kernel(const float* __restrict__ w, bf16* __restrict__ wp, int cout) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cout * 64) return;
+  const int o = i >> 6, k = i & 63;
+  wp[i] = __float2bfloat16_rn(k < 36 ? w[o * 36 + k] : 0.f);
+}
+__global__ void unpad_dw0_kernel(const float* __restrict__ dwp, float* __restrict__ dw, int cout) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cout * 36) return;
+  dw[i] = dwp[(i / 36) * 64 + i % 36];
+}
+
+// ------------------------------------------------------------------------------------------------
+// BatchNorm backward, apply pass (after a reduce pass that left S1 = sum dz, S2 = sum dz * xhat per channel in sums):
+// draw = gamma*rstd * (dz - S1/n - xhat * S2/n)   (batch statistics)   or   gamma*rstd * dz   (running statistics),
+// written over d (+ optional 16-bit copy);  dgamma = S2, dbeta = S1
+// ------------------------------------------------------------------------------------------------
+__global__ void bn_bwd_apply_kernel(const float* __restrict__ raw, float* __restrict__ d, const float* __restrict__ ss,
+                                    const float* __restrict__ mr, const double* __restrict__ sums, double count,
+                                    int use_batch, float* __restrict__ dgamma, float* __restrict__ dbeta, int C, long total,
+                                    bf16* __restrict__ d16) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < C) { dgamma[i] = (float)sums[i * 2 + 1]; dbeta[i] = (float)sums[i * 2]; }
+  if (i >= total) return;
+  const int c = (int)(i % C);
+  float dz = d[i];
+  if (use_batch) {
+    const float xh = (raw[i] - mr[c * 2]) * mr[c * 2 + 1];
+    dz = dz - (float)(sums[c * 2] / count) - xh * (float)(sums[c * 2 + 1] / count);
+  }
+  const float v = ss[c * 2] * dz;
+  d[i] = v;
+  if (d16) d16[i] = __float2bfloat16_rn(v);
 }
 }  // namespace
