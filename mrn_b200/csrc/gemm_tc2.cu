@@ -9,7 +9,8 @@
 //     ('b d p c -> b (d p) c', 'b d p c -> b (d c) p') are box orientations, not copies;
 //   * two-level output addressing (same MrnbAxis as gemm_f32.cu), split-K with fp32 atomics, and an epilogue with
 //     bias over n or m, exact GELU, an elementwise multiplier and a residual at the output address.
-// bf16 operands, fp32 accumulation in TMEM.  One 128 x BN output tile per CTA (router GEMMs have K >= 256).
+// bf16 operands, fp32 accumulation in TMEM.  128 x BN output tiles, BN = 128 for N >= 128 and 64 below, walked by two
+// persistent CTAs per SM (router GEMMs have K >= 256).
 #include "gemm_f32.h"
 #include "gemm_tc2.h"
 #include "sm100.cuh"
@@ -17,8 +18,7 @@
 namespace {
 
 constexpr int BM = 128, BK = 64, UMMA_K = 16;
-// operand ring depth: 3 x 32 KiB for the two co-resident CTAs of the <= 128-wide tiles, 4 x 48 KiB for the single 256-wide CTA
-__host__ __device__ constexpr int stages_for(int bn) { return bn > 128 ? 4 : 3; }
+constexpr int STAGES = 3;              // operand ring: 3 x <= 32 KiB, so that two CTAs fit one SM
 constexpr int A_BYTES = BM * BK * 2;
 
 __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
@@ -74,7 +74,6 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   extern __shared__ uint8_t smem_raw[];
   constexpr int B_BYTES = BN * BK * 2;
   constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  constexpr int STAGES = stages_for(BN);
   uint8_t* smem = smem_raw + align_smem_1024_offset(smem_raw);
   __shared__ __align__(8) uint64_t full_bar[STAGES];
   __shared__ __align__(8) uint64_t empty_bar[STAGES];
@@ -382,7 +381,7 @@ int launch2(const MrnbTcGemm2& p, cudaStream_t st) {
   ep.kb_per_split = (ep.KB_total + splits - 1) / splits;
   splits = (ep.KB_total + ep.kb_per_split - 1) / ep.kb_per_split;     // no empty split
   ep.splits = splits;
-  const size_t smem = 1024 + (size_t)stages_for(BN) * (A_BYTES + BN * BK * 2);
+  const size_t smem = 1024 + (size_t)STAGES * (A_BYTES + BN * BK * 2);
   static bool attr = false;
   if (!attr) { cudaFuncSetAttribute(tc_gemm2_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); attr = true; }
   ep.simple = (p.cn.si == 1 && p.cn.inner >= p.N && p.cm.inner >= p.M) ? 1 : 0;
@@ -393,8 +392,8 @@ int launch2(const MrnbTcGemm2& p, cudaStream_t st) {
   ep.total_tiles = (long)ep.tiles_n * ep.tiles_m * p.groups * splits;
   static int n_sm = 0;
   if (!n_sm) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); if (n_sm <= 0) n_sm = 148; }
-  // BN <= 128: two CTAs per SM (2 x (2 x BN <= 256) TMEM columns, 2 x <= 97 KiB smem); BN = 256: one (512 columns, 145 KiB)
-  const long cap = (BN > 128 ? 1L : 2L) * n_sm;
+  // two CTAs per SM: 2 x (2 x BN <= 256) TMEM columns, 2 x <= 97 KiB smem
+  const long cap = 2L * n_sm;
   const int grid = (int)(ep.total_tiles < cap ? ep.total_tiles : cap);
   tc_gemm2_kernel<BN, A_MN, B_MN><<<grid, 192, smem, st>>>(tmA, tmB, p.a.recipe, p.b.recipe, ep);
   MRNB_CHECK_LAUNCH("tc_gemm2_kernel");
@@ -410,14 +409,12 @@ int mrnb_tc_gemm2(const MrnbTcGemm2& p, cudaStream_t st) {
                  "tc_gemm2: split-K supports a raw fp32 accumulate only");
   MrnbProfScope prof(MRNB_PROF_TCGEMM2, st, 2.0 * p.M * p.N * p.K * p.groups,
                      (double)p.groups * (2.0 * p.M * p.K + 2.0 * p.N * p.K + 4.0 * p.M * p.N));
-  const int bn = p.bn ? p.bn : (p.N >= 128 ? 128 : 64);
-  MRNB_CHECK_ARG(bn == 64 || bn == 128 || bn == 256, "tc_gemm2: tile width %d", bn);
 #define GO(BN_)                                                                                   \
   if (p.a.mn_major && p.b.mn_major) return launch2<BN_, true, true>(p, st);                       \
   if (p.a.mn_major) return launch2<BN_, true, false>(p, st);                                      \
   if (p.b.mn_major) return launch2<BN_, false, true>(p, st);                                      \
   return launch2<BN_, false, false>(p, st);
-  if (bn == 256) { GO(256) } else if (bn == 128) { GO(128) } else { GO(64) }
+  if (p.N >= 128) { GO(128) } else { GO(64) }
 #undef GO
 }
 

@@ -29,9 +29,6 @@ struct MrnbTcGemm2 {
   float* pre32;                         // optional fp32 copy of the value before `mul` / `res` (same element offsets)
   int M, N, K, groups, splitk, gelu;
   float alpha;
-  int bn;                               // output tile width: 0 = auto (128 for N >= 128, else 64); 256 = one CTA per SM, for the
-                                        // large-K / large-N contractions whose 128-wide tiles are L2-traffic bound (a K-major B
-                                        // operand must then carry box rows = 256)
 };
 
 // [groups][rows][K] with k contiguous

@@ -11,8 +11,10 @@
 //   gn[b,k,:] = LN_T(y[b,k,:]);  g2[b,k,t] = sum_j Wc[k,j] gn[b,j,t] + bc[k];  y2 = y*g2;  out = y2 W3^T + b3 + x
 //   s[b,t,j] = sum_k out[b,k,t] Wcr[j,k] + bcr[j];  r[b,j] = sum_t wr[t] s[b,t,j] + br;  gate = softmax(r)
 // Every rearrange/permute of the reference is a two-level stride of the GEMM descriptors (no copies).
-// v1 engine: fp32 CUDA-core GEMM (gemm_f32.cu) for both precisions -- gate weights are an fp32 quantity
-// (1e-4 tolerance); the tensor-core port of these contractions is tracked in DESIGN.md.
+// Two GEMM engines.  fp32: the CUDA-core GEMM (gemm_f32.cu), the parity mode held to 1e-4.  bf16 with 32 <= T <= 64:
+// tcgen05 (gemm_tc.cu for the forward row Linears, gemm_tc2.cu for the token / channel mixing and every backward GEMM)
+// with bf16 operands and fp32 accumulation, CRNN's T = 63 padded to 64 frames.  The gate head (N = I) is an fp32 GEMV in
+// both.
 #include "common.cuh"
 #include <stdlib.h>
 #include "gemm_f32.h"
@@ -27,10 +29,17 @@ constexpr int RD = 256;   // router channel width (opt.hidden_size)
 enum { R_ROUTE_W, R_ROUTE_B, R_CR_W, R_CR_B, R_N_W, R_N_B, R_P1_W, R_P1_B, R_SN_W, R_SN_B, R_SP_W, R_SP_B,
        R_CN_W, R_CN_B, R_CP_W, R_CP_B, R_P2_W, R_P2_B, R_P3_W, R_P3_B };
 
+// element count of each parameter slot, in R_* order
+void router_sizes(int I, int T, int D, long* sz) {
+  const long s[MRNB_ROUTER_NPARAMS] = {T, 1, (long)I * I * D, I, D, D, 2L * D * D, 2L * D, D, D,
+                                       (long)I * T * I * T, (long)I * T, T, T, (long)I * D * I * D, (long)I * D,
+                                       (long)D * D, D, (long)D * D, D};
+  for (int k = 0; k < MRNB_ROUTER_NPARAMS; ++k) sz[k] = s[k];
+}
+
 long router_offsets(int I, int T, int D, long* off) {
-  const long sz[MRNB_ROUTER_NPARAMS] = {T, 1, (long)I * I * D, I, D, D, 2L * D * D, 2L * D, D, D,
-                                        (long)I * T * I * T, (long)I * T, T, T, (long)I * D * I * D, (long)I * D,
-                                        (long)D * D, D, (long)D * D, D};
+  long sz[MRNB_ROUTER_NPARAMS];
+  router_sizes(I, T, D, sz);
   // every slot starts on a 32-byte boundary (8 floats) so the bf16 shadow of a weight is a legal TMA base;
   // padding elements stay zero (zero gradient, untouched by Adam)
   long o = 0;
@@ -641,6 +650,8 @@ RouterWs carve(char* base, int B, int I, int T, int D, bool bwd) {
     kernel<<<cdiv((n), 256), 256, 0, st>>>(__VA_ARGS__);               \
     MRNB_CHECK_LAUNCH(#kernel);                                        \
   } while (0)
+// grid of the grid-stride row kernels (ln_rows_bwd_kernel, dg1_fused_kernel): 8 warps per block, 16 rows per warp
+inline int rows16_grid(long rows) { const int g = (int)((rows + 8 * 16 - 1) / (8 * 16)); return g > 0 ? g : 1; }
 
 // column sums for n-contiguous layouts: 64 x float4 columns per block, 4 row lanes, 4 rows in flight per thread
 __global__ void __launch_bounds__(256)
@@ -960,12 +971,7 @@ MrnbTcOperand nogroup(MrnbTcOperand o) {          // shared weight: ignore the g
 inline int bn_for(int N) { return N >= 128 ? 128 : 64; }
 // split-K factor of a weight-gradient GEMM with `tiles` output tiles: the largest split whose tiles x split work items
 // still fit ONE wave of the 2 x 148 persistent CTAs (a second, partly filled wave costs a whole tile duration)
-inline int splitk_for(int tiles, int ctas = 296) { const int s = ctas / (tiles > 0 ? tiles : 1); return s < 1 ? 1 : s; }
-// channel mixing (K = N = I*D >= 1024): 128 x 256 tiles, one CTA per SM
-// 128 x 256 tiles (one CTA per SM, 4-stage ring) measured against 128 x 128 (two CTAs per SM): forward 137 vs 135 us,
-// dgn 204 vs 164 us, dWc 218 vs 165 us -- the second co-resident CTA hides more latency than the wider tile saves in L2 traffic
-inline int bn_chan(long) { return 128; }   // 128 x 256 tiles at one CTA per SM measured slower (175 -> 246 us forward): the
-                                            // second co-resident CTA hides more latency than the wider tile saves in L2 traffic
+inline int splitk_for(int tiles) { const int s = 296 / (tiles > 0 ? tiles : 1); return s < 1 ? 1 : s; }
 
 // out[rows, Nout] = A[rows, K] . W[Nout, K]^T (+bias, +res)   -- plain row-major Linear
 int linear_rows(const Dims& d, const float* A32, const bf16* A16, long lda, const float* W32, const bf16* W16, int Nout, int K,
@@ -1022,12 +1028,121 @@ int dw_rows(const Dims& d, const float* dY32, const bf16* dY16, long ldy, int No
   return mrnb_sgemm(g, st);
 }
 
+// v2[b] = Ws . vn[b] + bs   (token mixing over n = i*T+t)
+int token_mix_fwd(const Dims& d, const float* Ws32, const bf16* Ws16, const float* bs, const float* vn32, const bf16* vn16,
+                  float* v2, cudaStream_t st) {
+  if (d.tc) {
+    MrnbTcGemm2 g{};
+    g.a = nogroup(mrnb_operand_k2d(Ws16, d.IT, d.IT, d.IT, 128, 1));
+    g.b = op_tok_c_mnmajor(vn16, d);
+    g.out32 = v2; g.cm = mrnb_axis(d.D); g.cn = mrnb_axis(1); g.c_gstride = d.ITD;
+    g.bias_m = bs; g.M = (int)d.IT; g.N = d.D; g.K = (int)d.IT; g.groups = d.B; g.alpha = 1.f;
+    return mrnb_tc_gemm2(g, st);
+  }
+  MrnbGemm g{};
+  g.A = Ws32; g.am = mrnb_axis(d.IT); g.ak = mrnb_axis(1); g.a_kfast = 1; g.sAb = 0;
+  g.B = vn32; g.bk = mrnb_axis(d.D); g.bn = mrnb_axis(1); g.b_kfast = 0; g.sBb = d.ITD;
+  g.C = v2; g.cm = mrnb_axis(d.D); g.cn = mrnb_axis(1); g.sCb = d.ITD;
+  g.M = (int)d.IT; g.N = d.D; g.K = (int)d.IT; g.batch = d.B; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
+  g.bias_m = bs;
+  return mrnb_sgemm(g, st);
+}
+// dvn[b,m,:] = sum_n Ws[n,m] dv2[b,n,:] ;  dWs[n,m] += sum_(b,c) dv2[b,n,c] vn[b,m,c]
+int token_mix_bwd(const Dims& d, const float* Ws32, const bf16* Ws16, const float* dv2_32, const bf16* dv2_16,
+                  const float* vn32, const bf16* vn16, float* dvn, float* dWs, cudaStream_t st) {
+  if (d.tc) {
+    MrnbTcGemm2 g{};
+    g.a = nogroup(mrnb_operand_mn2d(Ws16, d.IT, d.IT, d.IT, 1));
+    g.b = op_tok_c_mnmajor(dv2_16, d);
+    g.out32 = dvn; g.cm = mrnb_axis(d.D); g.cn = mrnb_axis(1); g.c_gstride = d.ITD;
+    g.M = (int)d.IT; g.N = d.D; g.K = (int)d.IT; g.groups = d.B; g.alpha = 1.f;
+    MRNB_TRY(mrnb_tc_gemm2(g, st));
+    MrnbTcGemm2 h{};
+    h.a = op_tok_bc_kmajor(dv2_16, d, 128);
+    h.b = op_tok_bc_kmajor(vn16, d, bn_for((int)d.IT));
+    h.out32 = dWs; h.cm = mrnb_axis(d.IT); h.cn = mrnb_axis(1);
+    h.M = (int)d.IT; h.N = (int)d.IT; h.K = d.B * d.D; h.groups = 1; h.alpha = 1.f;
+    h.splitk = splitk_for(cdiv(d.IT, 128) * cdiv(d.IT, bn_for((int)d.IT)));
+    return mrnb_tc_gemm2(h, st);
+  }
+  MrnbGemm g{};
+  g.A = Ws32; g.am = mrnb_axis(1); g.ak = mrnb_axis(d.IT); g.a_kfast = 0; g.sAb = 0;
+  g.B = dv2_32; g.bk = mrnb_axis(d.D); g.bn = mrnb_axis(1); g.b_kfast = 0; g.sBb = d.ITD;
+  g.C = dvn; g.cm = mrnb_axis(d.D); g.cn = mrnb_axis(1); g.sCb = d.ITD;
+  g.M = (int)d.IT; g.N = d.D; g.K = (int)d.IT; g.batch = d.B; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
+  MRNB_TRY(mrnb_sgemm(g, st));
+  MrnbGemm h{};
+  h.A = dv2_32; h.am = mrnb_axis(d.D); h.ak = mrnb_axis2(d.D, 1, d.ITD); h.a_kfast = 1;
+  h.B = vn32; h.bn = mrnb_axis(d.D); h.bk = mrnb_axis2(d.D, 1, d.ITD); h.b_kfast = 1;
+  h.C = dWs; h.cm = mrnb_axis(d.IT); h.cn = mrnb_axis(1);
+  h.M = (int)d.IT; h.N = (int)d.IT; h.K = d.B * d.D; h.batch = 1; h.alpha = 1.f; h.rows_per_scale = 1;
+  h.splitk = (d.B * d.D + 2047) / 2048; if (h.splitk > 32) h.splitk = 32; if (h.splitk < 1) h.splitk = 1;
+  return mrnb_sgemm(h, st);
+}
+
+// g2[(b,t),(i,c)] = sum_(i',c') gn[(b,t),(i',c')] Wc[(i,c),(i',c')] + bc   (channel mixing over k = i*D+c, K = N = I*D)
+// On tcgen05 every channel-mix GEMM runs 128 x 128 tiles at two CTAs per SM.  128 x 256 tiles at one CTA per SM (4-stage
+// ring) measured slower: forward 135 -> 137 us, dgn 164 -> 204 us, dWc 165 -> 218 us, and in an earlier measurement
+// forward 175 -> 246 us.  The second co-resident CTA hides more latency than the wider tile saves in L2 traffic.
+int channel_mix_fwd(const Dims& d, const float* Wc32, const bf16* Wc16, const float* bc, const float* gn32, const bf16* gn16,
+                    float* g2, cudaStream_t st) {
+  if (d.tc) {
+    MrnbTcGemm2 g{};
+    g.a = op_bt_ic_kmajor(gn16, d);
+    g.b = mrnb_operand_k2d(Wc16, d.ID, d.ID, d.ID, 128, 1);
+    g.out32 = g2; g.cm = mrnb_axis2(d.T, d.D, d.ITD); g.cn = mrnb_axis2(d.D, 1, d.TD);
+    g.bias_n = bc; g.M = d.B * d.T; g.N = (int)d.ID; g.K = (int)d.ID; g.groups = 1; g.alpha = 1.f;
+    return mrnb_tc_gemm2(g, st);
+  }
+  MrnbGemm g{};
+  g.A = gn32; g.am = mrnb_axis2(d.T, d.D, d.ITD); g.ak = mrnb_axis2(d.D, 1, d.TD); g.a_kfast = 1;
+  g.B = Wc32; g.bn = mrnb_axis(d.ID); g.bk = mrnb_axis(1); g.b_kfast = 1;
+  g.C = g2; g.cm = mrnb_axis2(d.T, d.D, d.ITD); g.cn = mrnb_axis2(d.D, 1, d.TD);
+  g.M = d.B * d.T; g.N = (int)d.ID; g.K = (int)d.ID; g.batch = 1; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
+  g.bias_n = bc;
+  return mrnb_sgemm(g, st);
+}
+// dgn[(b,t), j] = sum_k dg2[(b,t),k] Wc[k,j] ;  dWc[k,j] += sum_(b,t) dg2[(b,t),k] gn[(b,t),j]
+int channel_mix_bwd(const Dims& d, const float* Wc32, const bf16* Wc16, const float* dg2_32, const bf16* dg2_16,
+                    const float* gn32, const bf16* gn16, float* dgn, float* dWc, cudaStream_t st) {
+  if (d.tc) {
+    MrnbTcGemm2 g{};
+    g.a = op_bt_ic_kmajor(dg2_16, d);
+    g.b = mrnb_operand_mn2d(Wc16, d.ID, d.ID, d.ID, 1);
+    g.out32 = dgn; g.cm = mrnb_axis2(d.T, d.D, d.ITD); g.cn = mrnb_axis2(d.D, 1, d.TD);
+    g.M = d.B * d.T; g.N = (int)d.ID; g.K = (int)d.ID; g.groups = 1; g.alpha = 1.f;
+    MRNB_TRY(mrnb_tc_gemm2(g, st));
+    MrnbTcGemm2 h{};
+    h.a = op_ic_bt_mnmajor(dg2_16, d);
+    h.b = op_ic_bt_mnmajor(gn16, d);
+    h.out32 = dWc; h.cm = mrnb_axis(d.ID); h.cn = mrnb_axis(1);
+    h.M = (int)d.ID; h.N = (int)d.ID; h.K = d.B * d.T; h.groups = 1; h.alpha = 1.f;
+    h.splitk = splitk_for(cdiv(d.ID, 128) * cdiv(d.ID, 128));
+    return mrnb_tc_gemm2(h, st);
+  }
+  MrnbGemm g{};
+  g.A = dg2_32; g.am = mrnb_axis2(d.T, d.D, d.ITD); g.ak = mrnb_axis2(d.D, 1, d.TD); g.a_kfast = 1;
+  g.B = Wc32; g.bk = mrnb_axis(d.ID); g.bn = mrnb_axis(1); g.b_kfast = 0;
+  g.C = dgn; g.cm = mrnb_axis2(d.T, d.D, d.ITD); g.cn = mrnb_axis2(d.D, 1, d.TD);
+  g.M = d.B * d.T; g.N = (int)d.ID; g.K = (int)d.ID; g.batch = 1; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
+  MRNB_TRY(mrnb_sgemm(g, st));
+  MrnbGemm h{};
+  h.A = dg2_32; h.am = mrnb_axis2(d.D, 1, d.TD); h.ak = mrnb_axis2(d.T, d.D, d.ITD); h.a_kfast = 0;
+  h.B = gn32; h.bk = mrnb_axis2(d.T, d.D, d.ITD); h.bn = mrnb_axis2(d.D, 1, d.TD); h.b_kfast = 0;
+  h.C = dWc; h.cm = mrnb_axis(d.ID); h.cn = mrnb_axis(1);
+  h.M = (int)d.ID; h.N = (int)d.ID; h.K = d.B * d.T; h.batch = 1; h.alpha = 1.f; h.rows_per_scale = 1;
+  const int tiles = cdiv(d.ID, 128) * cdiv(d.ID, 128);
+  h.splitk = tiles >= 120 ? 1 : (tiles >= 30 ? 4 : 16);
+  if ((long)d.B * d.T < 64L * h.splitk) h.splitk = 1;
+  return mrnb_sgemm(h, st);
+}
+
 int router_forward(const float* P, const float* x, const Dims& d, float* out_user, float* scores, float* gate, int* index,
                    RouterWs& w, cudaStream_t st) {
   long off[MRNB_ROUTER_NPARAMS + 1];
   const long nparam = router_offsets(d.I, d.T, d.D, off);
   const int B = d.B, I = d.I, T = d.T, D = d.D;
-  const long M = d.M, IT = d.IT, ID = d.ID, TD = d.TD, ITD = d.ITD;
+  const long M = d.M;
   const bool tc = d.tc;
   const bf16* W16 = w.w16;
   float* out = w.out;   // kept in the workspace for the backward; copied to the caller's buffer at the end
@@ -1053,23 +1168,7 @@ int router_forward(const float* P, const float* x, const Dims& d, float* out_use
     else gelu_ln_fwd_kernel<false><<<cdiv(M, 8), 256, 0, st>>>(w.a1, P + off[R_SN_W], P + off[R_SN_B], w.u, w.vn, nullptr, w.stats2, M, 1e-5f);
     MRNB_CHECK_LAUNCH("gelu_ln_fwd_kernel");
   }
-  // v2[b] = Ws . vn[b] + bs  (token mixing over n = i*T+t)
-  if (tc) {
-    MrnbTcGemm2 g{};
-    g.a = nogroup(mrnb_operand_k2d(W16 + off[R_SP_W], IT, IT, IT, 128, 1));
-    g.b = op_tok_c_mnmajor(w.vn16, d);
-    g.out32 = w.v2; g.cm = mrnb_axis(D); g.cn = mrnb_axis(1); g.c_gstride = ITD;
-    g.bias_m = P + off[R_SP_B]; g.M = (int)IT; g.N = D; g.K = (int)IT; g.groups = B; g.alpha = 1.f;
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  } else {
-    MrnbGemm g{};
-    g.A = P + off[R_SP_W]; g.am = mrnb_axis(IT); g.ak = mrnb_axis(1); g.a_kfast = 1; g.sAb = 0;
-    g.B = w.vn; g.bk = mrnb_axis(D); g.bn = mrnb_axis(1); g.b_kfast = 0; g.sBb = ITD;
-    g.C = w.v2; g.cm = mrnb_axis(D); g.cn = mrnb_axis(1); g.sCb = ITD;
-    g.M = (int)IT; g.N = D; g.K = (int)IT; g.batch = B; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-    g.bias_m = P + off[R_SP_B];
-    MRNB_TRY(mrnb_sgemm(g, st));
-  }
+  MRNB_TRY(token_mix_fwd(d, P + off[R_SP_W], W16 + off[R_SP_W], P + off[R_SP_B], w.vn, w.vn16, w.v2, st));
   {   // g1 = u * v2 (a separate streaming pass: measured faster than a multiplier read in the GEMM's row-per-thread epilogue)
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     LAUNCH_EW(mul_kernel, M * D / 4, w.u, w.v2, tc ? nullptr : w.g1, tc ? w.g116 : nullptr, M * D / 4);
@@ -1086,24 +1185,7 @@ int router_forward(const float* P, const float* x, const Dims& d, float* out_use
                                            w.statsT, T, d.Tv, 1e-5f);
     MRNB_CHECK_LAUNCH("lnT_fwd_kernel");
   }
-  // g2[(b,t),(i,c)] = sum_(i',c') gn[(b,t),(i',c')] Wc[(i,c),(i',c')] + bc   (channel mixing over k = i*D+c)
-  if (tc) {
-    MrnbTcGemm2 g{};
-    g.a = op_bt_ic_kmajor(w.gn16, d);
-    g.bn = bn_chan(ID);
-    g.b = mrnb_operand_k2d(W16 + off[R_CP_W], ID, ID, ID, g.bn, 1);
-    g.out32 = w.g2; g.cm = mrnb_axis2(T, D, ITD); g.cn = mrnb_axis2(D, 1, TD);
-    g.bias_n = P + off[R_CP_B]; g.M = B * T; g.N = (int)ID; g.K = (int)ID; g.groups = 1; g.alpha = 1.f;
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  } else {
-    MrnbGemm g{};
-    g.A = w.gn; g.am = mrnb_axis2(T, D, ITD); g.ak = mrnb_axis2(D, 1, TD); g.a_kfast = 1;
-    g.B = P + off[R_CP_W]; g.bn = mrnb_axis(ID); g.bk = mrnb_axis(1); g.b_kfast = 1;
-    g.C = w.g2; g.cm = mrnb_axis2(T, D, ITD); g.cn = mrnb_axis2(D, 1, TD);
-    g.M = B * T; g.N = (int)ID; g.K = (int)ID; g.batch = 1; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-    g.bias_n = P + off[R_CP_B];
-    MRNB_TRY(mrnb_sgemm(g, st));
-  }
+  MRNB_TRY(channel_mix_fwd(d, P + off[R_CP_W], W16 + off[R_CP_W], P + off[R_CP_B], w.gn, w.gn16, w.g2, st));
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     LAUNCH_EW(mul_kernel, M * D / 4, w.y, w.g2, tc ? nullptr : w.y2, tc ? w.y216 : nullptr, M * D / 4);
@@ -1152,46 +1234,7 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     LAUNCH_EW(mul2_kernel, n4, w.dy2, w.g2, w.y, w.dy, w.dg2, tc ? w.dg216 : nullptr, n4);
   }
-  if (tc) {
-    {  // dgn[(b,t), j] = sum_k dg2[(b,t),k] Wc[k,j]
-      MrnbTcGemm2 g{};
-      g.a = op_bt_ic_kmajor(w.dg216, d);
-      g.b = mrnb_operand_mn2d(W16 + off[R_CP_W], ID, ID, ID, 1);
-      g.out32 = w.dgn; g.cm = mrnb_axis2(T, D, ITD); g.cn = mrnb_axis2(D, 1, TD);
-      g.M = B * T; g.N = (int)ID; g.K = (int)ID; g.groups = 1; g.alpha = 1.f; g.bn = bn_chan(ID);
-      MRNB_TRY(mrnb_tc_gemm2(g, st));
-    }
-    {  // dWc[k,j] = sum_(b,t) dg2[(b,t),k] gn[(b,t),j]
-      MrnbTcGemm2 g{};
-      g.a = op_ic_bt_mnmajor(w.dg216, d);
-      g.b = op_ic_bt_mnmajor(w.gn16, d);
-      g.out32 = G + off[R_CP_W]; g.cm = mrnb_axis(ID); g.cn = mrnb_axis(1);
-      g.M = (int)ID; g.N = (int)ID; g.K = B * T; g.groups = 1; g.alpha = 1.f;
-      g.bn = bn_chan(ID);
-      g.splitk = g.bn == 256 ? splitk_for(cdiv(ID, 128) * cdiv(ID, 256), 148) : splitk_for(cdiv(ID, 128) * cdiv(ID, 128));
-      MRNB_TRY(mrnb_tc_gemm2(g, st));
-    }
-  } else {
-    {
-      MrnbGemm g{};
-      g.A = w.dg2; g.am = mrnb_axis2(T, D, ITD); g.ak = mrnb_axis2(D, 1, TD); g.a_kfast = 1;
-      g.B = P + off[R_CP_W]; g.bk = mrnb_axis(ID); g.bn = mrnb_axis(1); g.b_kfast = 0;
-      g.C = w.dgn; g.cm = mrnb_axis2(T, D, ITD); g.cn = mrnb_axis2(D, 1, TD);
-      g.M = B * T; g.N = (int)ID; g.K = (int)ID; g.batch = 1; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-      MRNB_TRY(mrnb_sgemm(g, st));
-    }
-    {
-      MrnbGemm g{};
-      g.A = w.dg2; g.am = mrnb_axis2(D, 1, TD); g.ak = mrnb_axis2(T, D, ITD); g.a_kfast = 0;
-      g.B = w.gn; g.bk = mrnb_axis2(T, D, ITD); g.bn = mrnb_axis2(D, 1, TD); g.b_kfast = 0;
-      g.C = G + off[R_CP_W]; g.cm = mrnb_axis(ID); g.cn = mrnb_axis(1);
-      g.M = (int)ID; g.N = (int)ID; g.K = B * T; g.batch = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-      const int tiles = cdiv(ID, 128) * cdiv(ID, 128);
-      g.splitk = tiles >= 120 ? 1 : (tiles >= 30 ? 4 : 16);
-      if ((long)B * T < 64L * g.splitk) g.splitk = 1;
-      MRNB_TRY(mrnb_sgemm(g, st));
-    }
-  }
+  MRNB_TRY(channel_mix_bwd(d, P + off[R_CP_W], W16 + off[R_CP_W], w.dg2, w.dg216, w.gn, w.gn16, w.dgn, G + off[R_CP_W], st));
   MRNB_TRY(colsum(w.dg2, mrnb_axis2(T, D, ITD), mrnb_axis2(D, 1, TD), B * T, (int)ID, G + off[R_CP_B], st));
   {  // gn = LN_T(y)
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
@@ -1207,44 +1250,7 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     LAUNCH_EW(mul2_kernel, n4, w.dg1, w.v2, w.u, w.du, w.dv2, tc ? w.dv216 : nullptr, n4);
   }
-  if (tc) {
-    {  // dvn[b,m,:] = sum_n Ws[n,m] dv2[b,n,:]
-      MrnbTcGemm2 g{};
-      g.a = nogroup(mrnb_operand_mn2d(W16 + off[R_SP_W], IT, IT, IT, 1));
-      g.b = op_tok_c_mnmajor(w.dv216, d);
-      g.out32 = w.dvn; g.cm = mrnb_axis(D); g.cn = mrnb_axis(1); g.c_gstride = ITD;
-      g.M = (int)IT; g.N = D; g.K = (int)IT; g.groups = B; g.alpha = 1.f;
-      MRNB_TRY(mrnb_tc_gemm2(g, st));
-    }
-    {  // dWs[n,m] = sum_(b,c) dv2[b,n,c] vn[b,m,c]
-      MrnbTcGemm2 g{};
-      g.a = op_tok_bc_kmajor(w.dv216, d, 128);
-      g.b = op_tok_bc_kmajor(w.vn16, d, bn_for((int)IT));
-      g.out32 = G + off[R_SP_W]; g.cm = mrnb_axis(IT); g.cn = mrnb_axis(1);
-      g.M = (int)IT; g.N = (int)IT; g.K = B * D; g.groups = 1; g.alpha = 1.f;
-      g.splitk = splitk_for(cdiv(IT, 128) * cdiv(IT, bn_for((int)IT)));
-      MRNB_TRY(mrnb_tc_gemm2(g, st));
-    }
-  } else {
-    {
-      MrnbGemm g{};
-      g.A = P + off[R_SP_W]; g.am = mrnb_axis(1); g.ak = mrnb_axis(IT); g.a_kfast = 0; g.sAb = 0;
-      g.B = w.dv2; g.bk = mrnb_axis(D); g.bn = mrnb_axis(1); g.b_kfast = 0; g.sBb = ITD;
-      g.C = w.dvn; g.cm = mrnb_axis(D); g.cn = mrnb_axis(1); g.sCb = ITD;
-      g.M = (int)IT; g.N = D; g.K = (int)IT; g.batch = B; g.splitk = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-      MRNB_TRY(mrnb_sgemm(g, st));
-    }
-    {
-      MrnbGemm g{};
-      g.A = w.dv2; g.am = mrnb_axis(D); g.ak = mrnb_axis2(D, 1, ITD); g.a_kfast = 1;
-      g.B = w.vn; g.bn = mrnb_axis(D); g.bk = mrnb_axis2(D, 1, ITD); g.b_kfast = 1;
-      g.C = G + off[R_SP_W]; g.cm = mrnb_axis(IT); g.cn = mrnb_axis(1);
-      g.M = (int)IT; g.N = (int)IT; g.K = B * D; g.batch = 1; g.alpha = 1.f; g.rows_per_scale = 1;
-      g.splitk = (B * D + 2047) / 2048; if (g.splitk > 32) g.splitk = 32; if (g.splitk < 1) g.splitk = 1;
-      MRNB_TRY(mrnb_sgemm(g, st));
-    }
-  }
-  // dbs[n] = sum_(b,c) dv2[b,n,c]
+  MRNB_TRY(token_mix_bwd(d, P + off[R_SP_W], W16 + off[R_SP_W], w.dv2, w.dv216, w.vn, w.vn16, w.dvn, G + off[R_SP_W], st));
   {  // dbs[n] = sum_(b,c) dv2[b,n,c]
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     rowsum256_kernel<<<dim3((int)IT, B >= 64 ? 2 : 1), 256, 0, st>>>(w.dv2, (int)IT, B, G + off[R_SP_B]);
@@ -1252,13 +1258,12 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
   }
   {  // vn = LN_D(GELU(a1v)); u = GELU(a1u)
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const int grid = (int)((M + 8 * 16 - 1) / (8 * 16));
-    if (tc) ln_rows_bwd_kernel<true, true><<<grid > 0 ? grid : 1, 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn, w.da1 + D,
-                                                                                 w.da116 + D, 2 * D, nullptr, nullptr,
-                                                                                 G + off[R_SN_W], G + off[R_SN_B], M);
-    else ln_rows_bwd_kernel<true><<<grid > 0 ? grid : 1, 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn, w.da1 + D,
-                                                                        nullptr, 2 * D, nullptr, nullptr,
-                                                                        G + off[R_SN_W], G + off[R_SN_B], M);
+    if (tc) ln_rows_bwd_kernel<true, true><<<rows16_grid(M), 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn,
+                                                                           w.da1 + D, w.da116 + D, 2 * D, nullptr, nullptr,
+                                                                           G + off[R_SN_W], G + off[R_SN_B], M);
+    else ln_rows_bwd_kernel<true><<<rows16_grid(M), 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn, w.da1 + D,
+                                                                  nullptr, 2 * D, nullptr, nullptr,
+                                                                  G + off[R_SN_W], G + off[R_SN_B], M);
     MRNB_CHECK_LAUNCH("ln_rows_bwd_kernel");
     LAUNCH_EW(gelu_bwd_kernel, M * D, w.a1, w.du, w.da1, tc ? w.da116 : nullptr, M);
   }
@@ -1269,9 +1274,8 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
     if (dx) {   // dxhat = da1 (W1 diag(gamma)): the folded bf16 weights already carry gamma
       MRNB_TRY(dx_rows(d, w.da1, w.da116, 2 * D, 2 * D, P + off[R_P1_W], W16 + off[R_P1_W], D, w.dxn, D, st));
       MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-      const int grid = (int)((M + 8 * 16 - 1) / (8 * 16));
-      ln_rows_bwd_kernel<false><<<grid > 0 ? grid : 1, 256, 0, st>>>(x, D, w.stats1, nullptr, w.dxn, dx, nullptr, D, w.dy, w.dout,
-                                                                       nullptr, nullptr, M);
+      ln_rows_bwd_kernel<false><<<rows16_grid(M), 256, 0, st>>>(x, D, w.stats1, nullptr, w.dxn, dx, nullptr, D, w.dy, w.dout,
+                                                                nullptr, nullptr, M);
       MRNB_CHECK_LAUNCH("ln_rows_bwd_kernel");
     }
     return MRNB_OK;
@@ -1280,13 +1284,30 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
   MRNB_TRY(dx_rows(d, w.da1, w.da116, 2 * D, 2 * D, P + off[R_P1_W], W16 + off[R_P1_W], D, w.dxn, D, st));
   {  // xn = LN_D(x): dgamma/dbeta (+ dx = LNbwd + dy + dout when requested)
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const int grid = (int)((M + 8 * 16 - 1) / (8 * 16));
-    ln_rows_bwd_kernel<false><<<grid > 0 ? grid : 1, 256, 0, st>>>(x, D, w.stats1, P + off[R_N_W], w.dxn, dx, nullptr, D,
-                                                                     dx ? w.dy : nullptr, dx ? w.dout : nullptr,
-                                                                     G + off[R_N_W], G + off[R_N_B], M);
+    ln_rows_bwd_kernel<false><<<rows16_grid(M), 256, 0, st>>>(x, D, w.stats1, P + off[R_N_W], w.dxn, dx, nullptr, D,
+                                                              dx ? w.dy : nullptr, dx ? w.dout : nullptr,
+                                                              G + off[R_N_W], G + off[R_N_B], M);
     MRNB_CHECK_LAUNCH("ln_rows_bwd_kernel");
   }
   return MRNB_OK;
+}
+
+// Training-step backward in fp32 mode: gate head from dL/ds (w.ds), then the generic DM_Router backward on the
+// materialised dout.  G = zeroed gradient arena.
+int router_backward_gate_f32(const float* P, const float* x, const Dims& d, float* G, RouterWs& w, cudaStream_t st) {
+  long off[MRNB_ROUTER_NPARAMS + 1];
+  router_offsets(d.I, d.T, d.D, off);
+  {  // dWcr[j,(i,c)] = sum_(b,t) ds[(b,t),j] out[b,i,t,c]
+    MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
+    MRNB_DISPATCH_I(launch_gate_head_dw, d.I, w.ds, w.out, d.B, d.T, G + off[R_CR_W], st);
+  }
+  MRNB_TRY(colsum(w.ds, mrnb_axis(d.I), mrnb_axis(1), d.B * d.T, d.I, G + off[R_CR_B], st));
+  {  // dout[b,i,t,c] = sum_j ds[(b,t),j] Wcr[j,(i,c)]
+    MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
+    const long total4 = d.M * d.D / 4;
+    LAUNCH_EW(dout_kernel, total4, w.ds, P + off[R_CR_W], d.I, d.T, total4, w.dout, nullptr);
+  }
+  return dm_router_backward_core(P, x, d, G, nullptr, w, st);
 }
 
 // Training-step backward in tensor-core mode: gate head + DM_Router parameter gradients from dL/dr (w.dr), with the
@@ -1296,7 +1317,7 @@ int router_backward_gate_tc(const float* P, const float* x, const Dims& d, float
   long off[MRNB_ROUTER_NPARAMS + 1];
   router_offsets(d.I, d.T, d.D, off);
   const int B = d.B, I = d.I, T = d.T, D = d.D;
-  const long M = d.M, IT = d.IT, ID = d.ID, TD = d.TD, ITD = d.ITD;
+  const long M = d.M, IT = d.IT, ID = d.ID;
   const bf16* W16 = w.w16;
   const float* wr = P + off[R_ROUTE_W];
   Dims dq = d;                        // the collapsed last Linear: B*I rows (zero-padded to a 128-row tile) instead of B*I*T
@@ -1321,24 +1342,7 @@ int router_backward_gate_tc(const float* P, const float* x, const Dims& d, float
   }
   // dW3[n,k] = sum_(b,i) q[(b,i),n] y2w[(b,i),k]
   MRNB_TRY(dw_rows(dq, nullptr, w.gq16, D, D, nullptr, w.y2w16, D, D, G + off[R_P3_W], st));
-  {  // dgn[(b,t), j] = sum_k dg2[(b,t),k] Wc[k,j]
-    MrnbTcGemm2 g{};
-    g.a = op_bt_ic_kmajor(w.dg216, d);
-    g.b = mrnb_operand_mn2d(W16 + off[R_CP_W], ID, ID, ID, 1);
-    g.out32 = w.dgn; g.cm = mrnb_axis2(T, D, ITD); g.cn = mrnb_axis2(D, 1, TD);
-    g.M = B * T; g.N = (int)ID; g.K = (int)ID; g.groups = 1; g.alpha = 1.f; g.bn = bn_chan(ID);
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  }
-  {  // dWc[k,j] = sum_(b,t) dg2[(b,t),k] gn[(b,t),j]
-    MrnbTcGemm2 g{};
-    g.a = op_ic_bt_mnmajor(w.dg216, d);
-    g.b = op_ic_bt_mnmajor(w.gn16, d);
-    g.out32 = G + off[R_CP_W]; g.cm = mrnb_axis(ID); g.cn = mrnb_axis(1);
-    g.M = (int)ID; g.N = (int)ID; g.K = B * T; g.groups = 1; g.alpha = 1.f;
-    g.bn = bn_chan(ID);
-    g.splitk = g.bn == 256 ? splitk_for(cdiv(ID, 128) * cdiv(ID, 256), 148) : splitk_for(cdiv(ID, 128) * cdiv(ID, 128));
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  }
+  MRNB_TRY(channel_mix_bwd(d, nullptr, W16 + off[R_CP_W], nullptr, w.dg216, nullptr, w.gn16, w.dgn, G + off[R_CP_W], st));
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     // (capping the resident blocks so that the second pass over y / dgn hits L2 cut the DRAM reads from 500 to 400 MB but
@@ -1352,34 +1356,16 @@ int router_backward_gate_tc(const float* P, const float* x, const Dims& d, float
   MRNB_TRY(dw_rows(d, nullptr, w.dy16, D, D, nullptr, w.g116, D, D, G + off[R_P2_W], st));
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const int grid = (int)((M + 8 * 16 - 1) / (8 * 16));
-    dg1_fused_kernel<<<grid > 0 ? grid : 1, 256, 0, st>>>(w.dg1, w.v2, w.u, w.a1, w.da116, w.dv216, G + off[R_SP_B],
-                                                          G + off[R_P1_B], M, (int)IT);
+    dg1_fused_kernel<<<rows16_grid(M), 256, 0, st>>>(w.dg1, w.v2, w.u, w.a1, w.da116, w.dv216, G + off[R_SP_B],
+                                                     G + off[R_P1_B], M, (int)IT);
     MRNB_CHECK_LAUNCH("dg1_fused_kernel");
   }
-  {  // dvn[b,m,:] = sum_n Ws[n,m] dv2[b,n,:]
-    MrnbTcGemm2 g{};
-    g.a = nogroup(mrnb_operand_mn2d(W16 + off[R_SP_W], IT, IT, IT, 1));
-    g.b = op_tok_c_mnmajor(w.dv216, d);
-    g.out32 = w.dvn; g.cm = mrnb_axis(D); g.cn = mrnb_axis(1); g.c_gstride = ITD;
-    g.M = (int)IT; g.N = D; g.K = (int)IT; g.groups = B; g.alpha = 1.f;
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  }
-  {  // dWs[n,m] = sum_(b,c) dv2[b,n,c] vn[b,m,c]
-    MrnbTcGemm2 g{};
-    g.a = op_tok_bc_kmajor(w.dv216, d, 128);
-    g.b = op_tok_bc_kmajor(w.vn16, d, bn_for((int)IT));
-    g.out32 = G + off[R_SP_W]; g.cm = mrnb_axis(IT); g.cn = mrnb_axis(1);
-    g.M = (int)IT; g.N = (int)IT; g.K = B * D; g.groups = 1; g.alpha = 1.f;
-    g.splitk = splitk_for(cdiv(IT, 128) * cdiv(IT, bn_for((int)IT)));
-    MRNB_TRY(mrnb_tc_gemm2(g, st));
-  }
+  MRNB_TRY(token_mix_bwd(d, nullptr, W16 + off[R_SP_W], nullptr, w.dv216, nullptr, w.vn16, w.dvn, G + off[R_SP_W], st));
   {  // vn = LN_D(GELU(a1v)): da1[:, D:] (bf16 only), db1[D:], dgamma / dbeta
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const int grid = (int)((M + 8 * 16 - 1) / (8 * 16));
-    ln_rows_bwd_kernel<true, true><<<grid > 0 ? grid : 1, 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn, nullptr,
-                                                                          w.da116 + D, 2 * D, nullptr, nullptr, G + off[R_SN_W],
-                                                                          G + off[R_SN_B], M, G + off[R_P1_B] + D);
+    ln_rows_bwd_kernel<true, true><<<rows16_grid(M), 256, 0, st>>>(w.a1 + D, 2 * D, w.stats2, P + off[R_SN_W], w.dvn, nullptr,
+                                                                   w.da116 + D, 2 * D, nullptr, nullptr, G + off[R_SN_W],
+                                                                   G + off[R_SN_B], M, G + off[R_P1_B] + D);
     MRNB_CHECK_LAUNCH("ln_rows_bwd_kernel");
   }
   // a1 = xhat (W1 gamma)^T + b1f: proj_1 and LayerNorm 1 gradients from S = da1^T xhat (no M-row dxn GEMM, no pass over x)
@@ -1456,18 +1442,17 @@ RepackTable make_table(int I, int T, int Tp, int D) {
   RepackTable tb{};
   router_offsets(I, T, D, tb.off);
   router_offsets(I, Tp, D, tb.offp);
-  const long sz[MRNB_ROUTER_NPARAMS] = {T, 1, (long)I * I * D, I, D, D, 2L * D * D, 2L * D, D, D,
-                                        (long)I * T * I * T, (long)I * T, T, T, (long)I * D * I * D, (long)I * D,
-                                        (long)D * D, D, (long)D * D, D};
-  for (int k = 0; k < MRNB_ROUTER_NPARAMS; ++k) tb.sz[k] = sz[k];
+  router_sizes(I, T, D, tb.sz);
   return tb;
 }
 
-// workspace tail of the padded mode: padded input, padded parameters, padded gradients
+// workspace tail of the padded mode: padded input, padded parameters, padded gradients.  It sits behind the
+// backward-sized carve whatever the call, so that both backward entry points find Pp / xp where mrnb_router_forward
+// wrote them.
 struct PadWs { float *xp, *Pp, *Gp; size_t bytes; };
-PadWs carve_pad(char* base, size_t start, int B, int I, int Tp, int D) {
+PadWs carve_pad(char* base, int B, int I, int Tp, int D) {
   PadWs p{};
-  size_t o = al(start);
+  size_t o = al(carve(nullptr, B, I, Tp, D, true).bytes);
   long offp[MRNB_ROUTER_NPARAMS + 1];
   const size_t np = (size_t)router_offsets(I, Tp, D, offp);
   auto take = [&](size_t n) { float* q = base ? (float*)(base + o) : nullptr; o = al(o + n * 4); return q; };
@@ -1476,53 +1461,68 @@ PadWs carve_pad(char* base, size_t start, int B, int I, int Tp, int D) {
   return p;
 }
 
-int pad_inputs(const float* params, const float* x, int B, int I, int T, int Tp, int D, const PadWs& pw, cudaStream_t st) {
+// One call's engine, frame count and workspace: T -> Tp, the carve, the padded tail and the bytes they need.
+struct RouterRun {
+  Dims d;               // d.T = frames as run (Tp), d.Tv = the caller's frames
+  RouterWs w;
+  PadWs pw;             // padded mode only
+  bool padded;
+  size_t bytes;
+  RouterRun(void* ws, int B, int I, int T, int D, int prec, bool bwd)
+      : d(B, I, padded_T(prec, T), D, use_tc(prec, T), T), w(carve((char*)ws, B, I, d.T, D, bwd)), pw{}, padded(d.T != T) {
+    if (padded) pw = carve_pad((char*)ws, B, I, d.T, D);
+    bytes = padded ? pw.bytes : w.bytes;
+  }
+};
+
+int pad_inputs(const float* params, const float* x, const RouterRun& r, cudaStream_t st) {
   MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-  const RepackTable tb = make_table(I, T, Tp, D);
-  cudaMemsetAsync(pw.Pp, 0, (size_t)tb.offp[MRNB_ROUTER_NPARAMS] * sizeof(float), st);
+  const Dims& d = r.d;
+  const RepackTable tb = make_table(d.I, d.Tv, d.T, d.D);
+  cudaMemsetAsync(r.pw.Pp, 0, (size_t)tb.offp[MRNB_ROUTER_NPARAMS] * sizeof(float), st);
   const long n = tb.off[MRNB_ROUTER_NPARAMS];
-  LAUNCH_EW(repack_arena_kernel, n, params, pw.Pp, tb, I, T, Tp, n, 1);
-  const long total4 = (long)B * I * Tp * D / 4;
-  LAUNCH_EW(pad_frames_kernel, total4, x, pw.xp, T, Tp, total4, 1);
+  LAUNCH_EW(repack_arena_kernel, n, params, r.pw.Pp, tb, d.I, d.Tv, d.T, n, 1);
+  const long total4 = d.M * d.D / 4;
+  LAUNCH_EW(pad_frames_kernel, total4, x, r.pw.xp, d.Tv, d.T, total4, 1);
+  return MRNB_OK;
+}
+
+// padded [B*I, Tp, D] activations -> the caller's [B*I, T, D]
+int unpad_frames(const RouterRun& r, const float* src, float* dst, cudaStream_t st) {
+  MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
+  const long total4 = r.d.M * r.d.D / 4;
+  LAUNCH_EW(pad_frames_kernel, total4, src, dst, r.d.Tv, r.d.T, total4, 0);
+  return MRNB_OK;
+}
+
+// padded gradient arena -> the caller's arena
+int unpad_grads(const RouterRun& r, float* grads, cudaStream_t st) {
+  MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
+  const RepackTable tb = make_table(r.d.I, r.d.Tv, r.d.T, r.d.D);
+  const long n = tb.off[MRNB_ROUTER_NPARAMS];
+  LAUNCH_EW(repack_arena_kernel, n, r.pw.Gp, grads, tb, r.d.I, r.d.Tv, r.d.T, n, 0);
   return MRNB_OK;
 }
 
 }  // namespace
 
 extern "C" size_t mrnb_router_workspace_bytes(int B, int n_experts, int T, int D, int with_backward) {
-  const size_t plain = carve(nullptr, B, n_experts, T, D, with_backward != 0).bytes;
-  if (T == padded_T(MRNB_PREC_BF16, T)) return plain;
-  const int Tp = padded_T(MRNB_PREC_BF16, T);
-  const size_t inner = carve(nullptr, B, n_experts, Tp, D, true).bytes;   // the padded tail always sits behind the full carve
-  const size_t padded = carve_pad(nullptr, inner, B, n_experts, Tp, D).bytes;
-  return plain > padded ? plain : padded;
+  // enough for either precision: the fp32 engine never pads the frames, the tensor-core engine may
+  const size_t f32 = RouterRun(nullptr, B, n_experts, T, D, MRNB_PREC_FP32, with_backward != 0).bytes;
+  const size_t b16 = RouterRun(nullptr, B, n_experts, T, D, MRNB_PREC_BF16, with_backward != 0).bytes;
+  return f32 > b16 ? f32 : b16;
 }
 
 extern "C" int mrnb_router_forward(const float* params, const float* x, int B, int n_experts, int T, int D, int prec,
                                    float* out, float* scores, float* gate, int* index, void* workspace,
                                    size_t workspace_bytes, cudaStream_t stream) {
   ROUTER_ARGCHECK("router_forward");
-  const int Tp = padded_T(prec, T);
-  RouterWs w = carve((char*)workspace, B, n_experts, Tp, D, false);
-  if (Tp == T) {
-    MRNB_CHECK_ARG(workspace_bytes >= w.bytes, "router_forward: workspace too small (%zu < %zu)", workspace_bytes, w.bytes);
-    Dims d(B, n_experts, T, D, use_tc(prec, T));
-    return router_forward(params, x, d, out, scores, gate, index, w, stream);
-  }
-  // padded tensor-core mode (the padded tail sits behind the backward-sized carve so forward and backward agree)
-  const size_t inner = carve(nullptr, B, n_experts, Tp, D, true).bytes;
-  PadWs pw = carve_pad((char*)workspace, inner, B, n_experts, Tp, D);
-  MRNB_CHECK_ARG(workspace_bytes >= pw.bytes, "router_forward: workspace too small (%zu < %zu)", workspace_bytes, pw.bytes);
-  MRNB_TRY(pad_inputs(params, x, B, n_experts, T, Tp, D, pw, stream));
-  Dims d(B, n_experts, Tp, D, true, T);
-  MRNB_TRY(router_forward(pw.Pp, pw.xp, d, nullptr, scores, gate, index, w, stream));
-  if (out) {
-    MrnbProfScope prof(MRNB_PROF_ROUTER_EW, stream);
-    cudaStream_t st = stream;
-    const long total4 = (long)B * n_experts * Tp * D / 4;
-    LAUNCH_EW(pad_frames_kernel, total4, w.out, out, T, Tp, total4, 0);
-  }
-  return MRNB_OK;
+  RouterRun r(workspace, B, n_experts, T, D, prec, false);
+  MRNB_CHECK_ARG(workspace_bytes >= r.bytes, "router_forward: workspace too small (%zu < %zu)", workspace_bytes, r.bytes);
+  if (!r.padded) return router_forward(params, x, r.d, out, scores, gate, index, r.w, stream);
+  MRNB_TRY(pad_inputs(params, x, r, stream));
+  MRNB_TRY(router_forward(r.pw.Pp, r.pw.xp, r.d, nullptr, scores, gate, index, r.w, stream));
+  return out ? unpad_frames(r, r.w.out, out, stream) : MRNB_OK;
 }
 
 extern "C" int mrnb_router_backward(const float* params, const float* x, const float* gate, const float* dgate_ctc,
@@ -1530,59 +1530,28 @@ extern "C" int mrnb_router_backward(const float* params, const float* x, const f
                                     float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   ROUTER_ARGCHECK("router_backward");
   MRNB_CHECK_ARG(gate && domain && grads && taski_loss, "router_backward: null argument");
-  const int Tu = T;                                  // caller's frame count
-  const int Tp = padded_T(prec, T);
-  const bool padded = Tp != T;
-  RouterWs w = carve((char*)workspace, B, n_experts, Tp, D, true);
-  PadWs pw{};
-  if (padded) {
-    pw = carve_pad((char*)workspace, w.bytes, B, n_experts, Tp, D);
-    MRNB_CHECK_ARG(workspace_bytes >= pw.bytes, "router_backward: workspace too small (%zu < %zu)", workspace_bytes, pw.bytes);
-    params = pw.Pp; x = pw.xp;                       // written by mrnb_router_forward on the same workspace
-  } else {
-    MRNB_CHECK_ARG(workspace_bytes >= w.bytes, "router_backward: workspace too small (%zu < %zu)", workspace_bytes, w.bytes);
-  }
-  float* user_grads = grads;
-  if (padded) grads = pw.Gp;
-  T = Tp;
-  const int I = n_experts;
+  RouterRun r(workspace, B, n_experts, T, D, prec, true);
+  MRNB_CHECK_ARG(workspace_bytes >= r.bytes, "router_backward: workspace too small (%zu < %zu)", workspace_bytes, r.bytes);
+  if (r.padded) { params = r.pw.Pp; x = r.pw.xp; }   // written by mrnb_router_forward on the same workspace
+  float* G = r.padded ? r.pw.Gp : grads;
+  const Dims& d = r.d;
+  RouterWs& w = r.w;
   cudaStream_t st = stream;
-  Dims d(B, I, T, D, use_tc(prec, Tu), Tu);
   long off[MRNB_ROUTER_NPARAMS + 1];
-  const long nparam = router_offsets(I, T, D, off);
-  const long ID = d.ID, TD = d.TD, ITD = d.ITD;
-  cudaMemsetAsync(grads, 0, nparam * sizeof(float), st);
+  const long nparam = router_offsets(d.I, d.T, d.D, off);
+  cudaMemsetAsync(G, 0, nparam * sizeof(float), st);
   cudaMemsetAsync(taski_loss, 0, sizeof(float), st);
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    gate_bwd_kernel<<<cdiv(B, 256), 256, 0, st>>>(gate, dgate_ctc, domain, B, I, w.dr, taski_loss);
+    gate_bwd_kernel<<<cdiv(B, 256), 256, 0, st>>>(gate, dgate_ctc, domain, B, d.I, w.dr, taski_loss);
     MRNB_CHECK_LAUNCH("gate_bwd_kernel");
-    route_bwd_kernel<<<T, 256, 0, st>>>(w.dr, w.s, params + off[R_ROUTE_W], B, T, I, w.ds, grads + off[R_ROUTE_W],
-                                        grads + off[R_ROUTE_B]);
+    route_bwd_kernel<<<d.T, 256, 0, st>>>(w.dr, w.s, params + off[R_ROUTE_W], B, d.T, d.I, w.ds, G + off[R_ROUTE_W],
+                                          G + off[R_ROUTE_B]);
     MRNB_CHECK_LAUNCH("route_bwd_kernel");
   }
-  if (d.tc) {
-    MRNB_TRY(router_backward_gate_tc(params, x, d, grads, w, st));
-  } else {
-    {  // dWcr[j,(i,c)] = sum_(b,t) ds[(b,t),j] out[b,i,t,c]
-      MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-      MRNB_DISPATCH_I(launch_gate_head_dw, I, w.ds, w.out, B, T, grads + off[R_CR_W], st);
-    }
-    MRNB_TRY(colsum(w.ds, mrnb_axis(I), mrnb_axis(1), B * T, I, grads + off[R_CR_B], st));
-    {  // dout[b,i,t,c] = sum_j ds[(b,t),j] Wcr[j,(i,c)]
-      MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-      const long total4 = d.M * D / 4;
-      LAUNCH_EW(dout_kernel, total4, w.ds, params + off[R_CR_W], I, T, total4, w.dout, nullptr);
-    }
-    MRNB_TRY(dm_router_backward_core(params, x, d, grads, nullptr, w, st));
-  }
-  if (padded) {
-    MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const RepackTable tb = make_table(I, Tu, Tp, D);
-    const long n = tb.off[MRNB_ROUTER_NPARAMS];
-    LAUNCH_EW(repack_arena_kernel, n, pw.Gp, user_grads, tb, I, Tu, Tp, n, 0);
-  }
-  return MRNB_OK;
+  if (d.tc) MRNB_TRY(router_backward_gate_tc(params, x, d, G, w, st));
+  else MRNB_TRY(router_backward_gate_f32(params, x, d, G, w, st));
+  return r.padded ? unpad_grads(r, grads, st) : MRNB_OK;
 }
 
 extern "C" int mrnb_dm_router_backward(const float* params, const float* x, const float* d_out, int B, int n_experts,
@@ -1590,40 +1559,27 @@ extern "C" int mrnb_dm_router_backward(const float* params, const float* x, cons
                                        size_t workspace_bytes, cudaStream_t stream) {
   ROUTER_ARGCHECK("dm_router_backward");
   MRNB_CHECK_ARG(d_out && grads, "dm_router_backward: null argument");
-  const int Tp = padded_T(prec, T);
-  const bool padded = Tp != T;
-  RouterWs w = carve((char*)workspace, B, n_experts, Tp, D, true);
+  RouterRun r(workspace, B, n_experts, T, D, prec, true);
+  MRNB_CHECK_ARG(workspace_bytes >= r.bytes, "dm_router_backward: workspace too small (%zu < %zu)", workspace_bytes, r.bytes);
+  const Dims& d = r.d;
+  RouterWs& w = r.w;
   cudaStream_t st = stream;
-  if (!padded) {
-    MRNB_CHECK_ARG(workspace_bytes >= w.bytes, "dm_router_backward: workspace too small");
-    Dims d(B, n_experts, T, D, use_tc(prec, T));
-    long off[MRNB_ROUTER_NPARAMS + 1];
-    const long nparam = router_offsets(n_experts, T, D, off);
-    cudaMemsetAsync(grads, 0, nparam * sizeof(float), st);
+  long off[MRNB_ROUTER_NPARAMS + 1];
+  const long nparam = router_offsets(d.I, d.T, d.D, off);
+  cudaMemsetAsync(r.padded ? r.pw.Gp : grads, 0, nparam * sizeof(float), st);
+  if (!r.padded) {
     cudaMemcpyAsync(w.dout, d_out, (size_t)d.M * D * sizeof(float), cudaMemcpyDeviceToDevice, st);
     if (d.tc) LAUNCH_EW(cast16_kernel, d.M * D, d_out, w.dout16, d.M * D);
     return dm_router_backward_core(params, x, d, grads, dx, w, st);
   }
-  PadWs pw = carve_pad((char*)workspace, w.bytes, B, n_experts, Tp, D);
-  MRNB_CHECK_ARG(workspace_bytes >= pw.bytes, "dm_router_backward: workspace too small");
-  Dims d(B, n_experts, Tp, D, true, T);
-  long offp[MRNB_ROUTER_NPARAMS + 1];
-  const long np = router_offsets(n_experts, Tp, D, offp);
-  cudaMemsetAsync(pw.Gp, 0, np * sizeof(float), st);
-  const long total4 = d.M * D / 4;
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    LAUNCH_EW(pad_frames_kernel, total4, d_out, w.dout, T, Tp, total4, 1);
+    const long total4 = d.M * D / 4;
+    LAUNCH_EW(pad_frames_kernel, total4, d_out, w.dout, T, d.T, total4, 1);
     LAUNCH_EW(cast16_kernel, d.M * D, w.dout, w.dout16, d.M * D);
   }
   float* dxp = dx ? w.dg2 : nullptr;        // padded dx: dg2 is dead by the time the core's last kernel writes dx
-  MRNB_TRY(dm_router_backward_core(pw.Pp, pw.xp, d, pw.Gp, dxp, w, st));
-  {
-    MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
-    const RepackTable tb = make_table(n_experts, T, Tp, D);
-    const long n = tb.off[MRNB_ROUTER_NPARAMS];
-    LAUNCH_EW(repack_arena_kernel, n, pw.Gp, grads, tb, n_experts, T, Tp, n, 0);
-    if (dx) LAUNCH_EW(pad_frames_kernel, total4, dxp, dx, T, Tp, total4, 0);
-  }
-  return MRNB_OK;
+  MRNB_TRY(dm_router_backward_core(r.pw.Pp, r.pw.xp, d, r.pw.Gp, dxp, w, st));
+  MRNB_TRY(unpad_grads(r, grads, st));
+  return dx ? unpad_frames(r, dxp, dx, st) : MRNB_OK;
 }
