@@ -22,7 +22,7 @@ import torch
 
 from .. import dist as mdist
 from .. import ops
-from ..modules.model import MRNNet, _arch, _precision, sample_drop_scales
+from ..modules.model import MRNNet, _arch, _expert_bns, _precision, _train_forward_ran, sample_drop_scales
 from ..utils import Averager, CTCLabelConverter, DevicePrefetcher
 
 
@@ -52,6 +52,26 @@ def _domain_ids(indexs):
     if isinstance(indexs, (list, tuple)) and indexs and isinstance(indexs[0], torch.Tensor):
         return torch.cat([t.reshape(-1) for t in indexs]).to(torch.long).cpu()
     return torch.as_tensor(indexs, dtype=torch.long).reshape(-1).cpu()
+
+
+def _capture(fn, inputs):
+    """CUDA graph of fn(*static), `static` being clones of `inputs`.  Returns the graph-cache entry (graph, static,
+    out); `out` is what fn returned, device tensors that every replay overwrites."""
+    static = tuple(t.clone() for t in inputs)
+    torch.cuda.synchronize()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        out = fn(*static)
+    return graph, static, out
+
+
+def _replay(entry, inputs):
+    """Copies `inputs` into the static inputs of a _capture entry, replays its graph and returns its outputs."""
+    graph, static, out = entry
+    for dst, src in zip(static, inputs):
+        dst.copy_(src, non_blocking=True)
+    graph.replay()
+    return out
 
 
 def edit_distance(a, b):
@@ -302,14 +322,8 @@ class MRN(object):
             own = dict(expert.named_parameters())
             for key, t in tp.state().items():
                 own[key].copy_(t)                       # bumps the version counter -> inference packs are rebuilt
-            cn = expert.model.FeatureExtraction.ConvNet
-            if getattr(tp, "arch", "svtr") == "crnn":
-                pairs = ((cn[12], tp.bn_stats[(0, "mean")], tp.bn_stats[(0, "var")]),
-                         (cn[15], tp.bn_stats[(1, "mean")], tp.bn_stats[(1, "var")]))
-            else:
-                pairs = ((cn.patch_embed.proj[1], tp.bn_stats[ops.L.P_BN0_MEAN], tp.bn_stats[ops.L.P_BN0_VAR]),
-                         (cn.patch_embed.proj[4], tp.bn_stats[ops.L.P_BN1_MEAN], tp.bn_stats[ops.L.P_BN1_VAR]))
-            for bn, mean, var in pairs:
+            m0, v0, m1, v1 = tp.bn_running_stats()
+            for bn, mean, var in zip(_expert_bns(expert, tp.arch), (m0, m1), (v0, v1)):
                 bn.running_mean.copy_(mean.reshape(-1))
                 bn.running_var.copy_(var.reshape(-1))
                 bn.num_batches_tracked += self._tp_steps
@@ -324,7 +338,7 @@ class MRN(object):
         expert = self.net.model[-1]
         train_mode = bool(expert.training)
         B = image.shape[0]
-        crnn = getattr(tp, "arch", "svtr") == "crnn"
+        crnn = tp.arch == "crnn"
         if not crnn and train_mode and drop_scales is None and getattr(self.opt, "drop_path", True):
             rates = expert.model.FeatureExtraction.ConvNet.drop_path_rates()
             drop_scales = sample_drop_scales(1, B, rates, image.device)[0].contiguous()
@@ -370,16 +384,8 @@ class MRN(object):
             cache[key] = "warm"
             return self.train_step_stage0(image, labels_index, labels_length)
         if ent == "warm":
-            st_in = tuple(t.clone() for t in (image, labels_index, labels_length))
-            torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                loss = self._stage0_device(*st_in)
-            ent = cache[key] = (graph, st_in, loss)
-        graph, st_in, loss = ent
-        for dst, src in zip(st_in, (image, labels_index, labels_length)):
-            dst.copy_(src, non_blocking=True)
-        graph.replay()
+            ent = cache[key] = _capture(self._stage0_device, (image, labels_index, labels_length))
+        loss = _replay(ent, (image, labels_index, labels_length))
         mdist.allreduce_mean_(self._tp.grads)
         self.optimizer.step()
         if key[3]:
@@ -436,22 +442,28 @@ class MRN(object):
             p.requires_grad = False
         self.net.model[-1].eval()
 
-    def train_step_stage1(self, image, labels_index, labels_length, indexs, drop_scales=None):
-        """One router-training iteration (il_modules/mrn.py:338-371) entirely on the device.
-        image [B,4,32,256] fp32, labels_index [B,25] int64 (pad 1), labels_length [B] int32, indexs [B] int64.
-        Returns (loss_clf, taski_loss) as 1-element device tensors."""
+    def _stage1_device(self, image, labels_index, labels_length, indexs, drop_scales=None):
+        """Experts, router forward, fused combine + CTC, analytic gate gradient and router backward into the router's
+        gradient arena.  Pure device work on the current stream (capturable in a CUDA graph).  Returns (loss_clf,
+        taski_loss) as 1-element tensors."""
         net = self.net
         B = image.shape[0]
         r = net.route_and_combine(image, is_train=True, want_logits=False, targets=labels_index, lengths=labels_length,
                                   want_E=True, with_backward=True, drop_scales=drop_scales)
         c = ops.ctc_lattice(r["lpe"], labels_index, labels_length, r["zlab"], r["E"], grad_scale=float(self.pi) / B,
                             want_dgate=True)
-        grads = net.router_grad_arena()
-        taski_loss = ops.router_backward(net.router_arena(), r["features"], r["gate"], c["dgate"], indexs, grads, net._rws,
-                                         prec=_precision(net.opt))
-        mdist.allreduce_mean_(grads)                     # the ONE exchange step (replaces nn.DataParallel)
-        self.optimizer.step()                            # clip_grad_norm_(5) + Adam + OneCycle
+        taski_loss = ops.router_backward(net.router_arena(), r["features"], r["gate"], c["dgate"], indexs,
+                                         net.router_grad_arena(), net._rws, prec=_precision(net.opt))
         return c["loss"], taski_loss
+
+    def train_step_stage1(self, image, labels_index, labels_length, indexs, drop_scales=None):
+        """One router-training iteration (il_modules/mrn.py:338-371) entirely on the device.
+        image [B,4,32,256] fp32, labels_index [B,25] int64 (pad 1), labels_length [B] int32, indexs [B] int64.
+        Returns (loss_clf, taski_loss) as 1-element device tensors."""
+        loss, taski_loss = self._stage1_device(image, labels_index, labels_length, indexs, drop_scales)
+        mdist.allreduce_mean_(self.net.router_grad_arena())     # the ONE exchange step (replaces nn.DataParallel)
+        self.optimizer.step()                            # clip_grad_norm_(5) + Adam + OneCycle
+        return loss, taski_loss
 
     def train_step_stage1_graphed(self, image, labels_index, labels_length, indexs):
         """train_step_stage1 with the device work up to the router gradients (experts, router forward, combine + CTC,
@@ -460,33 +472,18 @@ class MRN(object):
         for a batch size runs eagerly (lazy allocations, attribute setup), the second captures, later ones replay.
         Steady-state loop only: re-capture (`reset_graphs()`) after the experts' weights or train / eval mode change."""
         net = self.net
-        B = int(image.shape[0])
+        modes = net._experts_train_mode()
         cache = self.__dict__.setdefault("_train_graphs", {})
-        key = (B, str(image.device), net._experts_train_mode())
+        key = (int(image.shape[0]), str(image.device), modes)
         ent = cache.get(key)
         if ent is None:
             cache[key] = "warm"
             return self.train_step_stage1(image, labels_index, labels_length, indexs)
         if ent == "warm":
-            st_in = tuple(t.clone() for t in (image, labels_index, labels_length, indexs))
-            torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                r = net.route_and_combine(st_in[0], is_train=True, want_logits=False, targets=st_in[1], lengths=st_in[2],
-                                          want_E=True, with_backward=True)
-                c = ops.ctc_lattice(r["lpe"], st_in[1], st_in[2], r["zlab"], r["E"], grad_scale=float(self.pi) / B,
-                                    want_dgate=True)
-                taski_loss = ops.router_backward(net.router_arena(), r["features"], r["gate"], c["dgate"], st_in[3],
-                                                 net.router_grad_arena(), net._rws, prec=_precision(net.opt))
-            ent = cache[key] = (graph, st_in, c["loss"], taski_loss)
-        graph, st_in, loss, taski_loss = ent
-        for dst, src in zip(st_in, (image, labels_index, labels_length, indexs)):
-            dst.copy_(src, non_blocking=True)
-        graph.replay()
-        if any(key[2]) and net._cache.pack is not None:
-            net._cache.pack.bn_dirty = True              # train-mode experts updated their BN running statistics
-            from ..modules.model import _count_bn_steps
-            _count_bn_steps(net._cache.pack, key[2])
+            ent = cache[key] = _capture(self._stage1_device, (image, labels_index, labels_length, indexs))
+        loss, taski_loss = _replay(ent, (image, labels_index, labels_length, indexs))
+        if any(modes) and net._cache.pack is not None:
+            _train_forward_ran(net._cache, list(net.model), modes)
         mdist.allreduce_mean_(net.router_grad_arena())
         self.optimizer.step()
         return loss, taski_loss
@@ -573,22 +570,14 @@ class MRN(object):
         cache = self.__dict__.setdefault("_infer_graphs", {})
         ent = cache.get(key)
         if ent is None:
-            static_in = image.clone()
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):             # warm-up on a side stream: lazy allocations, attribute setup, packs
                 for _ in range(2):
-                    self.infer_batch(static_in, val_choose, **dec)
+                    self.infer_batch(image, val_choose, **dec)
             torch.cuda.current_stream().wait_stream(side)
-            torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                out = self.infer_batch(static_in, val_choose, **dec)
-            ent = cache[key] = (graph, static_in, out)
-        graph, static_in, out = ent
-        static_in.copy_(image, non_blocking=True)
-        graph.replay()
-        return out
+            ent = cache[key] = _capture(lambda x: self.infer_batch(x, val_choose, **dec), (image,))
+        return _replay(ent, (image,))
 
     def validation(self, eval_loader, val_choose="TF"):
         """test.py:139-279 with the decode / confidence on the device.  opt.decode ("greedy", the default, or "beam"),

@@ -174,10 +174,7 @@ def _experts_forward(experts, image, opt, train_mode, cache=None, drop_scales=No
         feats, logits = ops.crnn_experts_forward(pack, image.contiguous().float(), bn_batch_stats=mask,
                                                  update_running=mask, want_logits=want_logits)
         if train_mode:
-            pack.bn_dirty = True
-            _count_bn_steps(pack, modes)
-            if cache is _solo_cache:
-                _writeback_bn(experts, pack)
+            _train_forward_ran(cache, experts, modes)
         return feats, logits
     if chunk is None:
         chunk = int(getattr(opt, "expert_chunk", 0) or 0)
@@ -192,11 +189,18 @@ def _experts_forward(experts, image, opt, train_mode, cache=None, drop_scales=No
                                              update_running=mask, drop_scales=drop_scales, chunk=chunk,
                                              want_logits=want_logits)
     if train_mode:
-        pack.bn_dirty = True
-        _count_bn_steps(pack, modes)
-        if cache is _solo_cache:
-            _writeback_bn(experts, pack)
+        _train_forward_ran(cache, experts, modes)
     return feats, logits
+
+
+def _train_forward_ran(cache, experts, modes):
+    """Bookkeeping after an expert forward (eager or replayed from a CUDA graph) in which the experts flagged in
+    `modes` were in .train(): their BN running statistics changed inside cache.pack.  The solo cache (single-expert
+    forwards) belongs to no MRNNet whose state_dict() would sync it, so its experts' buffers are written back at once."""
+    cache.pack.bn_dirty = True
+    _count_bn_steps(cache.pack, modes)
+    if cache is _solo_cache:
+        _writeback_bn(experts, cache.pack)
 
 
 _RATES_CACHE = {}
@@ -213,14 +217,19 @@ def sample_drop_scales(n_experts, B, rates, device, generator=None):
     return (keep / (1.0 - rates_t)).contiguous()
 
 
+def _expert_bns(expert, arch):
+    """The expert's two BatchNorm2d modules: VGG's after conv4 and conv5 (crnn), the patch embedding's two (svtr)."""
+    cn = expert.model.FeatureExtraction.ConvNet
+    return (cn[12], cn[15]) if arch == "crnn" else (cn.patch_embed.proj[1], cn.patch_embed.proj[4])
+
+
 def _writeback_bn(experts, pack):
     """Train-mode forwards update BN running statistics inside the pack; mirror them into the module buffers so
     state_dict() / checkpoints see what nn.BatchNorm2d in .train() would have produced (reference quirk 4)."""
     m0, v0, m1, v1 = pack.bn_running_stats()
     with torch.no_grad():
         for i, m in enumerate(experts):
-            cn = m.model.FeatureExtraction.ConvNet
-            bns = (cn[12], cn[15]) if pack.arch == "crnn" else (cn.patch_embed.proj[1], cn.patch_embed.proj[4])
+            bns = _expert_bns(m, pack.arch)
             steps = getattr(pack, "bn_steps", None)
             n_fwd = steps[i] if steps is not None else 1     # train-mode forwards of this expert since the last write-back
             if n_fwd == 0:

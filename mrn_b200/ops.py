@@ -6,6 +6,7 @@ libmrn_b200.so.  All wrappers require CUDA tensors and raise otherwise -- there 
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Dict, List, Optional, Sequence
 
 import torch
@@ -218,6 +219,14 @@ def round_up(v, a):
     return (v + a - 1) // a * a
 
 
+def _grow_workspace(pack, need):
+    """pack._ws, reallocated only when it holds fewer than `need` bytes: later calls (and CUDA-graph replays) keep
+    using the same buffer."""
+    if pack._ws is None or pack._ws.numel() < need:
+        pack._ws = torch.empty(need, dtype=torch.uint8, device=pack.device)
+    return pack._ws
+
+
 class SvtrPack:
     """Device-resident, expert-stacked copy of the SVTR expert parameters in the layout the kernels consume
     (include/mrn_b200.h: MRNB_P_* slots).  Built from a reference-format state_dict; rebuilt when experts change
@@ -320,13 +329,12 @@ class SvtrPack:
         return tuple(self.slot_tensors[s] for s in (L.P_BN0_MEAN, L.P_BN0_VAR, L.P_BN1_MEAN, L.P_BN1_VAR))
 
     def workspace(self, B, chunk):
-        need = int(L.load().mrnb_svtr_workspace_bytes(self.n_experts, B, chunk, self.prec))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self._ws
+        return _grow_workspace(self, int(L.load().mrnb_svtr_workspace_bytes(self.n_experts, B, chunk, self.prec)))
 
 
-def _logit_buffers(pack, B, device, want, T=T_FRAMES):
+def _logit_buffers(pack, B, device, want):
+    """Per-expert logit buffers [B, pack.n_frames, C_i rounded up to 4] for the grouped heads.  Returns (ptrs, lds,
+    [logits_i [B,T,C_i] views]); with want=False the pointers are NULL (no logits written) and the views None."""
     I = pack.n_experts
     ptrs = (C.c_void_p * I)()
     lds = (C.c_long * I)()
@@ -335,7 +343,7 @@ def _logit_buffers(pack, B, device, want, T=T_FRAMES):
         ld = round_up(pack.n_class[i], 4)
         lds[i] = ld
         if want:
-            buf = torch.empty(B, T, ld, device=device, dtype=torch.float32)
+            buf = torch.empty(B, pack.n_frames, ld, device=device, dtype=torch.float32)
             ptrs[i] = buf.data_ptr()
             logits.append(buf[:, :, :pack.n_class[i]])
         else:
@@ -360,26 +368,12 @@ def svtr_heads(pack: SvtrPack, B: int, route_index: Optional[torch.Tensor] = Non
 
 
 def svtr_experts_forward(pack: SvtrPack, image: torch.Tensor, bn_batch_stats: bool = False, update_running: bool = False,
-                         drop_scales: Optional[torch.Tensor] = None, chunk: int = 0, want_logits: bool = True,
-                         experts_with_logits: Optional[Sequence[int]] = None):
+                         drop_scales: Optional[torch.Tensor] = None, chunk: int = 0, want_logits: bool = True):
     """Runs every expert on `image` [B,4,32,256].  Returns (features [B,I,64,256], [logits_i [B,64,C_i] views])."""
     _chk_f32(image, drop_scales)
     B = image.shape[0]
-    I = pack.n_experts
-    feats = torch.empty(B, I, T_FRAMES, D_FEAT, device=image.device, dtype=torch.float32)
-    ptrs = (C.c_void_p * I)()
-    lds = (C.c_long * I)()
-    logits = []
-    for i in range(I):
-        ld = round_up(pack.n_class[i], 4)
-        lds[i] = ld
-        if want_logits and (experts_with_logits is None or i in experts_with_logits):
-            buf = torch.empty(B, T_FRAMES, ld, device=image.device, dtype=torch.float32)
-            ptrs[i] = buf.data_ptr()
-            logits.append(buf[:, :, :pack.n_class[i]])
-        else:
-            ptrs[i] = None
-            logits.append(None)
+    feats = torch.empty(B, pack.n_experts, T_FRAMES, D_FEAT, device=image.device, dtype=torch.float32)
+    ptrs, lds, logits = _logit_buffers(pack, B, image.device, want_logits)
     ws = pack.workspace(B, chunk)
     pack._ws_key = (B, int(chunk) if 0 < int(chunk) < B else 0)
     rc = L.load().mrnb_svtr_experts_forward(C.byref(pack.struct), _p(image), B, int(chunk), pack.prec, _mask(bn_batch_stats),
@@ -391,7 +385,7 @@ def svtr_experts_forward(pack: SvtrPack, image: torch.Tensor, bn_batch_stats: bo
 
 # ------------------------------------------------------------------------------------------------ stage-0 expert training
 def _train_slots():
-    """[(slot, key relative to the expert's Model, permute)] for every trainable SVTR slot, in arena order."""
+    """The SVTR arena's slot table: every trainable MrnbSvtrPack slot, then the classifier head ("fc_w", "fc_b")."""
     cn = "model.FeatureExtraction.ConvNet."
     out = [(L.P_POS_EMBED, cn + "pos_embed", None), (L.P_CONV0_W, cn + "patch_embed.proj.0.weight", None),
            (L.P_CONV0_B, cn + "patch_embed.proj.0.bias", None), (L.P_BN0_W, cn + "patch_embed.proj.1.weight", None),
@@ -407,76 +401,61 @@ def _train_slots():
                 (base + L.PS_CONV_B, f"{cn}sub_sample{s_ + 1}.conv.bias", None),
                 (base + L.PS_NORM_W, f"{cn}sub_sample{s_ + 1}.norm.weight", None),
                 (base + L.PS_NORM_B, f"{cn}sub_sample{s_ + 1}.norm.bias", None)]
-    out += [(L.P_SEQ_W, "model.SequenceModeling.0.weight", None), (L.P_SEQ_B, "model.SequenceModeling.0.bias", None)]
-    return out
+    out += [(L.P_SEQ_W, "model.SequenceModeling.0.weight", None), (L.P_SEQ_B, "model.SequenceModeling.0.bias", None),
+            ("fc_w", "fc.weight", None), ("fc_b", "fc.bias", None)]
+    return [(slot, [(key, perm)]) for slot, key, perm in out]
 
 
 _BN_STAT_SLOTS = ((L.P_BN0_MEAN, "patch_embed.proj.1.running_mean"), (L.P_BN0_VAR, "patch_embed.proj.1.running_var"),
                   (L.P_BN1_MEAN, "patch_embed.proj.4.running_mean"), (L.P_BN1_VAR, "patch_embed.proj.4.running_var"))
 
 
-class SvtrTrainPack:
-    """ONE expert's trainable parameters in a single flat fp32 arena laid out in MrnbSvtrPack slots (n_experts = 1;
-    conv weights as [Cout,kh,kw,Cin]), a gradient arena with the same layout, and the BatchNorm running statistics.
-    The arena is what mrnb_clip_adam updates and what the data-parallel all-reduce averages (stage 0,
-    il_modules/mrn.py:225-279).  `entries` maps each arena slice back to its state_dict key."""
+class _TrainPack:
+    """ONE expert's trainable parameters in a single flat fp32 arena, a gradient arena with the same layout, in bf16
+    mode a bf16 shadow of the arena at the same element offsets (refreshed before every forward), and the expert's
+    BatchNorm running statistics.  The arena is what mrnb_clip_adam updates and what the data-parallel all-reduce
+    averages (stage 0, il_modules/mrn.py:225-279).  `entries` maps each arena slice back to its state_dict key.
 
-    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32):
+    A subclass passes its slot table [(slot, [(key, permute), ...])] in arena order (the parts of a slot adjacent, each
+    slot padded to 8 floats), names its C struct (_Struct) and puts a slot's pointers into it (_point)."""
+
+    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec, slots):
         self.device = torch.device(device)
         self.prec = prec
-        slots = _train_slots() + [("fc_w", "fc.weight", None), ("fc_b", "fc.bias", None)]
         self.entries = []                         # (slot, key, permute, offset, kernel-layout shape)
+        self.slot_offset = {}
         off = 0
-        for slot, key, perm in slots:
-            shp = tuple(expert_sd[key].shape)
-            if perm is not None:
-                shp = tuple(shp[a] for a in perm)
-            self.entries.append((slot, key, perm, off, shp))
-            n = 1
-            for v in shp:
-                n *= v
-            off += round_up(n, 8)
+        for slot, parts in slots:
+            self.slot_offset[slot] = off
+            for key, perm in parts:
+                shp = tuple(expert_sd[key].shape)
+                if perm is not None:
+                    shp = tuple(shp[a] for a in perm)
+                self.entries.append((slot, key, perm, off, shp))
+                n = math.prod(shp)
+                assert n % 8 == 0 or len(parts) == 1, key
+                off += n
+            off = round_up(off, 8)
         self.numel = off
         self.params = torch.zeros(off, device=self.device, dtype=torch.float32)
         self.grads = torch.zeros(off, device=self.device, dtype=torch.float32)
-        cn = "model.FeatureExtraction.ConvNet."
-        self.bn_stats = {slot: expert_sd[cn + key].detach().to(self.device, torch.float32).clone().contiguous()
-                         for slot, key in _BN_STAT_SLOTS}
+        self.shadow16 = torch.zeros(off, device=self.device, dtype=torch.bfloat16) if prec == L.PREC_BF16 else None
         self.n_class = int(expert_sd["fc.weight"].shape[0])
-        self.struct = L.MrnbSvtrPack()
-        self.gstruct = L.MrnbSvtrPack()
-        for st_, arena in ((self.struct, self.params), (self.gstruct, self.grads)):
-            st_.n_experts = 1
-            st_.n_class[0] = self.n_class
-            for slot, key, perm, o, shp in self.entries:
-                ptr = arena.data_ptr() + 4 * o
-                if slot == "fc_w":
-                    st_.fc_w[0] = ptr
-                elif slot == "fc_b":
-                    st_.fc_b[0] = ptr
-                else:
-                    st_.p[slot] = ptr
-        for slot, t in self.bn_stats.items():
-            self.struct.p[slot] = t.data_ptr()
-        self.shadow16: Optional[torch.Tensor] = None
-        if prec == L.PREC_BF16:
-            # bf16 copies of the GEMM weights at the same element offsets (refreshed after every optimiser step)
-            self.shadow16 = torch.zeros(off, device=self.device, dtype=torch.bfloat16)
-            for slot, key, perm, o, shp in self.entries:
-                ptr = self.shadow16.data_ptr() + 2 * o
-                if slot == "fc_w":
-                    self.struct.fc_w16[0] = ptr
-                elif slot != "fc_b":
-                    self.struct.h[slot] = ptr
+        self.struct = self._Struct()
+        self.gstruct = self._Struct()
+        for slot, o in self.slot_offset.items():
+            self._point(self.struct, slot, self.params.data_ptr() + 4 * o,
+                        None if self.shadow16 is None else self.shadow16.data_ptr() + 2 * o)
+            self._point(self.gstruct, slot, self.grads.data_ptr() + 4 * o, None)
         self.load_state(expert_sd)
         self._ws: Optional[torch.Tensor] = None
 
+    def _bn_stat(self, expert_sd, key):
+        return expert_sd["model.FeatureExtraction.ConvNet." + key].detach().to(self.device, torch.float32).clone().contiguous()
+
     def view(self, arena, entry):
         slot, key, perm, o, shp = entry
-        n = 1
-        for v in shp:
-            n *= v
-        return arena[o:o + n].view(shp)
+        return arena[o:o + math.prod(shp)].view(shp)
 
     def load_state(self, expert_sd):
         with torch.no_grad():
@@ -504,11 +483,38 @@ class SvtrTrainPack:
         if self.shadow16 is not None:
             L.check(L.load().mrnb_cast_f32_to_bf16(_p(self.params), _p(self.shadow16), self.numel, _stream()), "cast")
 
+
+class SvtrTrainPack(_TrainPack):
+    """An SVTR expert's training arena laid out in MrnbSvtrPack slots (n_experts = 1; conv weights as [Cout,kh,kw,Cin]);
+    the BatchNorm running statistics sit in their MrnbSvtrPack slots, keyed by slot in `bn_stats`."""
+
+    arch = "svtr"
+    _Struct = L.MrnbSvtrPack
+
+    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32):
+        super().__init__(expert_sd, device, prec, _train_slots())
+        for st_ in (self.struct, self.gstruct):
+            st_.n_experts = 1
+            st_.n_class[0] = self.n_class
+        self.bn_stats = {slot: self._bn_stat(expert_sd, key) for slot, key in _BN_STAT_SLOTS}
+        for slot, t in self.bn_stats.items():
+            self.struct.p[slot] = t.data_ptr()
+
+    def bn_running_stats(self):
+        """(mean0, var0, mean1, var1): updated in place by train-mode forwards."""
+        return tuple(self.bn_stats[s] for s in (L.P_BN0_MEAN, L.P_BN0_VAR, L.P_BN1_MEAN, L.P_BN1_VAR))
+
+    @staticmethod
+    def _point(st, slot, ptr, ptr16):
+        if slot == "fc_w":
+            st.fc_w[0], st.fc_w16[0] = ptr, ptr16
+        elif slot == "fc_b":
+            st.fc_b[0] = ptr                      # the bias has no bf16 copy
+        else:
+            st.p[slot], st.h[slot] = ptr, ptr16
+
     def workspace(self, B):
-        need = int(L.load().mrnb_svtr_train_workspace_bytes(B, self.n_class, self.prec))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self._ws
+        return _grow_workspace(self, int(L.load().mrnb_svtr_train_workspace_bytes(B, self.n_class, self.prec)))
 
 
 def svtr_train_forward(tp: SvtrTrainPack, image, bn_batch_stats=True, update_running=True, drop_scales=None):
@@ -537,17 +543,16 @@ def svtr_train_backward(tp: SvtrTrainPack, image, dlogits, bn_batch_stats=True, 
     return tp.grads
 
 
-class CrnnTrainPack:
-    """ONE CRNN expert's trainable parameters in a single flat fp32 arena (MrnbCrnnTrainPack slots: conv weights as
-    [Cout,kh,kw,Cin]; each LSTM tensor = forward direction then reverse direction), a gradient arena with the same
-    layout and the two BatchNorm running statistics.  `entries` maps arena slices back to state_dict keys."""
+class CrnnTrainPack(_TrainPack):
+    """A CRNN expert's training arena in MrnbCrnnTrainPack slots: conv weights as [Cout,kh,kw,Cin]; each LSTM tensor =
+    forward direction then reverse direction in one slot.  `bn_stats` holds the two BatchNorms' running statistics,
+    keyed (0 / 1, "mean" / "var")."""
 
     arch = "crnn"
     n_frames = 63
+    _Struct = L.MrnbCrnnTrainPack
 
     def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32):
-        self.device = torch.device(device)
-        self.prec = prec
         cn = "model.FeatureExtraction.ConvNet."
         hwc = (0, 2, 3, 1)
         slots = [(L.T_CONV0_W, [(cn + "0.weight", hwc)]), (L.T_CONV0_B, [(cn + "0.bias", None)]),
@@ -564,55 +569,27 @@ class CrnnTrainPack:
                 slots.append((base + sl, [(q + "rnn." + nm, None), (q + "rnn." + nm + "_reverse", None)]))
             slots += [(base + L.TL_LIN_W, [(q + "linear.weight", None)]), (base + L.TL_LIN_B, [(q + "linear.bias", None)])]
         slots += [(L.T_FC_W, [("fc.weight", None)]), (L.T_FC_B, [("fc.bias", None)])]
-        self.entries = []                         # (slot, key, permute, offset, kernel-layout shape)
-        self.slot_offset = {}
-        off = 0
-        for slot, parts in slots:
-            self.slot_offset[slot] = off
-            for key, perm in parts:
-                shp = tuple(expert_sd[key].shape)
-                if perm is not None:
-                    shp = tuple(shp[a] for a in perm)
-                self.entries.append((slot, key, perm, off, shp))
-                n = 1
-                for v in shp:
-                    n *= v
-                assert n % 8 == 0 or len(parts) == 1, key
-                off += n
-            off = round_up(off, 8)
-        self.numel = off
-        self.params = torch.zeros(off, device=self.device, dtype=torch.float32)
-        self.grads = torch.zeros(off, device=self.device, dtype=torch.float32)
-        self.shadow16 = torch.zeros(off, device=self.device, dtype=torch.bfloat16) if prec == L.PREC_BF16 else None
+        super().__init__(expert_sd, device, prec, slots)
         self.bn_stats = {}
         for q, idx in enumerate((12, 15)):
-            self.bn_stats[(q, "mean")] = expert_sd[cn + f"{idx}.running_mean"].detach().to(self.device, torch.float32).clone().contiguous()
-            self.bn_stats[(q, "var")] = expert_sd[cn + f"{idx}.running_var"].detach().to(self.device, torch.float32).clone().contiguous()
-        self.n_class = int(expert_sd["fc.weight"].shape[0])
-        self.struct = L.MrnbCrnnTrainPack()
-        self.gstruct = L.MrnbCrnnTrainPack()
-        for st_, arena in ((self.struct, self.params), (self.gstruct, self.grads)):
+            self.bn_stats[(q, "mean")] = self._bn_stat(expert_sd, f"{idx}.running_mean")
+            self.bn_stats[(q, "var")] = self._bn_stat(expert_sd, f"{idx}.running_var")
+        for st_ in (self.struct, self.gstruct):
             st_.n_class = self.n_class
-            for slot, o in self.slot_offset.items():
-                st_.p[slot] = arena.data_ptr() + 4 * o
-                if self.shadow16 is not None and st_ is self.struct:
-                    st_.h[slot] = self.shadow16.data_ptr() + 2 * o
             for q in range(2):
                 st_.bn_mean[q] = self.bn_stats[(q, "mean")].data_ptr()
                 st_.bn_var[q] = self.bn_stats[(q, "var")].data_ptr()
-        self.load_state(expert_sd)
-        self._ws: Optional[torch.Tensor] = None
 
-    view = SvtrTrainPack.view
-    load_state = SvtrTrainPack.load_state
-    state = SvtrTrainPack.state
-    refresh_shadow = SvtrTrainPack.refresh_shadow
+    def bn_running_stats(self):
+        """(mean4, var4, mean5, var5): updated in place by train-mode forwards."""
+        return tuple(self.bn_stats[(q, s)] for q in range(2) for s in ("mean", "var"))
+
+    @staticmethod
+    def _point(st, slot, ptr, ptr16):
+        st.p[slot], st.h[slot] = ptr, ptr16
 
     def workspace(self, B):
-        need = int(L.load().mrnb_crnn_train_workspace_bytes(B, self.n_class, self.prec))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self._ws
+        return _grow_workspace(self, int(L.load().mrnb_crnn_train_workspace_bytes(B, self.n_class, self.prec)))
 
 
 def crnn_train_forward(tp: CrnnTrainPack, image, bn_batch_stats=True, update_running=True):
@@ -731,10 +708,7 @@ class CrnnPack:
         return tuple(self.slot_tensors[s] for s in (L.C_BN4_MEAN, L.C_BN4_VAR, L.C_BN5_MEAN, L.C_BN5_VAR))
 
     def workspace(self, B, chunk=0):
-        need = int(L.load().mrnb_crnn_workspace_bytes(self.n_experts, B, self.prec))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        return self._ws
+        return _grow_workspace(self, int(L.load().mrnb_crnn_workspace_bytes(self.n_experts, B, self.prec)))
 
 
 def crnn_experts_forward(pack: CrnnPack, image: torch.Tensor, bn_batch_stats: bool = False, update_running: bool = False,
@@ -742,22 +716,8 @@ def crnn_experts_forward(pack: CrnnPack, image: torch.Tensor, bn_batch_stats: bo
     """Runs every CRNN expert on `image` [B,4,32,256].  Returns (features [B,I,63,256], [logits_i [B,63,C_i] views])."""
     _chk_f32(image)
     B = image.shape[0]
-    I = pack.n_experts
-    T = T_FRAMES_CRNN
-    feats = torch.empty(B, I, T, D_FEAT, device=image.device, dtype=torch.float32)
-    ptrs = (C.c_void_p * I)()
-    lds = (C.c_long * I)()
-    logits = []
-    for i in range(I):
-        ld = round_up(pack.n_class[i], 4)
-        lds[i] = ld
-        if want_logits:
-            buf = torch.empty(B, T, ld, device=image.device, dtype=torch.float32)
-            ptrs[i] = buf.data_ptr()
-            logits.append(buf[:, :, :pack.n_class[i]])
-        else:
-            ptrs[i] = None
-            logits.append(None)
+    feats = torch.empty(B, pack.n_experts, T_FRAMES_CRNN, D_FEAT, device=image.device, dtype=torch.float32)
+    ptrs, lds, logits = _logit_buffers(pack, B, image.device, want_logits)
     ws = pack.workspace(B)
     rc = L.load().mrnb_crnn_experts_forward(C.byref(pack.struct), _p(image), B, pack.prec, _mask(bn_batch_stats),
                                             _mask(update_running), _p(feats), ptrs, lds, _p(ws), ws.numel(), _stream())
