@@ -276,7 +276,9 @@ int mrnb_router_forward(const float* params, const float* x, int B, int n_expert
 /* Backward of the stage-1 objective w.r.t. every router parameter (il_modules/mrn.py:342,360,362):
  *   loss = pi * CTC + CrossEntropy(gate, domain)   -- CE applied to the already softmaxed gate (reference quirk).
  * dgate_ctc [B,I] is d(pi*CTC)/dgate from mrnb_ctc_lattice; domain [B] int64.  Writes grads (same arena layout,
- * overwritten) and taski_loss (scalar, the CE term).  Must follow mrnb_router_forward with the same workspace. */
+ * overwritten) and taski_loss (scalar, the CE term).  Must follow mrnb_router_forward with the same workspace.
+ * domain == NULL: dgate_ctc (required) is the complete dL/dgate of an arbitrary loss, no CE term is added and
+ * taski_loss may be NULL (autograd through MRNNet). */
 int mrnb_router_backward(const float* params, const float* x, const float* gate, const float* dgate_ctc,
                          const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
                          float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream);
@@ -300,6 +302,18 @@ int mrnb_dm_router_backward(const float* params, const float* x, const float* d_
 int mrnb_gate_combine(const float* const* z, const long* ld, const int* Ci, int n_experts, const float* gate, int B,
                       int T, float* logits, long ldo, float* lse, float* E, int* amax, float* maxprob,
                       const long long* targets, const int* tlen, int Lmax, float* lpe, float* zlab, cudaStream_t stream);
+
+/* Backward of mrnb_gate_combine for a dense upstream gradient (autograd through MRNNet's soft route): dY [B,T,ldy] fp32
+ * = dL/dlogits over the union charset C = Ci[n_experts-1] ->
+ *   dgate [B,I],  dgate[b,i] = sum_{t, c<C} dY[b,t,c] * (c < Ci[i] ? z_i[b,t,c] : 1.0)   (pad with ones, quirk 1).
+ * The gate is not an input: the combined logits are linear in it.  Every expert is read, a zero-gate one too.  Same
+ * expert table as mrnb_gate_combine (z, ld, Ci host arrays; Ci[i] <= C); z[i] and dY 16-byte aligned, ld[i] and ldy
+ * multiples of 4.  Deterministic (fixed reduction order, no atomics).
+ * workspace: >= mrnb_gate_combine_backward_workspace_bytes(B, T, n_experts) (per-row partials). */
+size_t mrnb_gate_combine_backward_workspace_bytes(int B, int T, int n_experts);
+int mrnb_gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
+                               const float* dY, long ldy, float* dgate, void* workspace, size_t workspace_bytes,
+                               cudaStream_t stream);
 
 /* CTC alpha-beta over all T frames, blank 0.  nll [B] (0 where infeasible: zero_infinity), loss_mean = mean_b(nll_b /
  * max(len_b,1)).  Optional: dgate [B,I] = grad_scale/max(len,1) * sum_t(E_i - sum_s occ_s * zlab_i[ext_s])  (pass

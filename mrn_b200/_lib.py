@@ -101,6 +101,9 @@ _SIGNATURES = {
     "mrnb_dm_router_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "mrnb_gate_combine": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _vp, _i, _i, _vp, _l, _vp, _vp, _vp,
                                _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "mrnb_gate_combine_backward_workspace_bytes": (_sz, [_i, _i, _i]),
+    "mrnb_gate_combine_backward": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _i, _i, _vp, _l, _vp, _vp, _sz,
+                                        _vp]),
     "mrnb_ctc_lattice": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp, _vp]),
     "mrnb_ctc_dense_grad": (_i, [_vp, _l, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _l, _vp]),
     "mrnb_greedy_decode": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),

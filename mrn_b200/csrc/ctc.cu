@@ -553,6 +553,140 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
 }
 
 // ---------------------------------------------------------------------------------------------
+// Backward of the gated combine for a dense upstream gradient dY [B,T,C]:
+//   dgate[b,i] = sum_{t, c<C} dY[b,t,c] * pad_i[b,t,c],   pad_i = z_i below C_i and 1.0 past it.
+// The logits do not depend on the gate beyond this product, so the gate itself is not an input.
+//
+// Persistent like combine_row_tma_kernel: one CTA per SM walks rows r = blockIdx.x, blockIdx.x + gridDim.x, ...  A
+// producer warp streams each row in chunks of BWD_CHUNK columns through a ring of stages ([I + 1][BWD_CHUNK] floats:
+// the I expert slices, then dY) with 1-D bulk copies on mbarriers; lane i copies expert i's slice, lane I the dY slice.
+// Every expert is loaded whatever its gate (a zero-gate expert still has a gradient); a slice past an expert's charset
+// is not copied and reads as the pad value.  Each consumer thread owns 4 columns of a chunk and keeps I running dot
+// products; a row's partials are reduced in a fixed order (warp shuffles, then warp 0 over the warps) into
+// rowout[row, I], and a second kernel sums the T rows of each sample in order: no atomics, the same bits every run.
+// ---------------------------------------------------------------------------------------------
+constexpr int BWD_CONSUMERS = 512;
+constexpr int BWD_CHUNK = 4 * BWD_CONSUMERS;
+constexpr int BWD_MAX_STAGES = 4;
+constexpr int BWD_THREADS = BWD_CONSUMERS + 32;
+constexpr size_t BWD_SMEM_BUDGET = 200 * 1024;
+
+template <int I>
+__global__ void __launch_bounds__(BWD_THREADS, 1)
+combine_bwd_tma_kernel(RowPtrs P, const float* __restrict__ dY, long ldy, int C, int rows, int nchunks, int nstages,
+                       float* __restrict__ rowout) {
+  extern __shared__ __align__(128) float stage[];              // [nstages][I + 1][BWD_CHUNK]
+  __shared__ __align__(8) uint64_t full_bar[BWD_MAX_STAGES], empty_bar[BWD_MAX_STAGES];
+  __shared__ float part[2][BWD_CONSUMERS / 32][I];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  constexpr size_t SLOT = (size_t)(I + 1) * BWD_CHUNK;
+  if (tid == 0) {
+    for (int s = 0; s < nstages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], BWD_CONSUMERS / 32); }
+    fence_mbarrier_init();
+  }
+  __syncthreads();
+
+  if (warp == BWD_CONSUMERS / 32) {
+    // ---------------- producer warp
+    const int myC = lane < I ? P.C[lane] : C;
+    const long myld = lane < I ? P.ld[lane] : ldy;
+    const float* myz = lane < I ? P.z[lane] : dY;
+    uint32_t q = 0;
+    for (int row = blockIdx.x; row < rows; row += gridDim.x) {
+      const float* src = myz + (long)row * myld;
+      for (int j = 0; j < nchunks; ++j, ++q) {
+        const int s = (int)(q % (uint32_t)nstages);
+        uint32_t total = 0;
+#pragma unroll
+        for (int i = 0; i <= I; ++i) {
+          int n = (i < I ? P.C[i] : C) - j * BWD_CHUNK;
+          n = n < 0 ? 0 : (n > BWD_CHUNK ? BWD_CHUNK : n);
+          total += (uint32_t)((n + 3) & ~3) * 4u;                 // whole 16-byte pieces (ld is padded to 4)
+        }
+        int n = myC - j * BWD_CHUNK;
+        n = n < 0 ? 0 : (n > BWD_CHUNK ? BWD_CHUNK : n);
+        const uint32_t nb = lane <= I ? (uint32_t)((n + 3) & ~3) * 4u : 0u;
+        mbar_wait(&empty_bar[s], ((q / (uint32_t)nstages) & 1u) ^ 1u);
+        if (lane == 0) mbar_expect_tx(&full_bar[s], total);        // total > 0: the dY slice of chunk j < nchunks
+        __syncwarp();
+        if (nb) bulk_load(stage + s * SLOT + (size_t)lane * BWD_CHUNK, src + (long)j * BWD_CHUNK, nb, &full_bar[s]);
+      }
+    }
+    return;
+  }
+
+  // ---------------- consumers (4 columns each per chunk)
+  uint32_t q = 0, it = 0;
+  for (int row = blockIdx.x; row < rows; row += gridDim.x, ++it) {
+    float acc[I];
+#pragma unroll
+    for (int i = 0; i < I; ++i) acc[i] = 0.f;
+    for (int j = 0; j < nchunks; ++j, ++q) {
+      const int s = (int)(q % (uint32_t)nstages);
+      mbar_wait(&full_bar[s], (q / (uint32_t)nstages) & 1u);
+      const float* st = stage + s * SLOT + tid * 4;
+      const int c0 = j * BWD_CHUNK + tid * 4;
+      float4 dy = make_float4(0.f, 0.f, 0.f, 0.f);
+      float4 v[I];
+#pragma unroll
+      for (int i = 0; i < I; ++i) {
+        v[i] = make_float4(1.f, 1.f, 1.f, 1.f);
+        if (c0 < P.C[i]) v[i] = *reinterpret_cast<const float4*>(st + (size_t)i * BWD_CHUNK);
+      }
+      if (c0 < C) dy = *reinterpret_cast<const float4*>(st + (size_t)I * BWD_CHUNK);
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&empty_bar[s]);                 // stage s may be refilled
+      if (c0 >= C) continue;
+      if (c0 + 4 > C) {                                          // the row's last, partial group: ld padding is not dY
+        if (c0 + 1 >= C) dy.y = 0.f;
+        if (c0 + 2 >= C) dy.z = 0.f;
+        dy.w = 0.f;
+      }
+      const float sdy = (dy.x + dy.y) + (dy.z + dy.w);
+#pragma unroll
+      for (int i = 0; i < I; ++i) {
+        const int Ci = P.C[i];
+        if (c0 >= Ci) {
+          acc[i] += sdy;                                         // pad value 1.0
+        } else {
+          if (c0 + 4 > Ci) {                                     // the group straddling C_i: re-impose the pad
+            if (c0 + 1 >= Ci) v[i].y = 1.f;
+            if (c0 + 2 >= Ci) v[i].z = 1.f;
+            v[i].w = 1.f;
+          }
+          acc[i] = fmaf(dy.x, v[i].x, fmaf(dy.y, v[i].y, fmaf(dy.z, v[i].z, fmaf(dy.w, v[i].w, acc[i]))));
+        }
+      }
+    }
+    // ---- row reduction in a fixed order: warp tree, then warp 0 over the consumer warps (double-buffered partials)
+#pragma unroll
+    for (int i = 0; i < I; ++i) acc[i] = warp_sum(acc[i]);
+    const int buf = it & 1u;
+    if (lane == 0) {
+#pragma unroll
+      for (int i = 0; i < I; ++i) part[buf][warp][i] = acc[i];
+    }
+    asm volatile("bar.sync 1, %0;" ::"r"(BWD_CONSUMERS) : "memory");
+    if (warp == 0 && lane < I) {
+      float sum = 0.f;
+#pragma unroll
+      for (int w = 0; w < BWD_CONSUMERS / 32; ++w) sum += part[buf][w][lane];
+      rowout[(long)row * I + lane] = sum;
+    }
+  }
+}
+
+// dgate[b,i] = sum_t rowout[b,t,i], t ascending
+__global__ void combine_bwd_finish_kernel(const float* __restrict__ rowout, int B, int T, int I, float* __restrict__ dgate) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= B * I) return;
+  const int b = k / I, i = k - b * I;
+  float s = 0.f;
+  for (int t = 0; t < T; ++t) s += rowout[((long)b * T + t) * I + i];
+  dgate[k] = s;
+}
+
+// ---------------------------------------------------------------------------------------------
 // CTC lattice: one warp per sequence; lane l owns states 2l (blank) and 2l+1 (label l+1).
 // ---------------------------------------------------------------------------------------------
 constexpr int CTC_WARPS = 4;
@@ -781,6 +915,30 @@ int launch_combine(const RowPtrs& P, const float* gate, int B, int T, int C, flo
   return MRNB_OK;
 }
 
+template <int I>
+int launch_combine_bwd(const RowPtrs& P, const float* dY, long ldy, int B, int T, int C, float* dgate, float* rowout,
+                       cudaStream_t st) {
+  const int nchunks = (C + BWD_CHUNK - 1) / BWD_CHUNK;
+  const size_t slot_bytes = (size_t)(I + 1) * BWD_CHUNK * sizeof(float);
+  const int nstages = (int)(BWD_SMEM_BUDGET / slot_bytes) < BWD_MAX_STAGES ? (int)(BWD_SMEM_BUDGET / slot_bytes) : BWD_MAX_STAGES;
+  static bool attr_set = false;
+  static int num_sms = 148;
+  if (!attr_set) {
+    cudaFuncSetAttribute(combine_bwd_tma_kernel<I>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BWD_SMEM_BUDGET);
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
+    attr_set = true;
+  }
+  const int rows = B * T;
+  const int grid = rows < num_sms ? rows : num_sms;
+  combine_bwd_tma_kernel<I><<<grid, BWD_THREADS, nstages * slot_bytes, st>>>(P, dY, ldy, C, rows, nchunks, nstages, rowout);
+  MRNB_CHECK_LAUNCH("combine_bwd_tma_kernel");
+  combine_bwd_finish_kernel<<<cdiv(B * I, 256), 256, 0, st>>>(rowout, B, T, I, dgate);
+  MRNB_CHECK_LAUNCH("combine_bwd_finish_kernel");
+  return MRNB_OK;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -806,6 +964,40 @@ extern "C" int mrnb_gate_combine(const float* const* z, const long* ld, const in
   for (int i = 0; i < n_experts; ++i) rb += (double)Ci[i];
   MrnbProfScope prof(MRNB_PROF_COMBINE, stream, 0.0, 4.0 * B * T * (rb + (logits ? C : 0)));
 #define MRNB_CASE(N) case N: return launch_combine<N>(P, gate, B, T, C, logits, ldo, lse, E, amax, maxprob, targets, tlen, Lmax, lpe, zlab, S1, stream);
+  switch (n_experts) {
+    MRNB_CASE(1) MRNB_CASE(2) MRNB_CASE(3) MRNB_CASE(4) MRNB_CASE(5) MRNB_CASE(6) MRNB_CASE(7) MRNB_CASE(8)
+  }
+#undef MRNB_CASE
+  return MRNB_ERR_ARG;
+}
+
+extern "C" size_t mrnb_gate_combine_backward_workspace_bytes(int B, int T, int n_experts) {
+  return (size_t)B * T * n_experts * sizeof(float);
+}
+
+extern "C" int mrnb_gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
+                                          const float* dY, long ldy, float* dgate, void* workspace,
+                                          size_t workspace_bytes, cudaStream_t stream) {
+  MRNB_CHECK_ARG(n_experts >= 1 && n_experts <= MRNB_MAX_EXPERTS, "gate_combine_backward: n_experts %d out of range",
+                 n_experts);
+  MRNB_CHECK_ARG(B > 0 && T > 0 && z && ld && Ci && dY && dgate && workspace, "gate_combine_backward: null/empty argument");
+  const int C = Ci[n_experts - 1];
+  RowPtrs P;
+  for (int i = 0; i < n_experts; ++i) {
+    P.z[i] = z[i]; P.ld[i] = ld[i]; P.C[i] = Ci[i];
+    MRNB_CHECK_ARG(z[i] && Ci[i] > 0 && Ci[i] <= C && ld[i] >= Ci[i] && ld[i] % 4 == 0 &&
+                   (reinterpret_cast<uintptr_t>(z[i]) & 15) == 0,
+                   "gate_combine_backward: expert %d needs C_i <= C, a 16-byte aligned base and ld %% 4 == 0", i);
+  }
+  MRNB_CHECK_ARG(ldy >= C && ldy % 4 == 0 && (reinterpret_cast<uintptr_t>(dY) & 15) == 0,
+                 "gate_combine_backward: dY needs ldy >= C, ldy %% 4 == 0 and a 16-byte aligned base");
+  MRNB_CHECK_ARG(workspace_bytes >= mrnb_gate_combine_backward_workspace_bytes(B, T, n_experts),
+                 "gate_combine_backward: workspace too small (%zu bytes)", workspace_bytes);
+  double rb = C;
+  for (int i = 0; i < n_experts; ++i) rb += (double)Ci[i];
+  MrnbProfScope prof(MRNB_PROF_COMBINE, stream, 0.0, 4.0 * B * T * rb);
+  float* rowout = static_cast<float*>(workspace);
+#define MRNB_CASE(N) case N: return launch_combine_bwd<N>(P, dY, ldy, B, T, C, dgate, rowout, stream);
   switch (n_experts) {
     MRNB_CASE(1) MRNB_CASE(2) MRNB_CASE(3) MRNB_CASE(4) MRNB_CASE(5) MRNB_CASE(6) MRNB_CASE(7) MRNB_CASE(8)
   }

@@ -546,13 +546,19 @@ gate_finish_kernel(const float* __restrict__ s, const float* __restrict__ wr, co
 }
 
 // dL/dr from dL/dgate (CTC part) + CrossEntropy(gate, domain) applied to the softmaxed gate; also the CE loss.
+// domain == NULL: dgate_ctc is the whole dL/dgate (no CE term, ce_loss untouched).
 __global__ void gate_bwd_kernel(const float* __restrict__ gate, const float* __restrict__ dgate_ctc,
                                 const long long* __restrict__ domain, int B, int I, float* __restrict__ dr,
                                 float* __restrict__ ce_loss) {
   __shared__ double sh[8];
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   double lossb = 0.0;
-  if (b < B) {
+  if (b < B && !domain) {
+    float g[MRNB_MAX_EXPERTS];
+    float dot = 0.f;
+    for (int j = 0; j < I; ++j) { g[j] = gate[b * I + j]; dot = fmaf(g[j], dgate_ctc[b * I + j], dot); }
+    for (int j = 0; j < I; ++j) dr[b * I + j] = g[j] * (dgate_ctc[b * I + j] - dot);
+  } else if (b < B) {
     float g[MRNB_MAX_EXPERTS], dg[MRNB_MAX_EXPERTS];
     float mx = -INFINITY;
     for (int j = 0; j < I; ++j) { g[j] = gate[b * I + j]; mx = fmaxf(mx, g[j]); }
@@ -571,7 +577,7 @@ __global__ void gate_bwd_kernel(const float* __restrict__ gate, const float* __r
   lossb = warp_sum_d(lossb);
   if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = lossb;
   __syncthreads();
-  if (threadIdx.x == 0) {
+  if (threadIdx.x == 0 && domain) {
     double t = 0.0;
     for (int k = 0; k < (int)(blockDim.x >> 5); ++k) t += sh[k];
     atomicAdd(ce_loss, (float)t);
@@ -1529,7 +1535,9 @@ extern "C" int mrnb_router_backward(const float* params, const float* x, const f
                                     const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
                                     float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   ROUTER_ARGCHECK("router_backward");
-  MRNB_CHECK_ARG(gate && domain && grads && taski_loss, "router_backward: null argument");
+  MRNB_CHECK_ARG(gate && grads, "router_backward: null argument");
+  MRNB_CHECK_ARG(domain ? taski_loss != nullptr : dgate_ctc != nullptr,
+                 "router_backward: a domain needs taski_loss; without one, dgate_ctc is the whole dL/dgate and is required");
   RouterRun r(workspace, B, n_experts, T, D, prec, true);
   MRNB_CHECK_ARG(workspace_bytes >= r.bytes, "router_backward: workspace too small (%zu < %zu)", workspace_bytes, r.bytes);
   if (r.padded) { params = r.pw.Pp; x = r.pw.xp; }   // written by mrnb_router_forward on the same workspace
@@ -1540,7 +1548,7 @@ extern "C" int mrnb_router_backward(const float* params, const float* x, const f
   long off[MRNB_ROUTER_NPARAMS + 1];
   const long nparam = router_offsets(d.I, d.T, d.D, off);
   cudaMemsetAsync(G, 0, nparam * sizeof(float), st);
-  cudaMemsetAsync(taski_loss, 0, sizeof(float), st);
+  if (taski_loss) cudaMemsetAsync(taski_loss, 0, sizeof(float), st);
   {
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     gate_bwd_kernel<<<cdiv(B, 256), 256, 0, st>>>(gate, dgate_ctc, domain, B, d.I, w.dr, taski_loss);

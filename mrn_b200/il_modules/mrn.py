@@ -10,7 +10,8 @@ What runs where
   * stage 0 (training the newest expert end to end, il_modules/mrn.py:225-279; SURVEY.md §8(f)3) for SVTR experts:
     activation-keeping forward -> fused log-softmax + CTC -> dense CTC gradient -> hand-written backward to every
     parameter of the expert (mrnb_svtr_train_forward / _backward) -> [NCCL all-reduce of the expert's gradient arena]
-    -> clip + Adam on the arena.  CRNN experts (VGG + BiLSTM BPTT) are not implemented and raise.
+    -> clip + Adam on the arena.  CRNN experts run the same step (VGG + BiLSTM BPTT, mrnb_crnn_train_forward /
+    _backward).
 Host-side schedule / logging logic follows il_modules/base.py.
 """
 import math
@@ -22,7 +23,7 @@ import torch
 
 from .. import dist as mdist
 from .. import ops
-from ..modules.model import MRNNet, _arch, _expert_bns, _precision, _train_forward_ran, sample_drop_scales
+from ..modules.model import MRNNet, _arch, _precision, _train_forward_ran, _writeback_train_pack_bn, sample_drop_scales
 from ..utils import Averager, CTCLabelConverter, DevicePrefetcher
 
 
@@ -322,11 +323,7 @@ class MRN(object):
             own = dict(expert.named_parameters())
             for key, t in tp.state().items():
                 own[key].copy_(t)                       # bumps the version counter -> inference packs are rebuilt
-            m0, v0, m1, v1 = tp.bn_running_stats()
-            for bn, mean, var in zip(_expert_bns(expert, tp.arch), (m0, m1), (v0, v1)):
-                bn.running_mean.copy_(mean.reshape(-1))
-                bn.running_var.copy_(var.reshape(-1))
-                bn.num_batches_tracked += self._tp_steps
+        _writeback_train_pack_bn(expert, tp, self._tp_steps)
         self._tp_steps = 0
         self.net._cache.key = None                      # BN buffers changed without a parameter version bump
         self.reset_graphs()

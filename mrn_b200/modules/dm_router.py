@@ -22,8 +22,9 @@ class ChannelDomainGating(nn.Module):
 
 
 class DM_Router(nn.Module):
-    def __init__(self, channel, d_ffn, patch, domain):
+    def __init__(self, channel, d_ffn, patch, domain, autograd=False):
         super().__init__()
+        self.autograd = autograd        # forward() builds an autograd graph (input and parameter gradients)
         self.patch = patch
         self.channel = channel
         self.domain = domain
@@ -47,8 +48,12 @@ class DM_Router(nn.Module):
         return arena
 
     def forward(self, x):
-        """x [B, D(omain), P(atch), C] -> same shape (modules/dm_router.py:50-67)."""
+        """x [B, D(omain), P(atch), C] -> same shape (modules/dm_router.py:50-67).  With autograd=True and grad mode on,
+        the output is differentiable with respect to x and every parameter (mrnb_dm_router_backward)."""
         if not x.is_cuda:
             raise RuntimeError("DM_Router.forward needs a CUDA tensor: mrn_b200 has no CPU fallback")
+        if self.autograd and torch.is_grad_enabled():
+            from ..autograd import DmRouter
+            return DmRouter.apply(self, x.contiguous().float(), *self.parameters())
         out, _, _, _ = ops.router_forward(self._standalone_arena(x.device), x.contiguous().float(), self._ws)
         return out

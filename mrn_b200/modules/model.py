@@ -100,7 +100,11 @@ class Model(nn.Module):
         self.fc.weight.data[-increment:, :] *= gamma
 
     def forward(self, image, text=None, is_train=True):
-        """-> {"predict": [B,T,C], "feature": [B,T,256]} (modules/model.py:133-148) via a single-expert pack."""
+        """-> {"predict": [B,T,C], "feature": [B,T,256]} (modules/model.py:133-148) via a single-expert pack.
+        With opt.autograd and grad mode on, "predict" is differentiable with respect to every parameter (training-pack
+        forward, see _expert_autograd_forward) and "feature" is None."""
+        if _autograd_on(self.opt):
+            return {"predict": _expert_autograd_forward(self, image, self.opt), "feature": None}
         feats, logits = _experts_forward([self], image, self.opt, train_mode=self.training)
         return {"predict": logits[0], "feature": feats[:, 0]}
 
@@ -203,6 +207,64 @@ def _train_forward_ran(cache, experts, modes):
         _writeback_bn(experts, cache.pack)
 
 
+def _autograd_on(opt):
+    """opt.autograd (absent = False) and torch grad mode: the forwards build an autograd graph over the kernels."""
+    return bool(getattr(opt, "autograd", False)) and torch.is_grad_enabled()
+
+
+def _writeback_train_pack_bn(expert, tp, n_fwd):
+    """A training pack's BatchNorm running statistics -> the expert's buffers, after `n_fwd` train-mode forwards."""
+    with torch.no_grad():
+        m0, v0, m1, v1 = tp.bn_running_stats()
+        for bn, mean, var in zip(_expert_bns(expert, tp.arch), (m0, m1), (v0, v1)):
+            bn.running_mean.copy_(mean.reshape(-1))
+            bn.running_var.copy_(var.reshape(-1))
+            bn.num_batches_tracked += n_fwd
+
+
+def _expert_autograd_forward(expert, image, opt, net=None):
+    """Forward of one expert that autograd differentiates (opt.autograd): the training pack's activation-keeping forward
+    (ops.SvtrTrainPack / ops.CrnnTrainPack) in the expert's current mode -- in .train() BatchNorm batch statistics with
+    the running-statistics update and DropPath drawn as the default forward draws it -- and, on backward, the pack's full
+    backward, mapped back to every parameter in the reference layout by the pack's arena <-> state_dict table."""
+    if not image.is_cuda:
+        raise RuntimeError("mrn_b200 needs CUDA tensors: there is no CPU fallback")
+    from ..autograd import ExpertTrain
+    if net is not None:
+        net._sync_bn()                      # BN statistics the grouped pack still holds -> the module buffers
+    arch = _arch(opt)
+    named = list(expert.named_parameters())
+
+    def run(x):
+        tp = (ops.SvtrTrainPack if arch == "svtr" else ops.CrnnTrainPack)(expert.state_dict(), x.device, _precision(opt))
+        train = bool(expert.training)
+        x = x.contiguous().float()
+        B = x.shape[0]
+        drop = None
+        if arch == "crnn":
+            logits = ops.crnn_train_forward(tp, x, bn_batch_stats=train, update_running=train)
+        else:
+            if train and getattr(opt, "drop_path", True):
+                rates = expert.model.FeatureExtraction.ConvNet.drop_path_rates()
+                drop = sample_drop_scales(1, B, rates, x.device)[0].contiguous()
+            logits = ops.svtr_train_forward(tp, x, bn_batch_stats=train, update_running=train, drop_scales=drop)
+        if train:
+            _writeback_train_pack_bn(expert, tp, 1)
+            _solo_cache.key = None          # packs hold BN statistics: rebuild them from the updated buffers
+            if net is not None:
+                net._cache.key = None
+
+        def backward(dlogits):
+            if arch == "crnn":
+                ops.crnn_train_backward(tp, dlogits, B, bn_batch_stats=train)
+            else:
+                ops.svtr_train_backward(tp, x, dlogits, bn_batch_stats=train, drop_scales=drop)
+            return tp.state(tp.grads)
+        return backward, logits
+
+    return ExpertTrain.apply(run, [n for n, _ in named], image, *[p for _, p in named])
+
+
 _RATES_CACHE = {}
 
 
@@ -278,7 +340,8 @@ class MRNNet(nn.Module):
             self.out_dim = self.model[-1].SequenceModeling_output
         self.route = nn.Linear(self.patch, 1)
         self.channel_route = nn.Linear(self.feature_dim, len(self.model))
-        block = DM_Router(self.out_dim, self.out_dim * 2, self.patch, len(self.model))
+        block = DM_Router(self.out_dim, self.out_dim * 2, self.patch, len(self.model),
+                          autograd=bool(getattr(self.opt, "autograd", False)))
         self.dm_router = nn.Sequential(*[block for _ in range(self.layer_num)])
         self._arena = None
         self._grad_arena = None
@@ -356,10 +419,30 @@ class MRNNet(nn.Module):
     # -- forward ---------------------------------------------------------------------------------
     def forward(self, image, cross=True, text=None, is_train=True):
         """-> {"logits": [B,T,C], "index": gate [B,I] (train) / argmax [B] (eval) / None, "aux_logits": None}
-        (modules/model.py:343-359)."""
+        (modules/model.py:343-359).
+
+        opt.autograd (default off) with grad mode on makes the outputs differentiable (INTEGRATION.md §A):
+          * cross=True, is_train=True (soft route): "logits" and "index" (the gate) with respect to route.*,
+            channel_route.* and dm_router.0.*; the experts are frozen and an expert parameter that requires grad
+            raises NotImplementedError;
+          * cross=True, is_train=False (hard route): "index" is an argmax and "logits" depends only on the frozen
+            experts -- outputs as without the switch, no router gradient;
+          * cross=False: "logits" with respect to every parameter of the newest expert (training-pack forward)."""
+        grad = _autograd_on(self.opt)
         if cross is False:
+            if grad:
+                return dict(logits=_expert_autograd_forward(self.model[-1], image, self.opt, net=self), index=None,
+                            aux_logits=None)
             feats, logits = _experts_forward([self.model[-1]], image, self.opt, self.model[-1].training)
             return dict(logits=logits[0], index=None, aux_logits=None)
+        if grad and is_train:
+            from ..autograd import RoutedSoft
+            if any(p.requires_grad for p in self.model.parameters()):
+                raise NotImplementedError(
+                    "autograd through the routed forward keeps the experts frozen, as MRN stage 1 does "
+                    "(il_modules/mrn.py:154-157): set requires_grad=False on every expert parameter")
+            logits, gate = RoutedSoft.apply(self, image, *self.router_parameters())
+            return dict(logits=logits, index=gate, aux_logits=None)
         r = self.route_and_combine(image, is_train=is_train, want_logits=True)
         return dict(logits=r["logits"], index=r["index"], aux_logits=None)
 
@@ -375,9 +458,9 @@ class MRNNet(nn.Module):
         raise RuntimeError("padding with ones is fused into mrnb_gate_combine; no padded tensor is materialised")
 
     def route_and_combine(self, image, is_train=True, want_logits=True, targets=None, lengths=None, want_E=False,
-                          want_decode=False, with_backward=False, drop_scales=None):
+                          want_decode=False, with_backward=False, drop_scales=None, rws=None):
         """Experts -> DM-Router -> gate -> fused combine.  Soft route when is_train (modules/model.py:397-423),
-        hard route otherwise (:366-395)."""
+        hard route otherwise (:366-395).  rws: router workspace to use instead of the module's own."""
         experts = list(self.model)
         # Hard route (eval): route FIRST, then evaluate only the routed expert's classifier head per sample (SURVEY K8e;
         # modules/model.py:383-393 keeps padded_{index[b]}[b] and discards the other five heads' logits).  The soft
@@ -386,7 +469,7 @@ class MRNNet(nn.Module):
         feats, logits = _experts_forward(experts, image, self.opt, self._experts_train_mode(), self._cache,
                                          drop_scales=drop_scales, want_logits=not sparse)
         arena = self.router_arena(image.device)
-        _, scores, gate, index = ops.router_forward(arena, feats, self._rws, with_backward=with_backward,
+        _, scores, gate, index = ops.router_forward(arena, feats, rws or self._rws, with_backward=with_backward,
                                                     prec=_precision(self.opt), want_out=False)
         if is_train:
             g, idx_out = gate, gate

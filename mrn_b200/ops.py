@@ -770,10 +770,12 @@ def router_forward(params: torch.Tensor, x: torch.Tensor, ws: RouterWorkspace, w
 
 
 def router_backward(params, x, gate, dgate_ctc, domain, grads, ws: RouterWorkspace, prec=L.PREC_FP32):
+    """domain [B] int64: loss = pi*CTC + CE(gate, domain), returns the CE term.  domain None: dgate_ctc is the whole
+    dL/dgate of an arbitrary loss (no CE term), returns None."""
     _chk_f32(params, x, gate, dgate_ctc, grads)
-    assert domain.dtype == torch.int64
+    assert domain is None or domain.dtype == torch.int64
     B, I, T, D = x.shape
-    taski = torch.empty(1, device=x.device, dtype=torch.float32)
+    taski = torch.empty(1, device=x.device, dtype=torch.float32) if domain is not None else None
     w = ws.get(B, I, T, D, True, x.device)
     L.check(L.load().mrnb_router_backward(_p(params), _p(x), _p(gate), _p(dgate_ctc), _p(domain), B, I, T, D, prec,
                                           _p(grads), _p(taski), _p(w), w.numel(), _stream()), "router_backward")
@@ -835,6 +837,26 @@ def gate_combine(logits: Sequence[torch.Tensor], gate: torch.Tensor, targets: Op
                                        _p(r.get("E")), _p(r.get("amax")), _p(r.get("maxprob")), _p(targets), _p(lengths),
                                        Lmax, _p(r.get("lpe")), _p(r.get("zlab")), _stream()), "gate_combine")
     return r
+
+
+def gate_combine_backward(logits: Sequence[torch.Tensor], dY: torch.Tensor, out: Optional[torch.Tensor] = None):
+    """dgate [B,I] = d<dY, combined logits>/dgate for a dense upstream gradient dY [B,T,C] over the union charset (same
+    expert table as gate_combine; the pad value 1.0 counts).  dY rows that are not 16-byte aligned are first copied
+    into a padded buffer.  `out` may supply dgate."""
+    B, T, _ = logits[0].shape
+    I, C = len(logits), logits[-1].shape[2]
+    ptrs, lds, cs = _expert_tables(logits)
+    if dY.dtype != torch.float32 or tuple(dY.shape) != (B, T, C) or not dY.is_cuda:
+        raise RuntimeError("gate_combine_backward: dY must be a CUDA float32 tensor [B,T,C] = %s" % ((B, T, C),))
+    if not (dY.stride(2) == 1 and dY.stride(1) % 4 == 0 and dY.stride(0) == T * dY.stride(1) and dY.data_ptr() % 16 == 0):
+        buf = torch.zeros(B, T, round_up(C, 4), device=dY.device, dtype=torch.float32)
+        buf[:, :, :C].copy_(dY)
+        dY = buf[:, :, :C]
+    dgate = _out(out, (B, I), dY.device, torch.float32)
+    ws = torch.empty(int(L.load().mrnb_gate_combine_backward_workspace_bytes(B, T, I)), dtype=torch.uint8, device=dY.device)
+    L.check(L.load().mrnb_gate_combine_backward(ptrs, lds, cs, I, B, T, _p(dY), dY.stride(1), _p(dgate), _p(ws), ws.numel(),
+                                                _stream()), "gate_combine_backward")
+    return dgate
 
 
 def ctc_lattice(lpe, targets, lengths, zlab=None, E=None, grad_scale=0.0, want_dgate=False, want_occ=False):
