@@ -1,4 +1,5 @@
-"""Deterministic synthetic weights and inputs shared by bench.py, the tests and the golden generator.
+"""Deterministic synthetic weights and inputs shared by bench.py, the tests and the golden generator, and the one
+set-up the tests and tools build the mirror's MRNNet / MRN learner with (make_opt, build_net, build_learner).
 
 Data generation only (no reference code, no oracle arithmetic): numpy PCG64 streams keyed by
 (seed, crc32(name)) so the same tensors can be rebuilt on the GPU box without shipping weights.
@@ -7,6 +8,7 @@ the reference modules by oracle/make_golden.py).
 """
 from __future__ import annotations
 
+import argparse
 import zlib
 from collections import OrderedDict
 from typing import Dict, List, Sequence, Tuple
@@ -200,19 +202,10 @@ def ctor_state_dict(class_counts: Sequence[int], seed: int = 111, arch: str = "s
     elsewhere; router rebuilt by update_fc, modules/model.py:437-452) -- the "random-init weights" BASELINE.json's
     tolerances and metric are quoted on.  Gates come out soft (~1/I), unlike the gate-spreading synth_state_dict.
     Deterministic on the CPU generator for a given (seed, class_counts, arch)."""
-    import argparse
-    from .modules.model import MRNNet
-    opt = argparse.Namespace(Transformation="None", FeatureExtraction="SVTR" if arch == "svtr" else "VGG",
-                             SequenceModeling="None" if arch == "svtr" else "BiLSTM", Prediction="CTC", num_fiducial=20,
-                             input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256, batch_max_length=25,
-                             precision="fp32")
     gen_state = torch.get_rng_state()
     torch.manual_seed(seed)
     try:
-        net = MRNNet(opt)
-        for c in class_counts:
-            net.update_fc(opt.hidden_size, c)
-            net.build_prediction(opt, c)
+        net = build_net(class_counts, arch=arch, device=None)
         sd = OrderedDict((k, v.detach().clone()) for k, v in net.state_dict().items())
         for k in sd:                        # non-trivial BatchNorm running statistics (eval-mode experts use them)
             if k.endswith("running_var"):
@@ -222,3 +215,47 @@ def ctor_state_dict(class_counts: Sequence[int], seed: int = 111, arch: str = "s
     finally:
         torch.set_rng_state(gen_state)
     return sd
+
+
+# ------------------------------------------------------------------------------------------------ set-up outside a run
+def make_opt(arch: str = "svtr", precision: str = "fp32", **overrides) -> argparse.Namespace:
+    """The reference's option namespace (config/svtr_mrn.py, config/crnn_mrn.py) for building MRNNet / MRN without the
+    data pipeline: the model fields of `arch`, the training fields the learner reads, `overrides` on top."""
+    opt = argparse.Namespace(Transformation="None", FeatureExtraction="SVTR" if arch == "svtr" else "VGG",
+                             SequenceModeling="None" if arch == "svtr" else "BiLSTM", Prediction="CTC", num_fiducial=20,
+                             input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256, batch_max_length=25,
+                             lr=5e-4, num_iter=10000, grad_clip=5, exp_name="test", precision=precision, drop_path=False,
+                             autograd=False, expert_chunk=0, lan_list=list("abcdef"), val_interval=5000, start_task=0,
+                             optimizer="adam", schedule="super")
+    vars(opt).update(overrides)
+    return opt
+
+
+def build_net(class_counts: Sequence[int], state_dict=None, opt=None, *, device="cuda", **opt_kw):
+    """MRNNet grown one expert per class count as the reference grows it per task (update_fc + build_prediction),
+    `state_dict` loaded strict=True when given, moved to `device` (None: left on the CPU).  Without `opt` the options
+    are make_opt(**opt_kw)."""
+    from .modules.model import MRNNet
+    assert opt is None or not opt_kw, "options come from opt or from make_opt keywords, not both"
+    if opt is None:
+        opt = make_opt(**opt_kw)
+    net = MRNNet(opt)
+    for c in class_counts:
+        net.update_fc(opt.hidden_size, c)
+        net.build_prediction(opt, c)
+    if state_dict is not None:
+        res = net.load_state_dict(state_dict, strict=True)      # the state_dict contract (SURVEY.md §8b)
+        assert not res.missing_keys and not res.unexpected_keys
+    return net if device is None else net.to(device)
+
+
+def build_learner(net, *, train: bool = True, total_steps=None, schedule: str = "const"):
+    """MRN learner over `net` with net.opt, its model in train or eval mode; with `total_steps` also the fused router
+    optimiser (lr and grad_clip from net.opt)."""
+    from .il_modules.mrn import MRN, RankLocal, FusedAdam
+    learner = MRN(net.opt)
+    learner.model = RankLocal(net)
+    learner.model.train(train)
+    if total_steps is not None:
+        learner.optimizer = FusedAdam(net, net.opt.lr, total_steps, grad_clip=net.opt.grad_clip, schedule=schedule)
+    return learner

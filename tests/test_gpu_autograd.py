@@ -2,40 +2,18 @@
 loop -- forward, log_softmax + F.ctc_loss, CE on the gate, loss.backward(), clip_grad_norm_, torch.optim.Adam
 (il_modules/mrn.py:338-367 and :236-267) -- on the fused kernels, against the reference goldens, the fused learner
 step and fp64; the combine backward kernel against fp64; the switch left off changes nothing."""
-import argparse
-
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
 from oracle import mrn_oracle as O
-from oracle import synth
-from conftest import load_golden, gview, rel_err
+from mrn_b200 import synth
+from conftest import gview, rel_err
+from golden_cases import golden_case
 from persistent_walk import assert_walk, combine_walk
 
 ROUTER_PREFIXES = ("route.", "channel_route.", "dm_router.0.")
-
-
-def _opt(arch, precision="fp32", autograd=True):
-    feat, seq = ("SVTR", "None") if arch == "svtr" else ("VGG", "BiLSTM")
-    return argparse.Namespace(Transformation="None", FeatureExtraction=feat, SequenceModeling=seq, Prediction="CTC",
-                              num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                              batch_max_length=25, lr=5e-4, num_iter=10000, grad_clip=5, exp_name="test", precision=precision,
-                              drop_path=True, lan_list=list("abcdef"), val_interval=5000, start_task=0, optimizer="adam",
-                              schedule="super", autograd=autograd)
-
-
-def _net(arch, cc, sd, precision="fp32", autograd=True):
-    from mrn_b200.modules.model import MRNNet
-    opt = _opt(arch, precision, autograd)
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    res = net.load_state_dict(sd, strict=True)
-    assert not res.missing_keys and not res.unexpected_keys
-    return net.cuda()
 
 
 def _freeze_experts(net):
@@ -68,13 +46,10 @@ def test_stage1_torch_loop_matches_reference_golden(name):
     """Router .grad within 1e-3 of each parameter's scale (the rule of test_stage1_step_matches_reference_golden), the
     total norm of clip_grad_norm_ within 5e-4 and one torch.optim.Adam step against adam1.*."""
     from mrn_b200 import ops
-    g = load_golden(name)
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
     arch = "crnn" if name.startswith("crnn") else "svtr"
     T = 63 if arch == "crnn" else 64
-    cc, B, seed = tuple(int(c) for c in g["class_counts"]), int(g["B"]), int(g["seed"])
-    sd = synth.synth_state_dict(cc, seed, arch=arch)
-    img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
-    net = _net(arch, cc, sd)
+    net = synth.build_net(cc, sd, arch=arch, autograd=True)
     net.eval()                                          # the goldens were made with eval-mode, frozen experts
     _freeze_experts(net)
     _stage1_loop(net, img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda())
@@ -114,23 +89,19 @@ def test_autograd_gradients_match_fused_stage1_step(arch, precision, mode, monke
     train: experts in .train() (BatchNorm batch statistics) with the same injected DropPath scales on both paths."""
     import mrn_b200.modules.model as M
     from mrn_b200 import ops
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
     cc, B, seed = (37, 61, 96), 4, 7
     sd = synth.ctor_state_dict(cc, seed) if precision == "bf16" else synth.synth_state_dict(cc, seed, arch=arch)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     drop = synth.synth_drop_scales(len(cc), B, O.svtr_drop_path_rates(), seed).cuda() if mode == "train" else None
     x, t, l, d = img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda()
 
-    fused = _net(arch, cc, sd, precision, autograd=False)
-    fused.train(mode == "train")
-    learner = MRN(fused.opt)
-    learner.model = RankLocal(fused)
-    learner.optimizer = FusedAdam(fused, 5e-4, 20000, grad_clip=5, schedule="const")
+    fused = synth.build_net(cc, sd, arch=arch, precision=precision)
+    learner = synth.build_learner(fused, train=mode == "train", total_steps=20000)
     learner.train_step_stage1(x, t, l, d, drop_scales=drop)
     n, off = ops.router_param_offsets(len(cc), 63 if arch == "crnn" else 64)
     arena = fused.router_grad_arena()
 
-    net = _net(arch, cc, sd, precision)
+    net = synth.build_net(cc, sd, arch=arch, precision=precision, drop_path=True, autograd=True)
     net.train(mode == "train")
     _freeze_experts(net)
     if drop is not None:
@@ -159,7 +130,7 @@ def test_stage0_torch_loop_matches_reference_golden(name, monkeypatch):
     from test_oracle_pinning import pview, stage0_case
     g, cc, B, sd, img, tgt, lens, bn_train, drop = stage0_case(name)
     arch = str(g["arch"]) if "arch" in g else "svtr"
-    net = _net(arch, cc, sd)
+    net = synth.build_net(cc, sd, arch=arch, drop_path=True, autograd=True)
     net.train(bn_train)
     if drop is not None:
         monkeypatch.setattr(M, "sample_drop_scales", lambda n_, b_, rates, dev, generator=None: drop.unsqueeze(0).to(dev))
@@ -272,8 +243,8 @@ def test_autograd_switch_off_is_inert_and_on_keeps_forward_values(arch):
     cc, B, seed = (37, 61, 96), 3, 111
     sd = synth.synth_state_dict(cc, seed, arch=arch)
     x = synth.synth_batch(B, cc, seed)[0].cuda()
-    off = _net(arch, cc, sd, autograd=False)
-    on = _net(arch, cc, sd)
+    off = synth.build_net(cc, sd, arch=arch)
+    on = synth.build_net(cc, sd, arch=arch, autograd=True)
     for n in (off, on):
         n.eval()
     _freeze_experts(on)
@@ -302,12 +273,7 @@ def test_autograd_switch_off_is_inert_and_on_keeps_forward_values(arch):
 # ------------------------------------------------------------------------------------------------ 7. errors
 def test_routed_autograd_refuses_experts_that_require_grad():
     """No device needed: the check runs before any kernel."""
-    from mrn_b200.modules.model import MRNNet
-    opt = _opt("svtr")
-    net = MRNNet(opt)
-    for c in (5, 9):
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
+    net = synth.build_net((5, 9), device=None, autograd=True)
     assert net.dm_router[0].autograd is True
     with pytest.raises(NotImplementedError, match="frozen"):
         net(torch.zeros(1, 4, 32, 256), True, None, True)

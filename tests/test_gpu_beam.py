@@ -2,15 +2,13 @@
 statement of the same selection, the beam kernel against the fp64 oracle (oracle/ctc_beam_oracle.py) and against exact
 labeling probabilities, and MRN.infer_batch(decode="beam") end to end.  Both kernels give every warp one row / one
 sample and are not persistent, so there is no multi-item walk to cover."""
-import argparse
-
 import pytest
 import torch
 
 from oracle import ctc_beam_oracle as BO
 from oracle import mrn_oracle as O
-from oracle import synth
-from conftest import load_golden
+from mrn_b200 import synth
+from golden_cases import golden_case
 
 pytestmark = pytest.mark.gpu
 MLT17 = (1899, 2224, 3844, 4968, 5041, 5153)
@@ -189,33 +187,11 @@ def test_argument_errors_raise_with_the_kernel_message():
         ops.ctc_beam_search(*top, 8, 9)
 
 
-def _learner(arch, name):
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
-    from mrn_b200.modules.model import MRNNet
-    g = load_golden(name)
-    cc = tuple(int(c) for c in g["class_counts"])
-    B, seed = int(g["B"]), int(g["seed"])
-    opt = argparse.Namespace(Transformation="None", FeatureExtraction="SVTR" if arch == "svtr" else "VGG",
-                             SequenceModeling="None" if arch == "svtr" else "BiLSTM", Prediction="CTC", num_fiducial=20,
-                             input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256, batch_max_length=25,
-                             lr=5e-4, num_iter=10000, grad_clip=5, exp_name="test", precision="fp32", drop_path=False,
-                             lan_list=["a", "b", "c", "d", "e", "f"], val_interval=5000, start_task=0, optimizer="adam",
-                             schedule="super")
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    net.load_state_dict(synth.synth_state_dict(cc, seed, arch=arch), strict=True)
-    learner = MRN(opt)
-    learner.model = RankLocal(net.cuda())
-    learner.model.eval()
-    return learner, cc, B
-
-
 @pytest.mark.parametrize("arch,name", [("svtr", "svtr_mrn_i3_b3"), ("crnn", "crnn_mrn_i2_b4")])
 @pytest.mark.parametrize("route", ["TF", "FF"])
 def test_infer_batch_beam_decode(arch, name, route):
-    learner, cc, B = _learner(arch, name)
+    g, cc, B, seed, sd, *_ = golden_case(name)
+    learner = synth.build_learner(synth.build_net(cc, sd, arch=arch), train=False)
     W = 8
     for k in range(2):
         x = synth.synth_batch(B, cc, 70 + k)[0].cuda()

@@ -1,52 +1,22 @@
 """CRNN-MRN (VGG + BiLSTM + CTC, T = 63; config/crnn_mrn.py, BASELINE.json configs[0-1]) on the GPU through the
 reference-facing API, against the golden fixtures produced by the unmodified reference and the CPU oracle."""
-import argparse
-
 import numpy as np
 import pytest
 import torch
 
 from oracle import mrn_oracle as O
-from oracle import synth
-from conftest import load_golden, gview, rel_err
+from mrn_b200 import synth
+from conftest import gview, rel_err
+from golden_cases import golden_case
 
 pytestmark = pytest.mark.gpu
 CASES = ["crnn_mrn_i2_b4", "crnn_mrn_i3_b2"]
 
 
-def make_opt(precision="fp32"):
-    return argparse.Namespace(Transformation="None", FeatureExtraction="VGG", SequenceModeling="BiLSTM", Prediction="CTC",
-                              num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                              batch_max_length=25, lr=5e-4, num_iter=10000, grad_clip=5, exp_name="test", precision=precision,
-                              drop_path=False, lan_list=["a", "b", "c", "d", "e", "f"], val_interval=5000, start_task=0,
-                              optimizer="adam", schedule="super")
-
-
-def build_net(cc, sd, precision="fp32"):
-    from mrn_b200.modules.model import MRNNet
-    opt = make_opt(precision)
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    res = net.load_state_dict(sd, strict=True)
-    assert not res.missing_keys and not res.unexpected_keys
-    return net.cuda(), opt
-
-
-def _case(name):
-    g = load_golden(name)
-    cc = tuple(int(c) for c in g["class_counts"])
-    B, seed = int(g["B"]), int(g["seed"])
-    sd = synth.synth_state_dict(cc, seed, arch="crnn")
-    img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
-    return g, cc, B, seed, sd, img, tgt, lens, dom
-
-
 @pytest.mark.parametrize("name", CASES)
 def test_crnn_forward_matches_reference_golden(name):
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    net = synth.build_net(cc, sd, arch="crnn")
     net.eval()
     x = img.cuda()
     r = net.route_and_combine(x, is_train=True, want_logits=True)
@@ -67,12 +37,8 @@ def test_crnn_forward_matches_reference_golden(name):
 
 @pytest.mark.parametrize("name", CASES)
 def test_crnn_eval_decode_and_loss_match_reference_golden(name):
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    learner = synth.build_learner(synth.build_net(cc, sd, arch="crnn"), train=False)
     r = learner.infer_batch(img.cuda(), "TF", tgt.cuda(), lens.cuda())
     for b in range(B):
         n = int(r["lens"][b])
@@ -86,13 +52,9 @@ def test_crnn_eval_decode_and_loss_match_reference_golden(name):
 def test_crnn_stage1_step_matches_reference_golden(name):
     """Router-training step with T = 63: loss, router gradients, clip + Adam (il_modules/mrn.py:338-367)."""
     from mrn_b200 import ops
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
-    learner.optimizer = FusedAdam(net, 5e-4, 20000, grad_clip=5, schedule="const")
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    net = synth.build_net(cc, sd, arch="crnn")
+    learner = synth.build_learner(net, train=False, total_steps=20000)
     loss_clf, taski = learner.train_step_stage1(img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda())
     assert abs(float(loss_clf) - float(g["loss_clf"])) / abs(float(g["loss_clf"])) < 1e-4
     assert abs(float(taski) - float(g["taski_loss"])) < 1e-4
@@ -110,8 +72,8 @@ def test_crnn_stage1_step_matches_reference_golden(name):
 
 
 def test_crnn_train_mode_batchnorm_matches_reference_golden():
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case("crnn_mrn_i2_b4")
-    net, opt = build_net(cc, sd)
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case("crnn_mrn_i2_b4")
+    net = synth.build_net(cc, sd, arch="crnn")
     net.train()
     r = net.route_and_combine(img.cuda(), is_train=True, want_logits=True)
     assert rel_err(gview(r["features"].cpu(), g), g["train_features"]) < 1e-4
@@ -124,33 +86,16 @@ def test_crnn_train_mode_batchnorm_matches_reference_golden():
     assert int(sd2["model.0.model.FeatureExtraction.ConvNet.12.num_batches_tracked"]) == 1
 
 
-def _random_init_state_dict(cc, seed):
-    from mrn_b200.modules.model import MRNNet
-    torch.manual_seed(seed)
-    opt = make_opt()
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
-    for k in sd:
-        if k.endswith("running_var"):
-            sd[k] = 0.5 + torch.rand_like(sd[k])
-        if k.endswith("running_mean"):
-            sd[k] = 0.1 * torch.randn_like(sd[k])
-    return sd
-
-
 def test_crnn_bf16_mode_within_north_star_budget():
     """Tensor-core mode (implicit-GEMM convolutions on tcgen05, bf16 LSTM GEMMs): logits within 2e-2 relative of the
     fp32 oracle on random-init weights; gate deviation and expert flips reported."""
     cc, B = (37, 61, 96), 4
-    sd = _random_init_state_dict(cc, 9)
+    sd = synth.ctor_state_dict(cc, 9, arch="crnn")
     img, tgt, lens, dom = synth.synth_batch(B, cc, 9)
     with torch.no_grad():
         o = O.mrn_forward(sd, len(cc), img, True, True)
         e = O.mrn_forward(sd, len(cc), img, True, False)
-    net, opt = build_net(cc, sd, precision="bf16")
+    net = synth.build_net(cc, sd, arch="crnn", precision="bf16")
     net.eval()
     out = net(img.cuda(), True, None, True)
     err = rel_err(out["logits"].cpu().numpy(), o["logits"].numpy())
@@ -174,9 +119,9 @@ def test_crnn_persistent_lstm_kernel_matches_per_step_launches(monkeypatch):
     budget of the fp32 oracle on a 4-sample slice.  modules/sequence_modeling.py:12-22."""
     import os
     cc, B = (37, 61), 128
-    sd = _random_init_state_dict(cc, 11)
+    sd = synth.ctor_state_dict(cc, 11, arch="crnn")
     img, tgt, lens, dom = synth.synth_batch(B, cc, 11)
-    net, opt = build_net(cc, sd, precision="bf16")
+    net = synth.build_net(cc, sd, arch="crnn", precision="bf16")
     net.eval()
     x = img.cuda()
     res = {}
@@ -201,7 +146,6 @@ def test_crnn_persistent_lstm_kernel_matches_per_step_launches(monkeypatch):
 def test_crnn_baseline_config0_two_tasks_batch64():
     """BASELINE.json configs[0]: CRNN-MRN forward + CTC loss, 2 tasks (Chinese + Latin class counts), batch 64,
     synthetic 32x256 crops -- the CUDA path against the CPU oracle on the same inputs."""
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
     cc, B = synth.MLT17_CLASS_COUNTS[:2], 64
     sd = synth.synth_state_dict(cc, 17, arch="crnn")
     img, tgt, lens, dom = synth.synth_batch(B, cc, 17)
@@ -211,14 +155,12 @@ def test_crnn_baseline_config0_two_tasks_batch64():
         loss_ref = float(O.ctc_loss_mean(o["logits"], tgt, lens))
         e = O.mrn_forward(sd, 2, img, True, False)
         raw, seqs, conf = O.greedy_decode(e["logits"])
-    net, opt = build_net(cc, sd)
+    net = synth.build_net(cc, sd, arch="crnn")
     net.eval()
     r = net.route_and_combine(img.cuda(), is_train=True, want_logits=True, targets=tgt.cuda(), lengths=lens.cuda())
     assert rel_err(r["logits"].cpu().numpy(), o["logits"].numpy()) < 1e-4
     assert float((r["gate"].cpu() - o["index"]).abs().max()) < 1e-4
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
+    learner = synth.build_learner(net, train=False)
     # CTC loss of the soft-routed logits (forward + loss of configs[0])
     from mrn_b200 import ops
     lat = ops.ctc_lattice(r["lpe"], tgt.cuda(), lens.cuda())
@@ -237,13 +179,9 @@ def test_crnn_stage1_step_bf16_tensor_core_router():
     """bf16 mode runs the T = 63 router on tcgen05 through the 64-frame padded problem; the step must stay within the
     bf16 budget of the reference's loss and router gradients (compared on the caller's un-padded arena)."""
     from mrn_b200 import ops
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case("crnn_mrn_i3_b2")
-    net, opt = build_net(cc, sd, precision="bf16")
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
-    learner.optimizer = FusedAdam(net, 5e-4, 20000, grad_clip=5, schedule="const")
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case("crnn_mrn_i3_b2")
+    net = synth.build_net(cc, sd, arch="crnn", precision="bf16")
+    learner = synth.build_learner(net, train=False, total_steps=20000)
     loss_clf, taski = learner.train_step_stage1(img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda())
     assert abs(float(loss_clf) - float(g["loss_clf"])) / abs(float(g["loss_clf"])) < 2e-2
     assert abs(float(taski) - float(g["taski_loss"])) < 2e-2
@@ -264,16 +202,16 @@ def test_crnn_fused_lstm_cell_path_batch128():
     """B % 128 == 0 in tensor-core mode switches the recurrence to the GEMM with the LSTM cell fused into its epilogue
     (interleaved gate columns); compare the expert outputs with the fp32 oracle and with the unfused fp32 CUDA path."""
     cc, B = (61,), 128
-    sd = _random_init_state_dict(cc, 13)
+    sd = synth.ctor_state_dict(cc, 13, arch="crnn")
     img, tgt, lens, dom = synth.synth_batch(B, cc, 13)
     with torch.no_grad():
         feat, pred = O.expert_forward(sd, 0, img)
-    net16, _ = build_net(cc, sd, precision="bf16")
+    net16 = synth.build_net(cc, sd, arch="crnn", precision="bf16")
     net16.eval()
     one16 = net16.model[0](img.cuda())
     assert rel_err(one16["feature"].cpu().numpy(), feat.numpy()) < 2e-2
     assert rel_err(one16["predict"].cpu().numpy(), pred.numpy()) < 2e-2
-    net32, _ = build_net(cc, sd, precision="fp32")
+    net32 = synth.build_net(cc, sd, arch="crnn", precision="fp32")
     net32.eval()
     one32 = net32.model[0](img[:8].cuda())
     assert rel_err(one32["predict"].cpu().numpy(), pred[:8].numpy()) < 1e-4

@@ -1,6 +1,5 @@
 """2-GPU data-parallel parity: two ranks, each on its shard, all-reduced (NCCL) gradient arena + identical clip/Adam
 == one GPU on the concatenated batch (SURVEY.md §4, §8e).  Skipped on boxes with fewer than 2 GPUs."""
-import argparse
 import os
 import socket
 
@@ -9,29 +8,6 @@ import torch
 import torch.multiprocessing as mp
 
 pytestmark = pytest.mark.gpu
-
-
-def _opt():
-    return argparse.Namespace(Transformation="None", FeatureExtraction="SVTR", SequenceModeling="None", Prediction="CTC",
-                              num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                              batch_max_length=25, lr=5e-4, num_iter=100, grad_clip=5, exp_name="dp", precision="fp32",
-                              drop_path=False, lan_list=["a", "b", "c"], val_interval=50, start_task=0)
-
-
-def _build(cc, sd, dev):
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    from mrn_b200.modules.model import MRNNet
-    opt = _opt()
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    net.load_state_dict(sd, strict=True)
-    net = net.to(dev).eval()
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.optimizer = FusedAdam(net, 5e-4, 200, schedule="const")
-    return net, learner
 
 
 def _worker(rank, world, port, out):
@@ -43,7 +19,8 @@ def _worker(rank, world, port, out):
     cc, B, seed = (37, 61, 96), 4, 21
     sd = synth.synth_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
-    net, learner = _build(cc, sd, dev)
+    net = synth.build_net(cc, sd, device=dev)
+    learner = synth.build_learner(net, train=False, total_steps=200)
     lo, hi = mdist.shard_bounds(B, rank, world)
     l1, l2 = learner.train_step_stage1(img[lo:hi].to(dev), tgt[lo:hi].to(dev), lens[lo:hi].to(dev), dom[lo:hi].to(dev))
     torch.cuda.synchronize()
@@ -62,7 +39,8 @@ def test_two_rank_step_equals_single_gpu_step():
     sd = synth.synth_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     dev = torch.device("cuda", 0)
-    net, learner = _build(cc, sd, dev)
+    net = synth.build_net(cc, sd, device=dev)
+    learner = synth.build_learner(net, train=False, total_steps=200)
     l1, l2 = learner.train_step_stage1(img.to(dev), tgt.to(dev), lens.to(dev), dom.to(dev))
     ref = net.router_arena().cpu()
     a0, a1 = out[0][0], out[1][0]
@@ -82,7 +60,8 @@ def _worker_stage0(rank, world, port, out):
     cc, B, seed = (37, 61), 4, 23
     sd = synth.synth_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
-    net, learner = _build(cc, sd, dev)
+    net = synth.build_net(cc, sd, device=dev)
+    learner = synth.build_learner(net, train=False, total_steps=200)
     learner.opt.schedule = "const"
     learner.begin_expert_training(total_steps=100)
     net.model[-1].eval()                      # running-statistics BatchNorm: shards and the full batch see the same network
@@ -104,7 +83,8 @@ def test_two_rank_stage0_step_equals_single_gpu_step():
     sd = synth.synth_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     dev = torch.device("cuda", 0)
-    net, learner = _build(cc, sd, dev)
+    net = synth.build_net(cc, sd, device=dev)
+    learner = synth.build_learner(net, train=False, total_steps=200)
     learner.opt.schedule = "const"
     learner.begin_expert_training(total_steps=100)
     net.model[-1].eval()

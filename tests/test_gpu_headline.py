@@ -19,22 +19,12 @@ TOL = 2e-2          # BASELINE.json north_star: logits / CTC loss within 2e-2 re
 
 
 def _learner(sd, drop_path=True, precision="bf16"):
+    """The bench's options (bench.make_opt) with DropPath on or off."""
     from bench import make_opt
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    from mrn_b200.modules.model import MRNNet
     opt = make_opt(precision, 0, "svtr")
     opt.drop_path = drop_path
-    net = MRNNet(opt)
-    for c in CC:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    net.load_state_dict(sd, strict=True)
-    net = net.cuda()
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.train()
-    learner.optimizer = FusedAdam(net, 5e-4, 20000, grad_clip=5, schedule="const")
-    return learner, net
+    net = psynth.build_net(CC, sd, opt)
+    return psynth.build_learner(net, total_steps=20000), net
 
 
 def _oracle_step(sd, state, batch, drop):

@@ -7,8 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import synth
-from test_gpu_step import make_opt
+from mrn_b200 import synth
 
 
 N_NEW = (12, 10)           # new characters per task
@@ -70,9 +69,8 @@ class _Valid:
 def test_two_task_incremental_run(tmp_path, monkeypatch):
     from mrn_b200 import tiny_train
     monkeypatch.chdir(tmp_path)
-    opt = make_opt()
-    opt.il, opt.exp_name, opt.lan_list = "mrn", "inc", ["A", "B"]
-    opt.num_iter, opt.val_interval, opt.batch_size, opt.memory, opt.memory_num, opt.drop_path = 4, 10, 4, "random", 8, True
+    opt = synth.make_opt(il="mrn", exp_name="inc", lan_list=["A", "B"], num_iter=4, val_interval=10, batch_size=4,
+                         memory="random", memory_num=8, drop_path=True)
     tiny_train.seed_everything(111)
     mgr = _Manager(opt.batch_size)
     best, ned = tiny_train.train(opt, mgr, lambda k: _Valid(mgr, k), lambda k: _chars(k),

@@ -6,9 +6,8 @@ import pytest
 import torch
 
 from oracle import mrn_oracle as O
-from oracle import synth
+from mrn_b200 import synth
 from conftest import load_golden, gview, rel_err
-from test_gpu_step import build_net, make_opt
 from test_oracle_pinning import STAGE0_CASES, STAGE0_CRNN_CASES, pview, stage0_case
 
 pytestmark = pytest.mark.gpu
@@ -198,10 +197,7 @@ def test_learner_init_train_follows_the_oracle_for_three_iterations(tmp_path, mo
     sd = synth.synth_state_dict(cc, seed, arch=arch)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     tgt[tgt == 2] = 4; tgt[tgt == 3] = 5      # [UNK] / ' ' are multi-character or stripped entries: keep plain characters
-    opt = make_opt()
-    if arch == "crnn":
-        opt.FeatureExtraction, opt.SequenceModeling = "VGG", "BiLSTM"
-    opt.num_iter, opt.val_interval, opt.lan_list, opt.drop_path = 3, 100, ["x"], True
+    opt = synth.make_opt(arch, num_iter=3, val_interval=100, lan_list=["x"], drop_path=True)
     opt.cuda_graph = False                    # eager steps: the injected DropPath masks must be consumed one per iteration
     learner = MRN(opt)
     learner.character = chars
@@ -292,11 +288,7 @@ def test_stage0_cuda_graph_replay_matches_eager(arch):
     batches = [synth.synth_batch(B, cc, 50 + k) for k in range(2)]
     outs = []
     for graphed in (False, True):
-        opt = make_opt()
-        opt.drop_path, opt.num_iter, opt.schedule = False, 100, "const"
-        if arch == "crnn":
-            opt.FeatureExtraction, opt.SequenceModeling = "VGG", "BiLSTM"
-        net, _ = build_net(cc, sd) if arch == "svtr" else (None, None)
+        opt = synth.make_opt(arch, num_iter=100, schedule="const")
         learner = MRN(opt)
         learner.model.update_fc(opt.hidden_size, cc[0]); learner.model.build_prediction(opt, cc[0])
         learner.model.load_state_dict(sd, strict=True)
@@ -326,10 +318,7 @@ def test_stage0_training_reduces_the_loss_on_a_fixed_batch(arch, precision):
     sd = synth.synth_state_dict(cc, 21, arch=arch)
     img, tgt, lens, _ = synth.synth_batch(B, cc, 77)
     lens = lens.clamp(max=8); tgt[:, 8:] = 1
-    opt = make_opt(precision)
-    opt.drop_path, opt.num_iter, opt.schedule, opt.lr = False, 1000, "const", 5e-4
-    if arch == "crnn":
-        opt.FeatureExtraction, opt.SequenceModeling = "VGG", "BiLSTM"
+    opt = synth.make_opt(arch, precision, num_iter=1000, schedule="const")
     learner = MRN(opt)
     learner.model.update_fc(opt.hidden_size, cc[0]); learner.model.build_prediction(opt, cc[0])
     learner.model.load_state_dict(sd, strict=True)

@@ -1,36 +1,15 @@
 """End-to-end GPU parity through the reference-facing API (mrn_b200.modules.model.MRNNet, mrn_b200.il_modules.mrn.MRN)
 against the golden fixtures produced by the unmodified reference and against the CPU oracle."""
-import argparse
-
 import numpy as np
 import pytest
 import torch
 
 from oracle import mrn_oracle as O
-from oracle import synth
-from conftest import load_golden, gview, rel_err
+from mrn_b200 import synth
+from conftest import gview, rel_err
+from golden_cases import golden_case
 
 pytestmark = pytest.mark.gpu
-
-
-def make_opt(precision="fp32"):
-    return argparse.Namespace(Transformation="None", FeatureExtraction="SVTR", SequenceModeling="None", Prediction="CTC",
-                              num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                              batch_max_length=25, lr=5e-4, num_iter=10000, grad_clip=5, exp_name="test", precision=precision,
-                              drop_path=False, lan_list=["a", "b", "c", "d", "e", "f"], val_interval=5000, start_task=0,
-                              optimizer="adam", schedule="super")
-
-
-def build_net(cc, sd, precision="fp32"):
-    from mrn_b200.modules.model import MRNNet
-    opt = make_opt(precision)
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    res = net.load_state_dict(sd, strict=True)          # the state_dict contract (SURVEY.md §8b)
-    assert not res.missing_keys and not res.unexpected_keys
-    return net.cuda(), opt
 
 
 def ref_numel(g, pname):
@@ -40,19 +19,10 @@ def ref_numel(g, pname):
     return int(np.prod(shapes[pname]))
 
 
-def _case(name):
-    g = load_golden(name)
-    cc = tuple(int(c) for c in g["class_counts"])
-    B, seed = int(g["B"]), int(g["seed"])
-    sd = synth.synth_state_dict(cc, seed)
-    img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
-    return g, cc, B, seed, sd, img, tgt, lens, dom
-
-
 @pytest.mark.parametrize("name", ["svtr_mrn_i3_b3", "svtr_mrn_i2_b4"])
 def test_mrnnet_forward_matches_reference_golden(name):
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    net = synth.build_net(cc, sd)
     net.eval()
     x = img.cuda()
     out = net(x, True, None, True)                      # soft route (modules/model.py:397-423)
@@ -67,12 +37,8 @@ def test_mrnnet_forward_matches_reference_golden(name):
 
 @pytest.mark.parametrize("name", ["svtr_mrn_i3_b3", "svtr_mrn_i2_b4"])
 def test_learner_eval_decode_matches_reference_golden(name):
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    learner = synth.build_learner(synth.build_net(cc, sd), train=False)
     r = learner.infer_batch(img.cuda(), "TF", tgt.cuda(), lens.cuda())
     ties = 0
     for b in range(B):
@@ -88,13 +54,9 @@ def test_learner_eval_decode_matches_reference_golden(name):
 def test_stage1_step_matches_reference_golden(name):
     """loss = 15*CTC + CE(gate, domain), router gradients, clip_grad_norm_(5) and one Adam step (il_modules/mrn.py:338-367)."""
     from mrn_b200 import ops
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case(name)
-    net, opt = build_net(cc, sd)
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()                                # the golden step used eval-mode (frozen) experts
-    learner.optimizer = FusedAdam(net, 5e-4, 20000, grad_clip=5, schedule="const")
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case(name)
+    net = synth.build_net(cc, sd)
+    learner = synth.build_learner(net, train=False, total_steps=20000)   # the golden step used eval-mode (frozen) experts
     loss_clf, taski = learner.train_step_stage1(img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda())
     assert abs(float(loss_clf) - float(g["loss_clf"])) / abs(float(g["loss_clf"])) < 1e-4
     assert abs(float(taski) - float(g["taski_loss"])) < 1e-4
@@ -116,8 +78,8 @@ def test_stage1_step_matches_reference_golden(name):
 
 def test_train_mode_experts_match_oracle():
     """BN batch statistics + injected DropPath masks (reference quirk 4) through the module API."""
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case("svtr_mrn_i3_b3")
-    net, opt = build_net(cc, sd)
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case("svtr_mrn_i3_b3")
+    net = synth.build_net(cc, sd)
     net.train()
     drop = synth.synth_drop_scales(len(cc), B, O.svtr_drop_path_rates(), seed)
     r = net.route_and_combine(img.cuda(), is_train=True, want_logits=True, drop_scales=drop.cuda())
@@ -129,36 +91,16 @@ def test_train_mode_experts_match_oracle():
     assert int(sd2["model.0.model.FeatureExtraction.ConvNet.patch_embed.proj.1.num_batches_tracked"]) == 1
 
 
-def _random_init_state_dict(cc, seed):
-    """Random-init weights drawn by the mirror's own constructors, which restate the reference's initialisers
-    (modules/svtr.py:488-498; nn.Linear defaults for the router, modules/model.py:437-452) -- the weight distribution
-    BASELINE.json's tolerances are quoted on."""
-    from mrn_b200.modules.model import MRNNet
-    torch.manual_seed(seed)
-    opt = make_opt()
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
-    for k in sd:                        # non-trivial BN running statistics
-        if k.endswith("running_var"):
-            sd[k] = 0.5 + torch.rand_like(sd[k])
-        if k.endswith("running_mean"):
-            sd[k] = 0.1 * torch.randn_like(sd[k])
-    return sd
-
-
 def test_bf16_mode_within_north_star_budget():
     """bf16 operands / fp32 accumulate for the expert GEMMs: logits within 2e-2 relative of the fp32 oracle on
     random-init weights (BASELINE.json north_star); gate deviation and expert flips are reported."""
     cc, B = (37, 61, 96), 4
-    sd = _random_init_state_dict(cc, 5)
+    sd = synth.ctor_state_dict(cc, 5)
     img, tgt, lens, dom = synth.synth_batch(B, cc, 5)
     with torch.no_grad():
         o = O.mrn_forward(sd, len(cc), img, True, True)
         e = O.mrn_forward(sd, len(cc), img, True, False)
-    net, opt = build_net(cc, sd, precision="bf16")
+    net = synth.build_net(cc, sd, precision="bf16")
     net.eval()
     out = net(img.cuda(), True, None, True)
     assert rel_err(out["logits"].cpu().numpy(), o["logits"].numpy()) < 2e-2           # logits within 2e-2 in bf16
@@ -168,7 +110,7 @@ def test_bf16_mode_within_north_star_budget():
     print("bf16: gate max abs deviation %.2e, expert flips %d of %d" % (gate_dev, flips, B))
     assert gate_dev < 2e-2
     # fp32 mode on the same weights meets the fp32 tolerances
-    net32, _ = build_net(cc, sd, precision="fp32")
+    net32 = synth.build_net(cc, sd, precision="fp32")
     net32.eval()
     out32 = net32(img.cuda(), True, None, True)
     assert rel_err(out32["logits"].cpu().numpy(), o["logits"].numpy()) < 1e-4
@@ -182,7 +124,7 @@ def test_full_size_properties_6_experts():
     cc = synth.MLT17_CLASS_COUNTS
     sd = synth.synth_state_dict(cc, 3)
     img, tgt, lens, dom = synth.synth_batch(32, cc, 3)
-    net, opt = build_net(cc, sd, precision="bf16")
+    net = synth.build_net(cc, sd, precision="bf16")
     net.eval()
     x = img.cuda()
     r = net.route_and_combine(x, is_train=True, want_logits=True, targets=tgt.cuda(), lengths=lens.cuda(), want_E=True,
@@ -210,12 +152,8 @@ def test_full_size_properties_6_experts():
 def test_infer_batch_cuda_graph_replay_matches_eager():
     """The per-batch-size CUDA graph of the hard-routed inference call returns exactly what the eager call returns, for
     fresh inputs on every replay."""
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case("svtr_mrn_i3_b3")
-    net, opt = build_net(cc, sd)
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case("svtr_mrn_i3_b3")
+    learner = synth.build_learner(synth.build_net(cc, sd), train=False)
     for k in range(3):
         x = synth.synth_batch(B, cc, 50 + k)[0].cuda()
         eager = learner.infer_batch(x, "TF")
@@ -230,15 +168,11 @@ def test_infer_batch_cuda_graph_replay_matches_eager():
 def test_train_step_cuda_graph_replay_matches_eager():
     """Stage-1 steps replayed from the CUDA graph update the router exactly like eager steps on the same batches
     (eval-mode experts: no DropPath randomness)."""
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
-    g, cc, B, seed, sd, img, tgt, lens, dom = _case("svtr_mrn_i2_b4")
+    g, cc, B, seed, sd, img, tgt, lens, dom = golden_case("svtr_mrn_i2_b4")
     arenas, losses = [], []
     for graphed in (False, True):
-        net, opt = build_net(cc, sd)
-        learner = MRN(opt)
-        learner.model = RankLocal(net)
-        learner.model.eval()
-        learner.optimizer = FusedAdam(net, 5e-4, 100, grad_clip=5, schedule="super")
+        net = synth.build_net(cc, sd)
+        learner = synth.build_learner(net, train=False, total_steps=100, schedule="super")
         step = learner.train_step_stage1_graphed if graphed else learner.train_step_stage1
         ls = []
         for k in range(4):
@@ -277,7 +211,7 @@ def test_bf16_train_mode_experts_match_oracle(weights):
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     drop = synth.synth_drop_scales(len(cc), B, O.svtr_drop_path_rates(), seed)
     ref, preds = _oracle_stage1(sd, cc, img, tgt, lens, dom, "batch", drop)
-    net, opt = build_net(cc, sd, precision="bf16")
+    net = synth.build_net(cc, sd, precision="bf16")
     net.train()
     r = net.route_and_combine(img.cuda(), is_train=True, want_logits=True, drop_scales=drop.cuda())
     for i, z in enumerate(r["expert_logits"]):
@@ -295,16 +229,12 @@ def test_bf16_stage1_step_matches_oracle():
     """bf16 twin of test_stage1_step_matches_reference_golden on random-init weights: losses within 2e-2, router
     gradients (bf16 router GEMMs, fp32 accumulation) within 5e-2 of the fp32 oracle's, grad norm within 2e-2."""
     from mrn_b200 import ops
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
     cc, B, seed = (37, 61, 96), 4, 7
     sd = synth.ctor_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     ref, _ = _oracle_stage1(sd, cc, img, tgt, lens, dom, "eval", None)
-    net, opt = build_net(cc, sd, precision="bf16")
-    learner = MRN(opt)
-    learner.model = RankLocal(net)
-    learner.model.eval()
-    learner.optimizer = FusedAdam(net, 5e-4, 20000, grad_clip=5, schedule="const")
+    net = synth.build_net(cc, sd, precision="bf16")
+    learner = synth.build_learner(net, train=False, total_steps=20000)
     loss_clf, taski = learner.train_step_stage1(img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda())
     assert abs(float(loss_clf) - float(ref["loss_clf"])) / abs(float(ref["loss_clf"])) < 2e-2
     assert abs(float(taski) - float(ref["taski_loss"])) < 2e-2
@@ -328,7 +258,7 @@ def test_mixed_expert_modes_follow_each_modules_flag():
     cc, B, seed = (37, 61, 96), 3, 111
     sd = synth.synth_state_dict(cc, seed)
     img = synth.synth_batch(B, cc, seed)[0]
-    net, opt = build_net(cc, sd)
+    net = synth.build_net(cc, sd)
     net.train()
     net.model[-1].eval()
     assert net._experts_train_mode() == (True, True, False)

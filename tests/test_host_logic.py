@@ -10,15 +10,6 @@ from oracle import mrn_oracle as O
 from oracle.ref_import import reference_available
 
 
-def make_opt(**kw):
-    d = dict(Transformation="None", FeatureExtraction="SVTR", SequenceModeling="None", Prediction="CTC", num_fiducial=20,
-             input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256, batch_max_length=25, lr=5e-4,
-             num_iter=100, grad_clip=5, exp_name="t", precision="fp32", drop_path=False, lan_list=["a", "b"],
-             val_interval=50, start_task=0)
-    d.update(kw)
-    return argparse.Namespace(**d)
-
-
 def test_ctc_label_converter_matches_reference_semantics():
     from mrn_b200.utils import CTCLabelConverter
     chars = list("abcdefg") + ["中", "文"]
@@ -54,7 +45,7 @@ def test_module_tree_keeps_the_reference_state_dict_contract():
     from mrn_b200.il_modules.mrn import RankLocal
     from mrn_b200.modules.model import MRNNet
     cc = (37, 61, 96)
-    opt = make_opt()
+    opt = synth.make_opt()
     net = MRNNet(opt)
     for i, c in enumerate(cc):
         net.update_fc(opt.hidden_size, c)
@@ -83,7 +74,7 @@ def test_module_tree_keeps_the_reference_state_dict_contract():
 def test_crnn_module_tree_keeps_the_reference_state_dict_contract():
     from mrn_b200.modules.model import MRNNet
     cc = (37, 61)
-    opt = make_opt(FeatureExtraction="VGG", SequenceModeling="BiLSTM")
+    opt = synth.make_opt("crnn")
     net = MRNNet(opt)
     for c in cc:
         net.update_fc(opt.hidden_size, c)
@@ -97,12 +88,8 @@ def test_crnn_module_tree_keeps_the_reference_state_dict_contract():
 
 
 def test_router_arena_views_share_storage():
-    from mrn_b200.modules.model import MRNNet
     from mrn_b200 import ops
-    opt = make_opt()
-    net = MRNNet(opt)
-    for c in (20, 30):
-        net.update_fc(256, c); net.build_prediction(opt, c)
+    net = synth.build_net((20, 30), device=None)
     arena = net.router_arena("cpu")
     n, off = ops.router_param_offsets(2)
     assert arena.numel() == n
@@ -115,21 +102,19 @@ def test_router_arena_views_share_storage():
 
 def test_no_cpu_fallback_and_unsupported_configs_fail_loudly():
     from mrn_b200.modules.model import MRNNet, Model
-    opt = make_opt()
-    net = MRNNet(opt)
-    net.update_fc(256, 12); net.build_prediction(opt, 12)
+    net = synth.build_net((12,), device=None)
     with pytest.raises(RuntimeError, match="no CPU fallback|CUDA"):
         net(torch.zeros(1, 4, 32, 256), True, None, True)
     with pytest.raises(NotImplementedError):
-        MRNNet(make_opt(FeatureExtraction="ResNet", SequenceModeling="BiLSTM"))
+        MRNNet(synth.make_opt(FeatureExtraction="ResNet", SequenceModeling="BiLSTM"))
     with pytest.raises(NotImplementedError):
-        MRNNet(make_opt(Transformation="TPS"))
+        MRNNet(synth.make_opt(Transformation="TPS"))
     with pytest.raises(NotImplementedError):
-        Model(make_opt(Prediction="Attn"))
+        Model(synth.make_opt(Prediction="Attn"))
     from mrn_b200.il_modules.mrn import MRN
     if not torch.cuda.is_available():
         with pytest.raises(RuntimeError, match="CUDA"):
-            MRN(opt)
+            MRN(net.opt)
 
 
 # ---- stage-0 training arenas, driver glue (host logic only) ---------------------------------------------------------
@@ -214,13 +199,9 @@ def test_model_eval_and_train_and_freeze_step1_set_the_reference_modes():
     again -- the earlier experts are back in TRAIN mode, the reference's quirk the stage-1 step reproduces -- and freezes
     the newest expert in eval mode while the router modules stay trainable."""
     from mrn_b200.il_modules.mrn import MRN
-    from mrn_b200.modules.model import MRNNet
-    opt = make_opt()
-    net = MRNNet(opt)
-    for c in (12, 20):
-        net.update_fc(256, c); net.build_prediction(opt, c)
+    net = synth.build_net((12, 20), device=None)
     learner = MRN.__new__(MRN)                      # host logic only: no device
-    learner.opt = opt
+    learner.opt = net.opt
     learner.model = net
     net.eval()
     learner.model_eval_and_train(1)

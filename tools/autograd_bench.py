@@ -26,22 +26,9 @@ import torch  # noqa: E402
 import torch.nn.functional as F  # noqa: E402
 
 
-def _opt(autograd):
-    return argparse.Namespace(Transformation="None", FeatureExtraction="SVTR", SequenceModeling="None", Prediction="CTC",
-                              num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                              batch_max_length=25, lr=5e-4, num_iter=10000, grad_clip=5, exp_name="bench", precision="bf16",
-                              drop_path=False, lan_list=list("abcdef"), val_interval=5000, start_task=0, autograd=autograd)
-
-
-def _net(cc, sd, autograd):
-    from mrn_b200.modules.model import MRNNet
-    opt = _opt(autograd)
-    net = MRNNet(opt)
-    for c in cc:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    net.load_state_dict(sd, strict=True)
-    net = net.cuda().eval()
+def _frozen_net(cc, sd, autograd):
+    from mrn_b200 import synth
+    net = synth.build_net(cc, sd, precision="bf16", autograd=autograd).eval()
     for p in net.model.parameters():
         p.requires_grad = False
     return net
@@ -74,18 +61,14 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("autograd_bench.py needs a CUDA device")
     from mrn_b200 import ops, synth
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
     cc, B, seed = synth.MLT17_CLASS_COUNTS, args.batch, 3
     sd = synth.ctor_state_dict(cc, seed)
     img, tgt, lens, dom = synth.synth_batch(B, cc, seed)
     x, t, l, d = img.cuda(), tgt.cuda(), lens.cuda(), dom.cuda()
 
-    fused = _net(cc, sd, False)
-    learner = MRN(fused.opt)
-    learner.model = RankLocal(fused)
-    learner.optimizer = FusedAdam(fused, 5e-4, 10 ** 6, grad_clip=5, schedule="const")
+    learner = synth.build_learner(_frozen_net(cc, sd, False), train=False, total_steps=10 ** 6)
 
-    net = _net(cc, sd, True)
+    net = _frozen_net(cc, sd, True)
     params = net.router_parameters()
     adam = torch.optim.Adam(params, lr=5e-4)
     T = net.patch

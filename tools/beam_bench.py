@@ -81,22 +81,8 @@ def kernels(B, T, iters):
 
 
 def infer(B, rounds, steps):
-    from mrn_b200.il_modules.mrn import MRN, RankLocal
-    from mrn_b200.modules.model import MRNNet
-    opt = argparse.Namespace(Transformation="None", FeatureExtraction="SVTR", SequenceModeling="None", Prediction="CTC",
-                             num_fiducial=20, input_channel=4, output_channel=512, hidden_size=256, imgH=32, imgW=256,
-                             batch_max_length=25, lr=5e-4, num_iter=10000, grad_clip=5, exp_name="beam_bench",
-                             precision="bf16", drop_path=True, expert_chunk=0,
-                             lan_list=["Chinese", "Latin", "Japanese", "Korean", "Arabic", "Bangla"], val_interval=5000,
-                             start_task=0, optimizer="adam", schedule="super")
-    net = MRNNet(opt)
-    for c in CLASS_COUNTS:
-        net.update_fc(opt.hidden_size, c)
-        net.build_prediction(opt, c)
-    net.load_state_dict(synth.synth_state_dict(CLASS_COUNTS, 111), strict=True)
-    learner = MRN(opt)
-    learner.model = RankLocal(net.cuda())
-    learner.model.eval()
+    net = synth.build_net(CLASS_COUNTS, synth.synth_state_dict(CLASS_COUNTS, 111), precision="bf16")
+    learner = synth.build_learner(net, train=False)
     imgs = [synth.synth_batch(B, CLASS_COUNTS, 2000 + k)[0].cuda() for k in range(2)]
     modes = {"greedy": dict(decode="greedy"), "beam_w8": dict(decode="beam", beam_width=8, beam_topk=K)}
     ms = {m: [] for m in modes}

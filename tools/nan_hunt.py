@@ -19,7 +19,7 @@ import torch  # noqa: E402
 from bench import CLASS_COUNTS, make_opt  # noqa: E402
 from mrn_b200 import _lib as L  # noqa: E402
 from mrn_b200 import ops, synth  # noqa: E402
-from mrn_b200.modules.model import MRNNet, sample_drop_scales  # noqa: E402
+from mrn_b200.modules.model import sample_drop_scales  # noqa: E402
 
 
 def fin(t):
@@ -42,17 +42,12 @@ def main():
     B = a.batch
     nets = {}
     for prec in ("bf16", "fp32"):
-        opt = make_opt(prec, 0, "svtr")
-        torch.manual_seed(111)
-        net = MRNNet(opt)
-        for c in CLASS_COUNTS:
-            net.update_fc(opt.hidden_size, c)
-            net.build_prediction(opt, c)
         if a.init == "synth":
-            net.load_state_dict(synth.synth_state_dict(CLASS_COUNTS, 111, arch="svtr"), strict=True)
-        elif prec == "fp32":
-            net.load_state_dict(nets["bf16"].state_dict(), strict=True)
-        nets[prec] = net.to(dev)
+            sd = synth.synth_state_dict(CLASS_COUNTS, 111, arch="svtr")
+        else:                                   # ctor: the bf16 net's constructor draws, shared by the fp32 net
+            sd = nets["bf16"].state_dict() if prec == "fp32" else None
+        torch.manual_seed(111)
+        nets[prec] = synth.build_net(CLASS_COUNTS, sd, make_opt(prec, 0, "svtr"), device=dev)
     rates = nets["bf16"].model[0].model.FeatureExtraction.ConvNet.drop_path_rates()
     for mode in ("eval", "train_nodrop", "train_drop"):
         for k in range(2):
@@ -107,19 +102,10 @@ def main():
 
 
     # ---- the learner's step, eager then graphed, losses of every step
-    from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam
     for graphed in (False, True):
         opt = make_opt("bf16", 0, "svtr")
-        net = MRNNet(opt)
-        for c in CLASS_COUNTS:
-            net.update_fc(opt.hidden_size, c)
-            net.build_prediction(opt, c)
-        net.load_state_dict(nets["bf16"].state_dict(), strict=True)
-        net = net.to(dev)
-        learner = MRN(opt)
-        learner.model = RankLocal(net)
-        learner.model.train()
-        learner.optimizer = FusedAdam(net, opt.lr, opt.num_iter * 2, grad_clip=opt.grad_clip, schedule="super")
+        net = synth.build_net(CLASS_COUNTS, nets["bf16"].state_dict(), opt, device=dev)
+        learner = synth.build_learner(net, total_steps=opt.num_iter * 2, schedule="super")
         losses = []
         for k in range(10):
             img, tgt, lens, dom = (t.to(dev) for t in synth.synth_batch(B, CLASS_COUNTS, 1000 + k % 4))

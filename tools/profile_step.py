@@ -14,25 +14,14 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 from bench import CLASS_COUNTS, make_opt  # noqa: E402
 from mrn_b200 import synth  # noqa: E402
-from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam  # noqa: E402
-from mrn_b200.modules.model import MRNNet  # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--steps", type=int, default=2)
 ap.add_argument("--batch", type=int, default=256)
 ap.add_argument("--mode", default="train", choices=["train", "infer"])
 a = ap.parse_args()
-opt = make_opt("bf16", 0, "svtr")
-net = MRNNet(opt)
-for c in CLASS_COUNTS:
-    net.update_fc(opt.hidden_size, c)
-    net.build_prediction(opt, c)
-net.load_state_dict(synth.ctor_state_dict(CLASS_COUNTS, 111), strict=True)
-net = net.cuda()
-learner = MRN(opt)
-learner.model = RankLocal(net)
-learner.model.train() if a.mode == "train" else learner.model.eval()
-learner.optimizer = FusedAdam(net, opt.lr, 20000, grad_clip=5, schedule="super")
+net = synth.build_net(CLASS_COUNTS, synth.ctor_state_dict(CLASS_COUNTS, 111), make_opt("bf16", 0, "svtr"))
+learner = synth.build_learner(net, train=a.mode == "train", total_steps=20000, schedule="super")
 batches = [tuple(t.cuda() for t in synth.synth_batch(a.batch, CLASS_COUNTS, 1000 + k)) for k in range(2)]
 
 

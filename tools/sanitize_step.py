@@ -9,22 +9,11 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 from bench import CLASS_COUNTS, make_opt  # noqa: E402
 from mrn_b200 import synth  # noqa: E402
-from mrn_b200.il_modules.mrn import MRN, RankLocal, FusedAdam  # noqa: E402
-from mrn_b200.modules.model import MRNNet  # noqa: E402
 
 ARCH = os.environ.get("ARCH", "svtr")
 B = int(os.environ.get("B", 4))
-opt = make_opt("bf16", 0, ARCH)
-net = MRNNet(opt)
-for c in CLASS_COUNTS:
-    net.update_fc(opt.hidden_size, c)
-    net.build_prediction(opt, c)
-net.load_state_dict(synth.ctor_state_dict(CLASS_COUNTS, 111, arch=ARCH), strict=True)
-net = net.cuda()
-learner = MRN(opt)
-learner.model = RankLocal(net)
-learner.model.train()
-learner.optimizer = FusedAdam(net, opt.lr, 100, grad_clip=5, schedule="const")
+net = synth.build_net(CLASS_COUNTS, synth.ctor_state_dict(CLASS_COUNTS, 111, arch=ARCH), make_opt("bf16", 0, ARCH))
+learner = synth.build_learner(net, total_steps=100)
 img, tgt, lens, dom = (t.cuda() for t in synth.synth_batch(B, CLASS_COUNTS, 1000))
 l1, l2 = learner.train_step_stage1(img, tgt, lens, dom)
 learner.model.eval()
