@@ -337,9 +337,9 @@ def test_stage0_training_reduces_the_loss_on_a_fixed_batch(arch, precision):
 
 @pytest.mark.parametrize("arch", ["svtr", "crnn"])
 def test_stage0_full_size_properties(arch):
-    """BASELINE.json's full size (B = 256, union charset C = 5153, bf16 tensor-core mode), where the oracle is too slow:
-    size-independent properties of the step.  (1) softmax - occupancy sums to zero over the classes of every frame, so
-    the fc.bias gradient sums to zero; (2) the gradient of the mean loss is linear in the per-sample weights: the step
+    """BASELINE.json's full size (B = 256, union charset C = 5153, bf16 tensor-core mode): size-independent properties
+    of the step, which hold without a reference (test_gpu_stage0_scale.py compares this size with the fp64 oracle).
+    (1) softmax - occupancy sums to zero over the classes of every frame, so the fc.bias gradient sums to zero; (2) the gradient of the mean loss is linear in the per-sample weights: the step
     on the batch equals the average of the steps on its two halves for every parameter that does not see batch
     statistics (eval-mode BatchNorm); (3) two runs agree up to the order of the split-K reductions."""
     from mrn_b200 import ops
