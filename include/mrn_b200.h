@@ -137,6 +137,20 @@ int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads
                              long ld_dlogits, int B, int prec, int bn_batch_stats, const float* drop_scales,
                              float* grad_arena, long n_arena, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
+/* The same two calls with the expert's feature exposed, for joint expert + router training through MRNNet's soft route
+ * (modules/model.py:397-423 with nothing detached between the experts and the DM-Router; the two entries above are these
+ * with NULL).  features: NULL or [B,64,256] fp32 (dense), the SequenceModeling Linear's output f (modules/model.py:141);
+ * in bf16 mode the bf16 value the classifier head reads, widened.  dfeatures: NULL or [B,64,256] fp32 (dense), a
+ * gradient dL/df from outside the expert (the DM-Router's input gradient), added to dlogits . W_fc before anything
+ * downstream reads it. */
+int mrnb_svtr_train_forward_features(const MrnbSvtrPack* pack, const float* image, int B, int prec, int bn_batch_stats,
+                                     int update_running, const float* drop_scales, float* logits, long ld_logits,
+                                     float* features, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+int mrnb_svtr_train_backward_features(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
+                                      const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                      int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
+                                      void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * CRNN expert recognisers (VGG + 2 x BidirectionalLSTM + CTC head), T = 63 frames.
  * Replaces modules/feature_extraction.py:19-47 (VGG_FeatureExtractor.forward), modules/sequence_modeling.py:12-22
@@ -250,6 +264,14 @@ int mrnb_crnn_train_forward(const MrnbCrnnTrainPack* pack, const float* image, i
 int mrnb_crnn_train_backward(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads, const float* dlogits,
                              long ld_dlogits, int B, int prec, int bn_batch_stats, float* grad_arena, long n_arena,
                              void* workspace, size_t workspace_bytes, cudaStream_t stream);
+/* As for SVTR: features / dfeatures NULL or [B,63,256] fp32 (dense), the second BiLSTM's output (modules/model.py:141). */
+int mrnb_crnn_train_forward_features(const MrnbCrnnTrainPack* pack, const float* image, int B, int prec, int bn_batch_stats,
+                                     int update_running, float* logits, long ld_logits, float* features, void* workspace,
+                                     size_t workspace_bytes, cudaStream_t stream);
+int mrnb_crnn_train_backward_features(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads, const float* dlogits,
+                                      long ld_dlogits, const float* dfeatures, int B, int prec, int bn_batch_stats,
+                                      float* grad_arena, long n_arena, void* workspace, size_t workspace_bytes,
+                                      cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * DM-Router + gate head.   Replaces modules/dm_router.py:50-67 (DM_Router.forward, both gating blocks) and
@@ -283,6 +305,15 @@ int mrnb_router_backward(const float* params, const float* x, const float* gate,
                          const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
                          float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
+/* mrnb_router_backward plus the input gradient dx [B,I,T,D] fp32 = dL/dx through the gate head and the DM-Router (both
+ * residuals included): the gradient reaching the experts' features when they are trained with the router
+ * (modules/model.py:400-406 with nothing detached).  Parameter gradients as mrnb_router_backward's; in bf16 mode they
+ * come from the materialised d_out (the generic DM-Router backward), not the rank-one gate-head path, so they agree
+ * with mrnb_router_backward's within the bf16 budget rather than bitwise. */
+int mrnb_router_backward_dx(const float* params, const float* x, const float* gate, const float* dgate_ctc,
+                            const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads, float* dx,
+                            float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* DM_Router alone with an explicit upstream gradient (tests): d_out [B,I,T,D] -> grads of the dm_router.0.*
  * slots (4..19) and, if dx != NULL, the input gradient. */
 int mrnb_dm_router_backward(const float* params, const float* x, const float* d_out, int B, int n_experts, int T, int D,
@@ -314,6 +345,14 @@ size_t mrnb_gate_combine_backward_workspace_bytes(int B, int T, int n_experts);
 int mrnb_gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
                                const float* dY, long ldy, float* dgate, void* workspace, size_t workspace_bytes,
                                cudaStream_t stream);
+/* mrnb_gate_combine_backward plus the per-expert logit gradients in the same pass (trainable experts,
+ * modules/model.py:410-423 differentiated w.r.t. z_i):  dz_i[b,t,c] = gate[b,i] * dY[b,t,c] for c < Ci[i].
+ * gate [B,I]; dz, ldz HOST arrays [n_experts]: dz[i] = NULL skips expert i (frozen), otherwise [B,T,ldz[i]] fp32,
+ * 16-byte aligned, ldz[i] >= Ci[i] a multiple of 4; columns Ci[i]..ldz[i] are never written.  dgate is bitwise the
+ * value mrnb_gate_combine_backward returns. */
+int mrnb_gate_combine_backward_experts(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
+                                       const float* dY, long ldy, const float* gate, float* const* dz, const long* ldz,
+                                       float* dgate, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 /* CTC alpha-beta over all T frames, blank 0.  nll [B] (0 where infeasible: zero_infinity), loss_mean = mean_b(nll_b /
  * max(len_b,1)).  Optional: dgate [B,I] = grad_scale/max(len,1) * sum_t(E_i - sum_s occ_s * zlab_i[ext_s])  (pass

@@ -87,10 +87,16 @@ _SIGNATURES = {
     "mrnb_svtr_train_forward": (_i, [C.POINTER(MrnbSvtrPack), _vp, _i, _i, _i, _i, _vp, _vp, _l, _vp, _sz, _vp]),
     "mrnb_svtr_train_backward": (_i, [C.POINTER(MrnbSvtrPack), C.POINTER(MrnbSvtrPack), _vp, _vp, _l, _i, _i, _i, _vp,
                                       _vp, _l, _vp, _sz, _vp]),
+    "mrnb_svtr_train_forward_features": (_i, [C.POINTER(MrnbSvtrPack), _vp, _i, _i, _i, _i, _vp, _vp, _l, _vp, _vp, _sz, _vp]),
+    "mrnb_svtr_train_backward_features": (_i, [C.POINTER(MrnbSvtrPack), C.POINTER(MrnbSvtrPack), _vp, _vp, _l, _vp, _i, _i,
+                                               _i, _vp, _vp, _l, _vp, _sz, _vp]),
     "mrnb_crnn_train_workspace_bytes": (_sz, [_i, _i, _i]),
     "mrnb_crnn_train_forward": (_i, [C.POINTER(MrnbCrnnTrainPack), _vp, _i, _i, _i, _i, _vp, _l, _vp, _sz, _vp]),
     "mrnb_crnn_train_backward": (_i, [C.POINTER(MrnbCrnnTrainPack), C.POINTER(MrnbCrnnTrainPack), _vp, _l, _i, _i, _i, _vp,
                                       _l, _vp, _sz, _vp]),
+    "mrnb_crnn_train_forward_features": (_i, [C.POINTER(MrnbCrnnTrainPack), _vp, _i, _i, _i, _i, _vp, _l, _vp, _vp, _sz, _vp]),
+    "mrnb_crnn_train_backward_features": (_i, [C.POINTER(MrnbCrnnTrainPack), C.POINTER(MrnbCrnnTrainPack), _vp, _l, _vp, _i,
+                                               _i, _i, _vp, _l, _vp, _sz, _vp]),
     "mrnb_crnn_workspace_bytes": (_sz, [_i, _i, _i]),
     "mrnb_crnn_experts_forward": (_i, [C.POINTER(MrnbCrnnPack), _vp, _i, _i, _i, _i, _vp, C.POINTER(_vp), C.POINTER(_l),
                                        _vp, _sz, _vp]),
@@ -98,12 +104,15 @@ _SIGNATURES = {
     "mrnb_router_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "mrnb_router_forward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mrnb_router_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "mrnb_router_backward_dx": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mrnb_dm_router_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "mrnb_gate_combine": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _vp, _i, _i, _vp, _l, _vp, _vp, _vp,
                                _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "mrnb_gate_combine_backward_workspace_bytes": (_sz, [_i, _i, _i]),
     "mrnb_gate_combine_backward": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _i, _i, _vp, _l, _vp, _vp, _sz,
                                         _vp]),
+    "mrnb_gate_combine_backward_experts": (_i, [C.POINTER(_vp), C.POINTER(_l), C.POINTER(_i), _i, _i, _i, _vp, _l, _vp,
+                                                C.POINTER(_vp), C.POINTER(_l), _vp, _vp, _sz, _vp]),
     "mrnb_ctc_lattice": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp, _vp]),
     "mrnb_ctc_dense_grad": (_i, [_vp, _l, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp, _l, _vp]),
     "mrnb_greedy_decode": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),

@@ -6,7 +6,10 @@ once_differentiable: a double backward raises.
 
   * RoutedSoft: MRNNet's soft route (experts -> DM-Router -> gate -> combine).  Gradients reach route.*,
     channel_route.* and dm_router.0.* through mrnb_gate_combine_backward and mrnb_router_backward (domain = NULL).
-    The experts are frozen, as in MRN stage 1 (il_modules/mrn.py:154-157,285-287).
+    The experts are frozen, as in MRN stage 1 (il_modules/mrn.py:154-157,285-287) -- unless opt.autograd_experts names
+    trainable experts: those run their training packs, and the backward is mrnb_gate_combine_backward_experts (dgate
+    and each trainable expert's logit gradient dz_i = g_i dY in one pass), mrnb_router_backward_dx (the router's input
+    gradient dx) and one training-pack backward per trainable expert with dz_i and dx[:, i] as the feature gradient.
   * ExpertTrain: one expert end to end through its training pack (activation-keeping forward, full backward).
   * DmRouter: DM_Router on its own through mrnb_dm_router_backward (input and parameter gradients).
 """
@@ -23,14 +26,27 @@ def _arena_grads(grads, params, names, n_experts, T, D):
     return tuple(grads[off[slot[n]]:off[slot[n]] + p.numel()].view(p.shape) for n, p in zip(names, params))
 
 
+def _expert_grads(grads, keys):
+    """{state_dict key: gradient} of a training-pack backward -> one tensor (or None: a tensor the forward never reads)
+    per key, copied: the pack's gradient arena is overwritten by another backward through the same graph."""
+    return tuple(None if grads.get(k) is None else grads[k].clone(memory_format=torch.contiguous_format) for k in keys)
+
+
 class RoutedSoft(torch.autograd.Function):
-    """(net, image, *net.router_parameters()) -> (combined logits [B,T,C], gate [B,I])."""
+    """(net, image, trainable, *net.router_parameters(), *parameters of the trainable experts in order) ->
+    (combined logits [B,T,C], gate [B,I]).  trainable: indices of the experts that train with the router (empty: the
+    experts are frozen and run the grouped forward alone)."""
 
     @staticmethod
-    def forward(ctx, net, image, *params):
+    def forward(ctx, net, image, trainable, *params):
         rws = ops.RouterWorkspace()          # the backward reads the activations this forward leaves in it
-        r = net.route_and_combine(image, is_train=True, want_logits=True, with_backward=True, rws=rws)
-        ctx.net, ctx.rws = net, rws
+        experts_out, ctx.expert_backward = None, {}
+        if trainable:
+            feats, logits, ctx.expert_backward = net.joint_experts_forward(image, trainable)
+            experts_out = (feats, logits)
+        r = net.route_and_combine(image, is_train=True, want_logits=True, with_backward=True, rws=rws,
+                                  experts_out=experts_out)
+        ctx.net, ctx.rws, ctx.trainable = net, rws, trainable
         ctx.expert_logits = r["expert_logits"]
         ctx.save_for_backward(net.router_arena(), r["features"], r["gate"])
         return r["logits"], r["gate"]
@@ -40,37 +56,45 @@ class RoutedSoft(torch.autograd.Function):
     def backward(ctx, d_logits, d_gate):
         from .modules.model import _precision
         arena, feats, gate = ctx.saved_tensors
-        net = ctx.net
+        net, trainable = ctx.net, ctx.trainable
         B, I, T, D = feats.shape
+        dz = [None] * I
+        for e in trainable:                  # rows padded to 4 floats, as the kernel writes them
+            z = ctx.expert_logits[e]
+            dz[e] = torch.zeros(B, T, ops.round_up(z.shape[2], 4), device=z.device)[:, :, :z.shape[2]]
         dgate = torch.zeros_like(gate)
         if d_logits is not None:
-            dgate = ops.gate_combine_backward(ctx.expert_logits, d_logits.float())
+            if trainable:
+                dgate = ops.gate_combine_backward_experts(ctx.expert_logits, d_logits.float(), gate, dz)
+            else:
+                dgate = ops.gate_combine_backward(ctx.expert_logits, d_logits.float())
         if d_gate is not None:
             dgate = dgate + d_gate.float()
         grads = torch.empty_like(arena)
-        ops.router_backward(arena, feats, gate, dgate.contiguous(), None, grads, ctx.rws, prec=_precision(net.opt))
-        params = net.router_parameters()
-        return (None, None) + _arena_grads(grads, params, ops.ROUTER_PARAM_NAMES, I, T, D)
+        dx = torch.empty_like(feats) if trainable else None
+        ops.router_backward(arena, feats, gate, dgate.contiguous(), None, grads, ctx.rws, prec=_precision(net.opt), dx=dx)
+        out = _arena_grads(grads, net.router_parameters(), ops.ROUTER_PARAM_NAMES, I, T, D)
+        for e in trainable:
+            keys = [k for k, _ in net.model[e].named_parameters()]
+            out += _expert_grads(ctx.expert_backward[e](dz[e], dx[:, e].contiguous()), keys)
+        return (None, None, None) + out
 
 
 class ExpertTrain(torch.autograd.Function):
-    """(run, keys, image, *params) -> logits [B,T,C].  `run(image)` runs the expert's training-pack forward and returns
-    (backward, logits), backward(dlogits) -> {state_dict key: gradient in the reference layout}; `params` are the
-    expert's parameters named by `keys`."""
+    """(run, keys, image, *params) -> logits [B,T,C].  `run(image)` is modules.model._train_pack_run for one expert:
+    (logits, features, backward), backward(dlogits) -> {state_dict key: gradient in the reference layout}; `params`
+    are the expert's parameters named by `keys`."""
 
     @staticmethod
     def forward(ctx, run, keys, image, *params):
-        backward, logits = run(image)
+        logits, _, backward = run(image)
         ctx.run_backward, ctx.keys = backward, keys
         return logits
 
     @staticmethod
     @once_differentiable
     def backward(ctx, d_logits):
-        grads = ctx.run_backward(d_logits.float().contiguous())
-        # copies: the pack's gradient arena is overwritten by another backward through the same graph
-        return (None, None, None) + tuple(None if grads.get(k) is None else grads[k].clone(memory_format=torch.contiguous_format)
-                                          for k in ctx.keys)
+        return (None, None, None) + _expert_grads(ctx.run_backward(d_logits.float().contiguous()), ctx.keys)
 
 
 class DmRouter(torch.autograd.Function):

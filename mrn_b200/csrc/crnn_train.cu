@@ -301,7 +301,7 @@ inline float* gpt(const MrnbCrnnTrainPack& G, int slot) { return const_cast<floa
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
 int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, int bn_batch, int update_running, float* logits,
-                         long ld, void* ws, size_t ws_bytes, cudaStream_t st) {
+                         long ld, float* features, void* ws, size_t ws_bytes, cudaStream_t st) {
   constexpr bool TC = sizeof(AT) == 2;
   CrnnWs<AT> w = carve_crnn_ws<AT>((char*)ws, B, P.n_class);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "crnn_train_forward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
@@ -426,6 +426,10 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
   }
   MRNB_TRY(lin<AT>(w.out16[1], 256, P.p[MRNB_T_FC_W], P.h[MRNB_T_FC_W], P.p[MRNB_T_FC_B], logits, ld, true, M, P.n_class, 256,
                    nullptr, nullptr, 1, st));
+  if (features) {
+    widen_kernel<AT><<<cdiv((long)M * 256, 256), 256, 0, st>>>(w.out16[1], features, (long)M * 256);
+    MRNB_CHECK_LAUNCH("widen_kernel");
+  }
   return MRNB_OK;
 }
 
@@ -433,8 +437,9 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
 // Backward
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
-int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G, const float* dlogits, long ldg, int B,
-                          int bn_batch, float* grad_arena, long n_arena, void* ws, size_t ws_bytes, cudaStream_t st) {
+int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G, const float* dlogits, long ldg,
+                          const float* dfeatures, int B, int bn_batch, float* grad_arena, long n_arena, void* ws, size_t ws_bytes,
+                          cudaStream_t st) {
   constexpr bool TC = sizeof(AT) == 2;
   CrnnWs<AT> w = carve_crnn_ws<AT>((char*)ws, B, P.n_class);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "crnn_train_backward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
@@ -451,7 +456,8 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
   MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, gpt(G, MRNB_T_FC_B), st));
   MRNB_TRY(gemm_dw<AT>(dlog, w.out16[1], 256, gpt(G, MRNB_T_FC_W), M, C, 256, st));
   bf16* dout16 = TC ? w.d16 : nullptr;
-  MRNB_TRY(gemm_dx<AT>(dlog, P.p[MRNB_T_FC_W], P.h[MRNB_T_FC_W], w.dout, dout16, 256, M, C, 256, st));
+  // d feature = dlogits W_fc (+ dfeatures, the gradient reaching the feature from outside the expert, in the epilogue)
+  MRNB_TRY(gemm_dx<AT>(dlog, P.p[MRNB_T_FC_W], P.h[MRNB_T_FC_W], w.dout, dout16, 256, M, C, 256, st, dfeatures));
   // ---- the two BidirectionalLSTMs, last first
   float* dxin = w.d0;                        // gradient w.r.t. the layer input [M, Kin]
   for (int k = 1; k >= 0; --k) {
@@ -580,34 +586,49 @@ extern "C" size_t mrnb_crnn_train_workspace_bytes(int B, int n_class, int prec) 
                                 : carve_crnn_ws<float>(nullptr, B, n_class).bytes;
 }
 
-extern "C" int mrnb_crnn_train_forward(const MrnbCrnnTrainPack* pack, const float* image, int B, int prec, int bn_batch_stats,
-                                       int update_running, float* logits, long ld_logits, void* workspace,
-                                       size_t workspace_bytes, cudaStream_t stream) {
+extern "C" int mrnb_crnn_train_forward_features(const MrnbCrnnTrainPack* pack, const float* image, int B, int prec,
+                                                int bn_batch_stats, int update_running, float* logits, long ld_logits,
+                                                float* features, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   MRNB_CHECK_ARG(pack && image && logits && workspace && B > 0, "crnn_train_forward: null/empty argument");
   MRNB_CHECK_ARG(ld_logits >= pack->n_class && pack->n_class > 0, "crnn_train_forward: ld_logits < n_class");
   for (int k = 0; k < MRNB_T_COUNT; ++k) MRNB_CHECK_ARG(pack->p[k], "crnn_train_forward: parameter slot %d is null", k);
   MRNB_CHECK_ARG(pack->bn_mean[0] && pack->bn_mean[1] && pack->bn_var[0] && pack->bn_var[1], "crnn_train_forward: BN statistics missing");
   if (prec == MRNB_PREC_FP32)
-    return crnn_train_forward_t<float>(*pack, image, B, bn_batch_stats, update_running, logits, ld_logits, workspace,
+    return crnn_train_forward_t<float>(*pack, image, B, bn_batch_stats, update_running, logits, ld_logits, features, workspace,
                                        workspace_bytes, stream);
   if (prec == MRNB_PREC_BF16)
-    return crnn_train_forward_t<__nv_bfloat16>(*pack, image, B, bn_batch_stats, update_running, logits, ld_logits, workspace,
-                                               workspace_bytes, stream);
+    return crnn_train_forward_t<__nv_bfloat16>(*pack, image, B, bn_batch_stats, update_running, logits, ld_logits, features,
+                                               workspace, workspace_bytes, stream);
   mrnb_set_error("crnn_train_forward: unknown precision %d", prec);
+  return MRNB_ERR_ARG;
+}
+
+extern "C" int mrnb_crnn_train_forward(const MrnbCrnnTrainPack* pack, const float* image, int B, int prec, int bn_batch_stats,
+                                       int update_running, float* logits, long ld_logits, void* workspace,
+                                       size_t workspace_bytes, cudaStream_t stream) {
+  return mrnb_crnn_train_forward_features(pack, image, B, prec, bn_batch_stats, update_running, logits, ld_logits, nullptr,
+                                          workspace, workspace_bytes, stream);
+}
+
+extern "C" int mrnb_crnn_train_backward_features(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads,
+                                                 const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                                 int bn_batch_stats, float* grad_arena, long n_arena, void* workspace,
+                                                 size_t workspace_bytes, cudaStream_t stream) {
+  MRNB_CHECK_ARG(pack && grads && dlogits && grad_arena && workspace && B > 0, "crnn_train_backward: null/empty argument");
+  for (int k = 0; k < MRNB_T_COUNT; ++k) MRNB_CHECK_ARG(grads->p[k], "crnn_train_backward: gradient slot %d is null", k);
+  if (prec == MRNB_PREC_FP32)
+    return crnn_train_backward_t<float>(*pack, *grads, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena, n_arena,
+                                        workspace, workspace_bytes, stream);
+  if (prec == MRNB_PREC_BF16)
+    return crnn_train_backward_t<__nv_bfloat16>(*pack, *grads, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena,
+                                                n_arena, workspace, workspace_bytes, stream);
+  mrnb_set_error("crnn_train_backward: unknown precision %d", prec);
   return MRNB_ERR_ARG;
 }
 
 extern "C" int mrnb_crnn_train_backward(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads, const float* dlogits,
                                         long ld_dlogits, int B, int prec, int bn_batch_stats, float* grad_arena, long n_arena,
                                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
-  MRNB_CHECK_ARG(pack && grads && dlogits && grad_arena && workspace && B > 0, "crnn_train_backward: null/empty argument");
-  for (int k = 0; k < MRNB_T_COUNT; ++k) MRNB_CHECK_ARG(grads->p[k], "crnn_train_backward: gradient slot %d is null", k);
-  if (prec == MRNB_PREC_FP32)
-    return crnn_train_backward_t<float>(*pack, *grads, dlogits, ld_dlogits, B, bn_batch_stats, grad_arena, n_arena, workspace,
-                                        workspace_bytes, stream);
-  if (prec == MRNB_PREC_BF16)
-    return crnn_train_backward_t<__nv_bfloat16>(*pack, *grads, dlogits, ld_dlogits, B, bn_batch_stats, grad_arena, n_arena,
-                                                workspace, workspace_bytes, stream);
-  mrnb_set_error("crnn_train_backward: unknown precision %d", prec);
-  return MRNB_ERR_ARG;
+  return mrnb_crnn_train_backward_features(pack, grads, dlogits, ld_dlogits, nullptr, B, prec, bn_batch_stats, grad_arena,
+                                           n_arena, workspace, workspace_bytes, stream);
 }

@@ -564,6 +564,11 @@ combine_row_tma_kernel(RowPtrs P, const float* __restrict__ gate, int T, int C, 
 // is not copied and reads as the pad value.  Each consumer thread owns 4 columns of a chunk and keeps I running dot
 // products; a row's partials are reduced in a fixed order (warp shuffles, then warp 0 over the warps) into
 // rowout[row, I], and a second kernel sums the T rows of each sample in order: no atomics, the same bits every run.
+//
+// DZ = true (mrnb_gate_combine_backward_experts) also writes the per-expert logit gradients from the same stage reads:
+//   dz_i[b,t,c] = gate[b,i] * dY[b,t,c]   for c < C_i, for every expert whose dz_i pointer is non-null;
+// a thread stores its 4 columns (a partial group at the charset edge element-wise), so the ld padding is never written.
+// The dgate reduction is the same code in both instantiations.
 // ---------------------------------------------------------------------------------------------
 constexpr int BWD_CONSUMERS = 512;
 constexpr int BWD_CHUNK = 4 * BWD_CONSUMERS;
@@ -571,10 +576,12 @@ constexpr int BWD_MAX_STAGES = 4;
 constexpr int BWD_THREADS = BWD_CONSUMERS + 32;
 constexpr size_t BWD_SMEM_BUDGET = 200 * 1024;
 
-template <int I>
+struct DzPtrs { float* dz[MRNB_MAX_EXPERTS]; long ld[MRNB_MAX_EXPERTS]; };   // dz[i] null: expert i gets no dz
+
+template <int I, bool DZ>
 __global__ void __launch_bounds__(BWD_THREADS, 1)
 combine_bwd_tma_kernel(RowPtrs P, const float* __restrict__ dY, long ldy, int C, int rows, int nchunks, int nstages,
-                       float* __restrict__ rowout) {
+                       float* __restrict__ rowout, const float* __restrict__ gate, DzPtrs Dz, int T) {
   extern __shared__ __align__(128) float stage[];              // [nstages][I + 1][BWD_CHUNK]
   __shared__ __align__(8) uint64_t full_bar[BWD_MAX_STAGES], empty_bar[BWD_MAX_STAGES];
   __shared__ float part[2][BWD_CONSUMERS / 32][I];
@@ -618,9 +625,12 @@ combine_bwd_tma_kernel(RowPtrs P, const float* __restrict__ dY, long ldy, int C,
   // ---------------- consumers (4 columns each per chunk)
   uint32_t q = 0, it = 0;
   for (int row = blockIdx.x; row < rows; row += gridDim.x, ++it) {
-    float acc[I];
+    float acc[I], g[I];
 #pragma unroll
-    for (int i = 0; i < I; ++i) acc[i] = 0.f;
+    for (int i = 0; i < I; ++i) {
+      acc[i] = 0.f;
+      if constexpr (DZ) g[i] = gate[(long)(row / T) * I + i];
+    }
     for (int j = 0; j < nchunks; ++j, ++q) {
       const int s = (int)(q % (uint32_t)nstages);
       mbar_wait(&full_bar[s], (q / (uint32_t)nstages) & 1u);
@@ -641,6 +651,22 @@ combine_bwd_tma_kernel(RowPtrs P, const float* __restrict__ dY, long ldy, int C,
         if (c0 + 1 >= C) dy.y = 0.f;
         if (c0 + 2 >= C) dy.z = 0.f;
         dy.w = 0.f;
+      }
+      if constexpr (DZ) {
+#pragma unroll
+        for (int i = 0; i < I; ++i) {
+          const int Ci = P.C[i];
+          if (!Dz.dz[i] || c0 >= Ci) continue;
+          float* dst = Dz.dz[i] + (long)row * Dz.ld[i] + c0;
+          const float4 o = make_float4(g[i] * dy.x, g[i] * dy.y, g[i] * dy.z, g[i] * dy.w);
+          if (c0 + 4 <= Ci) {
+            *reinterpret_cast<float4*>(dst) = o;
+          } else {
+            dst[0] = o.x;
+            if (c0 + 1 < Ci) dst[1] = o.y;
+            if (c0 + 2 < Ci) dst[2] = o.z;
+          }
+        }
       }
       const float sdy = (dy.x + dy.y) + (dy.z + dy.w);
 #pragma unroll
@@ -915,16 +941,16 @@ int launch_combine(const RowPtrs& P, const float* gate, int B, int T, int C, flo
   return MRNB_OK;
 }
 
-template <int I>
+template <int I, bool DZ>
 int launch_combine_bwd(const RowPtrs& P, const float* dY, long ldy, int B, int T, int C, float* dgate, float* rowout,
-                       cudaStream_t st) {
+                       const float* gate, const DzPtrs& Dz, cudaStream_t st) {
   const int nchunks = (C + BWD_CHUNK - 1) / BWD_CHUNK;
   const size_t slot_bytes = (size_t)(I + 1) * BWD_CHUNK * sizeof(float);
   const int nstages = (int)(BWD_SMEM_BUDGET / slot_bytes) < BWD_MAX_STAGES ? (int)(BWD_SMEM_BUDGET / slot_bytes) : BWD_MAX_STAGES;
   static bool attr_set = false;
   static int num_sms = 148;
   if (!attr_set) {
-    cudaFuncSetAttribute(combine_bwd_tma_kernel<I>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BWD_SMEM_BUDGET);
+    cudaFuncSetAttribute(combine_bwd_tma_kernel<I, DZ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BWD_SMEM_BUDGET);
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
@@ -932,7 +958,8 @@ int launch_combine_bwd(const RowPtrs& P, const float* dY, long ldy, int B, int T
   }
   const int rows = B * T;
   const int grid = rows < num_sms ? rows : num_sms;
-  combine_bwd_tma_kernel<I><<<grid, BWD_THREADS, nstages * slot_bytes, st>>>(P, dY, ldy, C, rows, nchunks, nstages, rowout);
+  combine_bwd_tma_kernel<I, DZ><<<grid, BWD_THREADS, nstages * slot_bytes, st>>>(P, dY, ldy, C, rows, nchunks, nstages, rowout,
+                                                                                 gate, Dz, T);
   MRNB_CHECK_LAUNCH("combine_bwd_tma_kernel");
   combine_bwd_finish_kernel<<<cdiv(B * I, 256), 256, 0, st>>>(rowout, B, T, I, dgate);
   MRNB_CHECK_LAUNCH("combine_bwd_finish_kernel");
@@ -975,19 +1002,28 @@ extern "C" size_t mrnb_gate_combine_backward_workspace_bytes(int B, int T, int n
   return (size_t)B * T * n_experts * sizeof(float);
 }
 
-extern "C" int mrnb_gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
-                                          const float* dY, long ldy, float* dgate, void* workspace,
-                                          size_t workspace_bytes, cudaStream_t stream) {
+// Both combine-backward entries: dz == nullptr is mrnb_gate_combine_backward (no gate read, no dz written).
+static int gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
+                                 const float* dY, long ldy, const float* gate, float* const* dz, const long* ldz,
+                                 float* dgate, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   MRNB_CHECK_ARG(n_experts >= 1 && n_experts <= MRNB_MAX_EXPERTS, "gate_combine_backward: n_experts %d out of range",
                  n_experts);
   MRNB_CHECK_ARG(B > 0 && T > 0 && z && ld && Ci && dY && dgate && workspace, "gate_combine_backward: null/empty argument");
   const int C = Ci[n_experts - 1];
   RowPtrs P;
+  DzPtrs Dz{};
+  double wb = 0;
   for (int i = 0; i < n_experts; ++i) {
     P.z[i] = z[i]; P.ld[i] = ld[i]; P.C[i] = Ci[i];
     MRNB_CHECK_ARG(z[i] && Ci[i] > 0 && Ci[i] <= C && ld[i] >= Ci[i] && ld[i] % 4 == 0 &&
                    (reinterpret_cast<uintptr_t>(z[i]) & 15) == 0,
                    "gate_combine_backward: expert %d needs C_i <= C, a 16-byte aligned base and ld %% 4 == 0", i);
+    if (dz && dz[i]) {
+      MRNB_CHECK_ARG(gate && ldz && ldz[i] >= Ci[i] && ldz[i] % 4 == 0 && (reinterpret_cast<uintptr_t>(dz[i]) & 15) == 0,
+                     "gate_combine_backward_experts: dz %d needs the gate, ldz >= C_i, ldz %% 4 == 0 and a 16-byte aligned base", i);
+      Dz.dz[i] = dz[i]; Dz.ld[i] = ldz[i];
+      wb += Ci[i];
+    }
   }
   MRNB_CHECK_ARG(ldy >= C && ldy % 4 == 0 && (reinterpret_cast<uintptr_t>(dY) & 15) == 0,
                  "gate_combine_backward: dY needs ldy >= C, ldy %% 4 == 0 and a 16-byte aligned base");
@@ -995,14 +1031,30 @@ extern "C" int mrnb_gate_combine_backward(const float* const* z, const long* ld,
                  "gate_combine_backward: workspace too small (%zu bytes)", workspace_bytes);
   double rb = C;
   for (int i = 0; i < n_experts; ++i) rb += (double)Ci[i];
-  MrnbProfScope prof(MRNB_PROF_COMBINE, stream, 0.0, 4.0 * B * T * rb);
+  MrnbProfScope prof(MRNB_PROF_COMBINE, stream, 0.0, 4.0 * B * T * (rb + wb));
   float* rowout = static_cast<float*>(workspace);
-#define MRNB_CASE(N) case N: return launch_combine_bwd<N>(P, dY, ldy, B, T, C, dgate, rowout, stream);
+#define MRNB_CASE(N) case N: return dz ? launch_combine_bwd<N, true>(P, dY, ldy, B, T, C, dgate, rowout, gate, Dz, stream) \
+                                       : launch_combine_bwd<N, false>(P, dY, ldy, B, T, C, dgate, rowout, nullptr, Dz, stream);
   switch (n_experts) {
     MRNB_CASE(1) MRNB_CASE(2) MRNB_CASE(3) MRNB_CASE(4) MRNB_CASE(5) MRNB_CASE(6) MRNB_CASE(7) MRNB_CASE(8)
   }
 #undef MRNB_CASE
   return MRNB_ERR_ARG;
+}
+
+extern "C" int mrnb_gate_combine_backward(const float* const* z, const long* ld, const int* Ci, int n_experts, int B, int T,
+                                          const float* dY, long ldy, float* dgate, void* workspace,
+                                          size_t workspace_bytes, cudaStream_t stream) {
+  return gate_combine_backward(z, ld, Ci, n_experts, B, T, dY, ldy, nullptr, nullptr, nullptr, dgate, workspace,
+                               workspace_bytes, stream);
+}
+
+extern "C" int mrnb_gate_combine_backward_experts(const float* const* z, const long* ld, const int* Ci, int n_experts, int B,
+                                                  int T, const float* dY, long ldy, const float* gate, float* const* dz,
+                                                  const long* ldz, float* dgate, void* workspace, size_t workspace_bytes,
+                                                  cudaStream_t stream) {
+  MRNB_CHECK_ARG(gate && dz && ldz, "gate_combine_backward_experts: null gate / dz table");
+  return gate_combine_backward(z, ld, Ci, n_experts, B, T, dY, ldy, gate, dz, ldz, dgate, workspace, workspace_bytes, stream);
 }
 
 extern "C" int mrnb_ctc_lattice(const float* lpe, const float* zlab, const float* E, const long long* targets,

@@ -1298,9 +1298,10 @@ int dm_router_backward_core(const float* P, const float* x, const Dims& d, float
   return MRNB_OK;
 }
 
-// Training-step backward in fp32 mode: gate head from dL/ds (w.ds), then the generic DM_Router backward on the
-// materialised dout.  G = zeroed gradient arena.
-int router_backward_gate_f32(const float* P, const float* x, const Dims& d, float* G, RouterWs& w, cudaStream_t st) {
+// Training-step backward with d_out materialised: gate head from dL/ds (w.ds), then the generic DM_Router backward on
+// dout.  The fp32 engine always runs it; the tensor-core engine runs it when the input gradient dx [B,I,T,D] is asked for
+// (its own rank-one path never forms dx).  G = zeroed gradient arena.
+int router_backward_gate_dout(const float* P, const float* x, const Dims& d, float* G, float* dx, RouterWs& w, cudaStream_t st) {
   long off[MRNB_ROUTER_NPARAMS + 1];
   router_offsets(d.I, d.T, d.D, off);
   {  // dWcr[j,(i,c)] = sum_(b,t) ds[(b,t),j] out[b,i,t,c]
@@ -1311,9 +1312,9 @@ int router_backward_gate_f32(const float* P, const float* x, const Dims& d, floa
   {  // dout[b,i,t,c] = sum_j ds[(b,t),j] Wcr[j,(i,c)]
     MrnbProfScope prof(MRNB_PROF_ROUTER_EW, st);
     const long total4 = d.M * d.D / 4;
-    LAUNCH_EW(dout_kernel, total4, w.ds, P + off[R_CR_W], d.I, d.T, total4, w.dout, nullptr);
+    LAUNCH_EW(dout_kernel, total4, w.ds, P + off[R_CR_W], d.I, d.T, total4, w.dout, d.tc ? w.dout16 : nullptr);
   }
-  return dm_router_backward_core(P, x, d, G, nullptr, w, st);
+  return dm_router_backward_core(P, x, d, G, dx, w, st);
 }
 
 // Training-step backward in tensor-core mode: gate head + DM_Router parameter gradients from dL/dr (w.dr), with the
@@ -1531,9 +1532,11 @@ extern "C" int mrnb_router_forward(const float* params, const float* x, int B, i
   return out ? unpad_frames(r, r.w.out, out, stream) : MRNB_OK;
 }
 
-extern "C" int mrnb_router_backward(const float* params, const float* x, const float* gate, const float* dgate_ctc,
-                                    const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
-                                    float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+// Both training-step backward entries: dx == nullptr is mrnb_router_backward (the tensor-core engine keeps its rank-one
+// path, which forms no input gradient).
+static int router_backward(const float* params, const float* x, const float* gate, const float* dgate_ctc,
+                           const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads, float* dx,
+                           float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   ROUTER_ARGCHECK("router_backward");
   MRNB_CHECK_ARG(gate && grads, "router_backward: null argument");
   MRNB_CHECK_ARG(domain ? taski_loss != nullptr : dgate_ctc != nullptr,
@@ -1557,9 +1560,28 @@ extern "C" int mrnb_router_backward(const float* params, const float* x, const f
                                           G + off[R_ROUTE_B]);
     MRNB_CHECK_LAUNCH("route_bwd_kernel");
   }
-  if (d.tc) MRNB_TRY(router_backward_gate_tc(params, x, d, G, w, st));
-  else MRNB_TRY(router_backward_gate_f32(params, x, d, G, w, st));
-  return r.padded ? unpad_grads(r, grads, st) : MRNB_OK;
+  float* dxp = (dx && r.padded) ? w.dg2 : dx;   // padded dx: dg2 is dead by the time the core's last kernel writes dx
+  if (d.tc && !dx) MRNB_TRY(router_backward_gate_tc(params, x, d, G, w, st));
+  else MRNB_TRY(router_backward_gate_dout(params, x, d, G, dxp, w, st));
+  if (!r.padded) return MRNB_OK;
+  MRNB_TRY(unpad_grads(r, grads, st));
+  return dx ? unpad_frames(r, dxp, dx, st) : MRNB_OK;
+}
+
+extern "C" int mrnb_router_backward(const float* params, const float* x, const float* gate, const float* dgate_ctc,
+                                    const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
+                                    float* taski_loss, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  return router_backward(params, x, gate, dgate_ctc, domain, B, n_experts, T, D, prec, grads, nullptr, taski_loss, workspace,
+                         workspace_bytes, stream);
+}
+
+extern "C" int mrnb_router_backward_dx(const float* params, const float* x, const float* gate, const float* dgate_ctc,
+                                       const long long* domain, int B, int n_experts, int T, int D, int prec, float* grads,
+                                       float* dx, float* taski_loss, void* workspace, size_t workspace_bytes,
+                                       cudaStream_t stream) {
+  MRNB_CHECK_ARG(dx, "router_backward_dx: null dx");
+  return router_backward(params, x, gate, dgate_ctc, domain, B, n_experts, T, D, prec, grads, dx, taski_loss, workspace,
+                         workspace_bytes, stream);
 }
 
 extern "C" int mrnb_dm_router_backward(const float* params, const float* x, const float* d_out, int B, int n_experts,

@@ -694,8 +694,8 @@ inline float* gp(const MrnbSvtrPack& G, int slot) { return const_cast<float*>(G.
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
 int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_batch, int update_running,
-                    const float* drop /*[12,2,B] or null*/, float* logits, long ld, void* ws, size_t ws_bytes,
-                    cudaStream_t st) {
+                    const float* drop /*[12,2,B] or null*/, float* logits, long ld, float* features, void* ws,
+                    size_t ws_bytes, cudaStream_t st) {
   TrainWs<AT> w = carve_train_ws<AT>((char*)ws, B, P.n_class[0]);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "svtr_train_forward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
   const long u = (long)B * 32768;
@@ -798,6 +798,10 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
   MRNB_TRY(lin<AT>(w.vis, 512, P.p[MRNB_P_SEQ_W], P.h[MRNB_P_SEQ_W], P.p[MRNB_P_SEQ_B], w.feat, 256, false, M, 256, 512,
                    nullptr, nullptr, 1, st));
   MRNB_TRY(lin<AT>(w.feat, 256, P.fc_w[0], P.fc_w16[0], P.fc_b[0], logits, ld, true, M, P.n_class[0], 256, nullptr, nullptr, 1, st));
+  if (features) {
+    widen_kernel<AT><<<cdiv((long)M * 256, 256), 256, 0, st>>>(w.feat, features, (long)M * 256);
+    MRNB_CHECK_LAUNCH("widen_kernel");
+  }
   return MRNB_OK;
 }
 
@@ -807,8 +811,8 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
 int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* image, const float* dlogits, long ldg,
-                     int B, int bn_batch, const float* drop, float* grad_arena, long n_arena, void* ws, size_t ws_bytes,
-                     cudaStream_t st) {
+                     const float* dfeatures, int B, int bn_batch, const float* drop, float* grad_arena, long n_arena, void* ws,
+                     size_t ws_bytes, cudaStream_t st) {
   constexpr bool TC = sizeof(AT) == 2;
   TrainWs<AT> w = carve_train_ws<AT>((char*)ws, B, P.n_class[0]);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "svtr_train_backward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
@@ -826,7 +830,8 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
   }
   MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, const_cast<float*>(G.fc_b[0]), st));
   MRNB_TRY(gemm_dw<AT>(dlog, w.feat, 256, const_cast<float*>(G.fc_w[0]), M, C, 256, st));
-  MRNB_TRY(gemm_dx<AT>(dlog, P.fc_w[0], P.fc_w16[0], w.dfeat, w.dfeat16, 256, M, C, 256, st));
+  // d feature = dlogits W_fc (+ dfeatures, the gradient reaching the feature from outside the expert, in the epilogue)
+  MRNB_TRY(gemm_dx<AT>(dlog, P.fc_w[0], P.fc_w16[0], w.dfeat, w.dfeat16, 256, M, C, 256, st, dfeatures));
   Grad dfe{w.dfeat, w.dfeat16, 256};
   MRNB_TRY(launch_colsum<float>(w.dfeat, 256, M, 256, gp(G, MRNB_P_SEQ_B), st));
   MRNB_TRY(gemm_dw<AT>(dfe, w.vis, 512, gp(G, MRNB_P_SEQ_W), M, 256, 512, st));
@@ -989,28 +994,36 @@ extern "C" size_t mrnb_svtr_train_workspace_bytes(int B, int n_class, int prec) 
                                 : carve_train_ws<float>(nullptr, B, n_class).bytes;
 }
 
-extern "C" int mrnb_svtr_train_forward(const MrnbSvtrPack* pack, const float* image, int B, int prec, int bn_batch_stats,
-                                       int update_running, const float* drop_scales, float* logits, long ld_logits,
-                                       void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+extern "C" int mrnb_svtr_train_forward_features(const MrnbSvtrPack* pack, const float* image, int B, int prec,
+                                                int bn_batch_stats, int update_running, const float* drop_scales,
+                                                float* logits, long ld_logits, float* features, void* workspace,
+                                                size_t workspace_bytes, cudaStream_t stream) {
   MRNB_CHECK_ARG(pack && image && logits && workspace && B > 0, "svtr_train_forward: null/empty argument");
   MRNB_CHECK_ARG(pack->n_experts == 1, "svtr_train_forward: the training pack holds exactly one expert");
   MRNB_CHECK_ARG(ld_logits >= pack->n_class[0], "svtr_train_forward: ld_logits < n_class");
   MRNB_CHECK_ARG(!bn_batch_stats || (long)B * 512 > 1, "svtr_train_forward: batch statistics need more than one value");
   for (int k = 0; k < MRNB_P_COUNT; ++k) MRNB_CHECK_ARG(pack->p[k], "svtr_train_forward: parameter slot %d is null", k);
   if (prec == MRNB_PREC_FP32)
-    return train_forward_t<float>(*pack, image, B, bn_batch_stats, update_running, drop_scales, logits, ld_logits, workspace,
-                                  workspace_bytes, stream);
+    return train_forward_t<float>(*pack, image, B, bn_batch_stats, update_running, drop_scales, logits, ld_logits, features,
+                                  workspace, workspace_bytes, stream);
   if (prec == MRNB_PREC_BF16)
     return train_forward_t<__nv_bfloat16>(*pack, image, B, bn_batch_stats, update_running, drop_scales, logits, ld_logits,
-                                          workspace, workspace_bytes, stream);
+                                          features, workspace, workspace_bytes, stream);
   mrnb_set_error("svtr_train_forward: unknown precision %d", prec);
   return MRNB_ERR_ARG;
 }
 
-extern "C" int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
-                                        const float* dlogits, long ld_dlogits, int B, int prec, int bn_batch_stats,
-                                        const float* drop_scales, float* grad_arena, long n_arena, void* workspace,
-                                        size_t workspace_bytes, cudaStream_t stream) {
+extern "C" int mrnb_svtr_train_forward(const MrnbSvtrPack* pack, const float* image, int B, int prec, int bn_batch_stats,
+                                       int update_running, const float* drop_scales, float* logits, long ld_logits,
+                                       void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  return mrnb_svtr_train_forward_features(pack, image, B, prec, bn_batch_stats, update_running, drop_scales, logits, ld_logits,
+                                          nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mrnb_svtr_train_backward_features(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
+                                                 const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                                 int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
+                                                 void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   MRNB_CHECK_ARG(pack && grads && image && dlogits && grad_arena && workspace && B > 0, "svtr_train_backward: null/empty argument");
   MRNB_CHECK_ARG(pack->n_experts == 1 && grads->n_experts == 1, "svtr_train_backward: the training pack holds exactly one expert");
   for (int k = 0; k < MRNB_P_COUNT; ++k) {
@@ -1019,13 +1032,21 @@ extern "C" int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtr
   }
   MRNB_CHECK_ARG(grads->fc_w[0] && grads->fc_b[0], "svtr_train_backward: classifier gradient slots are null");
   if (prec == MRNB_PREC_FP32)
-    return train_backward_t<float>(*pack, *grads, image, dlogits, ld_dlogits, B, bn_batch_stats, drop_scales, grad_arena,
-                                   n_arena, workspace, workspace_bytes, stream);
+    return train_backward_t<float>(*pack, *grads, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, drop_scales,
+                                   grad_arena, n_arena, workspace, workspace_bytes, stream);
   if (prec == MRNB_PREC_BF16)
-    return train_backward_t<__nv_bfloat16>(*pack, *grads, image, dlogits, ld_dlogits, B, bn_batch_stats, drop_scales,
-                                           grad_arena, n_arena, workspace, workspace_bytes, stream);
+    return train_backward_t<__nv_bfloat16>(*pack, *grads, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats,
+                                           drop_scales, grad_arena, n_arena, workspace, workspace_bytes, stream);
   mrnb_set_error("svtr_train_backward: unknown precision %d", prec);
   return MRNB_ERR_ARG;
+}
+
+extern "C" int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
+                                        const float* dlogits, long ld_dlogits, int B, int prec, int bn_batch_stats,
+                                        const float* drop_scales, float* grad_arena, long n_arena, void* workspace,
+                                        size_t workspace_bytes, cudaStream_t stream) {
+  return mrnb_svtr_train_backward_features(pack, grads, image, dlogits, ld_dlogits, nullptr, B, prec, bn_batch_stats,
+                                           drop_scales, grad_arena, n_arena, workspace, workspace_bytes, stream);
 }
 
 // ---- C-ABI test entries: the bf16 training attention of one stage, forwarded unchanged to attn_tc_forward /

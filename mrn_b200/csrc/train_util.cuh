@@ -119,8 +119,11 @@ int lin(const AT* A, long lda, const float* W32, const void* W16, const float* b
   return linear<AT>(a, st);
 }
 
-int gemm_dx_f32(const float* dY, long ldy, const float* W, float* dX, long ldx, int M, int N, int K, cudaStream_t st) {
+// res (optional, dX's addressing): added to the product in the epilogue, before any 16-bit copy is written
+int gemm_dx_f32(const float* dY, long ldy, const float* W, float* dX, long ldx, int M, int N, int K, cudaStream_t st,
+                const float* res = nullptr) {
   MrnbGemm g{};
+  g.res = res;
   g.A = dY; g.am = mrnb_axis(ldy); g.ak = mrnb_axis(1); g.a_kfast = 1;
   g.B = W; g.bk = mrnb_axis(K); g.bn = mrnb_axis(1); g.b_kfast = 0;
   g.C = dX; g.cm = mrnb_axis(ldx); g.cn = mrnb_axis(1);
@@ -142,8 +145,10 @@ int gemm_dw_f32(const float* dY, long ldy, const float* X, long ldx, float* dW, 
   g.splitk = (int)sk;
   return mrnb_sgemm(g, st);
 }
-int gemm_dx_tc(const bf16* dY, long ldy, const void* W16, float* dX, bf16* dX16, long ldx, int M, int N, int K, cudaStream_t st) {
+int gemm_dx_tc(const bf16* dY, long ldy, const void* W16, float* dX, bf16* dX16, long ldx, int M, int N, int K, cudaStream_t st,
+               const float* res = nullptr) {
   MrnbTcGemm2 g{};
+  g.res = res;
   g.a = mrnb_operand_k2d(dY, M, N, ldy, 128, 1);
   g.b = mrnb_operand_mn2d(W16, K, N, K, 1);
   g.out32 = dX; g.out16 = dX16; g.cm = mrnb_axis(ldx); g.cn = mrnb_axis(1);
@@ -169,9 +174,18 @@ int gemm_dw_tc(const bf16* dY, long ldy, const bf16* X, long ldx, float* dW, int
 struct Grad { const float* f; const bf16* h; long ld; };
 
 template <typename AT>
-int gemm_dx(const Grad& dY, const float* W32, const void* W16, float* dX, bf16* dX16, long ldx, int M, int N, int K, cudaStream_t st) {
-  if constexpr (sizeof(AT) == 4) return gemm_dx_f32(dY.f, dY.ld, W32, dX, ldx, M, N, K, st);
-  else return gemm_dx_tc(dY.h, dY.ld, W16, dX, dX16, ldx, M, N, K, st);
+int gemm_dx(const Grad& dY, const float* W32, const void* W16, float* dX, bf16* dX16, long ldx, int M, int N, int K, cudaStream_t st,
+            const float* res = nullptr) {
+  if constexpr (sizeof(AT) == 4) return gemm_dx_f32(dY.f, dY.ld, W32, dX, ldx, M, N, K, st, res);
+  else return gemm_dx_tc(dY.h, dY.ld, W16, dX, dX16, ldx, M, N, K, st, res);
+}
+
+// a training pack's feature [rows, 256] (AT) -> the caller's fp32 buffer: a copy in fp32 mode, the widened bf16 value
+// (the operand the classifier head reads) in bf16 mode
+template <typename AT>
+__global__ void widen_kernel(const AT* __restrict__ x, float* __restrict__ y, long n) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) y[i] = to_f32<AT>(x[i]);
 }
 template <typename AT>
 int gemm_dw(const Grad& dY, const AT* X, long ldx, float* dW, int rows, int N, int K, cudaStream_t st) {

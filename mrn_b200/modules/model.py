@@ -222,47 +222,53 @@ def _writeback_train_pack_bn(expert, tp, n_fwd):
             bn.num_batches_tracked += n_fwd
 
 
+def _train_pack_run(expert, x, opt, net=None, drop=None, want_features=False):
+    """One expert's training-pack forward, the step autograd differentiates (opt.autograd): ops.SvtrTrainPack /
+    ops.CrnnTrainPack built from the expert's state_dict, run in the expert's current mode -- in .train() BatchNorm batch
+    statistics with the running-statistics update (written back to the expert's buffers once, here) and DropPath `drop`
+    [12,2,B] (None: drawn as the default forward draws it).  Returns (logits, features or None, backward);
+    backward(dlogits, dfeatures=None) runs the pack's full backward and returns {state_dict key: gradient in the reference
+    layout} (views of the pack's gradient arena)."""
+    arch = _arch(opt)
+    tp = (ops.SvtrTrainPack if arch == "svtr" else ops.CrnnTrainPack)(expert.state_dict(), x.device, _precision(opt))
+    train = bool(expert.training)
+    x = x.contiguous().float()
+    B = x.shape[0]
+    if arch == "crnn":
+        out = ops.crnn_train_forward(tp, x, bn_batch_stats=train, update_running=train, want_features=want_features)
+    else:
+        if drop is None and train and getattr(opt, "drop_path", True):
+            rates = expert.model.FeatureExtraction.ConvNet.drop_path_rates()
+            drop = sample_drop_scales(1, B, rates, x.device)[0].contiguous()
+        out = ops.svtr_train_forward(tp, x, bn_batch_stats=train, update_running=train, drop_scales=drop,
+                                     want_features=want_features)
+    logits, feats = out if want_features else (out, None)
+    if train:
+        _writeback_train_pack_bn(expert, tp, 1)
+        _solo_cache.key = None              # packs hold BN statistics: rebuild them from the updated buffers
+        if net is not None:
+            net._cache.key = None
+
+    def backward(dlogits, dfeatures=None):
+        if arch == "crnn":
+            ops.crnn_train_backward(tp, dlogits, B, bn_batch_stats=train, dfeatures=dfeatures)
+        else:
+            ops.svtr_train_backward(tp, x, dlogits, bn_batch_stats=train, drop_scales=drop, dfeatures=dfeatures)
+        return tp.state(tp.grads)
+    return logits, feats, backward
+
+
 def _expert_autograd_forward(expert, image, opt, net=None):
-    """Forward of one expert that autograd differentiates (opt.autograd): the training pack's activation-keeping forward
-    (ops.SvtrTrainPack / ops.CrnnTrainPack) in the expert's current mode -- in .train() BatchNorm batch statistics with
-    the running-statistics update and DropPath drawn as the default forward draws it -- and, on backward, the pack's full
-    backward, mapped back to every parameter in the reference layout by the pack's arena <-> state_dict table."""
+    """Forward of one expert that autograd differentiates (opt.autograd): _train_pack_run and, on backward, the pack's
+    full backward, mapped back to every parameter by the pack's arena <-> state_dict table."""
     if not image.is_cuda:
         raise RuntimeError("mrn_b200 needs CUDA tensors: there is no CPU fallback")
     from ..autograd import ExpertTrain
     if net is not None:
         net._sync_bn()                      # BN statistics the grouped pack still holds -> the module buffers
-    arch = _arch(opt)
     named = list(expert.named_parameters())
-
-    def run(x):
-        tp = (ops.SvtrTrainPack if arch == "svtr" else ops.CrnnTrainPack)(expert.state_dict(), x.device, _precision(opt))
-        train = bool(expert.training)
-        x = x.contiguous().float()
-        B = x.shape[0]
-        drop = None
-        if arch == "crnn":
-            logits = ops.crnn_train_forward(tp, x, bn_batch_stats=train, update_running=train)
-        else:
-            if train and getattr(opt, "drop_path", True):
-                rates = expert.model.FeatureExtraction.ConvNet.drop_path_rates()
-                drop = sample_drop_scales(1, B, rates, x.device)[0].contiguous()
-            logits = ops.svtr_train_forward(tp, x, bn_batch_stats=train, update_running=train, drop_scales=drop)
-        if train:
-            _writeback_train_pack_bn(expert, tp, 1)
-            _solo_cache.key = None          # packs hold BN statistics: rebuild them from the updated buffers
-            if net is not None:
-                net._cache.key = None
-
-        def backward(dlogits):
-            if arch == "crnn":
-                ops.crnn_train_backward(tp, dlogits, B, bn_batch_stats=train)
-            else:
-                ops.svtr_train_backward(tp, x, dlogits, bn_batch_stats=train, drop_scales=drop)
-            return tp.state(tp.grads)
-        return backward, logits
-
-    return ExpertTrain.apply(run, [n for n, _ in named], image, *[p for _, p in named])
+    return ExpertTrain.apply(lambda x: _train_pack_run(expert, x, opt, net=net), [n for n, _ in named], image,
+                             *[p for _, p in named])
 
 
 _RATES_CACHE = {}
@@ -320,6 +326,7 @@ class MRNNet(nn.Module):
         self.layer_num = 1
         self.beta = 1
         self._cache = _PackCache()
+        self._frozen_cache = _PackCache()   # the frozen experts' grouped pack when some experts train (opt.autograd_experts)
         self._arena: Optional[torch.Tensor] = None
         self._grad_arena: Optional[torch.Tensor] = None
         self._rws = ops.RouterWorkspace()
@@ -423,8 +430,12 @@ class MRNNet(nn.Module):
 
         opt.autograd (default off) with grad mode on makes the outputs differentiable (INTEGRATION.md §A):
           * cross=True, is_train=True (soft route): "logits" and "index" (the gate) with respect to route.*,
-            channel_route.* and dm_router.0.*; the experts are frozen and an expert parameter that requires grad
-            raises NotImplementedError;
+            channel_route.* and dm_router.0.*.  The experts are frozen: an expert parameter that requires grad raises
+            NotImplementedError -- unless opt.autograd_experts is set, in which case every parameter of each expert
+            with a parameter that requires grad (a trainable expert) gets its gradient too, along both paths of the
+            reference (its logits through the gated combine, its feature through the DM-Router and the gate head);
+            trainable experts run their training packs (BatchNorm / DropPath as cross=False), the others the grouped
+            forward;
           * cross=True, is_train=False (hard route): "index" is an argmax and "logits" depends only on the frozen
             experts -- outputs as without the switch, no router gradient;
           * cross=False: "logits" with respect to every parameter of the newest expert (training-pack forward)."""
@@ -437,11 +448,14 @@ class MRNNet(nn.Module):
             return dict(logits=logits[0], index=None, aux_logits=None)
         if grad and is_train:
             from ..autograd import RoutedSoft
-            if any(p.requires_grad for p in self.model.parameters()):
+            trainable = tuple(e for e, m in enumerate(self.model) if any(p.requires_grad for p in m.parameters()))
+            if trainable and not getattr(self.opt, "autograd_experts", False):
                 raise NotImplementedError(
                     "autograd through the routed forward keeps the experts frozen, as MRN stage 1 does "
-                    "(il_modules/mrn.py:154-157): set requires_grad=False on every expert parameter")
-            logits, gate = RoutedSoft.apply(self, image, *self.router_parameters())
+                    "(il_modules/mrn.py:154-157): set requires_grad=False on every expert parameter, or set "
+                    "opt.autograd_experts to train the experts that require grad together with the router")
+            expert_params = [p for e in trainable for p in self.model[e].parameters()]
+            logits, gate = RoutedSoft.apply(self, image, trainable, *self.router_parameters(), *expert_params)
             return dict(logits=logits, index=gate, aux_logits=None)
         r = self.route_and_combine(image, is_train=is_train, want_logits=True)
         return dict(logits=r["logits"], index=r["index"], aux_logits=None)
@@ -457,17 +471,63 @@ class MRNNet(nn.Module):
     def pad_zeros_features(self, feature, total):
         raise RuntimeError("padding with ones is fused into mrnb_gate_combine; no padded tensor is materialised")
 
+    def joint_experts_forward(self, image, trainable):
+        """Expert outputs of the soft route when the experts in `trainable` (indices) train with the router
+        (opt.autograd_experts): the frozen ones through one grouped forward built over them alone, each trainable one
+        through its training pack.  DropPath is drawn once for all experts, as the grouped forward draws it.  Returns
+        (features [B,I,T,D], [logits_i], {expert index: training-pack backward})."""
+        if not image.is_cuda:
+            raise RuntimeError("mrn_b200 needs CUDA tensors: there is no CPU fallback")
+        full = self._cache.pack
+        if full is not None and getattr(full, "bn_dirty", False):
+            self._sync_bn()                 # BN statistics the full grouped pack holds -> the module buffers
+            self._frozen_cache.key = None
+        I, B = len(self.model), image.shape[0]
+        modes = self._experts_train_mode()
+        drop = None
+        if _arch(self.opt) == "svtr" and any(modes) and getattr(self.opt, "drop_path", True):
+            rates = self.model[0].model.FeatureExtraction.ConvNet.drop_path_rates()
+            drop = sample_drop_scales(I, B, rates, image.device)
+            for e, t in enumerate(modes):
+                if not t:
+                    drop[e].fill_(1.0)
+        feats = torch.empty(B, I, self.patch, self.out_dim, device=image.device, dtype=torch.float32)
+        logits = [None] * I
+        frozen = [e for e in range(I) if e not in trainable]
+        if frozen:
+            experts = [self.model[e] for e in frozen]
+            f, z = _experts_forward(experts, image, self.opt, tuple(modes[e] for e in frozen), self._frozen_cache,
+                                    drop_scales=None if drop is None else drop[frozen].contiguous())
+            feats[:, frozen] = f
+            for k, e in enumerate(frozen):
+                logits[e] = z[k]
+            if any(modes[e] for e in frozen):
+                _writeback_bn(experts, self._frozen_cache.pack)
+                self._cache.key = None      # the full grouped pack's BN statistics are stale now
+        backward = {}
+        for e in trainable:
+            z, f, backward[e] = _train_pack_run(self.model[e], image, self.opt, net=self, want_features=True,
+                                                drop=drop[e].contiguous() if drop is not None and modes[e] else None)
+            feats[:, e] = f
+            logits[e] = z
+        return feats, logits, backward
+
     def route_and_combine(self, image, is_train=True, want_logits=True, targets=None, lengths=None, want_E=False,
-                          want_decode=False, with_backward=False, drop_scales=None, rws=None):
+                          want_decode=False, with_backward=False, drop_scales=None, rws=None, experts_out=None):
         """Experts -> DM-Router -> gate -> fused combine.  Soft route when is_train (modules/model.py:397-423),
-        hard route otherwise (:366-395).  rws: router workspace to use instead of the module's own."""
+        hard route otherwise (:366-395).  rws: router workspace to use instead of the module's own.  experts_out:
+        (features [B,I,T,D], [logits_i]) computed by the caller (joint_experts_forward) instead of the grouped forward."""
         experts = list(self.model)
         # Hard route (eval): route FIRST, then evaluate only the routed expert's classifier head per sample (SURVEY K8e;
         # modules/model.py:383-393 keeps padded_{index[b]}[b] and discards the other five heads' logits).  The soft
         # route needs every head.
         sparse = (not is_train) and _arch(self.opt) == "svtr" and not int(getattr(self.opt, "expert_chunk", 0) or 0)
-        feats, logits = _experts_forward(experts, image, self.opt, self._experts_train_mode(), self._cache,
-                                         drop_scales=drop_scales, want_logits=not sparse)
+        if experts_out is not None:
+            assert not sparse, "precomputed expert outputs serve the soft route"
+            feats, logits = experts_out
+        else:
+            feats, logits = _experts_forward(experts, image, self.opt, self._experts_train_mode(), self._cache,
+                                             drop_scales=drop_scales, want_logits=not sparse)
         arena = self.router_arena(image.device)
         _, scores, gate, index = ops.router_forward(arena, feats, rws or self._rws, with_backward=with_backward,
                                                     prec=_precision(self.opt), want_out=False)

@@ -517,29 +517,46 @@ class SvtrTrainPack(_TrainPack):
         return _grow_workspace(self, int(L.load().mrnb_svtr_train_workspace_bytes(B, self.n_class, self.prec)))
 
 
-def svtr_train_forward(tp: SvtrTrainPack, image, bn_batch_stats=True, update_running=True, drop_scales=None):
-    """Activation-keeping forward of the expert being trained.  Returns logits [B,64,C] (a view of a padded buffer)."""
+def _features_out(B, T, device):
+    """The training packs' feature output [B,T,256] fp32 (dense)."""
+    return torch.empty(B, T, D_FEAT, device=device, dtype=torch.float32)
+
+
+def _chk_dfeatures(dfeatures, B, T):
+    if dfeatures is not None:
+        _chk_f32(dfeatures)
+        assert tuple(dfeatures.shape) == (B, T, D_FEAT) and dfeatures.is_contiguous(), "dfeatures must be dense [B,T,256]"
+
+
+def svtr_train_forward(tp: SvtrTrainPack, image, bn_batch_stats=True, update_running=True, drop_scales=None,
+                       want_features=False):
+    """Activation-keeping forward of the expert being trained.  Returns logits [B,64,C] (a view of a padded buffer), or
+    (logits, features [B,64,256]) with want_features."""
     _chk_f32(image, drop_scales)
     B = image.shape[0]
     ld = round_up(tp.n_class, 4)
     buf = torch.empty(B, T_FRAMES, ld, device=image.device, dtype=torch.float32)
+    feats = _features_out(B, T_FRAMES, image.device) if want_features else None
     ws = tp.workspace(B)
     tp.refresh_shadow()
-    L.check(L.load().mrnb_svtr_train_forward(C.byref(tp.struct), _p(image), B, tp.prec, int(bn_batch_stats),
-                                             int(update_running), _p(drop_scales), _p(buf), ld, _p(ws), ws.numel(),
-                                             _stream()), "svtr_train_forward")
-    return buf[:, :, :tp.n_class]
+    L.check(L.load().mrnb_svtr_train_forward_features(C.byref(tp.struct), _p(image), B, tp.prec, int(bn_batch_stats),
+                                                      int(update_running), _p(drop_scales), _p(buf), ld, _p(feats), _p(ws),
+                                                      ws.numel(), _stream()), "svtr_train_forward")
+    return (buf[:, :, :tp.n_class], feats) if want_features else buf[:, :, :tp.n_class]
 
 
-def svtr_train_backward(tp: SvtrTrainPack, image, dlogits, bn_batch_stats=True, drop_scales=None):
-    """Fills tp.grads (overwritten) from d loss / d logits [B,64,C]; must follow svtr_train_forward on the same batch."""
+def svtr_train_backward(tp: SvtrTrainPack, image, dlogits, bn_batch_stats=True, drop_scales=None, dfeatures=None):
+    """Fills tp.grads (overwritten) from d loss / d logits [B,64,C] (+ d loss / d features [B,64,256] reaching the
+    feature from outside the expert); must follow svtr_train_forward on the same batch."""
     _chk_f32(image, drop_scales)
     assert dlogits.dtype == torch.float32 and dlogits.stride(2) == 1 and dlogits.stride(0) == dlogits.shape[1] * dlogits.stride(1)
     B = image.shape[0]
+    _chk_dfeatures(dfeatures, B, T_FRAMES)
     ws = tp.workspace(B)
-    L.check(L.load().mrnb_svtr_train_backward(C.byref(tp.struct), C.byref(tp.gstruct), _p(image), _p(dlogits),
-                                              dlogits.stride(1), B, tp.prec, int(bn_batch_stats), _p(drop_scales),
-                                              _p(tp.grads), tp.numel, _p(ws), ws.numel(), _stream()), "svtr_train_backward")
+    L.check(L.load().mrnb_svtr_train_backward_features(C.byref(tp.struct), C.byref(tp.gstruct), _p(image), _p(dlogits),
+                                                       dlogits.stride(1), _p(dfeatures), B, tp.prec, int(bn_batch_stats),
+                                                       _p(drop_scales), _p(tp.grads), tp.numel, _p(ws), ws.numel(),
+                                                       _stream()), "svtr_train_backward")
     return tp.grads
 
 
@@ -592,25 +609,29 @@ class CrnnTrainPack(_TrainPack):
         return _grow_workspace(self, int(L.load().mrnb_crnn_train_workspace_bytes(B, self.n_class, self.prec)))
 
 
-def crnn_train_forward(tp: CrnnTrainPack, image, bn_batch_stats=True, update_running=True):
-    """Activation-keeping forward of the CRNN expert being trained.  Returns logits [B,63,C]."""
+def crnn_train_forward(tp: CrnnTrainPack, image, bn_batch_stats=True, update_running=True, want_features=False):
+    """Activation-keeping forward of the CRNN expert being trained.  Returns logits [B,63,C], or (logits, features
+    [B,63,256]) with want_features."""
     _chk_f32(image)
     B = image.shape[0]
     ld = round_up(tp.n_class, 4)
     buf = torch.empty(B, T_FRAMES_CRNN, ld, device=image.device, dtype=torch.float32)
+    feats = _features_out(B, T_FRAMES_CRNN, image.device) if want_features else None
     ws = tp.workspace(B)
     tp.refresh_shadow()
-    L.check(L.load().mrnb_crnn_train_forward(C.byref(tp.struct), _p(image), B, tp.prec, int(bn_batch_stats), int(update_running),
-                                             _p(buf), ld, _p(ws), ws.numel(), _stream()), "crnn_train_forward")
-    return buf[:, :, :tp.n_class]
+    L.check(L.load().mrnb_crnn_train_forward_features(C.byref(tp.struct), _p(image), B, tp.prec, int(bn_batch_stats),
+                                                      int(update_running), _p(buf), ld, _p(feats), _p(ws), ws.numel(),
+                                                      _stream()), "crnn_train_forward")
+    return (buf[:, :, :tp.n_class], feats) if want_features else buf[:, :, :tp.n_class]
 
 
-def crnn_train_backward(tp: CrnnTrainPack, dlogits, B, bn_batch_stats=True):
+def crnn_train_backward(tp: CrnnTrainPack, dlogits, B, bn_batch_stats=True, dfeatures=None):
     assert dlogits.dtype == torch.float32 and dlogits.stride(2) == 1 and dlogits.stride(0) == dlogits.shape[1] * dlogits.stride(1)
+    _chk_dfeatures(dfeatures, B, T_FRAMES_CRNN)
     ws = tp.workspace(B)
-    L.check(L.load().mrnb_crnn_train_backward(C.byref(tp.struct), C.byref(tp.gstruct), _p(dlogits), dlogits.stride(1), B, tp.prec,
-                                              int(bn_batch_stats), _p(tp.grads), tp.numel, _p(ws), ws.numel(), _stream()),
-            "crnn_train_backward")
+    L.check(L.load().mrnb_crnn_train_backward_features(C.byref(tp.struct), C.byref(tp.gstruct), _p(dlogits), dlogits.stride(1),
+                                                       _p(dfeatures), B, tp.prec, int(bn_batch_stats), _p(tp.grads), tp.numel,
+                                                       _p(ws), ws.numel(), _stream()), "crnn_train_backward")
     return tp.grads
 
 
@@ -769,16 +790,23 @@ def router_forward(params: torch.Tensor, x: torch.Tensor, ws: RouterWorkspace, w
     return out, scores, gate, index
 
 
-def router_backward(params, x, gate, dgate_ctc, domain, grads, ws: RouterWorkspace, prec=L.PREC_FP32):
+def router_backward(params, x, gate, dgate_ctc, domain, grads, ws: RouterWorkspace, prec=L.PREC_FP32, dx=None):
     """domain [B] int64: loss = pi*CTC + CE(gate, domain), returns the CE term.  domain None: dgate_ctc is the whole
-    dL/dgate of an arbitrary loss (no CE term), returns None."""
+    dL/dgate of an arbitrary loss (no CE term), returns None.  dx (optional, like x): also the input gradient dL/dx
+    (mrnb_router_backward_dx)."""
     _chk_f32(params, x, gate, dgate_ctc, grads)
     assert domain is None or domain.dtype == torch.int64
     B, I, T, D = x.shape
     taski = torch.empty(1, device=x.device, dtype=torch.float32) if domain is not None else None
     w = ws.get(B, I, T, D, True, x.device)
-    L.check(L.load().mrnb_router_backward(_p(params), _p(x), _p(gate), _p(dgate_ctc), _p(domain), B, I, T, D, prec,
-                                          _p(grads), _p(taski), _p(w), w.numel(), _stream()), "router_backward")
+    if dx is None:
+        L.check(L.load().mrnb_router_backward(_p(params), _p(x), _p(gate), _p(dgate_ctc), _p(domain), B, I, T, D, prec,
+                                              _p(grads), _p(taski), _p(w), w.numel(), _stream()), "router_backward")
+    else:
+        _chk_f32(dx)
+        assert dx.shape == x.shape and dx.is_contiguous()
+        L.check(L.load().mrnb_router_backward_dx(_p(params), _p(x), _p(gate), _p(dgate_ctc), _p(domain), B, I, T, D, prec,
+                                                 _p(grads), _p(dx), _p(taski), _p(w), w.numel(), _stream()), "router_backward_dx")
     return taski
 
 
@@ -839,10 +867,8 @@ def gate_combine(logits: Sequence[torch.Tensor], gate: torch.Tensor, targets: Op
     return r
 
 
-def gate_combine_backward(logits: Sequence[torch.Tensor], dY: torch.Tensor, out: Optional[torch.Tensor] = None):
-    """dgate [B,I] = d<dY, combined logits>/dgate for a dense upstream gradient dY [B,T,C] over the union charset (same
-    expert table as gate_combine; the pad value 1.0 counts).  dY rows that are not 16-byte aligned are first copied
-    into a padded buffer.  `out` may supply dgate."""
+def _aligned_dY(logits: Sequence[torch.Tensor], dY: torch.Tensor):
+    """dY [B,T,C] checked and, when its rows are not 16-byte aligned, copied into a padded buffer."""
     B, T, _ = logits[0].shape
     I, C = len(logits), logits[-1].shape[2]
     ptrs, lds, cs = _expert_tables(logits)
@@ -852,10 +878,42 @@ def gate_combine_backward(logits: Sequence[torch.Tensor], dY: torch.Tensor, out:
         buf = torch.zeros(B, T, round_up(C, 4), device=dY.device, dtype=torch.float32)
         buf[:, :, :C].copy_(dY)
         dY = buf[:, :, :C]
-    dgate = _out(out, (B, I), dY.device, torch.float32)
     ws = torch.empty(int(L.load().mrnb_gate_combine_backward_workspace_bytes(B, T, I)), dtype=torch.uint8, device=dY.device)
+    return dY, ptrs, lds, cs, ws
+
+
+def gate_combine_backward(logits: Sequence[torch.Tensor], dY: torch.Tensor, out: Optional[torch.Tensor] = None):
+    """dgate [B,I] = d<dY, combined logits>/dgate for a dense upstream gradient dY [B,T,C] over the union charset (same
+    expert table as gate_combine; the pad value 1.0 counts).  dY rows that are not 16-byte aligned are first copied
+    into a padded buffer.  `out` may supply dgate."""
+    dY, ptrs, lds, cs, ws = _aligned_dY(logits, dY)
+    B, T, I = dY.shape[0], dY.shape[1], len(logits)
+    dgate = _out(out, (B, I), dY.device, torch.float32)
     L.check(L.load().mrnb_gate_combine_backward(ptrs, lds, cs, I, B, T, _p(dY), dY.stride(1), _p(dgate), _p(ws), ws.numel(),
                                                 _stream()), "gate_combine_backward")
+    return dgate
+
+
+def gate_combine_backward_experts(logits: Sequence[torch.Tensor], dY: torch.Tensor, gate: torch.Tensor,
+                                  dz: Sequence[Optional[torch.Tensor]], out: Optional[torch.Tensor] = None):
+    """gate_combine_backward plus, in the same pass, dz[i] = gate[:, i] * dY[:, :, :C_i] for every dz[i] given (fp32
+    [B,T,C_i] views with a dense row layout, 16-byte aligned rows); a None entry (a frozen expert) is skipped.
+    Returns dgate."""
+    dY, ptrs, lds, cs, ws = _aligned_dY(logits, dY)
+    B, T, I = dY.shape[0], dY.shape[1], len(logits)
+    _chk_f32(gate)
+    assert tuple(gate.shape) == (B, I) and len(dz) == I
+    dzp = (C.c_void_p * I)()
+    ldz = (C.c_long * I)()
+    for i, t in enumerate(dz):
+        if t is not None:
+            if t.dtype != torch.float32 or tuple(t.shape) != (B, T, cs[i]) or t.stride(2) != 1 or t.stride(0) != T * t.stride(1):
+                raise RuntimeError("gate_combine_backward_experts: dz[%d] must be fp32 [B,T,C_i] with a dense row layout" % i)
+            dzp[i], ldz[i] = t.data_ptr(), t.stride(1)
+    dgate = _out(out, (B, I), dY.device, torch.float32)
+    L.check(L.load().mrnb_gate_combine_backward_experts(ptrs, lds, cs, I, B, T, _p(dY), dY.stride(1), _p(gate), dzp, ldz,
+                                                        _p(dgate), _p(ws), ws.numel(), _stream()),
+            "gate_combine_backward_experts")
     return dgate
 
 
