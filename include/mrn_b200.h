@@ -151,6 +151,21 @@ int mrnb_svtr_train_backward_features(const MrnbSvtrPack* pack, const MrnbSvtrPa
                                       int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
                                       void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
+/* The backward with the gradient with respect to the input image, for any differentiable module in front of the
+ * recogniser (a rectification front end such as the reference's Transformation="TPS" stage, modules/transformation.py:9-216;
+ * learned augmentation; inversion of a frozen expert; saliency maps).  Arguments as mrnb_svtr_train_backward_features
+ * (which is this call with dimage = NULL), plus:
+ *   dimage: NULL or [B,4,32,256] fp32 NCHW (dense), overwritten with dL/dimage -- the input gradient of the patch
+ *           embedding's conv0 (modules/svtr.py PatchEmbed.proj[0], Conv2d(4, 32, 3, 2, 1)), read from the fp32 gradient
+ *           at conv0's output in both precision modes.
+ *   grads / grad_arena: both NULL selects the input-only backward of a frozen expert -- no parameter gradient is
+ *           computed (every launch whose only product is one is skipped); the BatchNorm batch statistics the input
+ *           gradient needs are kept.  At least one of grad_arena and dimage must be non-NULL (else MRNB_ERR_ARG). */
+int mrnb_svtr_train_backward_input(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
+                                   const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                   int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
+                                   float* dimage, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * CRNN expert recognisers (VGG + 2 x BidirectionalLSTM + CTC head), T = 63 frames.
  * Replaces modules/feature_extraction.py:19-47 (VGG_FeatureExtractor.forward), modules/sequence_modeling.py:12-22
@@ -272,6 +287,13 @@ int mrnb_crnn_train_backward_features(const MrnbCrnnTrainPack* pack, const MrnbC
                                       long ld_dlogits, const float* dfeatures, int B, int prec, int bn_batch_stats,
                                       float* grad_arena, long n_arena, void* workspace, size_t workspace_bytes,
                                       cudaStream_t stream);
+/* As mrnb_svtr_train_backward_input: the image gradient dimage (NULL or [B,4,32,256] fp32 NCHW, overwritten) is the input
+ * gradient of VGG's conv0 (modules/feature_extraction.py:27, Conv2d(4, 64, 3, 1, 1)), returned in the caller's NCHW
+ * layout although the forward runs on an NHWC copy of the image; grads = grad_arena = NULL: input-only backward. */
+int mrnb_crnn_train_backward_input(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads, const float* dlogits,
+                                   long ld_dlogits, const float* dfeatures, int B, int prec, int bn_batch_stats,
+                                   float* grad_arena, long n_arena, float* dimage, void* workspace, size_t workspace_bytes,
+                                   cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * DM-Router + gate head.   Replaces modules/dm_router.py:50-67 (DM_Router.forward, both gating blocks) and
@@ -447,6 +469,12 @@ int mrnb_attn_tc_train_forward(const void* qkv, void* P, void* O, int B, int N, 
                                cudaStream_t stream);
 int mrnb_attn_tc_train_backward(const void* qkv, const void* O, const float* dO, const void* dO16, const void* P, void* dS,
                                 void* dqkv, int B, int N, int d, int heads, cudaStream_t stream);
+/* conv0 input-gradient kernels of the two backwards above, on their own: d = the fp32 gradient at conv0's output, NHWC
+ * ([B,16,128,32] SVTR / [B,32,256,64] CRNN); w = the training pack's conv0 weight ([32,4,3,3] nn.Conv2d layout / [64,3,3,4]);
+ * dimage [B,4,32,256] fp32 NCHW, every element overwritten.  One thread per pixel sums its taps and channels in a fixed
+ * order: bitwise repeatable.  B <= 65535. */
+int mrnb_svtr_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t stream);
+int mrnb_crnn_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t stream);
 int mrnb_cast_f32_to_bf16(const float* x, void* y, long n, cudaStream_t stream);
 int mrnb_cast_f32_to_f16(const float* x, void* y, long n, cudaStream_t stream);
 

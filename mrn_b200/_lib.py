@@ -97,6 +97,12 @@ _SIGNATURES = {
     "mrnb_crnn_train_forward_features": (_i, [C.POINTER(MrnbCrnnTrainPack), _vp, _i, _i, _i, _i, _vp, _l, _vp, _vp, _sz, _vp]),
     "mrnb_crnn_train_backward_features": (_i, [C.POINTER(MrnbCrnnTrainPack), C.POINTER(MrnbCrnnTrainPack), _vp, _l, _vp, _i,
                                                _i, _i, _vp, _l, _vp, _sz, _vp]),
+    "mrnb_svtr_train_backward_input": (_i, [C.POINTER(MrnbSvtrPack), C.POINTER(MrnbSvtrPack), _vp, _vp, _l, _vp, _i, _i,
+                                            _i, _vp, _vp, _l, _vp, _vp, _sz, _vp]),
+    "mrnb_crnn_train_backward_input": (_i, [C.POINTER(MrnbCrnnTrainPack), C.POINTER(MrnbCrnnTrainPack), _vp, _l, _vp, _i,
+                                            _i, _i, _vp, _l, _vp, _vp, _sz, _vp]),
+    "mrnb_svtr_conv0_dimage": (_i, [_vp, _vp, _vp, _i, _vp]),
+    "mrnb_crnn_conv0_dimage": (_i, [_vp, _vp, _vp, _i, _vp]),
     "mrnb_crnn_workspace_bytes": (_sz, [_i, _i, _i]),
     "mrnb_crnn_experts_forward": (_i, [C.POINTER(MrnbCrnnPack), _vp, _i, _i, _i, _i, _vp, C.POINTER(_vp), C.POINTER(_l),
                                        _vp, _sz, _vp]),

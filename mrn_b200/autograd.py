@@ -10,7 +10,10 @@ once_differentiable: a double backward raises.
     trainable experts: those run their training packs, and the backward is mrnb_gate_combine_backward_experts (dgate
     and each trainable expert's logit gradient dz_i = g_i dY in one pass), mrnb_router_backward_dx (the router's input
     gradient dx) and one training-pack backward per trainable expert with dz_i and dx[:, i] as the feature gradient.
-  * ExpertTrain: one expert end to end through its training pack (activation-keeping forward, full backward).
+    An image that requires grad makes every expert run its training pack: the frozen ones take the input-only backward
+    (no parameter gradient), and the image gradient is the sum of the experts' image gradients in expert order.
+  * ExpertTrain: one expert end to end through its training pack (activation-keeping forward, full backward, or the
+    input-only backward when no expert parameter requires grad); logits, and the feature when asked for.
   * DmRouter: DM_Router on its own through mrnb_dm_router_backward (input and parameter gradients).
 """
 import torch
@@ -41,8 +44,9 @@ class RoutedSoft(torch.autograd.Function):
     def forward(ctx, net, image, trainable, *params):
         rws = ops.RouterWorkspace()          # the backward reads the activations this forward leaves in it
         experts_out, ctx.expert_backward = None, {}
-        if trainable:
-            feats, logits, ctx.expert_backward = net.joint_experts_forward(image, trainable)
+        if trainable or ctx.needs_input_grad[1]:
+            feats, logits, ctx.expert_backward = net.joint_experts_forward(image, trainable,
+                                                                           input_grad=ctx.needs_input_grad[1])
             experts_out = (feats, logits)
         r = net.route_and_combine(image, is_train=True, want_logits=True, with_backward=True, rws=rws,
                                   experts_out=experts_out)
@@ -57,44 +61,59 @@ class RoutedSoft(torch.autograd.Function):
         from .modules.model import _precision
         arena, feats, gate = ctx.saved_tensors
         net, trainable = ctx.net, ctx.trainable
+        packs = sorted(ctx.expert_backward)  # the experts that ran a training pack: trainable ones, or all for the image
         B, I, T, D = feats.shape
         dz = [None] * I
-        for e in trainable:                  # rows padded to 4 floats, as the kernel writes them
+        for e in packs:                      # rows padded to 4 floats, as the kernel writes them
             z = ctx.expert_logits[e]
             dz[e] = torch.zeros(B, T, ops.round_up(z.shape[2], 4), device=z.device)[:, :, :z.shape[2]]
         dgate = torch.zeros_like(gate)
         if d_logits is not None:
-            if trainable:
+            if packs:
                 dgate = ops.gate_combine_backward_experts(ctx.expert_logits, d_logits.float(), gate, dz)
             else:
                 dgate = ops.gate_combine_backward(ctx.expert_logits, d_logits.float())
         if d_gate is not None:
             dgate = dgate + d_gate.float()
         grads = torch.empty_like(arena)
-        dx = torch.empty_like(feats) if trainable else None
+        dx = torch.empty_like(feats) if packs else None
         ops.router_backward(arena, feats, gate, dgate.contiguous(), None, grads, ctx.rws, prec=_precision(net.opt), dx=dx)
         out = _arena_grads(grads, net.router_parameters(), ops.ROUTER_PARAM_NAMES, I, T, D)
-        for e in trainable:
-            keys = [k for k, _ in net.model[e].named_parameters()]
-            out += _expert_grads(ctx.expert_backward[e](dz[e], dx[:, e].contiguous()), keys)
-        return (None, None, None) + out
+        dimage = None
+        for e in packs:
+            g, di = ctx.expert_backward[e](dz[e], dx[:, e].contiguous(), dimage=ctx.needs_input_grad[1])
+            if e in trainable:
+                out += _expert_grads(g, [k for k, _ in net.model[e].named_parameters()])
+            if di is not None:               # summed in expert order
+                dimage = di if dimage is None else dimage.add_(di)
+        return (None, dimage, None) + out
 
 
 class ExpertTrain(torch.autograd.Function):
-    """(run, keys, image, *params) -> logits [B,T,C].  `run(image)` is modules.model._train_pack_run for one expert:
-    (logits, features, backward), backward(dlogits) -> {state_dict key: gradient in the reference layout}; `params`
-    are the expert's parameters named by `keys`."""
+    """(run, keys, want_features, image, *params) -> logits [B,T,C], or (logits, features [B,T,256]) with
+    want_features.  `run(image, want_features=, param_grads=)` is modules.model._train_pack_run for one expert:
+    (logits, features, backward), backward(dlogits, dfeatures, dimage=) -> ({state_dict key: gradient in the reference
+    layout} or None, image gradient or None); `params` are the expert's parameters named by `keys`.  The pack is built
+    without a gradient arena (input-only backward) when none of `params` requires grad."""
 
     @staticmethod
-    def forward(ctx, run, keys, image, *params):
-        logits, _, backward = run(image)
-        ctx.run_backward, ctx.keys = backward, keys
-        return logits
+    def forward(ctx, run, keys, want_features, image, *params):
+        param_grads = any(ctx.needs_input_grad[4:])
+        logits, feats, backward = run(image, want_features=want_features, param_grads=param_grads)
+        ctx.run_backward, ctx.keys, ctx.param_grads = backward, keys, param_grads
+        ctx.set_materialize_grads(False)
+        ctx.logits_shape = logits.shape
+        return (logits, feats) if want_features else logits
 
     @staticmethod
     @once_differentiable
-    def backward(ctx, d_logits):
-        return (None, None, None) + _expert_grads(ctx.run_backward(d_logits.float().contiguous()), ctx.keys)
+    def backward(ctx, d_logits, d_features=None):
+        if d_logits is None:                 # only the feature reached the loss
+            d_logits = torch.zeros(ctx.logits_shape, device=d_features.device)
+        dfeat = None if d_features is None else d_features.float().contiguous()
+        grads, dimage = ctx.run_backward(d_logits.float().contiguous(), dfeat, dimage=ctx.needs_input_grad[3])
+        pgrads = _expert_grads(grads, ctx.keys) if ctx.param_grads else (None,) * len(ctx.keys)
+        return (None, None, None, dimage) + pgrads
 
 
 class DmRouter(torch.autograd.Function):

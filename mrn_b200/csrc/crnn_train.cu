@@ -434,16 +434,19 @@ int crnn_train_forward_t(const MrnbCrnnTrainPack& P, const float* image, int B, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Backward
+// Backward.  grad_arena NULL (G all NULL): the input-only backward -- every launch whose only product is a parameter
+// gradient is skipped, the BatchNorm apply pass gets NULL gamma / beta outputs.  dimage: NULL or the image gradient
+// [B,4,32,256] (NCHW, overwritten).
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
 int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G, const float* dlogits, long ldg,
-                          const float* dfeatures, int B, int bn_batch, float* grad_arena, long n_arena, void* ws, size_t ws_bytes,
-                          cudaStream_t st) {
+                          const float* dfeatures, int B, int bn_batch, float* grad_arena, long n_arena, float* dimage, void* ws,
+                          size_t ws_bytes, cudaStream_t st) {
   constexpr bool TC = sizeof(AT) == 2;
+  const bool pg = grad_arena != nullptr;
   CrnnWs<AT> w = carve_crnn_ws<AT>((char*)ws, B, P.n_class);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "crnn_train_backward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
-  cudaMemsetAsync(grad_arena, 0, (size_t)n_arena * sizeof(float), st);
+  if (pg) cudaMemsetAsync(grad_arena, 0, (size_t)n_arena * sizeof(float), st);
   const int M = B * T63, C = P.n_class;
   // ---- CTC head
   Grad dlog{dlogits, nullptr, ldg};
@@ -453,8 +456,10 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
     MRNB_CHECK_LAUNCH("cast_pad_rows_kernel");
     dlog = Grad{dlogits, w.dlog16, ld16};
   }
-  MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, gpt(G, MRNB_T_FC_B), st));
-  MRNB_TRY(gemm_dw<AT>(dlog, w.out16[1], 256, gpt(G, MRNB_T_FC_W), M, C, 256, st));
+  if (pg) {
+    MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, gpt(G, MRNB_T_FC_B), st));
+    MRNB_TRY(gemm_dw<AT>(dlog, w.out16[1], 256, gpt(G, MRNB_T_FC_W), M, C, 256, st));
+  }
   bf16* dout16 = TC ? w.d16 : nullptr;
   // d feature = dlogits W_fc (+ dfeatures, the gradient reaching the feature from outside the expert, in the epilogue)
   MRNB_TRY(gemm_dx<AT>(dlog, P.p[MRNB_T_FC_W], P.h[MRNB_T_FC_W], w.dout, dout16, 256, M, C, 256, st, dfeatures));
@@ -465,8 +470,10 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
     const int Kin = k == 0 ? 512 : 256;
     Grad gout{w.dout, dout16, 256};
     const AT* r = TC ? w.rec16[k] : reinterpret_cast<const AT*>(w.rec[k]);
-    MRNB_TRY(launch_colsum<float>(w.dout, 256, M, 256, gpt(G, s0 + MRNB_TL_LIN_B), st));
-    MRNB_TRY(gemm_dw<AT>(gout, r, 512, gpt(G, s0 + MRNB_TL_LIN_W), M, 256, 512, st));
+    if (pg) {
+      MRNB_TRY(launch_colsum<float>(w.dout, 256, M, 256, gpt(G, s0 + MRNB_TL_LIN_B), st));
+      MRNB_TRY(gemm_dw<AT>(gout, r, 512, gpt(G, s0 + MRNB_TL_LIN_W), M, 256, 512, st));
+    }
     MRNB_TRY(gemm_dx<AT>(gout, P.p[s0 + MRNB_TL_LIN_W], P.h[s0 + MRNB_TL_LIN_W], w.drec, nullptr, 512, M, 256, 512, st));
     // BPTT: direction 0 from t = 62 down, direction 1 from t = 0 up
     for (int s = 0; s < T63; ++s) {
@@ -503,13 +510,15 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
     // G now holds d(gate pre-activations) [M, 2048] for both directions
     Grad gG{w.G[k], nullptr, 2048};
     if (TC) gG.h = w.dG16;                     // written step by step by the cell kernel
-    MRNB_TRY(launch_colsum<float>(w.G[k], 2048, M, 2048, gpt(G, s0 + MRNB_TL_BIH), st));
-    cudaMemcpyAsync(gpt(G, s0 + MRNB_TL_BHH), gpt(G, s0 + MRNB_TL_BIH), 2048 * sizeof(float), cudaMemcpyDeviceToDevice, st);
-    const AT* xin = k == 0 ? (TC ? w.vis16 : reinterpret_cast<const AT*>(w.act[6])) : w.out16[0];
-    MRNB_TRY(gemm_dw<AT>(gG, xin, Kin, gpt(G, s0 + MRNB_TL_WIH), M, 2048, Kin, st));
-    for (int dir = 0; dir < 2; ++dir) {
-      Grad gd{w.G[k] + dir * 1024, TC ? w.dG16 + dir * 1024 : nullptr, 2048};
-      MRNB_TRY(gemm_dw<AT>(gd, w.hseq[k] + dir * HID, 512, gpt(G, s0 + MRNB_TL_WHH) + (long)dir * 1024 * HID, M, 1024, HID, st));
+    if (pg) {
+      MRNB_TRY(launch_colsum<float>(w.G[k], 2048, M, 2048, gpt(G, s0 + MRNB_TL_BIH), st));
+      cudaMemcpyAsync(gpt(G, s0 + MRNB_TL_BHH), gpt(G, s0 + MRNB_TL_BIH), 2048 * sizeof(float), cudaMemcpyDeviceToDevice, st);
+      const AT* xin = k == 0 ? (TC ? w.vis16 : reinterpret_cast<const AT*>(w.act[6])) : w.out16[0];
+      MRNB_TRY(gemm_dw<AT>(gG, xin, Kin, gpt(G, s0 + MRNB_TL_WIH), M, 2048, Kin, st));
+      for (int dir = 0; dir < 2; ++dir) {
+        Grad gd{w.G[k] + dir * 1024, TC ? w.dG16 + dir * 1024 : nullptr, 2048};
+        MRNB_TRY(gemm_dw<AT>(gd, w.hseq[k] + dir * HID, 512, gpt(G, s0 + MRNB_TL_WHH) + (long)dir * 1024 * HID, M, 1024, HID, st));
+      }
     }
     float* dx = k == 0 ? dxin : w.dout;        // layer 1's input gradient is layer 0's output gradient
     MRNB_TRY(gemm_dx<AT>(gG, P.p[s0 + MRNB_TL_WIH], P.h[s0 + MRNB_TL_WIH], dx, k == 1 ? dout16 : nullptr, Kin, M, 2048, Kin, st));
@@ -529,7 +538,7 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
       maxpool_relu_bwd_kernel<<<cdiv(np / 4, 256), 256, 0, st>>>(w.act[l], d, other, Ho, Wo, L.Cout, L.ph, L.pw, np / 4);
       MRNB_CHECK_LAUNCH("maxpool_relu_bwd_kernel");
       float* t = d; d = other; other = t;
-      if (d16 && L.bn < 0) {
+      if (d16 && L.bn < 0 && (l > 0 || pg)) {      // conv0's 16-bit gradient feeds only its weight gradient
         cast_kernel<bf16><<<cdiv(n, 256), 256, 0, st>>>(d, d16, n);
         MRNB_CHECK_LAUNCH("cast_kernel");
       }
@@ -548,26 +557,30 @@ int crnn_train_backward_t(const MrnbCrnnTrainPack& P, const MrnbCrnnTrainPack& G
       MRNB_CHECK_LAUNCH("bn_bwd_apply_kernel");
     }
     // conv backward
-    if (L.b_slot >= 0) MRNB_TRY(launch_colsum<float>(d, L.Cout, rows, L.Cout, gpt(G, L.b_slot), st));
+    if (pg && L.b_slot >= 0) MRNB_TRY(launch_colsum<float>(d, L.Cout, rows, L.Cout, gpt(G, L.b_slot), st));
     const float* in = l == 0 ? w.img4 : w.pool[l - 1];
-    if (l == 0 && TC) {
-      im2col_c4_pad64_kernel<<<cdiv((long)rows * 8, 256), 256, 0, st>>>(in, reinterpret_cast<bf16*>(w.col), L.H, L.W, rows);
-      MRNB_CHECK_LAUNCH("im2col_c4_pad64_kernel");
-      cudaMemsetAsync(w.dw0pad, 0, 64 * 64 * sizeof(float), st);
-      MRNB_TRY(gemm_dw_tc(d16, 64, reinterpret_cast<const bf16*>(w.col), 64, w.dw0pad, rows, 64, 64, st));
-      unpad_dw0_kernel<<<9, 256, 0, st>>>(w.dw0pad, gpt(G, L.w_slot), 64);
-      MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
+    if (l == 0) {
+      if (pg && TC) {
+        im2col_c4_pad64_kernel<<<cdiv((long)rows * 8, 256), 256, 0, st>>>(in, reinterpret_cast<bf16*>(w.col), L.H, L.W, rows);
+        MRNB_CHECK_LAUNCH("im2col_c4_pad64_kernel");
+        cudaMemsetAsync(w.dw0pad, 0, 64 * 64 * sizeof(float), st);
+        MRNB_TRY(gemm_dw_tc(d16, 64, reinterpret_cast<const bf16*>(w.col), 64, w.dw0pad, rows, 64, 64, st));
+        unpad_dw0_kernel<<<9, 256, 0, st>>>(w.dw0pad, gpt(G, L.w_slot), 64);
+        MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
+      } else if (pg) {
+        float* colf = w.dcol;
+        MRNB_TRY(launch_im2col<float>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
+        MRNB_TRY(gemm_dw_f32(d, L.Cout, colf, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
+      }
+      // the image gradient from the fp32 d (never its bf16 copy), back in the caller's NCHW layout
+      if (dimage) MRNB_TRY(launch_crnn_conv0_dimage(d, P.p[L.w_slot], dimage, B, st));
       break;
     }
-    if (l == 0) {
-      float* colf = w.dcol;
-      MRNB_TRY(launch_im2col<float>(in, colf, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
-      MRNB_TRY(gemm_dw_f32(d, L.Cout, colf, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
-      break;                                   // no gradient w.r.t. the image
-    }
     Grad gd{d, d16, L.Cout};
-    MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
-    MRNB_TRY(gemm_dw<AT>(gd, w.col, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
+    if (pg) {
+      MRNB_TRY(launch_im2col<AT>(in, w.col, L.H, L.W, L.Cin, L.KH, L.KW, L.pad, 1, 1, Ho, Wo, rows, st));
+      MRNB_TRY(gemm_dw<AT>(gd, w.col, K, gpt(G, L.w_slot), rows, L.Cout, K, st));
+    }
     MRNB_TRY(gemm_dx<AT>(gd, P.p[L.w_slot], P.h[L.w_slot], w.dcol, nullptr, K, rows, L.Cout, K, st));
     const long in4 = (long)B * L.H * L.W * L.Cin / 4;
     // LAYERS has 3 x 3 windows and the 2 x 2 of conv6
@@ -610,20 +623,34 @@ extern "C" int mrnb_crnn_train_forward(const MrnbCrnnTrainPack* pack, const floa
                                           workspace, workspace_bytes, stream);
 }
 
+extern "C" int mrnb_crnn_train_backward_input(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads,
+                                              const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                              int bn_batch_stats, float* grad_arena, long n_arena, float* dimage,
+                                              void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  MRNB_CHECK_ARG(pack && dlogits && workspace && B > 0, "crnn_train_backward: null/empty argument");
+  MRNB_CHECK_ARG(grad_arena || dimage, "crnn_train_backward: neither the gradient arena nor dimage given");
+  MRNB_CHECK_ARG(!grads == !grad_arena, "crnn_train_backward: grads and grad_arena are given together or both NULL");
+  if (grads)
+    for (int k = 0; k < MRNB_T_COUNT; ++k) MRNB_CHECK_ARG(grads->p[k], "crnn_train_backward: gradient slot %d is null", k);
+  static const MrnbCrnnTrainPack no_grads{};   // input-only backward: every parameter-gradient pointer NULL
+  const MrnbCrnnTrainPack& G = grads ? *grads : no_grads;
+  if (prec == MRNB_PREC_FP32)
+    return crnn_train_backward_t<float>(*pack, G, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena, n_arena,
+                                        dimage, workspace, workspace_bytes, stream);
+  if (prec == MRNB_PREC_BF16)
+    return crnn_train_backward_t<__nv_bfloat16>(*pack, G, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena,
+                                                n_arena, dimage, workspace, workspace_bytes, stream);
+  mrnb_set_error("crnn_train_backward: unknown precision %d", prec);
+  return MRNB_ERR_ARG;
+}
+
 extern "C" int mrnb_crnn_train_backward_features(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads,
                                                  const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
                                                  int bn_batch_stats, float* grad_arena, long n_arena, void* workspace,
                                                  size_t workspace_bytes, cudaStream_t stream) {
-  MRNB_CHECK_ARG(pack && grads && dlogits && grad_arena && workspace && B > 0, "crnn_train_backward: null/empty argument");
-  for (int k = 0; k < MRNB_T_COUNT; ++k) MRNB_CHECK_ARG(grads->p[k], "crnn_train_backward: gradient slot %d is null", k);
-  if (prec == MRNB_PREC_FP32)
-    return crnn_train_backward_t<float>(*pack, *grads, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena, n_arena,
-                                        workspace, workspace_bytes, stream);
-  if (prec == MRNB_PREC_BF16)
-    return crnn_train_backward_t<__nv_bfloat16>(*pack, *grads, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, grad_arena,
-                                                n_arena, workspace, workspace_bytes, stream);
-  mrnb_set_error("crnn_train_backward: unknown precision %d", prec);
-  return MRNB_ERR_ARG;
+  MRNB_CHECK_ARG(grads && grad_arena, "crnn_train_backward: null/empty argument");
+  return mrnb_crnn_train_backward_input(pack, grads, dlogits, ld_dlogits, dfeatures, B, prec, bn_batch_stats, grad_arena,
+                                        n_arena, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int mrnb_crnn_train_backward(const MrnbCrnnTrainPack* pack, const MrnbCrnnTrainPack* grads, const float* dlogits,
@@ -631,4 +658,11 @@ extern "C" int mrnb_crnn_train_backward(const MrnbCrnnTrainPack* pack, const Mrn
                                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   return mrnb_crnn_train_backward_features(pack, grads, dlogits, ld_dlogits, nullptr, B, prec, bn_batch_stats, grad_arena,
                                            n_arena, workspace, workspace_bytes, stream);
+}
+
+// ---- C-ABI test entry: VGG conv0's input gradient on its own (d [B,32,256,64] NHWC fp32, w [64,3,3,4] -> dimage
+// [B,4,32,256] NCHW fp32), as crnn_train_backward_t launches it
+extern "C" int mrnb_crnn_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t stream) {
+  MRNB_CHECK_ARG(d && w && dimage && B > 0 && B <= 65535, "crnn_conv0_dimage: bad argument");
+  return launch_crnn_conv0_dimage(d, w, dimage, B, stream);
 }

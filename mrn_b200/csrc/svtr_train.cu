@@ -181,6 +181,7 @@ int launch_ln_fwd(const float* x, OT* y, const float* gamma, const float* beta, 
 
 // dx = add + rstd * (g*dy - mean(g*dy) - xhat * mean(g*dy*xhat));  dgamma += sum dy*xhat;  dbeta += sum dy.
 // `add` (the gradient arriving over the residual connection) may be null and may alias dx.  Optional 16-bit copy of dx.
+// dgamma / dbeta both null: dx only (the input-only backward).
 template <int D>
 __global__ void __launch_bounds__(256)
 ln_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, const float* __restrict__ gamma,
@@ -220,6 +221,7 @@ ln_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, const f
       if (dx16) dx16[o] = __float2bfloat16_rn(scale16 ? r * scale16[row / rows_per_scale] : r);
     }
   }
+  if (dgamma == nullptr) return;                     // input-only backward: no dgamma / dbeta (uniform over the block)
 #pragma unroll
   for (int j = 0; j < VPT; ++j) red[wp][lane + 32 * j] = ag[j];
   __syncthreads();
@@ -807,16 +809,20 @@ int train_forward_t(const MrnbSvtrPack& P, const float* image, int B, int bn_bat
 
 // ------------------------------------------------------------------------------------------------
 // Backward.  G holds the gradient pointers in the same slots; the caller passes the flat gradient arena so that it is
-// zeroed with one memset (split-K GEMMs, LayerNorm / bias sums accumulate with atomics).
+// zeroed with one memset (split-K GEMMs, LayerNorm / bias sums accumulate with atomics).  grad_arena NULL (G all NULL):
+// the input-only backward -- every launch whose only product is a parameter gradient is skipped, the kernels that write
+// a dX and a parameter gradient in one pass (LayerNorm, BatchNorm apply) get NULL parameter outputs.  dimage: NULL or
+// the image gradient [B,4,32,256] (NCHW, overwritten).
 // ------------------------------------------------------------------------------------------------
 template <typename AT>
 int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* image, const float* dlogits, long ldg,
-                     const float* dfeatures, int B, int bn_batch, const float* drop, float* grad_arena, long n_arena, void* ws,
-                     size_t ws_bytes, cudaStream_t st) {
+                     const float* dfeatures, int B, int bn_batch, const float* drop, float* grad_arena, long n_arena,
+                     float* dimage, void* ws, size_t ws_bytes, cudaStream_t st) {
   constexpr bool TC = sizeof(AT) == 2;
+  const bool pg = grad_arena != nullptr;
   TrainWs<AT> w = carve_train_ws<AT>((char*)ws, B, P.n_class[0]);
   MRNB_CHECK_ARG(ws_bytes >= w.bytes, "svtr_train_backward: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
-  cudaMemsetAsync(grad_arena, 0, (size_t)n_arena * sizeof(float), st);
+  if (pg) cudaMemsetAsync(grad_arena, 0, (size_t)n_arena * sizeof(float), st);
   const long u = (long)B * 32768;
   const int M = B * 64, C = P.n_class[0];
   // ---- CTC head and the 512 -> 256 Linear
@@ -828,13 +834,17 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
     MRNB_CHECK_LAUNCH("cast_pad_rows_kernel");
     dlog = Grad{dlogits, w.dlog16, ld16};
   }
-  MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, const_cast<float*>(G.fc_b[0]), st));
-  MRNB_TRY(gemm_dw<AT>(dlog, w.feat, 256, const_cast<float*>(G.fc_w[0]), M, C, 256, st));
+  if (pg) {
+    MRNB_TRY(launch_colsum<float>(dlogits, ldg, M, C, const_cast<float*>(G.fc_b[0]), st));
+    MRNB_TRY(gemm_dw<AT>(dlog, w.feat, 256, const_cast<float*>(G.fc_w[0]), M, C, 256, st));
+  }
   // d feature = dlogits W_fc (+ dfeatures, the gradient reaching the feature from outside the expert, in the epilogue)
   MRNB_TRY(gemm_dx<AT>(dlog, P.fc_w[0], P.fc_w16[0], w.dfeat, w.dfeat16, 256, M, C, 256, st, dfeatures));
   Grad dfe{w.dfeat, w.dfeat16, 256};
-  MRNB_TRY(launch_colsum<float>(w.dfeat, 256, M, 256, gp(G, MRNB_P_SEQ_B), st));
-  MRNB_TRY(gemm_dw<AT>(dfe, w.vis, 512, gp(G, MRNB_P_SEQ_W), M, 256, 512, st));
+  if (pg) {
+    MRNB_TRY(launch_colsum<float>(w.dfeat, 256, M, 256, gp(G, MRNB_P_SEQ_B), st));
+    MRNB_TRY(gemm_dw<AT>(dfe, w.vis, 512, gp(G, MRNB_P_SEQ_W), M, 256, 512, st));
+  }
   MRNB_TRY(gemm_dx<AT>(dfe, P.p[MRNB_P_SEQ_W], P.h[MRNB_P_SEQ_W], w.dln, nullptr, 512, M, 256, 512, st));       // d vis
   float* dx = w.dxa;          // gradient w.r.t. the residual stream
   float* dcv = w.dy;          // gradient w.r.t. a SubSample conv output (+ its 16-bit copy in dy16)
@@ -855,9 +865,11 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
     // ---- SubSample conv backward (im2col recomputed from the stage output)
     {
       Grad gcv{dcv, w.dy16, Co};
-      MRNB_TRY(launch_colsum<float>(dcv, Co, orows, Co, gp(G, ps + MRNB_PS_CONV_B), st));
-      MRNB_TRY(launch_im2col<AT>(w.xout[blk - 1], w.big, H, Wd, d, 3, 3, 1, 2, 1, Ho, Wd, (long)orows, st));
-      MRNB_TRY(gemm_dw<AT>(gcv, w.big, 9 * d, gp(G, ps + MRNB_PS_CONV_W), orows, Co, 9 * d, st));
+      if (pg) {
+        MRNB_TRY(launch_colsum<float>(dcv, Co, orows, Co, gp(G, ps + MRNB_PS_CONV_B), st));
+        MRNB_TRY(launch_im2col<AT>(w.xout[blk - 1], w.big, H, Wd, d, 3, 3, 1, 2, 1, Ho, Wd, (long)orows, st));
+        MRNB_TRY(gemm_dw<AT>(gcv, w.big, 9 * d, gp(G, ps + MRNB_PS_CONV_W), orows, Co, 9 * d, st));
+      }
       MRNB_TRY(gemm_dx<AT>(gcv, P.p[ps + MRNB_PS_CONV_W], P.h[ps + MRNB_PS_CONV_W], w.dbig, nullptr, 9 * d, orows, Co, 9 * d, st));
       col2im_nhwc_kernel<3, 3><<<cdiv(u / 4, 256), 256, 0, st>>>(w.dbig, dx, H, Wd, d, 1, 2, 1, Ho, Wd, u / 4);
       MRNB_CHECK_LAUNCH("col2im_nhwc_kernel");
@@ -876,9 +888,11 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
         MRNB_CHECK_LAUNCH("scale_rows_kernel");
         if (drop && !TC) gy.f = w.dy;
       }
-      if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dy16, d, rows, d, gp(G, pb + MRNB_PB_FC2_B), st));
-      else MRNB_TRY(launch_colsum<float>(gy.f, d, rows, d, gp(G, pb + MRNB_PB_FC2_B), st));
-      MRNB_TRY(gemm_dw<AT>(gy, w.hact[blk], 4 * d, gp(G, pb + MRNB_PB_FC2_W), rows, d, 4 * d, st));
+      if (pg) {
+        if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dy16, d, rows, d, gp(G, pb + MRNB_PB_FC2_B), st));
+        else MRNB_TRY(launch_colsum<float>(gy.f, d, rows, d, gp(G, pb + MRNB_PB_FC2_B), st));
+        MRNB_TRY(gemm_dw<AT>(gy, w.hact[blk], 4 * d, gp(G, pb + MRNB_PB_FC2_W), rows, d, 4 * d, st));
+      }
       if constexpr (TC) {
         // d(GELU output) leaves the GEMM as bf16 only; GELU' is applied in place on the bf16 tensor
         MRNB_TRY(gemm_dx_tc(gy.h, gy.ld, P.h[pb + MRNB_PB_FC2_W], nullptr, w.dbig16, 4 * d, rows, d, 4 * d, st));
@@ -890,9 +904,11 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
         MRNB_CHECK_LAUNCH("gelu_bwd_kernel");
       }
       Grad gh{w.dbig, w.dbig16, 4L * d};
-      if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dbig16, 4 * d, rows, 4 * d, gp(G, pb + MRNB_PB_FC1_B), st));
-      else MRNB_TRY(launch_colsum<float>(w.dbig, 4 * d, rows, 4 * d, gp(G, pb + MRNB_PB_FC1_B), st));
-      MRNB_TRY(gemm_dw<AT>(gh, w.ln2[blk], d, gp(G, pb + MRNB_PB_FC1_W), rows, 4 * d, d, st));
+      if (pg) {
+        if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dbig16, 4 * d, rows, 4 * d, gp(G, pb + MRNB_PB_FC1_B), st));
+        else MRNB_TRY(launch_colsum<float>(w.dbig, 4 * d, rows, 4 * d, gp(G, pb + MRNB_PB_FC1_B), st));
+        MRNB_TRY(gemm_dw<AT>(gh, w.ln2[blk], d, gp(G, pb + MRNB_PB_FC1_W), rows, 4 * d, d, st));
+      }
       MRNB_TRY(gemm_dx<AT>(gh, P.p[pb + MRNB_PB_FC1_W], P.h[pb + MRNB_PB_FC1_W], w.dln, nullptr, d, rows, 4 * d, d, st));
       // (bf16 mode: the same pass emits the mixer branch's GEMM operand, dx * ds0, in bf16)
       MRNB_TRY(launch_ln_bwd(w.xmid[blk], w.dln, P.p[pb + MRNB_PB_NORM2_W], dx, dx, TC ? w.dy16 : nullptr,
@@ -905,20 +921,22 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
         MRNB_CHECK_LAUNCH("scale_rows_kernel");
         gy.f = w.dy;
       }
-      if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dy16, d, rows, d, gp(G, pb + MRNB_PB_PROJ_B), st));
-      else MRNB_TRY(launch_colsum<float>(gy.f, d, rows, d, gp(G, pb + MRNB_PB_PROJ_B), st));
-      MRNB_TRY(gemm_dw<AT>(gy, w.att[blk], d, gp(G, pb + MRNB_PB_PROJ_W), rows, d, d, st));
+      if (pg) {
+        if constexpr (TC) MRNB_TRY(launch_colsum<bf16>(w.dy16, d, rows, d, gp(G, pb + MRNB_PB_PROJ_B), st));
+        else MRNB_TRY(launch_colsum<float>(gy.f, d, rows, d, gp(G, pb + MRNB_PB_PROJ_B), st));
+        MRNB_TRY(gemm_dw<AT>(gy, w.att[blk], d, gp(G, pb + MRNB_PB_PROJ_W), rows, d, d, st));
+      }
       MRNB_TRY(gemm_dx<AT>(gy, P.p[pb + MRNB_PB_PROJ_W], P.h[pb + MRNB_PB_PROJ_W], w.datt, w.datt16, d, rows, d, d, st));
       Grad gq{w.dqkv, w.dqkv16, 3L * d};
       if constexpr (TC) {
         MRNB_TRY(attn_tc_backward(w.qkv[blk], w.att[blk], w.datt, w.datt16, w.P[blk], w.dS16, w.dqkv16, B, N, d, heads, st));
-        MRNB_TRY(launch_colsum<bf16>(w.dqkv16, 3 * d, rows, 3 * d, gp(G, pb + MRNB_PB_QKV_B), st));
+        if (pg) MRNB_TRY(launch_colsum<bf16>(w.dqkv16, 3 * d, rows, 3 * d, gp(G, pb + MRNB_PB_QKV_B), st));
       } else {
         MRNB_TRY((attention_train_bwd<AT, float>(w.qkv[blk], w.att[blk], w.datt, w.lse[blk], w.Dbuf, w.dqkv, B, N, d, heads,
                                                  H, Wd, blk < 6, st)));
-        MRNB_TRY(launch_colsum<float>(w.dqkv, 3 * d, rows, 3 * d, gp(G, pb + MRNB_PB_QKV_B), st));
+        if (pg) MRNB_TRY(launch_colsum<float>(w.dqkv, 3 * d, rows, 3 * d, gp(G, pb + MRNB_PB_QKV_B), st));
       }
-      MRNB_TRY(gemm_dw<AT>(gq, w.ln1[blk], d, gp(G, pb + MRNB_PB_QKV_W), rows, 3 * d, d, st));
+      if (pg) MRNB_TRY(gemm_dw<AT>(gq, w.ln1[blk], d, gp(G, pb + MRNB_PB_QKV_W), rows, 3 * d, d, st));
       MRNB_TRY(gemm_dx<AT>(gq, P.p[pb + MRNB_PB_QKV_W], P.h[pb + MRNB_PB_QKV_W], w.dln, nullptr, d, rows, 3 * d, d, st));
       // (bf16 mode, not the first block of the stage: also emit dx * ds1 of the previous block, its MLP branch's operand)
       dy16_ready = TC && j > 0;
@@ -937,8 +955,10 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
   {
     mrnb_prof_begin(MRNB_PROF_CONV, st, 0.0, 0.0);
     const long per = 512L * 64;
-    pos_grad_kernel<<<cdiv(per, 256), 256, 0, st>>>(dx, gp(G, MRNB_P_POS_EMBED), B, per);
-    MRNB_CHECK_LAUNCH("pos_grad_kernel");
+    if (pg) {
+      pos_grad_kernel<<<cdiv(per, 256), 256, 0, st>>>(dx, gp(G, MRNB_P_POS_EMBED), B, per);
+      MRNB_CHECK_LAUNCH("pos_grad_kernel");
+    }
     cudaMemsetAsync(w.bsums, 0, 96 * 2 * sizeof(double), st);
     const long r1 = (long)B * 512;
     int chunks = (int)(r1 / 256); if (chunks < 1) chunks = 1; if (chunks > 148) chunks = 148;
@@ -947,14 +967,18 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
     bn_bwd_apply_kernel<<<cdiv(u, 256), 256, 0, st>>>(w.raw1, dx, w.ss + 64, w.mr + 64, w.bsums + 64, (double)r1, bn_batch,
                                                       gp(G, MRNB_P_BN1_W), gp(G, MRNB_P_BN1_B), 64, u, TC ? w.dy16 : nullptr);
     MRNB_CHECK_LAUNCH("bn_bwd_apply_kernel");
-    MRNB_TRY(launch_colsum<float>(dx, 64, r1, 64, gp(G, MRNB_P_CONV1_B), st));
+    if (pg) MRNB_TRY(launch_colsum<float>(dx, 64, r1, 64, gp(G, MRNB_P_CONV1_B), st));
     if constexpr (TC) {
-      MRNB_TRY(launch_im2col<AT>(w.act0, w.big, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
-      MRNB_TRY(gemm_dw_tc(w.dy16, 64, w.big, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
+      if (pg) {
+        MRNB_TRY(launch_im2col<AT>(w.act0, w.big, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
+        MRNB_TRY(gemm_dw_tc(w.dy16, 64, w.big, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
+      }
       MRNB_TRY(gemm_dx_tc(w.dy16, 64, P.h[MRNB_P_CONV1_W], w.dbig, nullptr, 288, (int)r1, 64, 288, st));
     } else {
-      MRNB_TRY(launch_im2col<float>(w.act0, w.colf, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
-      MRNB_TRY(gemm_dw_f32(dx, 64, w.colf, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
+      if (pg) {
+        MRNB_TRY(launch_im2col<float>(w.act0, w.colf, 16, 128, 32, 3, 3, 1, 2, 2, 8, 64, r1, st));
+        MRNB_TRY(gemm_dw_f32(dx, 64, w.colf, 288, gp(G, MRNB_P_CONV1_W), (int)r1, 64, 288, st));
+      }
       MRNB_TRY(gemm_dx_f32(dx, 64, P.p[MRNB_P_CONV1_W], w.dbig, 288, (int)r1, 64, 288, st));
     }
     float* dact0 = w.dy;                                   // [B,16,128,32]
@@ -968,20 +992,24 @@ int train_backward_t(const MrnbSvtrPack& P, const MrnbSvtrPack& G, const float* 
     bn_bwd_apply_kernel<<<cdiv(n0, 256), 256, 0, st>>>(w.raw0, dact0, w.ss, w.mr, w.bsums, (double)r0, bn_batch,
                                                        gp(G, MRNB_P_BN0_W), gp(G, MRNB_P_BN0_B), 32, n0, TC ? w.dbig16 : nullptr);
     MRNB_CHECK_LAUNCH("bn_bwd_apply_kernel");
-    MRNB_TRY(launch_colsum<float>(dact0, 32, r0, 32, gp(G, MRNB_P_CONV0_B), st));
-    if constexpr (TC) {
-      im2col_img_pad64_kernel<<<cdiv(r0 * 8, 256), 256, 0, st>>>(image, w.big, r0);
-      MRNB_CHECK_LAUNCH("im2col_img_pad64_kernel");
-      cudaMemsetAsync(w.dw0pad, 0, 32 * 64 * sizeof(float), st);
-      MRNB_TRY(gemm_dw_tc(w.dbig16, 32, w.big, 64, w.dw0pad, (int)r0, 32, 64, st));
-      unpad_dw0_kernel<<<5, 256, 0, st>>>(w.dw0pad, gp(G, MRNB_P_CONV0_W), 32);
-      MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
-    } else {
-      const long total = r0 * 36;
-      im2col_img_kernel<<<cdiv(total, 256), 256, 0, st>>>(image, w.colf, total);
-      MRNB_CHECK_LAUNCH("im2col_img_kernel");
-      MRNB_TRY(gemm_dw_f32(dact0, 32, w.colf, 36, gp(G, MRNB_P_CONV0_W), (int)r0, 32, 36, st));
+    if (pg) {
+      MRNB_TRY(launch_colsum<float>(dact0, 32, r0, 32, gp(G, MRNB_P_CONV0_B), st));
+      if constexpr (TC) {
+        im2col_img_pad64_kernel<<<cdiv(r0 * 8, 256), 256, 0, st>>>(image, w.big, r0);
+        MRNB_CHECK_LAUNCH("im2col_img_pad64_kernel");
+        cudaMemsetAsync(w.dw0pad, 0, 32 * 64 * sizeof(float), st);
+        MRNB_TRY(gemm_dw_tc(w.dbig16, 32, w.big, 64, w.dw0pad, (int)r0, 32, 64, st));
+        unpad_dw0_kernel<<<5, 256, 0, st>>>(w.dw0pad, gp(G, MRNB_P_CONV0_W), 32);
+        MRNB_CHECK_LAUNCH("unpad_dw0_kernel");
+      } else {
+        const long total = r0 * 36;
+        im2col_img_kernel<<<cdiv(total, 256), 256, 0, st>>>(image, w.colf, total);
+        MRNB_CHECK_LAUNCH("im2col_img_kernel");
+        MRNB_TRY(gemm_dw_f32(dact0, 32, w.colf, 36, gp(G, MRNB_P_CONV0_W), (int)r0, 32, 36, st));
+      }
     }
+    // the image gradient from the fp32 dact0 (never its bf16 copy): conv0's input gradient, gathered per pixel
+    if (dimage) MRNB_TRY(launch_svtr_conv0_dimage(dact0, P.p[MRNB_P_CONV0_W], dimage, B, st));
     mrnb_prof_end(MRNB_PROF_CONV, st);
   }
   return MRNB_OK;
@@ -1020,25 +1048,41 @@ extern "C" int mrnb_svtr_train_forward(const MrnbSvtrPack* pack, const float* im
                                           nullptr, workspace, workspace_bytes, stream);
 }
 
+extern "C" int mrnb_svtr_train_backward_input(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
+                                              const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
+                                              int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
+                                              float* dimage, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  MRNB_CHECK_ARG(pack && image && dlogits && workspace && B > 0, "svtr_train_backward: null/empty argument");
+  MRNB_CHECK_ARG(grad_arena || dimage, "svtr_train_backward: neither the gradient arena nor dimage given");
+  MRNB_CHECK_ARG(!grads == !grad_arena, "svtr_train_backward: grads and grad_arena are given together or both NULL");
+  MRNB_CHECK_ARG(pack->n_experts == 1 && (!grads || grads->n_experts == 1),
+                 "svtr_train_backward: the training pack holds exactly one expert");
+  if (grads) {
+    for (int k = 0; k < MRNB_P_COUNT; ++k) {
+      const bool stat = k == MRNB_P_BN0_MEAN || k == MRNB_P_BN0_VAR || k == MRNB_P_BN1_MEAN || k == MRNB_P_BN1_VAR;
+      MRNB_CHECK_ARG(stat || grads->p[k], "svtr_train_backward: gradient slot %d is null", k);
+    }
+    MRNB_CHECK_ARG(grads->fc_w[0] && grads->fc_b[0], "svtr_train_backward: classifier gradient slots are null");
+  }
+  static const MrnbSvtrPack no_grads{};   // input-only backward: every parameter-gradient pointer NULL
+  const MrnbSvtrPack& G = grads ? *grads : no_grads;
+  if (prec == MRNB_PREC_FP32)
+    return train_backward_t<float>(*pack, G, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, drop_scales,
+                                   grad_arena, n_arena, dimage, workspace, workspace_bytes, stream);
+  if (prec == MRNB_PREC_BF16)
+    return train_backward_t<__nv_bfloat16>(*pack, G, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats,
+                                           drop_scales, grad_arena, n_arena, dimage, workspace, workspace_bytes, stream);
+  mrnb_set_error("svtr_train_backward: unknown precision %d", prec);
+  return MRNB_ERR_ARG;
+}
+
 extern "C" int mrnb_svtr_train_backward_features(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
                                                  const float* dlogits, long ld_dlogits, const float* dfeatures, int B, int prec,
                                                  int bn_batch_stats, const float* drop_scales, float* grad_arena, long n_arena,
                                                  void* workspace, size_t workspace_bytes, cudaStream_t stream) {
-  MRNB_CHECK_ARG(pack && grads && image && dlogits && grad_arena && workspace && B > 0, "svtr_train_backward: null/empty argument");
-  MRNB_CHECK_ARG(pack->n_experts == 1 && grads->n_experts == 1, "svtr_train_backward: the training pack holds exactly one expert");
-  for (int k = 0; k < MRNB_P_COUNT; ++k) {
-    const bool stat = k == MRNB_P_BN0_MEAN || k == MRNB_P_BN0_VAR || k == MRNB_P_BN1_MEAN || k == MRNB_P_BN1_VAR;
-    MRNB_CHECK_ARG(stat || grads->p[k], "svtr_train_backward: gradient slot %d is null", k);
-  }
-  MRNB_CHECK_ARG(grads->fc_w[0] && grads->fc_b[0], "svtr_train_backward: classifier gradient slots are null");
-  if (prec == MRNB_PREC_FP32)
-    return train_backward_t<float>(*pack, *grads, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats, drop_scales,
-                                   grad_arena, n_arena, workspace, workspace_bytes, stream);
-  if (prec == MRNB_PREC_BF16)
-    return train_backward_t<__nv_bfloat16>(*pack, *grads, image, dlogits, ld_dlogits, dfeatures, B, bn_batch_stats,
-                                           drop_scales, grad_arena, n_arena, workspace, workspace_bytes, stream);
-  mrnb_set_error("svtr_train_backward: unknown precision %d", prec);
-  return MRNB_ERR_ARG;
+  MRNB_CHECK_ARG(grads && grad_arena, "svtr_train_backward: null/empty argument");
+  return mrnb_svtr_train_backward_input(pack, grads, image, dlogits, ld_dlogits, dfeatures, B, prec, bn_batch_stats,
+                                        drop_scales, grad_arena, n_arena, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int mrnb_svtr_train_backward(const MrnbSvtrPack* pack, const MrnbSvtrPack* grads, const float* image,
@@ -1063,4 +1107,11 @@ extern "C" int mrnb_attn_tc_train_backward(const void* qkv, const void* O, const
                  "attn_tc_train_backward: bad argument");
   return attn_tc_backward((const bf16*)qkv, (const bf16*)O, dO, (const bf16*)dO16, (const bf16*)P, (bf16*)dS, (bf16*)dqkv, B, N,
                           d, heads, stream);
+}
+
+// ---- C-ABI test entry: the patch embedding's conv0 input gradient on its own (d [B,16,128,32] NHWC fp32, w [32,4,3,3]
+// -> dimage [B,4,32,256] NCHW fp32), as train_backward_t launches it
+extern "C" int mrnb_svtr_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t stream) {
+  MRNB_CHECK_ARG(d && w && dimage && B > 0 && B <= 65535, "svtr_conv0_dimage: bad argument");
+  return launch_svtr_conv0_dimage(d, w, dimage, B, stream);
 }

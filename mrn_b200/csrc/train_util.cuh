@@ -329,16 +329,84 @@ __global__ void unpad_dw0_kernel(const float* __restrict__ dwp, float* __restric
 }
 
 // ------------------------------------------------------------------------------------------------
+// conv0 input gradient: the gradient with respect to the image of the first convolution of an expert (4 input
+// channels, 3 x 3, pad 1, stride S, on the 32 x 256 image; Ho = 32 / S, Wo = 256 / S):
+//   dimage[b,c,ih,iw] = sum over the taps (kh, kw) and output channels o that read pixel (ih, iw) of d[b,oh,ow,o] w[o,c,kh,kw]
+// d: the gradient at conv0's output, NHWC [B,Ho,Wo,COUT] fp32.  dimage: NCHW [B,4,32,256] fp32, every element written.
+// A gather, one thread per image pixel computing its four channels: taps in ascending (kh, kw) order, output channels in
+// ascending order within a tap -- no atomics, so the result is bitwise repeatable.  The weight sits in shared memory as
+// one float4 (its four input channels) per (tap, o).  W_HWC: the weight is [COUT,3,3,4] (the CRNN training pack), else
+// nn.Conv2d's [COUT,4,3,3] (the SVTR pack).  Block = one image row (256 threads), grid (32, B).
+// ------------------------------------------------------------------------------------------------
+template <int COUT, int S, bool W_HWC>
+__global__ void __launch_bounds__(256)
+conv0_dimage_kernel(const float* __restrict__ d, const float* __restrict__ w, float* __restrict__ dimage) {
+  constexpr int H = 32, W = 256, Ho = H / S, Wo = W / S;
+  __shared__ float4 wsh[9 * COUT];                        // [tap][o]
+  for (int i = threadIdx.x; i < 9 * COUT; i += blockDim.x) {
+    const int o = i % COUT, tap = i / COUT;
+    float v[4];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) v[c] = W_HWC ? w[(o * 9 + tap) * 4 + c] : w[(o * 4 + c) * 9 + tap];
+    wsh[i] = make_float4(v[0], v[1], v[2], v[3]);
+  }
+  __syncthreads();
+  const int iw = threadIdx.x, ih = blockIdx.x;
+  const long b = blockIdx.y;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+  for (int kh = 0; kh < 3; ++kh) {
+    const int th = ih + 1 - kh;
+    if (th < 0 || th % S != 0 || th / S >= Ho) continue;
+    const int oh = th / S;
+#pragma unroll
+    for (int kw = 0; kw < 3; ++kw) {
+      const int tw = iw + 1 - kw;
+      if (tw < 0 || tw % S != 0 || tw / S >= Wo) continue;
+      const float4* src = reinterpret_cast<const float4*>(d + ((b * Ho + oh) * Wo + tw / S) * COUT);
+      const float4* wt = wsh + (kh * 3 + kw) * COUT;
+#pragma unroll 4
+      for (int o4 = 0; o4 < COUT / 4; ++o4) {
+        const float4 g = __ldg(src + o4);
+        const float gv[4] = {g.x, g.y, g.z, g.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float4 wv = wt[o4 * 4 + j];
+          acc.x = fmaf(gv[j], wv.x, acc.x); acc.y = fmaf(gv[j], wv.y, acc.y);
+          acc.z = fmaf(gv[j], wv.z, acc.z); acc.w = fmaf(gv[j], wv.w, acc.w);
+        }
+      }
+    }
+  }
+  float* out = dimage + (b * 4 * H + ih) * W + iw;
+  out[0] = acc.x; out[(long)H * W] = acc.y; out[2L * H * W] = acc.z; out[3L * H * W] = acc.w;
+}
+
+// SVTR patch embedding conv0 (4 -> 32, stride 2): d [B,16,128,32], w [32,4,3,3]
+int launch_svtr_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t st) {
+  conv0_dimage_kernel<32, 2, false><<<dim3(32, B), 256, 0, st>>>(d, w, dimage);
+  MRNB_CHECK_LAUNCH("conv0_dimage_kernel");
+  return MRNB_OK;
+}
+// CRNN VGG conv0 (4 -> 64, stride 1): d [B,32,256,64], w [64,3,3,4]
+int launch_crnn_conv0_dimage(const float* d, const float* w, float* dimage, int B, cudaStream_t st) {
+  conv0_dimage_kernel<64, 1, true><<<dim3(32, B), 256, 0, st>>>(d, w, dimage);
+  MRNB_CHECK_LAUNCH("conv0_dimage_kernel");
+  return MRNB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // BatchNorm backward, apply pass (after a reduce pass that left S1 = sum dz, S2 = sum dz * xhat per channel in sums):
 // draw = gamma*rstd * (dz - S1/n - xhat * S2/n)   (batch statistics)   or   gamma*rstd * dz   (running statistics),
-// written over d (+ optional 16-bit copy);  dgamma = S2, dbeta = S1
+// written over d (+ optional 16-bit copy);  dgamma = S2, dbeta = S1 (both NULL: no parameter gradient, the input-only
+// backward)
 // ------------------------------------------------------------------------------------------------
 __global__ void bn_bwd_apply_kernel(const float* __restrict__ raw, float* __restrict__ d, const float* __restrict__ ss,
                                     const float* __restrict__ mr, const double* __restrict__ sums, double count,
                                     int use_batch, float* __restrict__ dgamma, float* __restrict__ dbeta, int C, long total,
                                     bf16* __restrict__ d16) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < C) { dgamma[i] = (float)sums[i * 2 + 1]; dbeta[i] = (float)sums[i * 2]; }
+  if (dgamma && i < C) { dgamma[i] = (float)sums[i * 2 + 1]; dbeta[i] = (float)sums[i * 2]; }
   if (i >= total) return;
   const int c = (int)(i % C);
   float dz = d[i];

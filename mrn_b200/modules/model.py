@@ -101,10 +101,11 @@ class Model(nn.Module):
 
     def forward(self, image, text=None, is_train=True):
         """-> {"predict": [B,T,C], "feature": [B,T,256]} (modules/model.py:133-148) via a single-expert pack.
-        With opt.autograd and grad mode on, "predict" is differentiable with respect to every parameter (training-pack
-        forward, see _expert_autograd_forward) and "feature" is None."""
+        With opt.autograd and grad mode on, "predict" and "feature" are differentiable with respect to every parameter
+        and to the image (training-pack forward, see _expert_autograd_forward)."""
         if _autograd_on(self.opt):
-            return {"predict": _expert_autograd_forward(self, image, self.opt), "feature": None}
+            predict, feature = _expert_autograd_forward(self, image, self.opt, want_features=True)
+            return {"predict": predict, "feature": feature}
         feats, logits = _experts_forward([self], image, self.opt, train_mode=self.training)
         return {"predict": logits[0], "feature": feats[:, 0]}
 
@@ -222,15 +223,18 @@ def _writeback_train_pack_bn(expert, tp, n_fwd):
             bn.num_batches_tracked += n_fwd
 
 
-def _train_pack_run(expert, x, opt, net=None, drop=None, want_features=False):
+def _train_pack_run(expert, x, opt, net=None, drop=None, want_features=False, param_grads=True):
     """One expert's training-pack forward, the step autograd differentiates (opt.autograd): ops.SvtrTrainPack /
     ops.CrnnTrainPack built from the expert's state_dict, run in the expert's current mode -- in .train() BatchNorm batch
     statistics with the running-statistics update (written back to the expert's buffers once, here) and DropPath `drop`
     [12,2,B] (None: drawn as the default forward draws it).  Returns (logits, features or None, backward);
-    backward(dlogits, dfeatures=None) runs the pack's full backward and returns {state_dict key: gradient in the reference
-    layout} (views of the pack's gradient arena)."""
+    backward(dlogits, dfeatures=None, dimage=False) runs the pack's backward and returns (grads, dimage): grads =
+    {state_dict key: gradient in the reference layout} (views of the pack's gradient arena), dimage = d loss / d image
+    [B,4,32,256] when asked for.  param_grads=False (a frozen expert that only carries the image gradient): the pack has
+    no gradient arena, the backward is the input-only one and grads is None."""
     arch = _arch(opt)
-    tp = (ops.SvtrTrainPack if arch == "svtr" else ops.CrnnTrainPack)(expert.state_dict(), x.device, _precision(opt))
+    tp = (ops.SvtrTrainPack if arch == "svtr" else ops.CrnnTrainPack)(expert.state_dict(), x.device, _precision(opt),
+                                                                      param_grads=param_grads)
     train = bool(expert.training)
     x = x.contiguous().float()
     B = x.shape[0]
@@ -249,26 +253,32 @@ def _train_pack_run(expert, x, opt, net=None, drop=None, want_features=False):
         if net is not None:
             net._cache.key = None
 
-    def backward(dlogits, dfeatures=None):
+    def backward(dlogits, dfeatures=None, dimage=False):
+        if not (param_grads or dimage):
+            return None, None
+        di = torch.empty(B, 4, 32, 256, device=x.device, dtype=torch.float32) if dimage else None
         if arch == "crnn":
-            ops.crnn_train_backward(tp, dlogits, B, bn_batch_stats=train, dfeatures=dfeatures)
+            ops.crnn_train_backward(tp, dlogits, B, bn_batch_stats=train, dfeatures=dfeatures, dimage=di,
+                                    param_grads=param_grads)
         else:
-            ops.svtr_train_backward(tp, x, dlogits, bn_batch_stats=train, drop_scales=drop, dfeatures=dfeatures)
-        return tp.state(tp.grads)
+            ops.svtr_train_backward(tp, x, dlogits, bn_batch_stats=train, drop_scales=drop, dfeatures=dfeatures, dimage=di,
+                                    param_grads=param_grads)
+        return (tp.state(tp.grads) if param_grads else None), di
     return logits, feats, backward
 
 
-def _expert_autograd_forward(expert, image, opt, net=None):
+def _expert_autograd_forward(expert, image, opt, net=None, want_features=False):
     """Forward of one expert that autograd differentiates (opt.autograd): _train_pack_run and, on backward, the pack's
-    full backward, mapped back to every parameter by the pack's arena <-> state_dict table."""
+    backward, mapped back to every parameter by the pack's arena <-> state_dict table, and the image gradient when the
+    image requires grad.  Returns logits, or (logits, features) with want_features."""
     if not image.is_cuda:
         raise RuntimeError("mrn_b200 needs CUDA tensors: there is no CPU fallback")
     from ..autograd import ExpertTrain
     if net is not None:
         net._sync_bn()                      # BN statistics the grouped pack still holds -> the module buffers
     named = list(expert.named_parameters())
-    return ExpertTrain.apply(lambda x: _train_pack_run(expert, x, opt, net=net), [n for n, _ in named], image,
-                             *[p for _, p in named])
+    return ExpertTrain.apply(lambda x, **kw: _train_pack_run(expert, x, opt, net=net, **kw), [n for n, _ in named],
+                             want_features, image, *[p for _, p in named])
 
 
 _RATES_CACHE = {}
@@ -435,10 +445,12 @@ class MRNNet(nn.Module):
             with a parameter that requires grad (a trainable expert) gets its gradient too, along both paths of the
             reference (its logits through the gated combine, its feature through the DM-Router and the gate head);
             trainable experts run their training packs (BatchNorm / DropPath as cross=False), the others the grouped
-            forward;
+            forward.  An image that requires grad gets its gradient through every expert: then every expert runs a
+            training pack, the frozen ones with the input-only backward (their .grad stays None);
           * cross=True, is_train=False (hard route): "index" is an argmax and "logits" depends only on the frozen
-            experts -- outputs as without the switch, no router gradient;
-          * cross=False: "logits" with respect to every parameter of the newest expert (training-pack forward)."""
+            experts -- outputs as without the switch, no router or image gradient;
+          * cross=False: "logits" with respect to every parameter of the newest expert and to the image
+            (training-pack forward)."""
         grad = _autograd_on(self.opt)
         if cross is False:
             if grad:
@@ -471,11 +483,12 @@ class MRNNet(nn.Module):
     def pad_zeros_features(self, feature, total):
         raise RuntimeError("padding with ones is fused into mrnb_gate_combine; no padded tensor is materialised")
 
-    def joint_experts_forward(self, image, trainable):
+    def joint_experts_forward(self, image, trainable, input_grad=False):
         """Expert outputs of the soft route when the experts in `trainable` (indices) train with the router
         (opt.autograd_experts): the frozen ones through one grouped forward built over them alone, each trainable one
-        through its training pack.  DropPath is drawn once for all experts, as the grouped forward draws it.  Returns
-        (features [B,I,T,D], [logits_i], {expert index: training-pack backward})."""
+        through its training pack.  input_grad (the image requires grad): the frozen experts run training packs too,
+        without a gradient arena (input-only backward).  DropPath is drawn once for all experts, as the grouped forward
+        draws it.  Returns (features [B,I,T,D], [logits_i], {expert index: training-pack backward})."""
         if not image.is_cuda:
             raise RuntimeError("mrn_b200 needs CUDA tensors: there is no CPU fallback")
         full = self._cache.pack
@@ -494,7 +507,7 @@ class MRNNet(nn.Module):
         feats = torch.empty(B, I, self.patch, self.out_dim, device=image.device, dtype=torch.float32)
         logits = [None] * I
         frozen = [e for e in range(I) if e not in trainable]
-        if frozen:
+        if frozen and not input_grad:
             experts = [self.model[e] for e in frozen]
             f, z = _experts_forward(experts, image, self.opt, tuple(modes[e] for e in frozen), self._frozen_cache,
                                     drop_scales=None if drop is None else drop[frozen].contiguous())
@@ -505,9 +518,10 @@ class MRNNet(nn.Module):
                 _writeback_bn(experts, self._frozen_cache.pack)
                 self._cache.key = None      # the full grouped pack's BN statistics are stale now
         backward = {}
-        for e in trainable:
+        for e in (range(I) if input_grad else trainable):
             z, f, backward[e] = _train_pack_run(self.model[e], image, self.opt, net=self, want_features=True,
-                                                drop=drop[e].contiguous() if drop is not None and modes[e] else None)
+                                                drop=drop[e].contiguous() if drop is not None and modes[e] else None,
+                                                param_grads=e in trainable)
             feats[:, e] = f
             logits[e] = z
         return feats, logits, backward

@@ -417,9 +417,11 @@ class _TrainPack:
     averages (stage 0, il_modules/mrn.py:225-279).  `entries` maps each arena slice back to its state_dict key.
 
     A subclass passes its slot table [(slot, [(key, permute), ...])] in arena order (the parts of a slot adjacent, each
-    slot padded to 8 floats), names its C struct (_Struct) and puts a slot's pointers into it (_point)."""
+    slot padded to 8 floats), names its C struct (_Struct) and puts a slot's pointers into it (_point).
+    param_grads=False: no gradient arena (grads is None) -- the pack of a frozen expert that only carries the image
+    gradient, run by the input-only backward."""
 
-    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec, slots):
+    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec, slots, param_grads=True):
         self.device = torch.device(device)
         self.prec = prec
         self.entries = []                         # (slot, key, permute, offset, kernel-layout shape)
@@ -438,7 +440,7 @@ class _TrainPack:
             off = round_up(off, 8)
         self.numel = off
         self.params = torch.zeros(off, device=self.device, dtype=torch.float32)
-        self.grads = torch.zeros(off, device=self.device, dtype=torch.float32)
+        self.grads = torch.zeros(off, device=self.device, dtype=torch.float32) if param_grads else None
         self.shadow16 = torch.zeros(off, device=self.device, dtype=torch.bfloat16) if prec == L.PREC_BF16 else None
         self.n_class = int(expert_sd["fc.weight"].shape[0])
         self.struct = self._Struct()
@@ -446,7 +448,8 @@ class _TrainPack:
         for slot, o in self.slot_offset.items():
             self._point(self.struct, slot, self.params.data_ptr() + 4 * o,
                         None if self.shadow16 is None else self.shadow16.data_ptr() + 2 * o)
-            self._point(self.gstruct, slot, self.grads.data_ptr() + 4 * o, None)
+            if self.grads is not None:
+                self._point(self.gstruct, slot, self.grads.data_ptr() + 4 * o, None)
         self.load_state(expert_sd)
         self._ws: Optional[torch.Tensor] = None
 
@@ -491,8 +494,8 @@ class SvtrTrainPack(_TrainPack):
     arch = "svtr"
     _Struct = L.MrnbSvtrPack
 
-    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32):
-        super().__init__(expert_sd, device, prec, _train_slots())
+    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32, param_grads: bool = True):
+        super().__init__(expert_sd, device, prec, _train_slots(), param_grads)
         for st_ in (self.struct, self.gstruct):
             st_.n_experts = 1
             st_.n_class[0] = self.n_class
@@ -545,19 +548,34 @@ def svtr_train_forward(tp: SvtrTrainPack, image, bn_batch_stats=True, update_run
     return (buf[:, :, :tp.n_class], feats) if want_features else buf[:, :, :tp.n_class]
 
 
-def svtr_train_backward(tp: SvtrTrainPack, image, dlogits, bn_batch_stats=True, drop_scales=None, dfeatures=None):
+def _grad_args(tp, param_grads, dimage, B):
+    """(grads struct, arena, arena length) of a training-pack backward: NULLs for the input-only backward."""
+    if dimage is not None:
+        _chk_f32(dimage)
+        assert tuple(dimage.shape) == (B, 4, 32, 256), "dimage must be dense [B,4,32,256]"
+    if not param_grads:
+        assert dimage is not None, "the input-only backward (param_grads=False) needs dimage"
+        return None, None, 0
+    assert tp.grads is not None, "this training pack has no gradient arena (built with param_grads=False)"
+    return C.byref(tp.gstruct), tp.grads, tp.numel
+
+
+def svtr_train_backward(tp: SvtrTrainPack, image, dlogits, bn_batch_stats=True, drop_scales=None, dfeatures=None,
+                        dimage=None, param_grads=True):
     """Fills tp.grads (overwritten) from d loss / d logits [B,64,C] (+ d loss / d features [B,64,256] reaching the
-    feature from outside the expert); must follow svtr_train_forward on the same batch."""
+    feature from outside the expert); must follow svtr_train_forward on the same batch.  dimage: None or an output
+    tensor [B,4,32,256] fp32 that receives d loss / d image.  param_grads=False: the input-only backward (no parameter
+    gradient; dimage required).  Returns tp.grads, or None without parameter gradients."""
     _chk_f32(image, drop_scales)
     assert dlogits.dtype == torch.float32 and dlogits.stride(2) == 1 and dlogits.stride(0) == dlogits.shape[1] * dlogits.stride(1)
     B = image.shape[0]
     _chk_dfeatures(dfeatures, B, T_FRAMES)
+    gstruct, grads, n = _grad_args(tp, param_grads, dimage, B)
     ws = tp.workspace(B)
-    L.check(L.load().mrnb_svtr_train_backward_features(C.byref(tp.struct), C.byref(tp.gstruct), _p(image), _p(dlogits),
-                                                       dlogits.stride(1), _p(dfeatures), B, tp.prec, int(bn_batch_stats),
-                                                       _p(drop_scales), _p(tp.grads), tp.numel, _p(ws), ws.numel(),
-                                                       _stream()), "svtr_train_backward")
-    return tp.grads
+    L.check(L.load().mrnb_svtr_train_backward_input(C.byref(tp.struct), gstruct, _p(image), _p(dlogits), dlogits.stride(1),
+                                                    _p(dfeatures), B, tp.prec, int(bn_batch_stats), _p(drop_scales), _p(grads),
+                                                    n, _p(dimage), _p(ws), ws.numel(), _stream()), "svtr_train_backward")
+    return grads
 
 
 class CrnnTrainPack(_TrainPack):
@@ -569,7 +587,7 @@ class CrnnTrainPack(_TrainPack):
     n_frames = 63
     _Struct = L.MrnbCrnnTrainPack
 
-    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32):
+    def __init__(self, expert_sd: Dict[str, torch.Tensor], device, prec: int = L.PREC_FP32, param_grads: bool = True):
         cn = "model.FeatureExtraction.ConvNet."
         hwc = (0, 2, 3, 1)
         slots = [(L.T_CONV0_W, [(cn + "0.weight", hwc)]), (L.T_CONV0_B, [(cn + "0.bias", None)]),
@@ -586,7 +604,7 @@ class CrnnTrainPack(_TrainPack):
                 slots.append((base + sl, [(q + "rnn." + nm, None), (q + "rnn." + nm + "_reverse", None)]))
             slots += [(base + L.TL_LIN_W, [(q + "linear.weight", None)]), (base + L.TL_LIN_B, [(q + "linear.bias", None)])]
         slots += [(L.T_FC_W, [("fc.weight", None)]), (L.T_FC_B, [("fc.bias", None)])]
-        super().__init__(expert_sd, device, prec, slots)
+        super().__init__(expert_sd, device, prec, slots, param_grads)
         self.bn_stats = {}
         for q, idx in enumerate((12, 15)):
             self.bn_stats[(q, "mean")] = self._bn_stat(expert_sd, f"{idx}.running_mean")
@@ -625,14 +643,32 @@ def crnn_train_forward(tp: CrnnTrainPack, image, bn_batch_stats=True, update_run
     return (buf[:, :, :tp.n_class], feats) if want_features else buf[:, :, :tp.n_class]
 
 
-def crnn_train_backward(tp: CrnnTrainPack, dlogits, B, bn_batch_stats=True, dfeatures=None):
+def crnn_train_backward(tp: CrnnTrainPack, dlogits, B, bn_batch_stats=True, dfeatures=None, dimage=None, param_grads=True):
+    """As svtr_train_backward, for the CRNN expert (dimage in the caller's NCHW layout)."""
     assert dlogits.dtype == torch.float32 and dlogits.stride(2) == 1 and dlogits.stride(0) == dlogits.shape[1] * dlogits.stride(1)
     _chk_dfeatures(dfeatures, B, T_FRAMES_CRNN)
+    gstruct, grads, n = _grad_args(tp, param_grads, dimage, B)
     ws = tp.workspace(B)
-    L.check(L.load().mrnb_crnn_train_backward_features(C.byref(tp.struct), C.byref(tp.gstruct), _p(dlogits), dlogits.stride(1),
-                                                       _p(dfeatures), B, tp.prec, int(bn_batch_stats), _p(tp.grads), tp.numel,
-                                                       _p(ws), ws.numel(), _stream()), "crnn_train_backward")
-    return tp.grads
+    L.check(L.load().mrnb_crnn_train_backward_input(C.byref(tp.struct), gstruct, _p(dlogits), dlogits.stride(1), _p(dfeatures),
+                                                    B, tp.prec, int(bn_batch_stats), _p(grads), n, _p(dimage), _p(ws),
+                                                    ws.numel(), _stream()), "crnn_train_backward")
+    return grads
+
+
+def conv0_dimage(arch, d, w, out=None):
+    """The conv0 input-gradient kernel of an expert's training-pack backward on its own: d = the gradient at conv0's
+    output (NHWC [B,16,128,32] svtr / [B,32,256,64] crnn, fp32), w = the pack's conv0 weight ([32,4,3,3] / [64,3,3,4]).
+    Returns dimage [B,4,32,256] (NCHW; `out` when given, overwritten)."""
+    _chk_f32(d, w, out)
+    B = d.shape[0]
+    shape, wshape = ((B, 16, 128, 32), (32, 4, 3, 3)) if arch == "svtr" else ((B, 32, 256, 64), (64, 3, 3, 4))
+    assert tuple(d.shape) == shape and tuple(w.shape) == wshape, (tuple(d.shape), tuple(w.shape))
+    if out is None:
+        out = torch.empty(B, 4, 32, 256, device=d.device, dtype=torch.float32)
+    assert tuple(out.shape) == (B, 4, 32, 256)
+    fn = L.load().mrnb_svtr_conv0_dimage if arch == "svtr" else L.load().mrnb_crnn_conv0_dimage
+    L.check(fn(_p(d), _p(w), _p(out), B, _stream()), "conv0_dimage")
+    return out
 
 
 # ------------------------------------------------------------------------------------------------ CRNN experts
